@@ -3,10 +3,14 @@
 solver on BASELINE.json's synthetic configs, with the kernel roofline and the
 CPU baseline beside it.
 
-  python bench.py --gpus N --steps K --warmup W [--workload cfg5] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--workload cfg5] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one Levenberg-Marquardt iteration (linearisation + Schur linear
 solve + step evaluation) of the fixed-iteration-count solve on the workload.
+--dump-outputs DIR writes what the timed solve returned (poses, points,
+intrinsics, cost per iteration) as DIR/<name>.npy; the synthetic inputs are
+seeded, so two builds run with the same arguments can be compared array by
+array.
 Default workload: cfg5 of BASELINE.json (10k cameras, 2M points, 8M
 observations, reprojection only, implicit-Schur PCG) -- the config the metric's
 "1/2/4/8 B200" refers to; it fits one GPU.  With N > 1 (torchrun, one rank per
@@ -328,6 +332,24 @@ def n_blk_all(s):
     return s.sparse_stats()[1]
 
 
+DUMP_BYTES = 64e6
+
+
+def write_outputs(path, arrays):
+    """Writes every array as path/<name>.npy in float64.  When they would pass DUMP_BYTES together, the largest is cut
+    to a fixed, seeded sample of its rows (in row order) so that the files stay comparable between runs."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        big = max(arrays, key=lambda k: arrays[k].nbytes)
+        a = arrays[big]
+        keep = int((DUMP_BYTES - (total - a.nbytes)) // (a.nbytes // a.shape[0]))
+        arrays[big] = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -344,10 +366,15 @@ def main():
                     help="single GPU: also time the matrix-free implicit-Schur PCG solver on the same problem (adds its W + K LM iterations)")
     ap.add_argument("--write-golden", action="store_true", help="single GPU: store this run's LM trace as the reference of parity_vs_n1")
     ap.add_argument("--store", type=int, default=0, help="BA_JAC_* for the implicit solver (0 auto, 1 planes, 2 factored, 3 tiled)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single GPU: write the poses, points, intrinsics and per-iteration cost of the timed solve to DIR/<name>.npy "
+                         "(float64, at most 64 MB in all: a seeded sample of the points beyond that)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs needs --impl b200 on one GPU")
     wl = WORKLOADS[args.workload]
     K, W = args.steps, max(args.warmup, 0)
 
@@ -453,6 +480,9 @@ def main():
     spchol = s.spchol_info()
     n_iter = summ.num_iterations
     pcg_counts = [t["linear_iters"] for t in trace[1:]]
+    if args.dump_outputs:
+        pose_k, pt_k, intr_k = s.download()
+        outputs = {"pose7": pose_k, "points": pt_k, "intrinsics": intr_k, "cost_per_iteration": [t["cost"] for t in trace]}
     # ---- end to end through the C-ABI with host buffers (pinned, inputs and outputs): upload + solve + download
     out_bufs = (pinned_copy(np.zeros((problem.n_cam, 7))), pinned_copy(np.zeros((problem.n_pt, 3))), pinned_copy(np.zeros(4)))
     sync_all()
@@ -613,6 +643,8 @@ def main():
         sample_iters = min(K, 3 if full.n_obs > 100000 else K)
         line["cpu_baseline"] = cpu_reference_run(full, wl["mode"], sample_iters, os.cpu_count() or 1)
     print(json.dumps(line))
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     if dist is not None:
         dist.destroy_process_group()
     return 0

@@ -1,9 +1,12 @@
 """bench.py's reference arm runs on the CPU: check the JSON contract of the line it prints (the b200 arm
-prints the same keys plus roofline / clocks / gpu_launches; it needs a GPU and is exercised by the driver)."""
+prints the same keys plus roofline / clocks / gpu_launches; it needs a GPU, and its --dump-outputs is checked by a gpu test)."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -46,6 +49,56 @@ def test_reference_arm_non_zero_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "cfg1", "--gpus", "2"],
                          capture_output=True, text=True, timeout=300, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_stays_under_64_mb_with_a_fixed_sample(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(5)
+    points = rng.normal(size=(3000000, 3)).astype(np.float32)
+    points[:, 0] = np.arange(points.shape[0])   # row number, to check the sample against
+    arrays = {"pose7": rng.normal(size=(10, 7)), "points": points, "intrinsics": np.ones(4)}
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), arrays)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["intrinsics.npy", "points.npy", "pose7.npy"]
+    assert sum(np.load(tmp_path / "a" / n).nbytes for n in names) <= 64e6
+    pts = np.load(tmp_path / "a" / "points.npy")
+    assert pts.dtype == np.float64 and 2500000 < pts.shape[0] < 3000000 and pts.shape[1] == 3
+    assert np.array_equal(pts, np.load(tmp_path / "b" / "points.npy"))
+    # a sample of whole rows, in their original order
+    rows = pts[:, 0].astype(np.int64)
+    assert np.all(np.diff(rows) > 0) and np.array_equal(pts, points[rows].astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "a" / "pose7.npy"), arrays["pose7"])
+
+
+def test_dump_outputs_refused_by_the_reference_arm(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "cfg1",
+                          "--dump-outputs", str(tmp_path / "d")], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode != 0 and "--dump-outputs" in out.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_two_runs_are_identical(tmp_path):
+    """The b200 arm with --dump-outputs: the timed solve runs exactly --steps LM iterations, and two runs with the same
+    arguments write the same arrays."""
+    lines = []
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cfg1", "--steps", "4", "--warmup", "1",
+                              "--no-cpu-baseline", "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, timeout=600,
+                             cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads(out.stdout.strip().split("\n")[-1]))
+    assert lines[0]["steps"] == 4 and lines[0]["detail"]["lm_iterations"] == 4
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["cost_per_iteration.npy", "intrinsics.npy", "points.npy", "pose7.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, b), n
+    pose, pts = np.load(tmp_path / "a" / "pose7.npy"), np.load(tmp_path / "a" / "points.npy")
+    assert pose.shape == (7, 7) and pts.shape == (500, 3)
+    cost = np.load(tmp_path / "a" / "cost_per_iteration.npy")
+    assert cost.shape == (5,) and cost[-1] == lines[0]["final_cost"] and cost[0] == lines[0]["initial_cost"]
 
 
 def test_committed_gpu_bench_line_keeps_the_contract():

@@ -185,10 +185,6 @@ def test_no_raw_pointer_se3_constructor_anywhere():
     for f in ("OptimizationUtils_gpu.cpp", "TrajectoryIO.cpp", "ba_host_capi.cpp"):
         s = open(os.path.join(HOST_DIR, f)).read()
         assert re.search(r"SE3d\s*\(\s*(pose7|p7|initial7)", s) is None, f
-    ref = "/root/reference/headers/sophus/se3.hpp"
-    if os.path.exists(ref):  # (this container only; the GPU box has no /root/reference)
-        real = open(ref).read()
-        assert re.search(r"SE3\s*\(\s*(Scalar|double)\s+const\s*\*", real) is None and "Scalar* data()" in real
 
 
 # ---------------------------------------------------------------- device-resident store (SURVEY.md 8f row N1)
