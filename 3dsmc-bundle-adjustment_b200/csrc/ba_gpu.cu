@@ -171,6 +171,12 @@ struct ba_gpu_ctx {
   bool spc_tree = true;         // one persistent launch with dependency counters (BA_SPCHOL_LEVELS=1: one launch per tree level)
   size_t spc_smem_factor = 0, spc_smem_solve = 0, spc_smem_update = 0;
   double sym_ms = 0.0;          // host time of the symbolic phase (last upload)
+  // sparse Cholesky of the REF / depth-prior / free-intrinsics cost (solver = EXPLICIT_CHOLESKY's linearisation and W / WV,
+  // the block-sparse S and the tree instead of the dense S): right-hand-side rows of the tree (5 with the intrinsics border),
+  // B by camera [24 n_cam], Z = L^-1 B by position [24 n_cam], the corner C + b_k [20], the per-CTA border partials
+  bool sp_ref = false;
+  int spc_nrhs = 1;
+  Buf spb_B, spb_Z, spb_kk, spb_part;
   // phase timing of the large-problem solvers: CUDA events on the solver stream at the phase boundaries of every LM
   // iteration of the last solve (a few dozen event records per iteration: < 0.1 % of a multi-millisecond iteration)
   std::vector<cudaEvent_t> ph_ev;
@@ -495,7 +501,9 @@ extern "C" int ba_gpu_set_options(ba_gpu_ctx *ctx, const ba_gpu_options *o) {
 extern "C" int64_t ba_gpu_launch_count(const ba_gpu_ctx *ctx) { return ctx ? ctx->launches : 0; }
 extern "C" int ba_gpu_sparse_stats(const ba_gpu_ctx *ctx, int64_t *n_pairs, int32_t *n_blocks, int32_t *n_entries) {
   if (!ctx || !ctx->uploaded) return BA_ERR_STATE;
-  const bool sp = ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG;  // (also the Cholesky variant: ctx->spchol)
+  // block-sparse S in force: the NS solvers (PCG and Cholesky: ctx->solver == SPARSE_SCHUR_PCG) and the sparse Cholesky with
+  // depth prior / free intrinsics (ctx->sp_ref)
+  const bool sp = ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG || ctx->sp_ref;
   if (n_pairs) *n_pairs = sp ? ctx->n_pairs : 0;
   if (n_blocks) *n_blocks = sp ? ctx->n_sblk : 0;
   if (n_entries) *n_entries = sp ? ctx->n_ent : 0;
@@ -891,13 +899,14 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   // on one GPU BA_SPCHOL_PARTS=n runs the n parts one after the other (tests of the queues and of the exchange layout)
   int want_parts = ctx->n_ranks > 1 ? (getenv("BA_SPCHOL_REPLICATED") ? 1 : ctx->n_ranks)
                                     : (getenv("BA_SPCHOL_PARTS") ? std::min(BA_MAX_RANKS, std::max(1, atoi(getenv("BA_SPCHOL_PARTS")))) : 1);
-  if (getenv("BA_SPCHOL_LEVELS")) want_parts = 1;
+  if (getenv("BA_SPCHOL_LEVELS") || ctx->sp_ref) want_parts = 1;  // (the REF-cost path is single-GPU: one part)
+  const int R = ctx->spc_nrhs;
   const SpPartition part = spsym_partition(S, want_parts);
   ctx->spc_parts = part.parts;
   ctx->spc_dist = ctx->n_ranks > 1 && part.parts == ctx->n_ranks;
   // layout of spc_U (6x6 blocks): [update matrices of the subtree roots | right-hand-side updates of every node | the other
-  // update matrices]: the first two pieces are what the ranks exchange, one contiguous all-reduce
-  const int64_t ru_blocks = ((int64_t)S.bord.size() * 6 + 35) / 36 + 1;
+  // update matrices]: the first two pieces are what the ranks exchange, one contiguous all-reduce.  (R rows of 6 nb per node)
+  const int64_t ru_blocks = ((int64_t)S.bord.size() * 6 * R + 35) / 36 + 1;
   {
     SpSymbolic &W = ctx->sym;
     auto usize = [&](int id) { const int64_t nb = W.node[(size_t)id * SPSYM_NODE_INTS + SPN_NB]; return nb * nb; };
@@ -961,18 +970,24 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   size_t sf = 0, ss = 0, su = 0;
   for (int id = 0; id < S.n_nodes; ++id) {
     const int32_t *N = S.node.data() + (size_t)id * SPSYM_NODE_INTS;
-    sf = std::max(sf, spc_factor_smem(N[SPN_M], N[SPN_NB]));
+    sf = std::max(sf, spc_factor_smem(N[SPN_M], N[SPN_NB], R));
     ss = std::max(ss, spc_solve_smem(N[SPN_M], N[SPN_NB]));
-    su = std::max(su, spc_update_smem(N[SPN_M], N[SPN_NB]));
+    su = std::max(su, spc_update_smem(N[SPN_M], N[SPN_NB], R));
   }
+  // (at the front capacity, SPC_CAP_BLOCKS = 770 and SPC_MAX_OWN = 24, the five-row factor front needs 228,160 bytes)
   if (sf > 227 * 1024 || ss > 227 * 1024 || su > 227 * 1024)
     return fail(ctx, BA_ERR_STATE, "sparse Cholesky: front exceeds shared memory (%zu / %zu / %zu bytes)", sf, ss, su);
   ctx->spc_smem_factor = sf;
   ctx->spc_smem_solve = ss;
   ctx->spc_smem_update = su;
-  CK(cudaFuncSetAttribute(k_spchol_factor, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
+  if (R > 1) {
+    CK(cudaFuncSetAttribute(k_spchol_factor<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
+    CK(cudaFuncSetAttribute(k_spchol_update<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)su));
+  } else {
+    CK(cudaFuncSetAttribute(k_spchol_factor<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
+    CK(cudaFuncSetAttribute(k_spchol_update<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)su));
+  }
   CK(cudaFuncSetAttribute(k_spchol_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
-  CK(cudaFuncSetAttribute(k_spchol_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)su));
   // work queues of the persistent tree kernel.  Phase A (one queue per part): per level (bottom-up) the factor items of the
   // part's nodes, then their update tiles -- more tiles per node where the part has few nodes on a level.  Phase B: the same
   // for the top part, then the backward substitution level by level top-down (top part first, then the subtrees this GPU
@@ -1044,7 +1059,10 @@ static int build_spchol(ba_gpu_ctx *ctx) {
       return rc;
     RES(spc_cnt, ((size_t)3 * S.n_nodes + 16) * 4);
     const size_t st_ = std::max(std::max(sf, ss), su);
-    CK(cudaFuncSetAttribute(k_spchol_tree, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_));
+    if (R > 1)
+      CK(cudaFuncSetAttribute(k_spchol_tree<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_));
+    else
+      CK(cudaFuncSetAttribute(k_spchol_tree<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_));
     ctx->spc_tree = getenv("BA_SPCHOL_LEVELS") == nullptr;
     if (getenv("BA_SPCHOL_DEBUG"))
       fprintf(stderr, "[spchol] rank %d: %d parts%s, top %d nodes / %d cameras (%.1f %% of the work), heaviest part %.1f %%, "
@@ -1205,13 +1223,30 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   bool want_chol = solver == BA_SOLVER_SPARSE_SCHUR_CHOLESKY;
   if (want_chol) solver = BA_SOLVER_SPARSE_SCHUR_PCG;
   ctx->spchol = false;
+  // depth prior and / or free intrinsics through the sparse Cholesky: when asked for, and under AUTO when free intrinsics
+  // take the problem past the dense explicit limit.  It keeps the explicit solver's linearisation (planes store, W / WV) and
+  // replaces the dense S by the block-sparse one; the four intrinsics columns become a border of the tree's solve.
+  const bool sp_ref = (o.use_depth_prior || o.optimize_intrinsics) &&
+                      (want_chol || (solver == BA_SOLVER_AUTO && ctx->nk && ctx->n_red > BA_EXPLICIT_MAX_DIM && ctx->n_ranks == 1));
+  ctx->sp_ref = sp_ref;
+  // right-hand-side rows of the tree, decided by THIS upload (a context reused after set_options must not keep the border of an
+  // earlier REF problem: the NS path is the one-row tree)
+  ctx->spc_nrhs = sp_ref && ctx->nk ? 5 : 1;
+  if (sp_ref) {
+    if (ctx->n_ranks > 1)
+      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics is single-GPU");
+    if (o.jacobian_store == BA_JAC_FACTORED || o.jacobian_store == BA_JAC_TILED)
+      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics reads the planes Jacobian store");
+    solver = BA_SOLVER_EXPLICIT_CHOLESKY;
+    want_chol = false;
+  }
   if (solver == BA_SOLVER_AUTO)
     solver = (ctx->n_red <= o.explicit_max_dim || ctx->nk) ? BA_SOLVER_EXPLICIT_CHOLESKY : BA_SOLVER_IMPLICIT_PCG;
   if ((solver == BA_SOLVER_IMPLICIT_PCG || solver == BA_SOLVER_SPARSE_SCHUR_PCG) && ctx->nk)
     return fail(ctx, BA_ERR_UNSUPPORTED, "optimize_intrinsics needs the explicit solver (as ITERATIVE_SCHUR needs points only)");
   if (solver == BA_SOLVER_SPARSE_SCHUR_PCG && o.use_depth_prior)
     return fail(ctx, BA_ERR_UNSUPPORTED, "the block-sparse Schur solver needs NS mode (no depth prior, fixed intrinsics)");
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_red > BA_EXPLICIT_MAX_DIM)
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !sp_ref && ctx->n_red > BA_EXPLICIT_MAX_DIM)
     return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d)", BA_EXPLICIT_MAX_DIM,
                 ctx->n_red);
   if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks > 1)
@@ -1461,6 +1496,18 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     ctx->dist_pcg = false;
     if (!ctx->spchol && ctx->n_ranks > 1 && o.persistent_pcg == 1 && (rcs = setup_dist_pcg(ctx))) return rcs;
   }
+  if (sp_ref) {
+    prof.stamp("to sparse");
+    int rcs = build_sparse_structure(ctx);
+    if (!rcs) rcs = build_spchol(ctx);
+    if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) {
+      const std::string why = ctx->err;
+      return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d), and the sparse "
+                  "Cholesky cannot take it: %s", BA_EXPLICIT_MAX_DIM, ctx->n_red, why.c_str());
+    }
+    if (rcs) return rcs;
+    prof.stamp("sparse structure + symbolic");
+  }
   if (ctx->fact && !sparse && o.jacobian_store != BA_JAC_FACTORED && ctx->n_tiles > 0) {
     // tile-fused product: tile metadata, then (if the locality bounds hold) the tile-camera-major store
     RES(tmeta, (size_t)ctx->n_tiles * sizeof(TileMeta));
@@ -1520,7 +1567,17 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   LAUNCH(k_fill, cdiv(6 * n_cam, 256), 256, 0, P<double>(ctx->one_c), (size_t)6 * nc, 1.0);
   LAUNCH(k_fill, cdiv(3 * n_pt, 256), 256, 0, P<double>(ctx->one_p), (size_t)3 * np, 1.0);
   LAUNCH(k_fill, 1, 256, 0, P<double>(ctx->one_k), (size_t)4, 1.0);
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY) {
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && sp_ref) {
+    // no dense S, no pair list: the block-sparse structure of build_sparse_structure() holds S
+    RES(W, (no + 1) * 144);
+    RES(WV, (no + 1) * 144);
+    RES(spb_B, nc * 192 + 64);
+    RES(spb_Z, nc * 192 + 64);
+    RES(spb_kk, 20 * 8);
+    RES(spb_part, (size_t)(ctx->nblk_cam + 1) * 14 * 8);
+    CK(cudaMemsetAsync(ctx->yk.p, 0, 32, s));  // (no intrinsics: y_k stays 0)
+    prof.stamp("rest");
+  } else if (solver == BA_SOLVER_EXPLICIT_CHOLESKY) {
     RES(W, (no + 1) * 144);
     RES(WV, (no + 1) * 144);
     RES(S, (size_t)ctx->n_red * ctx->n_red * 8 + 64);
@@ -1896,7 +1953,19 @@ static SpChol spchol_args(ba_gpu_ctx *ctx) {
   a.ypos = P<double>(ctx->spc_ypos);
   a.yc = P<double>(ctx->yc);
   a.prof = getenv("BA_SPCHOL_PROF") ? P<unsigned long long>(ctx->spc_prof) : nullptr;
+  const bool border = ctx->spc_nrhs > 1;
+  a.Bc = border ? P<double>(ctx->spb_B) : nullptr;
+  a.Zb = border ? P<double>(ctx->spb_Z) : nullptr;
+  a.yk = border ? P<double>(ctx->yk) : nullptr;
   return a;
+}
+// intrinsics border between the forward and the backward substitution: T = C - Z^T Z, t = b_k - Z^T z, y_k = T^-1 t
+static void enqueue_spchol_border(ba_gpu_ctx *ctx, int gate) {
+  LmState *st = P<LmState>(ctx->st);
+  const int nblk = ctx->nblk_cam;
+  LAUNCH(k_spb_reduce, nblk, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->spb_Z), P<double>(ctx->spc_z), P<double>(ctx->spb_part), st,
+         gate);
+  LAUNCH(k_spb_solve, 1, 32, 0, nblk, P<double>(ctx->spb_part), P<double>(ctx->spb_kk), P<double>(ctx->yk), st, gate);
 }
 static void enqueue_spchol(ba_gpu_ctx *ctx, int gate) {
   LmState *st = P<LmState>(ctx->st);
@@ -1920,8 +1989,19 @@ static void enqueue_spchol(ba_gpu_ctx *ctx, int gate) {
       t.queue = P<int2>(ctx->spc_queue) + first;
       t.n_items = n;
       t.ticket = cnt + slot;
-      LAUNCH(k_spchol_tree, std::min(ctx->n_sm, n), SPC_THREADS, smem, a, t, st, gate);
+      if (ctx->spc_nrhs > 1)
+        LAUNCH((k_spchol_tree<5>), std::min(ctx->n_sm, n), SPC_THREADS, smem, a, t, st, gate);
+      else
+        LAUNCH((k_spchol_tree<1>), std::min(ctx->n_sm, n), SPC_THREADS, smem, a, t, st, gate);
     };
+    if (ctx->spc_parts == 1 && ctx->spc_nrhs > 1) {
+      // intrinsics border: the queue's factor / update prefix, the 4 x 4 border system, then the backward substitution
+      launch(0, ctx->spc_qB, 0);
+      enqueue_spchol_border(ctx, gate);
+      phase_mark(ctx, BA_PHASE_FACTOR);
+      launch(ctx->spc_qB, ctx->spc_qB_n, 1);
+      return;
+    }
     if (ctx->spc_parts == 1) {
       launch(0, ctx->spc_n_items, 0);
       phase_mark(ctx, BA_PHASE_FACTOR);
@@ -1947,12 +2027,19 @@ static void enqueue_spchol(ba_gpu_ctx *ctx, int gate) {
   ctx->pdl = !ctx->pdl_off;
   for (int l = 0; l < S.n_levels; ++l) {
     const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
-    LAUNCH(k_spchol_factor, nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, gate);
+    if (ctx->spc_nrhs > 1)
+      LAUNCH((k_spchol_factor<5>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, gate);
+    else
+      LAUNCH((k_spchol_factor<1>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, gate);
     if (l + 1 < S.n_levels) {  // (roots have no border)
       const int tiles = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
-      LAUNCH(k_spchol_update, nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, gate);
+      if (ctx->spc_nrhs > 1)
+        LAUNCH((k_spchol_update<5>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, gate);
+      else
+        LAUNCH((k_spchol_update<1>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, gate);
     }
   }
+  if (ctx->spc_nrhs > 1) enqueue_spchol_border(ctx, gate);
   phase_mark(ctx, BA_PHASE_FACTOR);
   for (int l = S.n_levels - 1; l >= 0; --l)
     LAUNCH(k_spchol_solve, S.level_ptr[l + 1] - S.level_ptr[l], SPC_THREADS, ctx->spc_smem_solve, a, S.level_ptr[l], st, gate);
@@ -2182,7 +2269,7 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
   LmState *st = P<LmState>(ctx->st);
   const int n = ctx->n_red;
   if (n == 0) return 0;
-  cudaMemsetAsync(ctx->S.p, 0, (size_t)n * n * 8, ctx->stream);
+  if (!ctx->sp_ref) cudaMemsetAsync(ctx->S.p, 0, (size_t)n * n * 8, ctx->stream);
   // side stream: point-block inverses (k_obs_W re-derives the inverse it needs), then -- once W is there -- borders +
   // right-hand side; main stream: W, then the camera-camera blocks (disjoint parts of S)
   fork_side(ctx);
@@ -2194,6 +2281,37 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
            P<double>(ctx->dp), P<double>(ctx->W), P<double>(ctx->WV), st, GATE_RUN);
   });
   side_after_main(ctx);
+  if (ctx->sp_ref) {
+    // sparse Cholesky: side stream -- camera-side vectors, then b_c, B, C and b_k by camera; main stream -- the blocks of S
+    if (ctx->nk) {
+      LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
+             P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
+             P<double>(ctx->part_ex), ctx->n_pt, P<double>(ctx->Vinv), P<double>(ctx->part_kk), st, GATE_RUN);
+      LAUNCH((k_spb_assemble<4>), cdiv(ctx->n_cam * 30 + 14, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
+             P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
+             P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
+             P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
+    } else {
+      LAUNCH((k_explicit_cam<0>), ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), P<int32_t>(ctx->pt_idx),
+             P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk), P<double>(ctx->part_ex), st, GATE_RUN);
+      LAUNCH((k_spb_assemble<0>), cdiv(ctx->n_cam * 6, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
+             P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
+             P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
+             P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
+    }
+    fork_main(ctx);
+    LAUNCH(k_sp_schur_planes, cdiv(ctx->n_sblk * 32, BA_THREADS), BA_THREADS, 0, ctx->n_sblk, P<int32_t>(ctx->sb_ptr),
+           P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->Sblk), st, GATE_RUN);
+    LAUNCH(k_sp_add_diag, cdiv(ctx->n_cam * 36, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->sp_diag), P<double>(ctx->U),
+           P<double>(ctx->Sblk), st, GATE_RUN);
+    join(ctx);
+    phase_mark(ctx, BA_PHASE_SCHUR);
+    // LM damping of the camera columns (b is already assembled), then factorisation, border and substitutions
+    LAUNCH(k_spchol_rhs, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->item_ptr), P<double>(ctx->part6), P<double>(ctx->gc),
+           P<double>(ctx->dc), P<double>(ctx->b), P<double>(ctx->dsq), st, GATE_RUN, 1);
+    enqueue_spchol(ctx, GATE_RUN);
+    return 0;
+  }
   if (ctx->nk) {
     LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
            P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
@@ -2383,10 +2501,10 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   const int64_t l0 = ctx->launches;
   CK(cudaEventRecord(ctx->ev0, ctx->stream));
   // windowed explicit solver on one GPU (single-CTA solve: every kernel is a small gated kernel): programmatic dependent launches
-  const bool pdl = !ctx->pdl_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks == 1 && ctx->n_red > 0 &&
+  const bool pdl = !ctx->pdl_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && !ctx->sp_ref && ctx->n_ranks == 1 && ctx->n_red > 0 &&
                    ctx->n_red <= BA_LDLT_MAX_N;
   ctx->pdl = pdl;
-  ctx->ph_on = ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY && getenv("BA_NO_PHASE_TIMES") == nullptr;
+  ctx->ph_on = (ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY || ctx->sp_ref) && getenv("BA_NO_PHASE_TIMES") == nullptr;
   ctx->ph_n = 0;
   phase_mark(ctx, BA_PHASE_START);
   enqueue_iteration_zero(ctx);
@@ -2396,7 +2514,7 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   int rc = 0;
   // windowed explicit solver on one GPU: the ~26 small kernels of an LM iteration (two streams, fork / join) are
   // captured once per upload and replayed
-  const bool graphed = !ctx->lm_graph_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks == 1 &&
+  const bool graphed = !ctx->lm_graph_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && !ctx->sp_ref && ctx->n_ranks == 1 &&
                        ctx->n_red > 0 && ctx->n_red <= BA_LDLT_MAX_N;
   for (int it = 1;; ++it) {
     if (graphed) {
@@ -2666,6 +2784,7 @@ extern "C" int ba_gpu_schur_matvec(ba_gpu_ctx *ctx, double radius, const double 
   if (!ctx || !x || !y) return BA_ERR_INVALID;
   if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_schur_matvec before ba_gpu_upload");
   if (ctx->nk) return fail(ctx, BA_ERR_UNSUPPORTED, "implicit Schur product needs optimize_intrinsics = 0");
+  if (ctx->sp_ref) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_matvec with the sparse Cholesky needs NS mode");
   CK(cudaSetDevice(ctx->device));
   ctx->sp_full_next = true;  // (the product needs every block of S on every rank)
   int rc = prepare_linear_system(ctx, radius);
@@ -2692,6 +2811,7 @@ extern "C" int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *
   if (!ctx || !rhs || !y) return BA_ERR_INVALID;
   if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_schur_solve before ba_gpu_upload");
   if (!ctx->spchol) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs the sparse Cholesky solver");
+  if (ctx->sp_ref) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs NS mode (no depth prior, fixed intrinsics)");
   CK(cudaSetDevice(ctx->device));
   int rc = prepare_linear_system(ctx, radius);
   if (rc) return rc;

@@ -13,7 +13,11 @@
 //     36 warp-broadcast loads of the pivot rows + a conflict-free read-modify-write of its six entries.
 //   * The 6x6 pivot block is factorised by warp 0 with shuffles (lane = row) while the other warps still run the
 //     trailing update of the previous step (look-ahead): two CTA barriers per eliminated camera.
-//   * The right-hand side rides along as one more row (forward substitution fused into the factorisation).
+//   * The right-hand side rides along as one more row (forward substitution fused into the factorisation).  With free
+//     intrinsics (REF cost) it is R = 5 rows: b_c and the four columns of the camera-intrinsics border B, so the forward
+//     substitution yields z = L^-1 b_c and Z = L^-1 B; the 4x4 border system T y_k = t (T = C - Z^T Z, t = b_k - Z^T z)
+//     is solved between factorisation and backward substitution (k_spb_reduce / k_spb_solve), and the backward
+//     substitution solves L^T y_c = z - Z y_k.  The symbolic phase, the tree and the supernodes are the same for R = 1, 5.
 //   * The panel goes to HBM/L2 for the backward substitution; the node's update matrix U = L_B L_B^T (+ what its children
 //     pass through) -- two thirds of the multiply-adds, no dependent chain -- is formed by a second launch per level with
 //     several thread blocks per node (k_spchol_update), for the parent's extend-add.
@@ -37,6 +41,11 @@ struct SpChol {
   double *z, *linv, *ypos;    // by elimination position: forward-substituted rhs [6], inverse pivot blocks [36], solution [6]
   double *yc;                 // solution by camera [6 n_cam]
   unsigned long long *prof;   // nullable (BA_SPCHOL_PROF=1): ns per phase of thread block 0 of every factor launch, summed
+  // intrinsics border (R = 5; nullptr otherwise): B by camera [24 n_cam] (6 x 4 row-major per camera), Z = L^-1 B by
+  // elimination position [24 n_cam] (6 x 4 row-major per position), y_k [4] (read by the backward substitution)
+  const double *Bc;
+  double *Zb;
+  const double *yk;
 };
 #define SPC_TICK(slot)                                          \
   if (a.prof && prof_block && tid == 0) {                       \
@@ -47,7 +56,8 @@ struct SpChol {
   }
 
 __host__ __device__ inline size_t spc_off(const int32_t *N, int lo) { return ((size_t)N[lo + 1] << 31) | (size_t)N[lo]; }
-inline size_t spc_factor_smem(int m, int nb) { return ((size_t)36 * (m + nb) * (m + 1) + 6 * m + 72 + 8) * 8; }
+// (R: right-hand-side rows, 1 or 5)
+inline size_t spc_factor_smem(int m, int nb, int R = 1) { return ((size_t)36 * (m + nb) * (m + 1) + 6 * m * R + 72 + 8) * 8; }
 inline size_t spc_solve_smem(int m, int nb) { return ((size_t)36 * m * m + 36 * m + 6 * nb + 12 * m + 8) * 8; }
 
 // right-hand side b = -g_c - sum (J_c^T J_p V^-1 g_p partials) and LM damping D^2 = (sqrt(diag / radius))^2 per camera column
@@ -160,6 +170,8 @@ __device__ __forceinline__ void spc_wait_ge(const int *flag, int want) {
 }
 // (udone / tiles: completion counters of the persistent tree kernel -- the node waits for its children's update matrices only
 //  AFTER it has assembled its stored blocks of S, which do not depend on them; nullptr: one launch per level, nothing to wait for)
+// NR right-hand-side rows (1: b; 5: b and the four border columns), row r of the own cameras at zf[r * C6 ..]
+template <int NR>
 __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool prof_block, LmState *st, double *spc_sm,
                                                 const int *udone = nullptr, const int32_t *tiles = nullptr) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -168,14 +180,18 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
   const int LD = 6 * (m + nb), C6 = 6 * m;
   double *P = spc_sm;                    // panel, column-major, LD x C6
   double *LT = P + (size_t)LD * C6;      // current pivot column block, row-major: LT[R * 6 + c]
-  double *zf = LT + (size_t)LD * 6;      // right-hand side of the own cameras
-  double *Tb = zf + C6;                  // two inverse pivot blocks (ping-pong)
+  double *zf = LT + (size_t)LD * 6;      // right-hand-side rows of the own cameras
+  double *Tb = zf + NR * C6;             // two inverse pivot blocks (ping-pong)
 
   unsigned long long t0_ = 0;
   if (a.prof && prof_block && tid == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0_));
   // ---- phase 0: clear, right-hand side
   for (int i = tid; i < LD * C6; i += SPC_THREADS) P[i] = 0.0;
-  for (int i = tid; i < C6; i += SPC_THREADS) zf[i] = a.b[6 * (size_t)a.perm[k0 + i / 6] + i % 6];
+  for (int i = tid; i < NR * C6; i += SPC_THREADS) {
+    const int r = i / C6, j = i - r * C6;
+    const int cam = a.perm[k0 + j / 6];
+    zf[i] = r == 0 ? a.b[6 * (size_t)cam + j % 6] : a.Bc[24 * (size_t)cam + (j % 6) * 4 + r - 1];
+  }
   __syncthreads();
   // ---- phase 1a: stored blocks of S (one thread per scalar, entry records through 16-byte broadcast loads), damping on
   //      the diagonal.  Independent iterations: unrolled so that several dependent load chains are in flight.
@@ -227,7 +243,7 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
       n_in = lo;
     }
     const double *Uc = a.U + 36 * spc_off(Cn, SPN_U_LO);
-    const double *ruc = a.ru + 6 * (size_t)Cn[SPN_BORD];
+    const double *ruc = a.ru + 6 * NR * (size_t)Cn[SPN_BORD];  // (row r of the child's rhs update at ruc[r * nbc6 ..])
     // one warp per scalar column of the child's update matrix (block lower triangle: rows from the column's own block
     // down), lanes along the rows: coalesced reads of the column from L2, up to four independent loads in flight per lane
     // before the first one is consumed (this gather was the longest piece of a node's critical path: one dependent
@@ -256,7 +272,10 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
           if (dst[u] >= 0) pcol[dst[u]] -= v[u];
       }
     }
-    for (int idx = tid; idx < 6 * n_in; idx += SPC_THREADS) zf[6 * __ldg(rel + idx / 6) + idx % 6] -= __ldcg(ruc + idx);
+    for (int idx = tid; idx < NR * 6 * n_in; idx += SPC_THREADS) {
+      const int r = idx / (6 * n_in), e = idx - r * 6 * n_in;
+      zf[r * C6 + 6 * __ldg(rel + e / 6) + e % 6] -= __ldcg(ruc + (size_t)r * nbc6 + e);
+    }
     __syncthreads();
   }
   SPC_TICK(1)
@@ -282,14 +301,17 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
       }
     }
     if (warp == 0) {
+      // lane = (rhs row r, component l): 6 NR <= 30 lanes
+      const int r = lane / 6, l = lane - 6 * r;
+      double *zr = zf + r * C6 + 6 * k;
       double v = 0.0;
-      if (lane < 6) {
+      if (lane < 6 * NR) {
 #pragma unroll
         for (int c = 0; c < 6; ++c)
-          if (c <= lane) v += T[lane * 6 + c] * zf[6 * k + c];
+          if (c <= l) v += T[l * 6 + c] * zr[c];
       }
       __syncwarp();
-      if (lane < 6) zf[6 * k + lane] = v;
+      if (lane < 6 * NR) zr[l] = v;
     }
     __syncthreads();
     if (k + 1 == m) break;
@@ -309,10 +331,13 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
           for (int c = 0; c < 6; ++c) s += x[c] * lj[c];
           P[(size_t)(6 * j + bb) * LD + R] -= s;
         }
-        double s = 0.0;
 #pragma unroll
-        for (int c = 0; c < 6; ++c) s += x[c] * zf[6 * k + c];
-        zf[R] -= s;
+        for (int r = 0; r < NR; ++r) {
+          double s = 0.0;
+#pragma unroll
+          for (int c = 0; c < 6; ++c) s += x[c] * zf[r * C6 + 6 * k + c];
+          zf[r * C6 + R] -= s;
+        }
       }
       __syncwarp();
       ok = spc_chol6(P, LD, k + 1, lane, Tb + ((k + 1) & 1) * 36, a.linv + 36 * (size_t)(k0 + k + 1)) && ok;
@@ -345,10 +370,13 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
               }
             }
             if (g == 0) {
-              double s = 0.0;
 #pragma unroll
-              for (int c = 0; c < 6; ++c) s += x[c] * zf[6 * k + c];
-              zf[R] -= s;
+              for (int r = 0; r < NR; ++r) {
+                double s = 0.0;
+#pragma unroll
+                for (int c = 0; c < 6; ++c) s += x[c] * zf[r * C6 + 6 * k + c];
+                zf[r * C6 + R] -= s;
+              }
             }
           } else {
             const int R1 = b0 + (u - n_own), R2 = R1 + n_pair;
@@ -385,16 +413,22 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
     double *Pg = a.panel + 36 * spc_off(N, SPN_PANEL_LO);
     for (int i = tid; i < LD * C6; i += SPC_THREADS) Pg[i] = P[i];
     for (int i = tid; i < C6; i += SPC_THREADS) a.z[6 * (size_t)k0 + i] = zf[i];
+    if (NR > 1)
+      for (int i = tid; i < (NR - 1) * C6; i += SPC_THREADS) {
+        const int q = i / C6, j = i - q * C6;
+        a.Zb[4 * (6 * (size_t)k0 + j) + q] = zf[(q + 1) * C6 + j];
+      }
   }
   __syncthreads();
   SPC_TICK(3)
   if (a.prof && prof_block && tid == 0) a.prof[4] += 1;
 }
+template <int NR>
 __global__ void __launch_bounds__(SPC_THREADS, 1)
 k_spchol_factor(SpChol a, int lvl_first, LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   extern __shared__ __align__(16) double spc_sm[];
-  spc_factor_node(a, a.level_nodes[lvl_first + blockIdx.x], blockIdx.x == 0, st, spc_sm);
+  spc_factor_node<NR>(a, a.level_nodes[lvl_first + blockIdx.x], blockIdx.x == 0, st, spc_sm);
 }
 
 // Update matrix of the nodes of one level, after their panels are factorised: U = L_B L_B^T + what the children pass through
@@ -403,9 +437,9 @@ k_spchol_factor(SpChol a, int lvl_first, LmState *st, int gate) {
 // levels of the tree have fewer nodes than the GPU has SMs.  Every block loads the node's border rows of the panel (L2-resident,
 // just written) into shared memory and takes every tiles-th chunk of the 3 x 6 output pieces.
 #define SPU_THREADS 256
-inline size_t spc_update_smem(int m, int nb) { return ((size_t)36 * nb * m + 6 * m + 8) * 8; }
-// tile `tile` of `tiles` of the update matrix of node `id`, by the calling thread block (NT threads)
-template <int NT>
+inline size_t spc_update_smem(int m, int nb, int R = 1) { return ((size_t)36 * nb * m + 6 * m * R + 8) * 8; }
+// tile `tile` of `tiles` of the update matrix of node `id`, by the calling thread block (NT threads); NR right-hand-side rows
+template <int NT, int NR>
 __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int tile, int tiles, double *spc_sm) {
   const int tid = threadIdx.x;
   const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
@@ -422,6 +456,11 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
       LB[idx] = __ldcg(Pg + (size_t)c * LD + r);  // (L2: written by another thread block of this or the previous launch)
     }
     for (int i = tid; i < C6; i += NT) zf[i] = __ldcg(a.z + 6 * (size_t)k0 + i);
+    if (NR > 1)
+      for (int i = tid; i < (NR - 1) * C6; i += NT) {
+        const int q = i / C6, j = i - q * C6;
+        zf[(q + 1) * C6 + j] = __ldcg(a.Zb + 4 * (6 * (size_t)k0 + j) + q);
+      }
   }
   __syncthreads();
   double *Ug = a.U + 36 * spc_off(N, SPN_U_LO);
@@ -469,24 +508,28 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
 #pragma unroll
       for (int x = 0; x < 3; ++x) Ug[(size_t)(rb + y) * NB6 + ra + x] = acc[x][y];
   }
-  double *rug = a.ru + 6 * (size_t)N[SPN_BORD];
-  for (int idx = tile * NT + tid; idx < NB6; idx += tiles * NT) {
+  // rhs updates: row r of the node at ru[6 NR bord + r NB6 ..]
+  double *rug = a.ru + 6 * NR * (size_t)N[SPN_BORD];
+  for (int idx = tile * NT + tid; idx < NR * NB6; idx += tiles * NT) {
+    const int r = idx / NB6, e = idx - r * NB6;
+    const double *zr = zf + r * C6;
     double s = 0.0;
-    for (int c = 0; c < C6; ++c) s += LB[(size_t)c * NB6 + idx] * zf[c];
+    for (int c = 0; c < C6; ++c) s += LB[(size_t)c * NB6 + e] * zr[c];
     for (int ci = 0; ci < nch; ++ci) {
       const int ch = a.children[N[SPN_CHILD] + ci];
       const int32_t *Cn = a.node + (size_t)ch * SPSYM_NODE_INTS;
-      const int ii = a.inv[Cn[SPN_INV] + idx / 6];
-      if (ii >= 0) s += __ldcg(a.ru + 6 * (size_t)Cn[SPN_BORD] + 6 * ii + idx % 6);
+      const int ii = a.inv[Cn[SPN_INV] + e / 6];
+      if (ii >= 0) s += __ldcg(a.ru + 6 * NR * (size_t)Cn[SPN_BORD] + (size_t)r * 6 * Cn[SPN_NB] + 6 * ii + e % 6);
     }
     rug[idx] = s;
   }
 }
+template <int NR>
 __global__ void __launch_bounds__(SPU_THREADS, 1)
 k_spchol_update(SpChol a, int lvl_first, int tiles, LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   extern __shared__ __align__(16) double spc_sm[];
-  spc_update_node<SPU_THREADS>(a, a.level_nodes[lvl_first + blockIdx.x / tiles], blockIdx.x % tiles, tiles, spc_sm);
+  spc_update_node<SPU_THREADS, NR>(a, a.level_nodes[lvl_first + blockIdx.x / tiles], blockIdx.x % tiles, tiles, spc_sm);
 }
 
 // backward substitution of one tree level (parents are done): y_O = L_OO^-T (z_O - L_BO^T y_B)
@@ -509,7 +552,12 @@ __device__ __forceinline__ void spc_solve_node(const SpChol &a, int id, LmState 
   for (int i = tid; i < 36 * m; i += SPC_THREADS) Ti[i] = __ldcg(a.linv + 36 * (size_t)k0 + i);
   for (int i = tid; i < NB6; i += SPC_THREADS) yB[i] = __ldcg(a.ypos + 6 * (size_t)bord[i / 6] + i % 6);
   for (int i = tid; i < C6; i += SPC_THREADS) {
-    w[i] = __ldcg(a.z + 6 * (size_t)k0 + i);
+    double v = __ldcg(a.z + 6 * (size_t)k0 + i);
+    if (a.Zb) {  // intrinsics border: L^T y_c = z - Z y_k
+      const double *zr = a.Zb + 4 * (6 * (size_t)k0 + i);
+      v -= ((__ldcg(zr) * __ldcg(a.yk) + __ldcg(zr + 1) * __ldcg(a.yk + 1)) + __ldcg(zr + 2) * __ldcg(a.yk + 2)) + __ldcg(zr + 3) * __ldcg(a.yk + 3);
+    }
+    w[i] = v;
     y[i] = 0.0;
   }
   __syncthreads();
@@ -580,6 +628,7 @@ struct SpTree {
   const int32_t *tiles;    // update tiles per node (0: no border)
   int *ticket, *fdone, *udone, *sdone;
 };
+template <int NR>
 __global__ void __launch_bounds__(SPC_THREADS, 1)
 k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
@@ -596,7 +645,7 @@ k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
     const int id = q.x;
     const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
     if (q.y == -1) {
-      spc_factor_node(a, id, it == 0, st, spc_sm, t.udone, t.tiles);
+      spc_factor_node<NR>(a, id, it == 0, st, spc_sm, t.udone, t.tiles);
       __syncthreads();
       if (tid == 0) {
         __threadfence();
@@ -605,7 +654,7 @@ k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
     } else if (q.y >= 0) {
       if (tid == 0) spc_wait_ge(t.fdone + id, 1);
       __syncthreads();
-      spc_update_node<SPC_THREADS>(a, id, q.y, t.tiles[id], spc_sm);
+      spc_update_node<SPC_THREADS, NR>(a, id, q.y, t.tiles[id], spc_sm);
       __syncthreads();
       if (tid == 0) {
         __threadfence();
@@ -645,4 +694,180 @@ __global__ void k_spchol_dist_pre(int n_cam, int n_top, const int32_t *topcams, 
 __global__ void k_spchol_dist_post(int n_cam, const double *yc, LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   if (threadIdx.x == 0 && yc[6 * (size_t)n_cam] != 0.0) st->lin_fail = 1;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Sparse Cholesky of the REF / DEPTH / INTR cost (depth prior and / or free intrinsics, planes store): the explicit path's
+// per-observation W = Jc^T Jp and WV = W V^-1 (k_obs_W, already Jacobi-scaled) summed into the device-built block structure
+// (build_sparse_structure), the camera-intrinsics border B, the corner C and the right-hand side assembled by camera, and the
+// 4 x 4 border system solved between the forward and the backward substitution.
+// ---------------------------------------------------------------------------------------------
+// values of S from the planes: one warp per block, S_b = -sum_pairs WV_a W_b^T in the fixed pair order of the block
+// (lanes stride the pairs, then the recursive-halving warp sum); k_sp_add_diag then puts U on the diagonal blocks
+__global__ void __launch_bounds__(BA_THREADS)
+k_sp_schur_planes(int n_blk, const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ pairs,
+                  const double *__restrict__ W, const double *__restrict__ WV, double *__restrict__ S, const LmState *st, int gate) {
+  if (!gate_open(st, gate)) return;
+  const int b = (int)((blockIdx.x * (size_t)BA_THREADS + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (b >= n_blk) return;
+  double acc[36];
+#pragma unroll
+  for (int k = 0; k < 36; ++k) acc[k] = 0.0;
+  const int e1 = blk_ptr[b + 1];
+  for (int e = blk_ptr[b] + lane; e < e1; e += 32) {
+    const unsigned long long pr = __ldg(pairs + e);
+    const double *wv = WV + 18 * (size_t)(pr >> 32), *w = W + 18 * (size_t)(pr & 0xffffffffu);
+    double A[18], B[18];
+#pragma unroll
+    for (int k = 0; k < 18; ++k) {
+      A[k] = __ldg(wv + k);
+      B[k] = __ldg(w + k);
+    }
+#pragma unroll
+    for (int r = 0; r < 6; ++r)
+#pragma unroll
+      for (int c = 0; c < 6; ++c) acc[r * 6 + c] += A[3 * r] * B[3 * c] + A[3 * r + 1] * B[3 * c + 1] + A[3 * r + 2] * B[3 * c + 2];
+  }
+  int idx, cnt;
+  sp_reduce_scatter36(acc, lane, idx, cnt);
+  double *Sb = S + 36 * (size_t)b + idx;
+  if (cnt > 0) Sb[0] = -acc[0];
+  if (cnt > 1) Sb[1] = -acc[1];
+}
+
+// right-hand side, border and corner by camera: k_explicit_assemble<NK>'s arithmetic with the destinations of the sparse
+// solve.  b[6 c] = -g_c + W V^-1 g_p; (NK) B[24 c] = U_ck - sum WV Wk^T (zero for the fixed camera), kk[0..15] = C (damped),
+// kk[16..19] = b_k.  Item partials are added in item order, point-tile partials in tile order.
+template <int NK>
+__global__ void __launch_bounds__(BA_THREADS)
+k_spb_assemble(int n_cam, int fixed_cam, const int32_t *__restrict__ item_ptr, const double *__restrict__ part_cam, int nblk_pt,
+               const double *__restrict__ part_kk, const double *__restrict__ gc, const double *__restrict__ Uck,
+               const double *__restrict__ Ukk, const double *__restrict__ gk, const double *__restrict__ dk, double *__restrict__ b,
+               double *__restrict__ Bc, double *__restrict__ kk, const LmState *st, int gate) {
+  if (!gate_open(st, gate)) return;
+  constexpr int NV = 6 + (NK ? 24 : 0);
+  const int idx = blockIdx.x * BA_THREADS + threadIdx.x;
+  if (idx < n_cam * NV) {
+    const int c = idx / NV, k = idx - c * NV;
+    const bool fixed = c == fixed_cam;
+    double acc = 0.0;
+    for (int it = item_ptr[c]; it < item_ptr[c + 1]; ++it) acc += part_cam[(size_t)it * NV + k];
+    if (k < 6)
+      b[6 * (size_t)c + k] = fixed ? 0.0 : -gc[6 * (size_t)c + k] + acc;
+    else if (NK)
+      Bc[24 * (size_t)c + k - 6] = fixed ? 0.0 : Uck[24 * (size_t)c + k - 6] - acc;
+  } else if (NK && idx < n_cam * NV + 14) {
+    const int k = idx - n_cam * NV;
+    double v = 0.0;
+    for (int t = 0; t < nblk_pt; ++t) v += part_kk[14 * (size_t)t + k];
+    if (k < 10) {
+      int a = 0, r = k;  // k-th entry of the row-major upper triangle of the 4 x 4 block -> (a, b)
+      while (r >= 4 - a) {
+        r -= 4 - a;
+        ++a;
+      }
+      const int b2 = a + r;
+      double x = Ukk[a * 4 + b2] - v;
+      if (a == b2) {
+        const double D = sqrt(dk[a] / st->radius);
+        x += D * D;
+      }
+      kk[a * 4 + b2] = x;
+      kk[b2 * 4 + a] = x;
+    } else {
+      kk[16 + k - 10] = -gk[k - 10] + v;
+    }
+  }
+}
+
+// border reduction after the forward substitution: per thread block, over its elimination positions (one per thread),
+// Z^T Z (10 upper entries) and Z^T z (4), block sums in a fixed tree -> part[14 blockIdx.x ..]
+__global__ void __launch_bounds__(BA_THREADS)
+k_spb_reduce(int n_pos, const double *__restrict__ Zb, const double *__restrict__ z, double *__restrict__ part, const LmState *st,
+             int gate) {
+  if (!gate_open(st, gate)) return;
+  __shared__ double red[BA_WARPS + 1];
+  const int p = blockIdx.x * BA_THREADS + threadIdx.x;
+  double v[14];
+#pragma unroll
+  for (int k = 0; k < 14; ++k) v[k] = 0.0;
+  if (p < n_pos) {
+#pragma unroll
+    for (int r = 0; r < 6; ++r) {
+      double zr[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) zr[q] = __ldcg(Zb + 4 * (6 * (size_t)p + r) + q);
+      const double zz = __ldcg(z + 6 * (size_t)p + r);
+      int u = 0;
+#pragma unroll
+      for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int c = a; c < 4; ++c) v[u++] += zr[a] * zr[c];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) v[10 + a] += zr[a] * zz;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 14; ++k) {
+    const double s = block_sum(v[k], red);
+    if (threadIdx.x == 0) part[14 * (size_t)blockIdx.x + k] = s;
+  }
+}
+
+// the border system, one warp: partials added in block order, T = C - Z^T Z, t = b_k - Z^T z, y_k = T^-1 t by a 4 x 4
+// Cholesky.  A non-positive or non-finite pivot sets lin_fail (y_k = 0 then).
+__global__ void __launch_bounds__(32)
+k_spb_solve(int nblk, const double *__restrict__ part, const double *__restrict__ kk, double *__restrict__ yk, LmState *st, int gate) {
+  if (!gate_open(st, gate)) return;
+  __shared__ double s[14];
+  const int lane = threadIdx.x;
+  if (lane < 14) {
+    double v = 0.0;
+    for (int b = 0; b < nblk; ++b) v += __ldcg(part + 14 * (size_t)b + lane);
+    s[lane] = v;
+  }
+  __syncwarp();
+  if (lane != 0) return;
+  double T[4][4], t[4];
+  int u = 0;
+  for (int a = 0; a < 4; ++a)
+    for (int c = a; c < 4; ++c) {
+      T[a][c] = kk[a * 4 + c] - s[u++];
+      T[c][a] = T[a][c];
+    }
+  for (int a = 0; a < 4; ++a) t[a] = kk[16 + a] - s[10 + a];
+  bool ok = true;
+  for (int j = 0; j < 4; ++j) {  // L in the lower triangle of T
+    double d = T[j][j];
+    for (int k = 0; k < j; ++k) d -= T[j][k] * T[j][k];
+    if (!(d > 0.0) || !isfinite(d)) {
+      ok = false;
+      break;
+    }
+    T[j][j] = sqrt(d);
+    for (int i = j + 1; i < 4; ++i) {
+      double x = T[i][j];
+      for (int k = 0; k < j; ++k) x -= T[i][k] * T[j][k];
+      T[i][j] = x / T[j][j];
+    }
+  }
+  double y[4] = {0.0, 0.0, 0.0, 0.0};
+  if (ok) {
+    for (int i = 0; i < 4; ++i) {
+      double x = t[i];
+      for (int k = 0; k < i; ++k) x -= T[i][k] * y[k];
+      y[i] = x / T[i][i];
+    }
+    for (int i = 3; i >= 0; --i) {
+      double x = y[i];
+      for (int k = i + 1; k < 4; ++k) x -= T[k][i] * y[k];
+      y[i] = x / T[i][i];
+    }
+    for (int i = 0; i < 4; ++i) ok = ok && isfinite(y[i]);
+  }
+  if (!ok) {
+    st->lin_fail = 1;
+    for (int i = 0; i < 4; ++i) y[i] = 0.0;
+  }
+  for (int i = 0; i < 4; ++i) yk[i] = y[i];
 }

@@ -45,7 +45,10 @@ enum {
 };
 
 enum {
-  BA_SOLVER_AUTO = 0,              /* dense explicit if reduced dim <= explicit_max_dim (or free intrinsics);
+  BA_SOLVER_AUTO = 0,              /* dense explicit if reduced dim <= explicit_max_dim, or with free intrinsics
+                                      up to reduced dim 16,384; free intrinsics beyond 16,384 (one GPU): the
+                                      sparse Cholesky with the intrinsics border (_SPARSE_SCHUR_CHOLESKY;
+                                      BA_ERR_UNSUPPORTED with the reason when its fronts do not fit);
                                       else block-sparse S if the co-visibility is sparse (NS mode), factorised
                                       exactly (_SPARSE_SCHUR_CHOLESKY) when its fronts fit, else with PCG;
                                       else implicit */
@@ -60,8 +63,13 @@ enum {
   BA_SOLVER_SPARSE_SCHUR_CHOLESKY = 4 /* the same block-sparse S factorised EXACTLY by a supernodal multifrontal
                                       Cholesky over a nested-dissection tree of the camera sequence
                                       (== Ceres SPARSE_SCHUR, the reference's own setting,
-                                      headers/BundleAdjustmentConfig.h:62). NS mode only; BA_ERR_UNSUPPORTED
-                                      when a front does not fit shared memory (AUTO then keeps PCG). */
+                                      headers/BundleAdjustmentConfig.h:62).  Every cost mode: with depth
+                                      prior and / or free intrinsics (REF, the reference's cost) S comes from
+                                      the planes store and the four intrinsics columns are a dense border,
+                                      solved by a 4x4 Schur complement between the forward and the backward
+                                      substitution; one GPU, jacobian_store AUTO or PLANES.  BA_ERR_UNSUPPORTED
+                                      when a front does not fit shared memory (AUTO on an NS problem then
+                                      keeps PCG). */
 };
 
 enum {
@@ -186,8 +194,9 @@ int ba_gpu_get_indices(ba_gpu_ctx *ctx, int32_t *perm_pt_major,
 /* y = S x (reduced camera system at the current state, given radius), unscaled
  * coordinates, x,y [n_cam*6] host buffers. Runs the implicit-Schur kernels. */
 int ba_gpu_schur_matvec(ba_gpu_ctx *ctx, double radius, const double *x, double *y);
-/* y = (S + D^2)^-1 rhs through the sparse Cholesky of the last upload (BA_SOLVER_SPARSE_SCHUR_CHOLESKY in force),
- * same conventions as ba_gpu_schur_matvec: ba_gpu_schur_matvec(radius, ba_gpu_schur_solve(radius, b)) == b */
+/* y = (S + D^2)^-1 rhs through the sparse Cholesky of the last upload (BA_SOLVER_SPARSE_SCHUR_CHOLESKY in force, NS mode:
+ * BA_ERR_UNSUPPORTED with depth prior or free intrinsics, as for ba_gpu_schur_matvec then), same conventions as
+ * ba_gpu_schur_matvec: ba_gpu_schur_matvec(radius, ba_gpu_schur_solve(radius, b)) == b */
 int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *rhs, double *y);
 /* structure of the sparse Cholesky of the last upload (zeros when another solver is in force): info[0..10] as
  * ba_sparse_symbolic_info, info[11] = host microseconds of the symbolic phase, info[12] = parts of the subtree-to-rank
@@ -242,8 +251,8 @@ const char *ba_gpu_phase_name(int32_t phase);
 int64_t ba_gpu_launch_count(const ba_gpu_ctx *ctx);
 /* BA_JAC_* in force after the last upload (what BA_JAC_AUTO resolved to) */
 int ba_gpu_jacobian_store_used(const ba_gpu_ctx *ctx);
-/* block-sparse Schur structure of the last upload (zeros for the other solvers): same-point
- * observation pairs, stored upper blocks, row entries (each off-diagonal block appears twice) */
+/* block-sparse Schur structure of the last upload (BA_SOLVER_SPARSE_SCHUR_PCG / _CHOLESKY in any cost mode; zeros for the
+ * other solvers): same-point observation pairs, stored upper blocks, row entries (each off-diagonal block appears twice) */
 int ba_gpu_sparse_stats(const ba_gpu_ctx *ctx, int64_t *n_pairs, int32_t *n_blocks, int32_t *n_entries);
 
 /* ---- device-resident keyframe / landmark store for sliding windows (SURVEY.md 8f row N1) ----
