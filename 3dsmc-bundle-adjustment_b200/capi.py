@@ -67,7 +67,7 @@ EXPORTS = [
     "ba_gpu_upload", "ba_gpu_solve", "ba_gpu_get_trace", "ba_gpu_download", "ba_gpu_eval", "ba_gpu_get_indices",
     "ba_gpu_schur_matvec", "ba_gpu_se3_plus", "ba_gpu_time_kernel", "ba_gpu_launch_count", "ba_gpu_comm_unique_id",
     "ba_gpu_comm_init", "ba_gpu_jacobian_store_used", "ba_gpu_sparse_stats", "ba_gpu_backproject",
-    "ba_gpu_schur_solve", "ba_gpu_spchol_info", "ba_gpu_phase_times", "ba_gpu_phase_name",
+    "ba_gpu_schur_solve", "ba_gpu_spchol_info", "ba_gpu_covariance", "ba_gpu_phase_times", "ba_gpu_phase_name",
     "ba_store_create", "ba_store_destroy", "ba_store_clear", "ba_store_set_keyframe", "ba_store_set_keyframes", "ba_store_set_poses", "ba_store_set_landmarks",
     "ba_store_window_solve",
     "ba_sparse_symbolic_create", "ba_sparse_symbolic_info", "ba_sparse_symbolic_get", "ba_sparse_symbolic_destroy",
@@ -118,6 +118,8 @@ def load():
     L.ba_gpu_phase_name.restype = C.c_char_p
     L.ba_gpu_schur_solve.argtypes = [vp, C.c_double, c_double_p, c_double_p]
     L.ba_gpu_spchol_info.argtypes = [vp, C.POINTER(C.c_int64)]
+    L.ba_gpu_covariance.argtypes = [vp, c_double_p, c_double_p, c_double_p, c_double_p, C.c_int32, c_int32_p, c_int32_p,
+                                    c_double_p]
     L.ba_store_create.argtypes = [vp, C.POINTER(vp)]
     L.ba_store_destroy.argtypes = [vp]
     L.ba_store_destroy.restype = None

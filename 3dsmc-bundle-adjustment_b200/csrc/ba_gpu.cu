@@ -14,6 +14,7 @@
 #include "ba_kernels_dist.cuh"
 #include "ba_kernels_chol.cuh"
 #include "ba_kernels_spchol.cuh"
+#include "ba_kernels_selinv.cuh"
 #include "ba_kernels_store.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -177,6 +178,14 @@ struct ba_gpu_ctx {
   bool sp_ref = false;
   int spc_nrhs = 1;
   Buf spb_B, spb_Z, spb_kk, spb_part;
+  // covariance (ba_gpu_covariance, ba_kernels_selinv.cuh), built by the first call after an upload: selected-inversion queue,
+  // Y scratch (panel-shaped), X = A^-1 B by position [4 x 6 n_cam], T^-1, Sigma on the stored blocks of S, Sigma_ck (scaled),
+  // block -> front records, camera -> position, outputs
+  bool cov_ready = false;
+  int cov_n_items = 0;
+  size_t cov_smem = 0;
+  Buf cov_Y, cov_X, cov_zq, cov_yscr, cov_Tinv, cov_S, cov_ck, cov_brec, cov_pos, cov_queue, cov_tiles, cov_cnt, cov_cam, cov_ci,
+      cov_pt, cov_pin, cov_pout, cov_bad;
   // phase timing of the large-problem solvers: CUDA events on the solver stream at the phase boundaries of every LM
   // iteration of the last solve (a few dozen event records per iteration: < 0.1 % of a multi-millisecond iteration)
   std::vector<cudaEvent_t> ph_ev;
@@ -1202,6 +1211,7 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   ctx->uploaded = false;
   ctx->lm_graph_stale = true;
   ctx->linearized = false;
+  ctx->cov_ready = false;
   const ba_gpu_options &o = ctx->opt;
   if (n_cam <= 0 || n_pt < 0 || n_obs < 0 || !pose7 || !intr4 || (n_pt > 0 && !pt3) ||
       (n_obs > 0 && (!cam_idx || !pt_idx || !uv2)))
@@ -2831,6 +2841,272 @@ extern "C" int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *
   CK(cudaGetLastError());
   if (ctx->h_st->lin_fail) return fail(ctx, BA_ERR_NUMERIC, "sparse Cholesky: non-positive pivot");
   for (size_t i = 0; i < n; ++i) y[i] = bs[i] * sc[i];
+  return BA_OK;
+}
+
+// ------------------------------------------------------------------ covariance
+// structure of ba_gpu_covariance, once per upload: under another solver (dense explicit, matrix-free PCG) the block structure and the symbolic tree
+// that solver = 4 builds (the sp_ref branch of the upload); then the selected-inversion queue, the block -> front records and
+// the scratch buffers.  Growing buffers a captured LM-iteration graph may point at marks that graph stale.
+static int cov_prepare(ba_gpu_ctx *ctx) {
+  if (ctx->cov_ready) return 0;
+  cudaStream_t s = ctx->stream;
+  int rc;
+  if (!ctx->sp_ref) {
+    ctx->lm_graph_stale = true;
+    if ((rc = build_sparse_structure(ctx))) return rc;
+    ctx->spc_nrhs = ctx->nk ? 5 : 1;
+    rc = build_spchol(ctx);
+    ctx->spchol = false;  // (the LM solve of this context stays the dense explicit one)
+    if (rc == BA_ERR_UNSUPPORTED) {
+      const std::string why = ctx->err;
+      return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance: %s", why.c_str());
+    }
+    if (rc) return rc;
+    const size_t nc = (size_t)ctx->n_cam;
+    RES(W, ((size_t)ctx->n_obs + 1) * 144);  // (the matrix-free PCG, AUTO on a large DEPTH problem, has no per-observation W)
+    RES(WV, ((size_t)ctx->n_obs + 1) * 144);
+    RES(spb_B, nc * 192 + 64);
+    RES(spb_Z, nc * 192 + 64);
+    RES(spb_kk, 20 * 8);
+    RES(spb_part, (size_t)(ctx->nblk_cam + 1) * 14 * 8);
+  }
+  const SpSymbolic &S = ctx->sym;
+  auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
+  // queue: levels top-down; per level the prepare items, the product tiles (more per node where the level has few nodes), the
+  // finish items
+  std::vector<int32_t> q, tiles((size_t)S.n_nodes, 0);
+  size_t smem = 0;
+  for (int l = S.n_levels - 1; l >= 0; --l) {
+    const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
+    const int t_lvl = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
+    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
+      const int id = S.level_nodes[e];
+      tiles[id] = N_(id, SPN_NB) > 0 ? t_lvl : 0;
+      smem = std::max(smem, si_smem(N_(id, SPN_M), N_(id, SPN_NB)));
+      q.push_back(id);
+      q.push_back(-1);
+    }
+    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
+      const int id = S.level_nodes[e];
+      for (int t = 0; t < tiles[id]; ++t) {
+        q.push_back(id);
+        q.push_back(t);
+      }
+    }
+    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
+      q.push_back(S.level_nodes[e]);
+      q.push_back(-3);
+    }
+  }
+  if (smem > 227 * 1024) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance: a front does not fit shared memory (%zu bytes)", smem);
+  // stored block of S -> (node, local row, local column, flags: 1 transposed, 2 diagonal) from the entry table
+  std::vector<int32_t> brec((size_t)ctx->n_sblk * 4 + 4, 0);
+  for (int id = 0; id < S.n_nodes; ++id)
+    for (int e = N_(id, SPN_AENT); e < N_(id, SPN_AENT) + N_(id, SPN_NAENT); ++e) {
+      const uint32_t code = (uint32_t)S.aent[4 * (size_t)e];
+      const uint32_t blk = code & 0x3fffffffu;
+      if (blk == 0x3fffffffu) continue;
+      if ((int)blk >= ctx->n_sblk) return fail(ctx, BA_ERR_STATE, "ba_gpu_covariance: inconsistent entry table");
+      int32_t *r = brec.data() + 4 * (size_t)blk;
+      r[0] = id;
+      r[1] = S.aent[4 * (size_t)e + 1];
+      r[2] = S.aent[4 * (size_t)e + 2];
+      r[3] = (code & 0x80000000u ? 1 : 0) | (code & 0x40000000u ? 2 : 0);
+    }
+  auto up = [&](Buf &b, const std::vector<int32_t> &v) -> int {
+    int rc2 = buf_reserve(ctx, b, (v.size() + 1) * 4);
+    if (rc2) return rc2;
+    if (!v.empty()) CK(cudaMemcpyAsync(b.p, v.data(), v.size() * 4, cudaMemcpyHostToDevice, s));
+    return 0;
+  };
+  if ((rc = up(ctx->cov_queue, q)) || (rc = up(ctx->cov_tiles, tiles)) || (rc = up(ctx->cov_brec, brec)) || (rc = up(ctx->cov_pos, S.pos)))
+    return rc;
+  ctx->cov_n_items = (int)(q.size() / 2);
+  ctx->cov_smem = smem;
+  CK(cudaFuncSetAttribute(k_selinv_tree, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t nc = (size_t)ctx->n_cam;
+  RES(cov_Y, ((size_t)S.panel_blocks + 1) * 288);
+  RES(cov_X, (4 * nc + 1) * 48);
+  RES(cov_zq, (nc + 1) * 48);
+  RES(cov_yscr, (nc + 1) * 48);
+  RES(cov_Tinv, 16 * 8);
+  RES(cov_S, ((size_t)ctx->n_sblk + 1) * 288);
+  RES(cov_ck, (nc + 1) * 192);
+  RES(cov_cnt, ((size_t)3 * S.n_nodes + 16) * 4);
+  RES(cov_cam, nc * 288);
+  RES(cov_ci, nc * 192);
+  RES(cov_pt, ((size_t)ctx->n_pt + 1) * 72);
+  RES(cov_bad, 16);
+  CK(cudaStreamSynchronize(s));  // (host vectors die here)
+  ctx->cov_ready = true;
+  return 0;
+}
+
+extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
+                                 int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs) {
+  if (!ctx) return BA_ERR_INVALID;
+  if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_covariance before ba_gpu_upload");
+  if (ctx->n_ranks > 1) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance is single-GPU");
+  if (!ctx->depth)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance needs the depth prior: without it (%s cost) the scale is free and the "
+                "Gauss-Newton Hessian is singular", ctx->nk ? "INTR" : "NS");
+  if (ctx->fixed_cam < 0)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance needs a fixed camera: with fixed_cam < 0 the gauge is free and the "
+                "Gauss-Newton Hessian is singular");
+  if (n_pairs < 0 || (n_pairs > 0 && (!cam_a || !cam_b || !cov_pairs))) return fail(ctx, BA_ERR_INVALID, "bad camera pair list");
+  for (int i = 0; i < n_pairs; ++i)
+    if (cam_a[i] < 0 || cam_a[i] >= ctx->n_cam || cam_b[i] < 0 || cam_b[i] >= ctx->n_cam)
+      return fail(ctx, BA_ERR_INVALID, "camera pair %d (%d, %d) out of range", i, cam_a[i], cam_b[i]);
+  CK(cudaSetDevice(ctx->device));
+  ctx->pdl = false;
+  ctx->cur = ctx->stream;
+  int rc = cov_prepare(ctx);
+  if (rc) return rc;
+  cudaStream_t s = ctx->stream;
+  LmState *st = P<LmState>(ctx->st);
+  const SpSymbolic &S = ctx->sym;
+  const size_t nc = (size_t)ctx->n_cam;
+  // linearisation at the current point, radius +inf: every LM damping D = sqrt(diag / radius) is exactly 0 (the next
+  // ba_gpu_solve starts from k_lm_init)
+  enqueue_iteration_zero(ctx, false);
+  LAUNCH(k_clear_done, 1, 1, 0, st);
+  LAUNCH(k_set_radius, 1, 1, 0, st, INFINITY);
+  enqueue_point_inverse(ctx, GATE_RUN);
+  DISPATCH_D(ctx->depth, {
+    LAUNCH((k_obs_W<DD>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->pt_idx), ctx->Jc_, P<double>(ctx->V),
+           P<double>(ctx->dp), P<double>(ctx->W), P<double>(ctx->WV), st, GATE_RUN);
+  });
+  if (ctx->nk) {
+    LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
+           P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
+           P<double>(ctx->part_ex), ctx->n_pt, P<double>(ctx->Vinv), P<double>(ctx->part_kk), st, GATE_RUN);
+    LAUNCH((k_spb_assemble<4>), cdiv(ctx->n_cam * 30 + 14, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
+           P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
+           P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
+           P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
+  }
+  LAUNCH(k_sp_schur_planes, cdiv(ctx->n_sblk * 32, BA_THREADS), BA_THREADS, 0, ctx->n_sblk, P<int32_t>(ctx->sb_ptr),
+         P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->Sblk), st, GATE_RUN);
+  LAUNCH(k_sp_add_diag, cdiv(ctx->n_cam * 36, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->sp_diag), P<double>(ctx->U),
+         P<double>(ctx->Sblk), st, GATE_RUN);
+  // no damping; the fixed camera (no block of S, no border row) gets a unit pivot so that the tree can eliminate it
+  CK(cudaMemsetAsync(ctx->dsq.p, 0, nc * 48, s));
+  LAUNCH(k_fill, 1, 32, 0, P<double>(ctx->dsq) + 6 * (size_t)ctx->fixed_cam, (size_t)6, 1.0);
+  // factorisation (forward substitution: Z = L^-1 B with the border)
+  SpChol a = spchol_args(ctx);
+  if (ctx->spc_tree && ctx->spc_parts == 1) {
+    SpTree t;
+    int *cnt = P<int>(ctx->spc_cnt);
+    t.tiles = P<int32_t>(ctx->spc_tiles);
+    t.fdone = cnt + 16;
+    t.udone = t.fdone + S.n_nodes;
+    t.sdone = t.udone + S.n_nodes;
+    CK(cudaMemcpyAsync(cnt, ctx->spc_cnt_init.p, ((size_t)3 * S.n_nodes + 16) * 4, cudaMemcpyDeviceToDevice, s));
+    const size_t smem = std::max(std::max(ctx->spc_smem_factor, ctx->spc_smem_solve), ctx->spc_smem_update);
+    t.queue = P<int2>(ctx->spc_queue);
+    t.n_items = ctx->spc_qB;
+    t.ticket = cnt;
+    if (ctx->spc_nrhs > 1)
+      LAUNCH((k_spchol_tree<5>), std::min(ctx->n_sm, t.n_items), SPC_THREADS, smem, a, t, st, GATE_RUN);
+    else
+      LAUNCH((k_spchol_tree<1>), std::min(ctx->n_sm, t.n_items), SPC_THREADS, smem, a, t, st, GATE_RUN);
+  } else {
+    for (int l = 0; l < S.n_levels; ++l) {
+      const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
+      if (ctx->spc_nrhs > 1)
+        LAUNCH((k_spchol_factor<5>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, GATE_RUN);
+      else
+        LAUNCH((k_spchol_factor<1>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, GATE_RUN);
+      if (l + 1 < S.n_levels) {
+        const int tiles = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
+        if (ctx->spc_nrhs > 1)
+          LAUNCH((k_spchol_update<5>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, GATE_RUN);
+        else
+          LAUNCH((k_spchol_update<1>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, GATE_RUN);
+      }
+    }
+  }
+  // intrinsics border: T^-1, then X = L^-T Z one column at a time (the backward substitution of the LM step, levels top-down)
+  const double *X = nullptr;
+  if (ctx->nk) {
+    LAUNCH(k_spb_reduce, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->spb_Z), P<double>(ctx->spc_z),
+           P<double>(ctx->spb_part), st, GATE_RUN);
+    LAUNCH(k_cov_border, 1, 32, 0, ctx->nblk_cam, P<double>(ctx->spb_part), P<double>(ctx->spb_kk), P<double>(ctx->cov_Tinv), st);
+    SpChol ax = a;
+    ax.Zb = nullptr;
+    ax.yk = nullptr;
+    ax.z = P<double>(ctx->cov_zq);
+    ax.yc = P<double>(ctx->cov_yscr);
+    for (int qc = 0; qc < 4; ++qc) {
+      LAUNCH(k_cov_zcol, cdiv(6 * ctx->n_cam, BA_THREADS), BA_THREADS, 0, 6 * ctx->n_cam, qc, P<double>(ctx->spb_Z), P<double>(ctx->cov_zq));
+      ax.ypos = P<double>(ctx->cov_X) + (size_t)qc * 6 * nc;
+      for (int l = S.n_levels - 1; l >= 0; --l)
+        LAUNCH(k_spchol_solve, S.level_ptr[l + 1] - S.level_ptr[l], SPC_THREADS, ctx->spc_smem_solve, ax, S.level_ptr[l], st, GATE_RUN);
+    }
+    X = P<double>(ctx->cov_X);
+  }
+  // selected inversion of A on the pattern of L (overwrites the panels and the update-matrix slots)
+  {
+    SelInv si;
+    si.node = a.node;
+    si.rel = a.rel;
+    si.linv = a.linv;
+    si.panel = a.panel;
+    si.U = a.U;
+    si.Y = P<double>(ctx->cov_Y);
+    si.queue = P<int2>(ctx->cov_queue);
+    si.n_items = ctx->cov_n_items;
+    si.tiles = P<int32_t>(ctx->cov_tiles);
+    int *cnt = P<int>(ctx->cov_cnt);
+    si.ticket = cnt;
+    si.pdone = cnt + 16;
+    si.tdone = si.pdone + S.n_nodes;
+    si.sdone = si.tdone + S.n_nodes;
+    CK(cudaMemsetAsync(cnt, 0, ((size_t)3 * S.n_nodes + 16) * 4, s));
+    LAUNCH(k_selinv_tree, std::min(ctx->n_sm, si.n_items), SPC_THREADS, ctx->cov_smem, si);
+  }
+  // Sigma on the stored blocks of S (+ border correction), per camera, pairs, points
+  LAUNCH(k_cov_blocks, cdiv(ctx->n_sblk * 36, BA_THREADS), BA_THREADS, 0, ctx->n_sblk, P<int4>(ctx->cov_brec), P<int32_t>(ctx->sb_i),
+         P<int32_t>(ctx->sb_j), a.node, a.panel, P<int32_t>(ctx->cov_pos), ctx->n_cam, X, P<double>(ctx->cov_Tinv), P<double>(ctx->cov_S));
+  LAUNCH(k_cov_cam, cdiv(ctx->n_cam * 60, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam, ctx->nk, P<int32_t>(ctx->sp_diag),
+         P<double>(ctx->cov_S), P<int32_t>(ctx->cov_pos), X, P<double>(ctx->cov_Tinv), P<double>(ctx->sc), P<double>(ctx->sk),
+         P<double>(ctx->cov_ck), P<double>(ctx->cov_cam), P<double>(ctx->cov_ci));
+  CK(cudaMemsetAsync(ctx->cov_bad.p, 0, 16, s));
+  if (n_pairs > 0) {
+    RES(cov_pin, (size_t)n_pairs * 8 + 16);
+    RES(cov_pout, (size_t)n_pairs * 288 + 16);
+    CK(cudaMemcpyAsync(ctx->cov_pin.p, cam_a, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(P<int32_t>(ctx->cov_pin) + n_pairs, cam_b, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
+    LAUNCH(k_cov_pairs, cdiv(n_pairs * 36, BA_THREADS), BA_THREADS, 0, n_pairs, P<int32_t>(ctx->cov_pin),
+           P<int32_t>(ctx->cov_pin) + n_pairs, ctx->fixed_cam, P<int32_t>(ctx->ent_ptr), P<int2>(ctx->ent), P<double>(ctx->cov_S),
+           P<double>(ctx->sc), P<double>(ctx->cov_pout), P<int>(ctx->cov_bad));
+  }
+  if (cov_pt && ctx->n_pt > 0)
+    LAUNCH(k_cov_points, ctx->nblk_pt, BA_THREADS, 0, ctx->n_pt, ctx->fixed_cam, ctx->nk, P<int32_t>(ctx->pt_rowptr),
+           P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->perm), P<double>(ctx->W), P<double>(ctx->Wk), P<double>(ctx->Vinv),
+           P<int32_t>(ctx->ent_ptr), P<int2>(ctx->ent), P<double>(ctx->cov_S), P<double>(ctx->cov_ck), P<double>(ctx->cov_Tinv),
+           P<double>(ctx->sp), P<double>(ctx->cov_pt));
+  if ((rc = poll_state(ctx))) return rc;
+  CK(cudaGetLastError());
+  if (ctx->h_st->eval_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-finite residual or Jacobian");
+  if (ctx->h_st->lin_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-positive pivot (the Hessian is not positive definite)");
+  int bad = 0;
+  CK(cudaMemcpy(&bad, ctx->cov_bad.p, 4, cudaMemcpyDeviceToHost));
+  if (bad) return fail(ctx, BA_ERR_INVALID, "ba_gpu_covariance: a requested camera pair shares no point (outside the pattern of S)");
+  if (cov_cam) CK(cudaMemcpy(cov_cam, ctx->cov_cam.p, nc * 288, cudaMemcpyDeviceToHost));
+  if (cov_cam_intr) CK(cudaMemcpy(cov_cam_intr, ctx->cov_ci.p, nc * 192, cudaMemcpyDeviceToHost));
+  if (cov_pt && ctx->n_pt > 0) CK(cudaMemcpy(cov_pt, ctx->cov_pt.p, (size_t)ctx->n_pt * 72, cudaMemcpyDeviceToHost));
+  if (n_pairs > 0) CK(cudaMemcpy(cov_pairs, ctx->cov_pout.p, (size_t)n_pairs * 288, cudaMemcpyDeviceToHost));
+  if (cov_intr) {
+    double ti[16] = {0.0}, sk[4] = {0.0};
+    if (ctx->nk) {
+      CK(cudaMemcpy(ti, ctx->cov_Tinv.p, 128, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(sk, ctx->sk.p, 32, cudaMemcpyDeviceToHost));
+    }
+    for (int i = 0; i < 4; ++i)
+      for (int j = 0; j < 4; ++j) cov_intr[4 * i + j] = ti[4 * i + j] * (sk[i] * sk[j]);
+  }
   return BA_OK;
 }
 

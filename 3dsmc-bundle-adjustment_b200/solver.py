@@ -161,6 +161,23 @@ class GpuSolver:
         self._check(self.lib.ba_gpu_schur_solve(self._ctx, float(radius), capi.dp(rhs), capi.dp(y)))
         return y
 
+    def covariance(self, points=True, pairs=None):
+        """Covariance of the estimate at the current state (after solve(), or right after upload()): the inverse of the
+        undamped Gauss-Newton Hessian per block in its tangent space, as ceres::Covariance (loss applied).  Needs the depth
+        prior and a fixed camera.  pairs: [n, 2] camera indices of co-visible cameras (or a == b).
+        -> {"cam": [n_cam,6,6], "cam_intr": [n_cam,6,4], "intr": [4,4], "pt": [n_pt,3,3] (None if not points),
+            "pairs": [n,6,6]}"""
+        if self._shape is None:  # (before upload: the library reports BA_ERR_STATE)
+            self._check(self.lib.ba_gpu_covariance(self._ctx, None, None, None, None, 0, None, None, None))
+        n_cam, n_pt, _ = self._shape
+        pr = np.zeros((0, 2), dtype=np.int32) if pairs is None else np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 2)
+        a, b = np.ascontiguousarray(pr[:, 0]), np.ascontiguousarray(pr[:, 1])
+        out = dict(cam=np.zeros((n_cam, 6, 6)), cam_intr=np.zeros((n_cam, 6, 4)), intr=np.zeros((4, 4)),
+                   pt=np.zeros((n_pt, 3, 3)) if points else None, pairs=np.zeros((len(a), 6, 6)))
+        self._check(self.lib.ba_gpu_covariance(self._ctx, capi.dp(out["cam"]), capi.dp(out["cam_intr"]), capi.dp(out["intr"]),
+                                               capi.dp(out["pt"]), len(a), capi.ip(a), capi.ip(b), capi.dp(out["pairs"])))
+        return out
+
     def spchol_info(self):
         """Structure of the sparse Cholesky of the last upload ({} when another solver is in force)."""
         info = (C.c_int64 * 24)()

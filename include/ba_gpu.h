@@ -198,6 +198,20 @@ int ba_gpu_schur_matvec(ba_gpu_ctx *ctx, double radius, const double *x, double 
  * BA_ERR_UNSUPPORTED with depth prior or free intrinsics, as for ba_gpu_schur_matvec then), same conventions as
  * ba_gpu_schur_matvec: ba_gpu_schur_matvec(radius, ba_gpu_schur_solve(radius, b)) == b */
 int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *rhs, double *y);
+/* Covariance of the estimate at the current device state (after ba_gpu_solve, or right after ba_gpu_upload):
+ * the inverse of the undamped Gauss-Newton Hessian of the cost in force, per block in its tangent space
+ * (== ceres::Covariance, GetCovarianceBlockInTangentSpace, loss applied).  Constant blocks have zero covariance.
+ *   cov_cam      [n_cam*36]  6x6 row-major per camera, columns ordered as Jc of ba_gpu_eval   (nullable)
+ *   cov_cam_intr [n_cam*24]  6x4 camera-intrinsics cross-covariance                            (nullable)
+ *   cov_intr     [16]        4x4                                                                (nullable)
+ *   cov_pt       [n_pt*9]    3x3 per point                                                      (nullable)
+ *   n_pairs, cam_a, cam_b -> cov_pairs [n_pairs*36]: Cov(delta_a, delta_b) for cameras that share a point (or a == b)
+ * Selected inversion over the supernodal tree of BA_SOLVER_SPARSE_SCHUR_CHOLESKY, whichever solver the upload resolved to
+ * (the first call after an upload builds that tree when another solver is in force).  A later ba_gpu_solve is unaffected.
+ * BA_ERR_UNSUPPORTED: no depth prior (scale free), fixed_cam < 0 (gauge free), more than one rank, or a front that does not
+ * fit; BA_ERR_INVALID: a pair that is not co-visible, an index out of range; BA_ERR_NUMERIC: a non-positive pivot. */
+int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
+                      int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs);
 /* structure of the sparse Cholesky of the last upload (zeros when another solver is in force): info[0..10] as
  * ba_sparse_symbolic_info, info[11] = host microseconds of the symbolic phase, info[12] = parts of the subtree-to-rank
  * partition in force (1: one queue), info[13] = 1 when the factorisation is distributed over the ranks of the communicator
