@@ -185,7 +185,8 @@ struct ba_gpu_ctx {
   int cov_n_items = 0;
   size_t cov_smem = 0;
   Buf cov_Y, cov_X, cov_zq, cov_yscr, cov_Tinv, cov_S, cov_ck, cov_brec, cov_pos, cov_queue, cov_tiles, cov_cnt, cov_cam, cov_ci,
-      cov_pt, cov_pin, cov_pout, cov_bad;
+      cov_pt, cov_pin, cov_pout, cov_bad, cov_piv;
+  double cov_ratio[2] = {0.0, 0.0};  // smallest pivot / diagonal of the last covariance call: cameras, intrinsics (0: none)
   // phase timing of the large-problem solvers: CUDA events on the solver stream at the phase boundaries of every LM
   // iteration of the last solve (a few dozen event records per iteration: < 0.1 % of a multi-millisecond iteration)
   std::vector<cudaEvent_t> ph_ev;
@@ -2938,6 +2939,7 @@ static int cov_prepare(ba_gpu_ctx *ctx) {
   RES(cov_ci, nc * 192);
   RES(cov_pt, ((size_t)ctx->n_pt + 1) * 72);
   RES(cov_bad, 16);
+  RES(cov_piv, sizeof(CovPivots));
   CK(cudaStreamSynchronize(s));  // (host vectors die here)
   ctx->cov_ready = true;
   return 0;
@@ -2973,6 +2975,8 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
   LAUNCH(k_clear_done, 1, 1, 0, st);
   LAUNCH(k_set_radius, 1, 1, 0, st, INFINITY);
   enqueue_point_inverse(ctx, GATE_RUN);
+  CovPivots *cp = P<CovPivots>(ctx->cov_piv);
+  LAUNCH(k_cov_pivots_init, 1, 1, 0, cp, st);
   DISPATCH_D(ctx->depth, {
     LAUNCH((k_obs_W<DD>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->pt_idx), ctx->Jc_, P<double>(ctx->V),
            P<double>(ctx->dp), P<double>(ctx->W), P<double>(ctx->WV), st, GATE_RUN);
@@ -3027,12 +3031,15 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
       }
     }
   }
+  LAUNCH(k_cov_pivots, cdiv(6 * ctx->n_cam, BA_THREADS), BA_THREADS, 0, ctx->n_cam, a.perm, P<int32_t>(ctx->sp_diag), a.S, a.dsq,
+         a.linv, BA_COV_MIN_PIVOT_RATIO, cp);
   // intrinsics border: T^-1, then X = L^-T Z one column at a time (the backward substitution of the LM step, levels top-down)
   const double *X = nullptr;
   if (ctx->nk) {
     LAUNCH(k_spb_reduce, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->spb_Z), P<double>(ctx->spc_z),
            P<double>(ctx->spb_part), st, GATE_RUN);
-    LAUNCH(k_cov_border, 1, 32, 0, ctx->nblk_cam, P<double>(ctx->spb_part), P<double>(ctx->spb_kk), P<double>(ctx->cov_Tinv), st);
+    LAUNCH(k_cov_border, 1, 32, 0, ctx->nblk_cam, P<double>(ctx->spb_part), P<double>(ctx->spb_kk), P<double>(ctx->cov_Tinv),
+           BA_COV_MIN_PIVOT_RATIO, cp, st);
     SpChol ax = a;
     ax.Zb = nullptr;
     ax.yk = nullptr;
@@ -3090,6 +3097,23 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
   if ((rc = poll_state(ctx))) return rc;
   CK(cudaGetLastError());
   if (ctx->h_st->eval_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-finite residual or Jacobian");
+  CovPivots piv;
+  CK(cudaMemcpy(&piv, cp, sizeof(piv), cudaMemcpyDeviceToHost));
+  memcpy(&ctx->cov_ratio[0], &piv.min_cam, 8);
+  memcpy(&ctx->cov_ratio[1], &piv.min_border, 8);
+  if (!ctx->nk) ctx->cov_ratio[1] = 0.0;
+  if (piv.bad_point)
+    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is singular: the 3x3 block of a point is singular (a point "
+                "without observations, or one its observations do not fix)");
+  if (piv.first_bad) {
+    const int k = ctx->n_cam - piv.first_bad;
+    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is rank-deficient: a pivot of camera %d (elimination position "
+                "%d) is below %g times its diagonal (a camera its observations do not fix, or cameras not connected to the fixed one)",
+                S.perm[k], k, BA_COV_MIN_PIVOT_RATIO);
+  }
+  if (piv.bad_border)
+    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is rank-deficient: intrinsics pivot %d is below %g times its "
+                "diagonal (the observations do not fix the intrinsics)", piv.bad_border - 1, BA_COV_MIN_PIVOT_RATIO);
   if (ctx->h_st->lin_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-positive pivot (the Hessian is not positive definite)");
   int bad = 0;
   CK(cudaMemcpy(&bad, ctx->cov_bad.p, 4, cudaMemcpyDeviceToHost));
@@ -3107,6 +3131,13 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
     for (int i = 0; i < 4; ++i)
       for (int j = 0; j < 4; ++j) cov_intr[4 * i + j] = ti[4 * i + j] * (sk[i] * sk[j]);
   }
+  return BA_OK;
+}
+
+extern "C" int ba_gpu_covariance_pivots(const ba_gpu_ctx *ctx, double ratio[2]) {
+  if (!ctx || !ratio) return BA_ERR_INVALID;
+  ratio[0] = ctx->cov_ratio[0];
+  ratio[1] = ctx->cov_ratio[1];
   return BA_OK;
 }
 

@@ -234,10 +234,47 @@ __global__ void __launch_bounds__(BA_THREADS) k_cov_zcol(int n6, int q, const do
   if (i < n6) zq[i] = Zb[4 * (size_t)i + q];
 }
 
-// T = C - Z^T Z (partials of k_spb_reduce added in block order) and T^-1 by a 4 x 4 Cholesky (one thread).  A non-positive or
-// non-finite pivot sets lin_fail.
+// Relative pivot test of the covariance factorisation.  A scalar pivot of an exactly rank-deficient Hessian is rounding: its
+// sign, and so the outcome of a `pivot > 0` test, is a coin flip.  The covariance is rejected when a pivot falls below tau times
+// its column's diagonal before elimination (healthy problems: 6e-4 .. 1e-1; rounding in a singular one: 1e-12 .. 1e-16).  The
+// LM step does not run this test.
+struct CovPivots {
+  unsigned long long min_cam, min_border;  // smallest pivot / diagonal, as the bits of a non-negative double (ordered as integers)
+  int first_bad;                           // n_cam - first elimination position that fails, 0: none
+  int bad_border;                          // 1 + first intrinsics column that fails, 0: none
+  int bad_point;                           // a 3x3 point block is singular
+  int pad;
+};
+
+__global__ void k_cov_pivots_init(CovPivots *cp, const LmState *st) {
+  CovPivots c;
+  c.min_cam = c.min_border = (unsigned long long)__double_as_longlong(INFINITY);
+  c.first_bad = c.bad_border = c.pad = 0;
+  c.bad_point = st->lin_fail;  // (called right after the point inverses: nothing else has set it yet)
+  *cp = c;
+}
+
+// one thread per scalar column of the camera system: the pivot from the stored inverse pivot block (diagonal 1 / sqrt(pivot)),
+// the diagonal before elimination from the stored diagonal block of S plus the damping
+__global__ void __launch_bounds__(BA_THREADS)
+k_cov_pivots(int n_cam, const int32_t *__restrict__ perm, const int32_t *__restrict__ sp_diag, const double *__restrict__ S,
+             const double *__restrict__ dsq, const double *__restrict__ linv, double tau, CovPivots *cp) {
+  const int i = blockIdx.x * BA_THREADS + threadIdx.x;
+  if (i >= 6 * n_cam) return;
+  const int k = i / 6, c = i - 6 * k, cam = perm[k], blk = sp_diag[cam];
+  const double d0 = (blk >= 0 ? S[36 * (size_t)blk + 7 * c] : 0.0) + dsq[6 * (size_t)cam + c];
+  const double li = linv[36 * (size_t)k + 7 * c];
+  const double piv = 1.0 / (li * li);
+  double r = piv / d0;
+  if (!(r > 0.0)) r = 0.0;  // (non-positive, NaN)
+  atomicMin(&cp->min_cam, (unsigned long long)__double_as_longlong(r));
+  if (!(piv > tau * d0) || !isfinite(piv)) atomicMax(&cp->first_bad, n_cam - k);
+}
+
+// T = C - Z^T Z (partials of k_spb_reduce added in block order) and T^-1 by a 4 x 4 Cholesky (one thread).  A pivot of T below
+// tau times the diagonal of C (the intrinsics columns before any elimination), or a non-finite one, sets lin_fail.
 __global__ void k_cov_border(int nblk, const double *__restrict__ part, const double *__restrict__ kk, double *__restrict__ Tinv,
-                             LmState *st) {
+                             double tau, CovPivots *cp, LmState *st) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   double s[10];
   for (int k = 0; k < 10; ++k) {
@@ -254,10 +291,16 @@ __global__ void k_cov_border(int nblk, const double *__restrict__ part, const do
     }
   double L[4][4] = {{0.0}}, Li[4][4] = {{0.0}};
   bool ok = true;
+  double rmin = INFINITY;
   for (int j = 0; j < 4; ++j) {
     double d = T[j][j];
     for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k];
-    if (!(d > 0.0) || !isfinite(d)) ok = false;
+    const double c0 = kk[5 * j], r = d / c0;
+    rmin = fmin(rmin, r > 0.0 ? r : 0.0);
+    if (ok && (!(d > tau * c0) || !isfinite(d))) {
+      ok = false;
+      cp->bad_border = 1 + j;
+    }
     L[j][j] = ok ? sqrt(d) : 1.0;
     for (int i = j + 1; i < 4; ++i) {
       double x = T[i][j];
@@ -278,6 +321,7 @@ __global__ void k_cov_border(int nblk, const double *__restrict__ part, const do
       Tinv[i * 4 + c] = v;
       Tinv[c * 4 + i] = v;
     }
+  cp->min_border = (unsigned long long)__double_as_longlong(rmin);
   if (!ok) st->lin_fail = 1;
 }
 

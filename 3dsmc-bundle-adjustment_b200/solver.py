@@ -178,6 +178,13 @@ class GpuSolver:
                                                capi.dp(out["pt"]), len(a), capi.ip(a), capi.ip(b), capi.dp(out["pairs"])))
         return out
 
+    def covariance_pivots(self):
+        """Smallest pivot / diagonal ratio of the last covariance() call, also a rejected one: {"cam": camera system,
+        "intr": intrinsics (0 when they are constant)}.  covariance() rejects a ratio below capi.BA_COV_MIN_PIVOT_RATIO."""
+        r = np.zeros(2)
+        self._check(self.lib.ba_gpu_covariance_pivots(self._ctx, capi.dp(r)))
+        return {"cam": float(r[0]), "intr": float(r[1])}
+
     def spchol_info(self):
         """Structure of the sparse Cholesky of the last upload ({} when another solver is in force)."""
         info = (C.c_int64 * 24)()

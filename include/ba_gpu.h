@@ -209,9 +209,20 @@ int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *rhs, double
  * Selected inversion over the supernodal tree of BA_SOLVER_SPARSE_SCHUR_CHOLESKY, whichever solver the upload resolved to
  * (the first call after an upload builds that tree when another solver is in force).  A later ba_gpu_solve is unaffected.
  * BA_ERR_UNSUPPORTED: no depth prior (scale free), fixed_cam < 0 (gauge free), more than one rank, or a front that does not
- * fit; BA_ERR_INVALID: a pair that is not co-visible, an index out of range; BA_ERR_NUMERIC: a non-positive pivot. */
+ * fit; BA_ERR_INVALID: a pair that is not co-visible, an index out of range.
+ * BA_ERR_NUMERIC: the Hessian is singular or numerically rank-deficient: a point's 3x3 block is singular (a point without
+ * observations), or a scalar pivot of the Jacobi-scaled camera system, or of the 4x4 intrinsics system T = C - Z^T Z, is below
+ * BA_COV_MIN_PIVOT_RATIO times its column's diagonal before elimination (a camera with too few observations to fix its pose,
+ * cameras not connected to the fixed one).  In an exactly rank-deficient Hessian such a pivot is rounding, of either sign, and
+ * the inverse would be of order 1e16: the relative test rejects it whatever the rounding.  This is the analogue of Ceres'
+ * Covariance::Options::min_reciprocal_condition_number.  The LM step (ba_gpu_solve) does not apply it: there the damping
+ * makes the system definite. */
+#define BA_COV_MIN_PIVOT_RATIO 1e-9
 int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
                       int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs);
+/* smallest pivot / diagonal ratio of the last ba_gpu_covariance call (also a rejected one): ratio[0] over the camera system,
+ * ratio[1] over the intrinsics (0 when they are constant); compare with BA_COV_MIN_PIVOT_RATIO */
+int ba_gpu_covariance_pivots(const ba_gpu_ctx *ctx, double ratio[2]);
 /* structure of the sparse Cholesky of the last upload (zeros when another solver is in force): info[0..10] as
  * ba_sparse_symbolic_info, info[11] = host microseconds of the symbolic phase, info[12] = parts of the subtree-to-rank
  * partition in force (1: one queue), info[13] = 1 when the factorisation is distributed over the ranks of the communicator

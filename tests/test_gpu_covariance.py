@@ -97,6 +97,13 @@ def _rel(a, b):
     return float(np.max(np.abs(np.asarray(a) - np.asarray(b))) / max(np.max(np.abs(b)), 1e-300))
 
 
+def _check_pivot_margin(name, mode, piv):
+    """A healthy Hessian passes the relative pivot test of the covariance with three orders of magnitude to spare."""
+    print("smallest pivot / diagonal %s %s: cameras %.3e intrinsics %.3e" % (name, mode, piv["cam"], piv["intr"]))
+    assert piv["cam"] > 1e3 * capi.BA_COV_MIN_PIVOT_RATIO
+    assert mode != "REF" or piv["intr"] > 1e3 * capi.BA_COV_MIN_PIVOT_RATIO
+
+
 def _pairs(p):
     bi, bj = covisibility_blocks(p.cam_idx, p.pt_idx, p.n_cam, p.fixed_cam)
     return np.stack([np.concatenate([bi, bj]), np.concatenate([bj, bi])], axis=1).astype(np.int32)
@@ -113,7 +120,9 @@ def test_matches_oracle_reference(name, mode):
     pose, pt, intr = (x.copy() for x in s.download())
     pr = _pairs(p)
     got = s.covariance(points=True, pairs=pr)
+    piv = s.covariance_pivots()
     s.close()
+    _check_pivot_margin(name, mode, piv)
     ref = _reference(p, mode, pose, pt, intr)
     err = dict(cam=_rel(got["cam"], ref["cam"]), pt=_rel(got["pt"], ref["pt"]),
                pairs=_rel(got["pairs"], np.stack([ref["pair"](a, b) for a, b in pr])))
@@ -252,8 +261,10 @@ def test_big_sequence_columns_against_sparse_lu():
     bi, bj = covisibility_blocks(p.cam_idx, p.pt_idx, p.n_cam, p.fixed_cam)
     pr = np.array([(a, b) for a, b in zip(bi, bj) if a in cams or b in cams], dtype=np.int32)
     got = s.covariance(points=False, pairs=pr)
+    piv = s.covariance_pivots()
     pose, pt, intr = (x.copy() for x in s.download())
     s.close()
+    _check_pivot_margin("big%d" % N_KF_BIG, "REF", piv)
     H, nR, nk, slot = _hessian(p, "REF", pose, pt, intr)
     S, _, _ = _reduced(H, nR, p.n_pt)
     lu = spla.splu(S)

@@ -19,7 +19,7 @@ def _solver(**kw):
     return ba_b200.GpuSolver(**kw)
 
 
-@pytest.mark.parametrize("solver", [1, 2, 3])
+@pytest.mark.parametrize("solver", [1, 2, 3, 4])
 def test_no_observations(solver):
     """An upload without observations: zero cost, nothing moves, no crash (any solver)."""
     p = _tiny()
@@ -41,7 +41,7 @@ def test_no_observations(solver):
         s.close()
 
 
-@pytest.mark.parametrize("solver", [1, 2, 3])
+@pytest.mark.parametrize("solver", [1, 2, 3, 4])
 def test_ragged_problem_matches_oracle(solver):
     """Cameras without observations, points seen once, points never seen, a camera seen only through the
     fixed pose's points: the solve still tracks the oracle."""

@@ -1,0 +1,287 @@
+"""The sparse Cholesky (solver = 4) and the covariance on co-visibility that is not a band (tests/irregular_problems.py): loop
+closures (a range with no cut, eliminated as one chain; a wide separator; several closures), a street loop whose tracks wrap
+around, two unconnected maps (a forest), ragged inputs (a camera without observations, points seen once or never, duplicate
+observations).  Extend-add maps with far cameras, several roots and cameras without a diagonal block of S only arise here.
+References: the oracle's SPARSE_SCHUR-equivalent exact solve, the dense explicit path on the GPU, the block-CSR product, and
+the float64 numpy covariance of test_gpu_covariance.  Rank-deficient Hessians are rejected by the covariance's relative pivot
+test whatever the rounding."""
+import functools
+
+import numpy as np
+import pytest
+
+import irregular_problems as ip
+from helpers import ba_b200, mode_opts, ora, pose_err, rel_err, to_oracle
+from spchol_emulation import covisibility_blocks
+from test_gpu_covariance import TOL, TOL_INTR, _pairs, _reference, _rel
+from test_gpu_spchol_border import _lockstep_oracle
+
+pytestmark = pytest.mark.gpu
+syn = ba_b200.synthetic
+capi = ba_b200.capi
+TAU = capi.BA_COV_MIN_PIVOT_RATIO
+
+
+@functools.lru_cache(maxsize=None)
+def _cached(name):
+    if name in ("closure_a", "closure_b", "closure_c"):
+        return ip.closure_problem(name[-1])
+    if name == "street":
+        return ip.closed_street()
+    if name == "two_maps":
+        return ip.two_maps(ip.tum_window(12, 5), ip.tum_window(10, 6))
+    if name == "ragged":  # a camera without observations, points seen once, unobserved points, duplicate observations
+        return ip.ragged(ip.closure_problem("c"), empty_cam=7, once=200, unobserved=50, duplicates=60)
+    if name == "dup_once":  # full rank: duplicate observations and points seen once only
+        return ip.ragged(ip.closure_problem("c"), once=200, duplicates=60)
+    if name == "one_obs_cam":
+        return ip.ragged(ip.tum_window(12, 5), one_obs_cam=7)
+    if name == "empty_cam":
+        return ip.ragged(ip.tum_window(12, 5), empty_cam=7)
+    if name == "unobserved_pt":
+        return ip.ragged(ip.tum_window(12, 5), unobserved=3)
+    raise KeyError(name)
+
+
+def _problem(name):
+    return _cached(name).copy()
+
+
+@pytest.fixture(scope="module")
+def solver_cache():
+    cache = {}
+    yield cache
+    for s in cache.values():
+        s.close()
+
+
+def _check_tree(s, p):
+    """The device's tree is the one the symbolic phase builds on the CPU for the same block list."""
+    sym = ip.gpu_symbolic(p)
+    info = s.spchol_info()
+    assert (info["nodes"], info["levels"], info["max_border"]) == (sym.n_nodes, sym.n_levels, sym.info[7])
+    return sym
+
+
+# ---------------------------------------------------------------- 1. NS: lock step with the oracle, solve inverts the product
+NS_CASES = ["closure_a", "closure_b", "closure_c", "street", "two_maps"]
+
+
+@pytest.mark.parametrize("name", NS_CASES)
+def test_ns_lockstep_oracle(name, solver_cache):
+    p = _problem(name)
+    s, summ = _lockstep_oracle(p, "NS", 8, solver_cache)
+    _check_tree(s, p)
+    assert summ.final_cost < 0.5 * summ.initial_cost
+
+
+@pytest.mark.parametrize("name", NS_CASES)
+def test_ns_solve_inverts_the_product(name, solver_cache):
+    p = _problem(name)
+    g, _ = mode_opts("NS", solver=4)
+    key = tuple(sorted(g.items()))
+    if key not in solver_cache:
+        solver_cache[key] = ba_b200.GpuSolver(**g)
+    s = solver_cache[key]
+    s.upload(p)
+    _check_tree(s, p)
+    rng = np.random.default_rng(11)
+    for radius in (1e4, 3.7):
+        b = rng.normal(size=6 * p.n_cam)
+        y = s.schur_solve(radius, b)
+        err = rel_err(s.schur_matvec(radius, y), b)
+        print("schur_solve residual %s radius %g: %.2e" % (name, radius, err))
+        # (as test_spchol_solve_inverts_the_product: the residual of a backward-stable solve grows with the condition number;
+        #  the closed street's free scale under the weak damping of radius 1e4 gives the largest, 2e-10 on a B200)
+        assert err < 1e-9, (name, radius, err)
+
+
+# ---------------------------------------------------------------- 2. REF / DEPTH / INTR: oracle, dense explicit path
+BORDER_CASES = ["closure_a", "closure_b", "closure_c", "two_maps", "ragged"]
+
+
+@pytest.mark.parametrize("mode", ["REF", "DEPTH", "INTR"])
+@pytest.mark.parametrize("name", BORDER_CASES)
+def test_border_lockstep_oracle(name, mode, solver_cache):
+    p = _problem(name)
+    s, summ = _lockstep_oracle(p, mode, 8, solver_cache)
+    _check_tree(s, p)
+    assert summ.final_cost < summ.initial_cost
+    if name == "ragged":  # the camera without observations does not move
+        pose, _, _ = s.download()
+        assert np.array_equal(pose[7], p.pose7[7])
+
+
+@pytest.mark.parametrize("name", ["closure_a", "closure_c", "ragged"])
+def test_border_sparse_vs_dense_explicit(name):
+    p = _problem(name)
+    out = []
+    for solver in (4, 1):
+        g, _ = mode_opts("REF", solver=solver, max_num_iterations=8)
+        s = ba_b200.GpuSolver(**g)
+        s.upload(p)
+        summ = s.solve()
+        out.append((summ, s.trace(), s.download()[0].copy()))
+        s.close()
+    (ss, ts, ps), (sd, td, pd) = out
+    assert ss.solver_used == capi.BA_SOLVER_SPARSE_SCHUR_CHOLESKY and sd.solver_used == capi.BA_SOLVER_EXPLICIT_CHOLESKY
+    assert len(ts) == len(td)
+    for a, b in zip(ts, td):
+        assert a["step_is_valid"] == b["step_is_valid"] and a["step_is_successful"] == b["step_is_successful"]
+        assert abs(a["cost"] - b["cost"]) <= 1e-10 * abs(b["cost"]), (a, b)
+    dt, dr = pose_err(ps, pd)
+    assert dt < 1e-8 and dr < 1e-8, (dt, dr)
+    if name == "ragged":
+        assert np.array_equal(ps[7], p.pose7[7]) and np.array_equal(pd[7], p.pose7[7])
+
+
+def test_single_camera_sparse_cholesky():
+    """One keyframe, fixed, through solver = 4 (REF cost): an empty camera system; the points are pulled back onto their
+    observation."""
+    p = syn.make_config(1)
+    keep = p.cam_idx == 0
+    q = p.copy()
+    q.pose7 = p.pose7[:1].copy()
+    q.cam_idx, q.pt_idx, q.uv2, q.depth = p.cam_idx[keep].copy(), p.pt_idx[keep].copy(), p.uv2[keep].copy(), p.depth[keep].copy()
+    seen = np.unique(q.pt_idx)
+    q.pt3 = q.pt3.copy()
+    q.pt3[seen] += np.random.default_rng(0).normal(size=(seen.size, 3)) * 0.01
+    g, o = mode_opts("REF", solver=4, max_num_iterations=8)
+    s = ba_b200.GpuSolver(**g)
+    try:
+        s.upload(q)
+        summ = s.solve()
+        pose, pt, intr = s.download()
+        assert summ.solver_used == capi.BA_SOLVER_SPARSE_SCHUR_CHOLESKY
+        assert np.array_equal(pose, q.pose7)
+        assert summ.initial_cost > 1e-8 and summ.final_cost < 1e-3 * summ.initial_cost
+        op = to_oracle(q)
+        rc, osum, _ = ora.solve(op, ora.default_options(**o))
+        assert rc == 0 and summ.num_iterations == osum.num_iterations
+        assert abs(summ.final_cost - osum.final_cost) <= 1e-8 * summ.initial_cost
+        assert np.max(np.abs(pt - op.pt3)) < 1e-6 and np.max(np.abs(intr - op.intr)) < 1e-5
+    finally:
+        s.close()
+
+
+# ---------------------------------------------------------------- 3. covariance on the full-rank cases
+COV_CASES = ["closure_a", "closure_b", "closure_c", "dup_once"]
+
+
+def _closure_pairs(p, min_gap=10):
+    """Co-visible camera pairs further apart than min_gap in the sequence, both orders: the loop closures."""
+    bi, bj = covisibility_blocks(p.cam_idx, p.pt_idx, p.n_cam, p.fixed_cam)
+    far = bj - bi > min_gap
+    pr = np.stack([np.concatenate([bi[far], bj[far]]), np.concatenate([bj[far], bi[far]])], axis=1).astype(np.int32)
+    assert len(pr) > 0
+    return pr
+
+
+def _covariance(p, mode, solver=4, iters=0, pairs=None):
+    g, _ = mode_opts(mode, solver=solver, max_num_iterations=max(iters, 1))
+    s = ba_b200.GpuSolver(**g)
+    try:
+        s.upload(p)
+        if iters:
+            s.solve()
+        got = s.covariance(points=True, pairs=pairs)
+        state = tuple(x.copy() for x in s.download())
+        return got, s.covariance_pivots(), s.spchol_info(), state
+    finally:
+        s.close()
+
+
+@pytest.mark.parametrize("mode", ["REF", "DEPTH"])
+@pytest.mark.parametrize("name", COV_CASES)
+def test_covariance_matches_numpy(name, mode):
+    p = _problem(name)
+    if name == "dup_once":  # points observed twice by one camera, points seen once
+        pairs = p.cam_idx.astype(np.int64) * p.n_pt + p.pt_idx
+        assert p.n_obs - np.unique(pairs).size > 0 and np.sum(np.bincount(p.pt_idx, minlength=p.n_pt) == 1) >= 200
+    far = _closure_pairs(p)
+    pr = np.concatenate([far, _pairs(p)])
+    got, piv, _, (pose, pt, intr) = _covariance(p, mode, iters=4, pairs=pr)
+    ref = _reference(p, mode, pose, pt, intr)
+    err = dict(cam=_rel(got["cam"], ref["cam"]), pt=_rel(got["pt"], ref["pt"]),
+               pairs=_rel(got["pairs"], np.stack([ref["pair"](a, b) for a, b in pr])),
+               closure_pairs=_rel(got["pairs"][:len(far)], np.stack([ref["pair"](a, b) for a, b in far])))
+    if mode == "REF":
+        err.update(cam_intr=_rel(got["cam_intr"], ref["cam_intr"]), intr=_rel(got["intr"], ref["intr"]))
+    else:
+        assert not got["cam_intr"].any() and not got["intr"].any()
+    print("covariance max relative error %s %s: %s; smallest pivot / diagonal: cameras %.3e intrinsics %.3e"
+          % (name, mode, " ".join("%s=%.2e" % kv for kv in sorted(err.items())), piv["cam"], piv["intr"]))
+    # In REF a camera (or pair) block is (A^-1)_cc + X_c T^-1 X_c^T: it carries the intrinsics border, the ill-conditioned
+    # direction, and its error follows the intrinsics blocks.  Measured on a B200 at closure_a: cam 1.06e-8 against numpy from
+    # the oracle's Jacobians, 9.6e-9 against numpy from the GPU's own Jacobians (so not the linearisation), intr 3.6e-8; the same
+    # problem in DEPTH (no border, the same tree) agrees to 5e-11.
+    intr_like = ("cam_intr", "intr") + (("cam", "pairs", "closure_pairs") if mode == "REF" else ())
+    for k, v in err.items():
+        assert v <= (TOL_INTR if k in intr_like else TOL), (k, v)
+    assert piv["cam"] > 1e3 * TAU and (mode == "DEPTH" or piv["intr"] > 1e3 * TAU), piv
+
+
+@pytest.mark.parametrize("name", ["closure_a", "dup_once"])
+def test_covariance_auto_and_sparse_cholesky_bit_identical(name):
+    p = _problem(name)
+    pr = np.concatenate([_closure_pairs(p), _pairs(p)])
+    (a, _, ia, _), (b, _, ib, _) = (_covariance(p, "REF", solver=sv, pairs=pr) for sv in (0, 4))
+    assert ia == {} and ib["nodes"] >= 1  # AUTO: the dense explicit solver is in force
+    for k in ("cam", "cam_intr", "intr", "pt", "pairs"):
+        assert np.array_equal(a[k], b[k]), k
+
+
+def test_covariance_other_tree_and_level_launches_agree(monkeypatch):
+    p = _problem("closure_c")
+    pr = np.concatenate([_closure_pairs(p), _pairs(p)])
+    base, _, ib, _ = _covariance(p, "REF", pairs=pr)
+    monkeypatch.setenv("BA_SPCHOL_LEAF", "6")
+    leaf, _, il, _ = _covariance(p, "REF", pairs=pr)
+    monkeypatch.delenv("BA_SPCHOL_LEAF")
+    monkeypatch.setenv("BA_SPCHOL_LEVELS", "1")
+    lev, _, _, _ = _covariance(p, "REF", pairs=pr)
+    assert il["nodes"] != ib["nodes"]  # really another tree
+    err = {k: (_rel(leaf[k], base[k]), _rel(lev[k], base[k])) for k in ("cam", "cam_intr", "intr", "pt", "pairs")}
+    for k, (e_leaf, e_lev) in err.items():
+        print("covariance closure_c %s: other tree %.2e, per-level launches %.2e" % (k, e_leaf, e_lev))
+    # (a point block amplifies the camera blocks by W V^-1: the largest difference, 2e-10 on a B200, is at a point seen by two
+    #  adjacent cameras at the far end of the chain, Sigma_pp about half the largest; both trees are as close to numpy there)
+    for k, (e_leaf, e_lev) in err.items():
+        tol = 1e-9 if k == "pt" else 1e-10
+        assert e_leaf <= tol and e_lev <= tol, (k, e_leaf, e_lev)
+
+
+# ---------------------------------------------------------------- 4. rank-deficient Hessians
+SINGULAR = {"two_maps": "camera", "one_obs_cam": "camera", "empty_cam": "camera", "unobserved_pt": "point"}
+
+
+@pytest.mark.parametrize("mode", ["REF", "DEPTH"])
+@pytest.mark.parametrize("name", sorted(SINGULAR))
+def test_rank_deficient_rejected(name, mode):
+    p = _problem(name)
+    g, _ = mode_opts(mode, solver=4)
+    s = ba_b200.GpuSolver(**g)
+    try:
+        s.upload(p)
+        with pytest.raises(ba_b200.BAError) as e:
+            s.covariance(points=True)
+        piv = s.covariance_pivots()
+    finally:
+        s.close()
+    print("rank-deficient %s %s: smallest pivot / diagonal: cameras %.3e intrinsics %.3e; %s"
+          % (name, mode, piv["cam"], piv["intr"], e.value))
+    assert e.value.code == capi.BA_ERR_NUMERIC
+    assert "singular" in str(e.value) or "rank-deficient" in str(e.value)
+    assert SINGULAR[name] in str(e.value)
+    if SINGULAR[name] == "camera":
+        assert piv["cam"] < TAU
+
+
+@pytest.mark.parametrize("name", sorted(SINGULAR))
+def test_rank_deficient_lm_tracks_oracle(name, solver_cache):
+    p = _problem(name)
+    s, summ = _lockstep_oracle(p, "REF", 8, solver_cache)
+    _check_tree(s, p)
+    assert summ.final_cost < summ.initial_cost
+    if name == "empty_cam":
+        assert np.array_equal(s.download()[0][7], p.pose7[7])
