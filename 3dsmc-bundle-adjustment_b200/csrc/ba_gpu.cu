@@ -137,6 +137,7 @@ struct ba_gpu_ctx {
   int64_t lm_graph_launches = 0;
   bool lm_graph_off = false, lm_graph_stale = true;
   bool spmv6 = false;  // BA_SPMV6=1: six-lanes-per-block product kernel in the launch-per-step PCG / product hook (experiment)
+  bool sps_simt = false;  // BA_SPS_SIMT=1: values of S by k_sp_schur_simt instead of the DMMA kernel (A/B comparisons only)
   bool pdl = false, pdl_off = false;  // programmatic dependent launches inside the windowed LM iteration (BA_NO_PDL=1: off)
   int legacy_chol = 0;  // BA_LEGACY_CHOL=1: left-looking single-CTA Cholesky, =2: shared-memory L D L^T, =3: grid-barrier blocked substitution (A/B timing only)
   Buf sp_lkeys, sp_gid, sp_gather, sp_gsorted, sp_diag, sp_scal;
@@ -435,6 +436,8 @@ extern "C" int ba_gpu_create(const ba_gpu_options *o, ba_gpu_ctx **out) {
   ctx->lm_graph_off = getenv("BA_NO_LM_GRAPH") != nullptr;
   ctx->pdl_off = getenv("BA_NO_PDL") != nullptr;
   ctx->spmv6 = getenv("BA_SPMV6") != nullptr;
+  ctx->sps_simt = getenv("BA_SPS_SIMT") && atoi(getenv("BA_SPS_SIMT")) != 0;
+  cudaFuncSetAttribute(k_sp_schur, cudaFuncAttributeMaxDynamicSharedMemorySize, BA_SPS_SMEM);
   cudaFuncSetAttribute(k_cholesky_solve<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 210 * 1024);
   cudaFuncSetAttribute(k_ldlt_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt_smem_bytes(BA_LDLT_MAX_N));
   cudaFuncSetAttribute(k_ldlt2_solve<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt2_smem_bytes(31));
@@ -767,7 +770,10 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
          P<int32_t>(ctx->pt_idx), P<int32_t>(ctx->sp_pair_pt));
   {
     int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, 0));
+    if (ctx->sps_simt)
+      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur_simt, BA_THREADS, 0));
+    else
+      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, BA_SPS_SMEM));
     ctx->sp_ctas_per_sm = std::max(1, per_sm);
   }
   RES(sp_ukeys, np8);
@@ -1918,10 +1924,17 @@ static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
   int *ticket = reinterpret_cast<int *>(P<char>(ctx->pcg_bar) + 16);
   cudaMemsetAsync(ticket, 0, 4, ctx->stream);
   // (pair records hold canonical observation indices: the kernel reads the CAMERA-major factored planes)
-  LAUNCH(k_sp_schur, std::min(cdiv(ctx->n_sblk_local, BA_SPS_CHUNK), ctx->n_sm * ctx->sp_ctas_per_sm), BA_THREADS, 0,
-         ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr), P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid),
-         P<unsigned long long>(ctx->sp_pairs), P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr),
-         P<double>(ctx->Vs), P<double>(ctx->Sblk), ticket, st, gate);
+  const int sps_grid = std::min(cdiv(ctx->n_sblk_local, BA_SPS_CHUNK), ctx->n_sm * ctx->sp_ctas_per_sm);
+  if (ctx->sps_simt)
+    LAUNCH(k_sp_schur_simt, sps_grid, BA_THREADS, 0, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
+           P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
+           P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
+           P<double>(ctx->Sblk), ticket, st, gate);
+  else
+    LAUNCH(k_sp_schur, sps_grid, BA_THREADS, BA_SPS_SMEM, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
+           P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
+           P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
+           P<double>(ctx->Sblk), ticket, st, gate);
   if (ctx->n_ranks > 1) {
     if (ctx->spchol && ctx->spc_dist && !ctx->sp_full_next) {
       // distributed factorisation: only the blocks another rank needs from this one (and the top part's) are summed

@@ -5,8 +5,9 @@
 // functors (:25-49, :72-94, :116-125) chained with the SE3 local
 // parameterisation (headers/sophus/local_parameterization_se3.hpp:17-37), Huber
 // correction, normal-equation blocks, Schur complement, linear solve and the
-// Levenberg-Marquardt controller.  fp64 throughout, no tensor cores, no global
-// floating-point atomics: every reduction has a fixed order.
+// Levenberg-Marquardt controller.  fp64 throughout, no global floating-point
+// atomics: every reduction has a fixed order.  Tensor cores only where a block is a
+// dense fp64 contraction: k_sp_schur (ba_kernels_sparse.cuh) sums with fp64 DMMA.
 //
 // Gating: every kernel of the LM pipeline first looks at the device-resident
 // controller state, so the host can enqueue whole iterations without waiting

@@ -350,8 +350,10 @@ __device__ __forceinline__ ObsGeo load_geo_l1(const FPlanes &F, int i, double fx
   o.wfy = b.y * fy;
   return o;
 }
+// The round-2 kernel: every lane holds the 36 accumulators of the block (238 registers, 8 warps per SM).  Kept only to
+// alternate with k_sp_schur in one process (BA_SPS_SIMT=1, read at create); no solver selects it.
 __global__ void __launch_bounds__(BA_THREADS)
-k_sp_schur(int n_blk, int n_cam, const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ lkeys,
+k_sp_schur_simt(int n_blk, int n_cam, const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ lkeys,
            const int32_t *__restrict__ gid, const unsigned long long *__restrict__ pairs, const int32_t *__restrict__ pair_pt,
            FPlanes F, const double *__restrict__ geo, const double *__restrict__ intr, const double *__restrict__ Vs,
            double *__restrict__ S, int *ticket, const LmState *st, int gate) {
@@ -436,6 +438,127 @@ k_sp_schur(int n_blk, int n_cam, const int32_t *__restrict__ blk_ptr, const unsi
       double *Sb = S + 36 * (size_t)gid[b] + idx;
       if (cnt > 0) Sb[0] = -acc[0];  // k_sp_add_diag puts U on the diagonal blocks
       if (cnt > 1) Sb[1] = -acc[1];
+    }
+  }
+}
+
+// Per block, S_b = -diag(s_i) [sum_pairs A_p^T H_p] diag(s_j) with A_p = [a0; a1] (2 x 6, rows of Jc in camera i) and
+// H_p = M_p [b0; b1] (2 x 6, the 2x2 core times the rows of Jc in camera j): a dense fp64 contraction of 6 x 2n by 2n x 6,
+// which is what mma.m8n8k4.f64 (DMMA) computes, two pairs per instruction, into an 8 x 8 accumulator (the 6 x 6 block
+// padded) of 2 registers per lane.  The warp walks the block's pairs in trips of 32: lane j stages pair e0 + j -- the
+// same gathers and arithmetic as k_sp_schur_simt -- as 12 double2 (a_t[r], h_t[r]) in its warp's slab, then the warp
+// runs ceil(n / 2) DMMA steps over the slab.  Lanes past the block's end stage zeros, so an odd tail's second pair adds 0.
+// Every block is summed in one fixed order (pair order, then the steps in order): bit-identical from run to run.
+// Slab: entry q = 6 t + r of pair p at q * BA_SPS_LD + p.  A lane stages with 12 stores of consecutive double2 across the
+// warp, and in step s lane (r = l >> 2, k = l & 3) reads entry (6 (k & 1) + r, 2 s + (k >> 1)) with one 16-byte load; with a
+// row stride of 34 (= 2 mod 8 in 16-byte bank groups) the 8 lanes of each quarter-warp hit 8 distinct bank groups, for the
+// stores and for the loads (a stride of 32 puts 4 of them on one group).
+// Registers: 122, no spills, two CTAs (16 warps) per SM.  Three CTAs (80 registers) spill even with the rotations moved to
+// shared memory and the pair-record prefetch dropped (16 to 40 bytes).
+#define BA_SPS_LD 34
+#define BA_SPS_SMEM (BA_THREADS / 32 * 12 * BA_SPS_LD * 16)
+__device__ __forceinline__ void dmma_m8n8k4(double &d0, double &d1, double a, double b) {
+  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
+}
+__global__ void __launch_bounds__(BA_THREADS, 2)
+k_sp_schur(int n_blk, int n_cam, const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ lkeys,
+           const int32_t *__restrict__ gid, const unsigned long long *__restrict__ pairs, const int32_t *__restrict__ pair_pt,
+           FPlanes F, const double *__restrict__ geo, const double *__restrict__ intr, const double *__restrict__ Vs,
+           double *__restrict__ S, int *ticket, const LmState *st, int gate) {
+  if (!gate_open(st, gate)) return;
+  extern __shared__ double2 sps_slab[];
+  __shared__ int s_chunk, s_next;
+  const int lane = threadIdx.x & 31, r = lane >> 2, k = lane & 3;
+  double2 *slab = sps_slab + (threadIdx.x >> 5) * (12 * BA_SPS_LD);
+  const double2 *frag = slab + (6 * (k & 1) + r) * BA_SPS_LD + (k >> 1);  // this lane's A / B operand in step 0
+  const double fx = ldg1(intr), fy = ldg1(intr + 1);
+  for (;;) {
+    __syncthreads();  // every warp is done with the previous chunk's counter
+    if (threadIdx.x == 0) {
+      s_chunk = atomicAdd(ticket, 1);
+      s_next = 0;
+    }
+    __syncthreads();
+    const int c0 = s_chunk * BA_SPS_CHUNK;
+    if (c0 >= n_blk) return;
+    const int cend = c0 + BA_SPS_CHUNK < n_blk ? c0 + BA_SPS_CHUNK : n_blk;
+    for (;;) {
+      int b = 0;
+      if (lane == 0) b = c0 + atomicAdd(&s_next, 1);
+      b = __shfl_sync(BA_FULL, b, 0);
+      if (b >= cend) break;
+      const unsigned long long key = lkeys[b];
+      const int ci = (int)(key / (unsigned long long)n_cam), cj = (int)(key % (unsigned long long)n_cam);
+      CamRec ri, rj;
+      load_camrec(geo, ci, ri);
+      load_camrec(geo, cj, rj);
+      double d0 = 0.0, d1 = 0.0;
+      const int e1 = blk_ptr[b + 1];
+      int e0 = blk_ptr[b];
+      unsigned long long pr = 0;
+      int p = 0;
+      if (e0 + lane < e1) {
+        pr = pairs[e0 + lane];
+        p = __ldg(pair_pt + e0 + lane);
+      }
+      for (; e0 < e1; e0 += 32) {
+        // the next trip's pair record is fetched before this trip's gathers are consumed
+        const int en = e0 + 32 + lane;
+        unsigned long long prn = 0;
+        int pn = 0;
+        if (en < e1) {
+          prn = pairs[en];
+          pn = __ldg(pair_pt + en);
+        }
+        // a lane past the block's end stages zeros: zero geometry (weights included) zeroes its rows and its core
+        ObsGeo ga = {0.0, 0.0, 0.0, 0.0, 0.0}, gb = ga;
+        double vs[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        if (e0 + lane < e1) {
+          // Vs as three 16-byte loads (the record is 48 B, 16-byte aligned): every load instruction of these gathers touches
+          // up to 32 different lines, and the L1 work of the six 8-byte loads was a third of the kernel's gather traffic
+          const double2 *v2 = reinterpret_cast<const double2 *>(Vs) + 3 * (size_t)p;
+          const double2 v01 = ldg2(v2), v23 = ldg2(v2 + 1), v45 = ldg2(v2 + 2);
+          vs[0] = v01.x; vs[1] = v01.y; vs[2] = v23.x; vs[3] = v23.y; vs[4] = v45.x; vs[5] = v45.y;
+          ga = load_geo_l1(F, (int)(pr >> 32), fx, fy);
+          gb = load_geo_l1(F, (int)(pr & 0xffffffffu), fx, fy);
+        }
+        double a0[6], a1[6], pa0[3], pa1[3], b0[6], b1[6], pb0[3], pb1[3];
+        sp_rows(ga, ri.R, a0, a1, pa0, pa1);
+        sp_rows(gb, rj.R, b0, b1, pb0, pb1);
+        double v0[3], v1[3];
+        sym3_mul(vs, pa0, v0);
+        sym3_mul(vs, pa1, v1);
+        const double m00 = v0[0] * pb0[0] + v0[1] * pb0[1] + v0[2] * pb0[2];
+        const double m01 = v0[0] * pb1[0] + v0[1] * pb1[1] + v0[2] * pb1[2];
+        const double m10 = v1[0] * pb0[0] + v1[1] * pb0[1] + v1[2] * pb0[2];
+        const double m11 = v1[0] * pb1[0] + v1[1] * pb1[1] + v1[2] * pb1[2];
+#pragma unroll
+        for (int c = 0; c < 6; ++c) {
+          slab[c * BA_SPS_LD + lane] = make_double2(a0[c], m00 * b0[c] + m01 * b1[c]);
+          slab[(6 + c) * BA_SPS_LD + lane] = make_double2(a1[c], m10 * b0[c] + m11 * b1[c]);
+        }
+        __syncwarp();
+        const int n_step = ((e1 - e0 < 32 ? e1 - e0 : 32) + 1) >> 1;
+        for (int s = 0; s < n_step; ++s) {
+          double av = 0.0, bv = 0.0;  // rows / columns 6 and 7 of the padded block
+          if (r < 6) {
+            const double2 v = frag[2 * s];
+            av = v.x;
+            bv = v.y;
+          }
+          dmma_m8n8k4(d0, d1, av, bv);
+        }
+        __syncwarp();  // the slab is read before the next trip overwrites it
+        pr = prn;
+        p = pn;
+      }
+      // lane l holds entries (r, 2k) and (r, 2k + 1) of the block: scales, then -S (k_sp_add_diag puts U on the diagonal)
+      if (r < 6 && k < 3) {
+        const double *si = geo + BA_CAMREC * (size_t)ci + 9, *sj = geo + BA_CAMREC * (size_t)cj + 9;
+        const double s_r = ldg1(si + r);
+        *reinterpret_cast<double2 *>(S + 36 * (size_t)gid[b] + 6 * r + 2 * k) =
+            make_double2(-(d0 * (s_r * ldg1(sj + 2 * k))), -(d1 * (s_r * ldg1(sj + 2 * k + 1))));
+      }
     }
   }
 }
