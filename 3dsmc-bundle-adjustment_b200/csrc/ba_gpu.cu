@@ -118,6 +118,7 @@ struct ba_gpu_ctx {
   bool fact = false, planes_ready = false;
   Buf fcm, fpm, geo, camx, Vs, ts, tgs, ys, tile_lo, tile_span;
   bool staged = false;
+  bool fp_store = false;  // point-major r / g records (Fp_) are kept: only the implicit solver's product reads them
   FPlanes Fc_, Fp_;
   // tile-fused product (ba_kernels_tile.cuh)
   Buf tmeta, tseg, tout, taux, tm_cam, tm_pt, tm_uv, ftm, cam_tmin, cam_tmax, tcnt, tpart_ptr, part6t;
@@ -1351,14 +1352,9 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     if (rcp) return rcp;
   } else {
     RES(fcm, n_pad * 48);
-    RES(fpm, n_pad * 48);
-    auto setf = [&](FPlanes &F, double *base) {
-      F.r = reinterpret_cast<double2 *>(base);
-      F.g0 = reinterpret_cast<double2 *>(base + 2 * n_pad);
-      F.g1 = reinterpret_cast<double2 *>(base + 4 * n_pad);
-    };
-    setf(ctx->Fc_, P<double>(ctx->fcm));
-    setf(ctx->Fp_, P<double>(ctx->fpm));
+    ctx->Fc_.r = P<double2>(ctx->fcm);
+    ctx->Fc_.g = reinterpret_cast<double4 *>(P<double2>(ctx->fcm) + n_pad);  // (n_pad is a multiple of 32: 32-byte aligned)
+    ctx->Fp_ = FPlanes{nullptr, nullptr};  // (allocated below once the solver is known)
     RES(geo, nc * BA_CAMREC * 8);
     RES(camx, nc * BA_CAMREC * 8);
     RES(Vs, np * 48);
@@ -1512,6 +1508,14 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     }
     ctx->dist_pcg = false;
     if (!ctx->spchol && ctx->n_ranks > 1 && o.persistent_pcg == 1 && (rcs = setup_dist_pcg(ctx))) return rcs;
+  }
+  // point-major records: only the implicit solver's product reads them (the block-sparse solvers, AUTO's included, reduce
+  // the point blocks straight from the projection and project again in the back-substitution)
+  ctx->fp_store = ctx->fact && !sparse;
+  if (ctx->fp_store) {
+    RES(fpm, n_pad * 48);
+    ctx->Fp_.r = P<double2>(ctx->fpm);
+    ctx->Fp_.g = reinterpret_cast<double4 *>(P<double2>(ctx->fpm) + n_pad);
   }
   if (sp_ref) {
     prof.stamp("to sparse");
@@ -1754,18 +1758,24 @@ static void enqueue_linearize(ba_gpu_ctx *ctx, int gate, const double *sc, const
            gate);
     // point-major branch on the side stream, camera-major branch on the main one (both need geo)
     fork_side(ctx);
-    LAUNCH((kf_linearize<0>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->pm_pt),
-           P<double2>(ctx->pm_uv), P<double>(ctx->pose), P<double>(ctx->pt), intr, ctx->cp, ctx->Fp_, (double *)nullptr, st,
-           gate);
-    LAUNCH(kf_pt_blocks, ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam), ctx->Fp_,
-           P<double>(ctx->geo), intr, sp, P<double>(ctx->V), P<double>(ctx->gp), P<double>(ctx->dp), ctx->lo, st, gate);
+#define PT_LIN(STORE, STAGED)                                                                                                   \
+  LAUNCH((kf_pt_linearize<STORE, STAGED>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr),                  \
+         P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->pm_pt), P<double2>(ctx->pm_uv), P<double>(ctx->pose), P<double>(ctx->pt),    \
+         P<double>(ctx->geo), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr, ctx->cp, sp, ctx->Fp_,               \
+         P<double>(ctx->V), P<double>(ctx->gp), P<double>(ctx->dp), ctx->lo, st, gate)
+    if (ctx->fp_store) {
+      if (ctx->staged) PT_LIN(1, 1); else PT_LIN(1, 0);
+    } else {
+      if (ctx->staged) PT_LIN(0, 1); else PT_LIN(0, 0);
+    }
+#undef PT_LIN
     if (ctx->tiled)
       LAUNCH(kt_linearize, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->tm_cam), P<int32_t>(ctx->tm_pt),
              P<double2>(ctx->tm_uv), P<double>(ctx->pose), P<double>(ctx->pt), intr, ctx->cp, ctx->Tg0, ctx->Tg1, st, gate);
     fork_main(ctx);
-    LAUNCH((kf_linearize<1>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
-           P<double2>(ctx->uv), P<double>(ctx->pose), P<double>(ctx->pt), intr, ctx->cp, ctx->Fc_, P<double>(ctx->pc_lin), st,
-           gate);
+    LAUNCH(kf_linearize, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
+           P<double2>(ctx->uv), P<double>(ctx->pose), P<double>(ctx->pt), P<double>(ctx->geo), intr, ctx->cp, ctx->Fc_,
+           P<double>(ctx->pc_lin), st, gate);
     LAUNCH(kf_cam_blocks, ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), ctx->Fc_, P<double>(ctx->geo), intr,
            P<double>(ctx->part_blk), st, gate);
     ItemRef ir = reduce_items<27>(ctx, P<double>(ctx->part_blk), ctx->red_blk, gate);
@@ -1889,12 +1899,14 @@ static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int pa
     if (passes & 1) {
       if (ctx->staged) {
         LAUNCH((kf_schur_pass1<0, 1>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-               ctx->Fp_, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
+               ctx->Fp_, (const int32_t *)nullptr, (const double2 *)nullptr, (const double *)nullptr, (const double *)nullptr,
+               ctx->cp, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
                P<double>(ctx->Vinv), P<double>(ctx->sp), (const double *)nullptr, (double *)nullptr, P<double>(ctx->ts), st, gate);
       } else {
         LAUNCH(k_pack_camx, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, v, P<double>(ctx->geo), P<double>(ctx->camx), st, gate);
         LAUNCH((kf_schur_pass1<0, 0>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-               ctx->Fp_, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
+               ctx->Fp_, (const int32_t *)nullptr, (const double2 *)nullptr, (const double *)nullptr, (const double *)nullptr,
+               ctx->cp, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
                P<double>(ctx->Vinv), P<double>(ctx->sp), (const double *)nullptr, (double *)nullptr, P<double>(ctx->ts), st, gate);
       }
     }
@@ -2450,14 +2462,23 @@ static int enqueue_lm_iteration(ba_gpu_ctx *ctx) {
   phase_mark(ctx, BA_PHASE_SUBSTITUTION);
   if (ctx->fact) {
     const double *intr = P<double>(ctx->intr);
-    LAUNCH(k_pack_camx, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->yc), P<double>(ctx->geo), P<double>(ctx->camx), st,
-           GATE_RUN);
-    LAUNCH((kf_schur_pass1<1, 0>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-           ctx->Fp_, P<double>(ctx->geo), P<double>(ctx->yc), P<double>(ctx->camx), P<int32_t>(ctx->tile_lo),
-           P<int32_t>(ctx->tile_span), intr, P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->gp), P<double>(ctx->yp),
-           P<double>(ctx->ys), st, GATE_RUN);
+    // (pass 1 projects every observation again instead of reading point-major records; the camera run staged as in the product)
+#define BACKSUB(STAGED)                                                                                                         \
+  LAUNCH((kf_schur_pass1<1, STAGED>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr),                      \
+         P<int32_t>(ctx->pm_cam), ctx->Fp_, P<int32_t>(ctx->pm_pt), P<double2>(ctx->pm_uv), P<double>(ctx->pose),             \
+         P<double>(ctx->pt), ctx->cp, P<double>(ctx->geo), P<double>(ctx->yc), P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), \
+         P<int32_t>(ctx->tile_span), intr, P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->gp), P<double>(ctx->yp),  \
+         P<double>(ctx->ys), st, GATE_RUN)
+    if (ctx->staged) {
+      BACKSUB(1);
+    } else {
+      LAUNCH(k_pack_camx, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->yc), P<double>(ctx->geo), P<double>(ctx->camx),
+             st, GATE_RUN);
+      BACKSUB(0);
+    }
+#undef BACKSUB
     LAUNCH(kf_model_cost, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx), ctx->Fc_,
-           P<double>(ctx->camx), intr, P<double>(ctx->ys), P<double>(ctx->pc_mcc), st, GATE_RUN);
+           P<double>(ctx->geo), P<double>(ctx->yc), intr, P<double>(ctx->ys), P<double>(ctx->pc_mcc), st, GATE_RUN);
   } else
   DISPATCH_DK(D, K, {
     // back-substitution y_p = V^-1 (-g_p - W^T y_c)
@@ -3285,18 +3306,22 @@ extern "C" int ba_gpu_time_kernel(ba_gpu_ctx *ctx, int32_t which, int32_t warmup
   if (rc) return rc;
   LmState *st = P<LmState>(ctx->st);
   LAUNCH(k_clear_done, 1, 1, 0, st);
+  // the two-pass product of the factored store reads the point-major records, which only the implicit solver keeps
+  const bool two_pass = !ctx->fact || ctx->fp_store;
+  if ((which == BA_KERNEL_SCHUR_PASS1 || which == BA_KERNEL_SCHUR_PASS2) && !two_pass)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "the two-pass product runs with the implicit solver only (solver = 2)");
   if (which != BA_KERNEL_LINEARIZE) {
     // t must hold a finite pass-1 result before a pass-2-only timing
     CK(cudaMemcpyAsync(ctx->p.p, ctx->gc.p, (size_t)ctx->n_cam * 48, cudaMemcpyDeviceToDevice, ctx->stream));
-    enqueue_matvec(ctx, P<double>(ctx->p), GATE_RUN, 7);
+    enqueue_matvec(ctx, P<double>(ctx->p), GATE_RUN, two_pass ? 7 : 3);
   }
   const size_t flush_n = (size_t)512 * 1024 * 1024 / 8;  // 512 MiB > 126 MB L2
   if (flush_l2) RES(flush, flush_n * 8);
   auto one = [&]() {
     if (which == BA_KERNEL_LINEARIZE && ctx->fact) {
-      LAUNCH((kf_linearize<1>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
-             P<double2>(ctx->uv), P<double>(ctx->pose), P<double>(ctx->pt), P<double>(ctx->intr), ctx->cp, ctx->Fc_,
-             P<double>(ctx->pc_lin), st, GATE_RUN);
+      LAUNCH(kf_linearize, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
+             P<double2>(ctx->uv), P<double>(ctx->pose), P<double>(ctx->pt), P<double>(ctx->geo), P<double>(ctx->intr), ctx->cp,
+             ctx->Fc_, P<double>(ctx->pc_lin), st, GATE_RUN);
     } else if (which == BA_KERNEL_LINEARIZE) {
       DISPATCH_DK(ctx->depth, ctx->nk, {
         LAUNCH((k_linearize<DD, KK, 1>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx),

@@ -9,24 +9,36 @@
 //     Jp = diag(w fx iz, w fy iz) [ R^T row0 - xz R^T row2 ] diag(s_p)
 //                                 [ R^T row1 - yz R^T row2 ]
 // (Appendix B of SURVEY.md; s_c, s_p = Jacobi column scales, R = R(q) of the
-// camera).  Instead of materialising 144 B of Jacobian per observation and
-// streaming it twice per PCG iteration, the store keeps g (32 B) and r (16 B)
-// and every consumer rebuilds the entries in registers: the implicit Schur
-// product reads 36 B/obs per pass instead of 148 B/obs.  The point scale s_p is
-// folded into per-point quantities (V^-1, t, y_p are kept pre-scaled) so the
-// camera-major kernels never gather it.
+// camera).  Instead of materialising 144 B of Jacobian per observation, the store
+// keeps per observation one 32-byte record g (one 256-bit load or store) and the
+// 16-byte residual r, and every consumer rebuilds the entries in registers.  The
+// point scale s_p is folded into per-point quantities (V^-1, t, y_p are kept
+// pre-scaled) so the camera-major kernels never gather it.
+//
+// Layout and readers:
+//   geo  per camera: R (from k_cam_geo, the one R every projection uses) and s_c.
+//   Fc_  camera-major r / g, written by kf_linearize; read by kf_cam_blocks,
+//        kf_schur_pass2, kf_schur_diag, kf_model_cost and k_sp_schur.
+//   Fp_  point-major r / g, only for the implicit solver (its PCG product runs
+//        kf_schur_pass1<0, .> every iteration); filled by kf_pt_linearize<1, .>.
+//        The block-sparse solvers neither allocate nor fill it: kf_pt_linearize<0, .>
+//        reduces V, g_p straight from the projection, and the back-substitution
+//        kf_schur_pass1<1, .> projects again.  All projections go through
+//        project_obs with R from geo, so a recomputed g equals the stored one bit for bit.
 #pragma once
 #include "ba_kernels.cuh"
 
 struct FPlanes {
-  double2 *r;   // robustified residual (r0, r1)
-  double2 *g0;  // (X/Z, Y/Z)
-  double2 *g1;  // (1/Z, w)
+  double2 *r;  // robustified residual (r0, r1)
+  double4 *g;  // (X/Z, Y/Z, 1/Z, w), 32-byte records
 };
 
 // per-camera record, 16 doubles = one 128-byte line: R (9, row-major), s (6, zero
 // for the constant pose :299 so that its Jacobian columns vanish), pad
 #define BA_CAMREC 16
+// shared-memory staging of a point tile's camera run (kf_pt_linearize, kf_schur_pass1): at most BA_STAGE_CAMS cameras
+#define BA_STAGE_CAMS 96
+#define BA_STAGE_REC 18
 struct CamRec {
   double R[9];
   double s[6];
@@ -106,59 +118,101 @@ __device__ __forceinline__ void jp_tmul(const ObsGeo &o, const double R[9], doub
   v[1] = (R[3] * al0 + R[4] * al1) + R[5] * al2;
   v[2] = (R[6] * al0 + R[7] * al1) + R[8] * al2;
 }
-__device__ __forceinline__ ObsGeo load_geo(const FPlanes &F, int i, double fx, double fy) {
-  const double2 a = lds2(F.g0 + i), b = lds2(F.g1 + i);
+// 256-bit accesses of the 32-byte g record (LDG.E.256 / STG.E.256 on sm_100a): streaming load, L1 load, streaming store
+__device__ __forceinline__ double4 lds4(const double4 *p) {
+  double4 v;
+  asm volatile("ld.global.nc.L1::no_allocate.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v.x), "=d"(v.y), "=d"(v.z), "=d"(v.w) : "l"(p));
+  return v;
+}
+__device__ __forceinline__ double4 ldg4(const double4 *p) {
+  double4 v;
+  asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v.x), "=d"(v.y), "=d"(v.z), "=d"(v.w) : "l"(p));
+  return v;
+}
+__device__ __forceinline__ void sts4(double4 *p, double4 v) {
+  asm volatile("st.global.L1::no_allocate.v4.f64 [%0], {%1,%2,%3,%4};" ::"l"(p), "d"(v.x), "d"(v.y), "d"(v.z), "d"(v.w));
+}
+__device__ __forceinline__ ObsGeo obs_geo(double4 g, double fx, double fy) {
   ObsGeo o;
-  o.xz = a.x;
-  o.yz = a.y;
-  o.iz = b.x;
-  o.wfx = b.y * fx;
-  o.wfy = b.y * fy;
+  o.xz = g.x;
+  o.yz = g.y;
+  o.iz = g.z;
+  o.wfx = g.w * fx;
+  o.wfy = g.w * fy;
   return o;
 }
+__device__ __forceinline__ ObsGeo load_geo(const FPlanes &F, int i, double fx, double fy) { return obs_geo(lds4(F.g + i), fx, fy); }
 
-// ------------------------------------------------------------------ linearise
-// 96 B/obs: uv 16 + idx 8 + point 24 read; r 16 + g 32 written
-template <int COST>
+// R of camera c as k_cam_geo stored it
+__device__ __forceinline__ void load_R(const double *__restrict__ geo, int c, double R[9]) {
+  const double2 *p = reinterpret_cast<const double2 *>(geo + (size_t)BA_CAMREC * c);
+  const double2 a = ldg2(p), b = ldg2(p + 1), d = ldg2(p + 2), e = ldg2(p + 3);
+  R[0] = a.x; R[1] = a.y; R[2] = b.x; R[3] = b.y; R[4] = d.x; R[5] = d.y; R[6] = e.x; R[7] = e.y;
+  R[8] = ldg1(geo + (size_t)BA_CAMREC * c + 8);
+}
+
+// The projection of one observation: camera rotation R (from geo) and centre C, point X, measurement m, intrinsics
+// K = (fx, fy, cx, cy).  Every linearisation of the factored store and the back-substitution's recompute go through this
+// one function, so the g they form agree bit for bit.
+struct ObsProj {
+  double r0, r1;       // robustified residual
+  double xz, yz, iz, w;  // the g record
+  double rho;          // rho(s), the cost term is rho / 2
+};
+__device__ __forceinline__ ObsProj project_obs(const double R[9], const double C[3], const double X3[3], double2 m,
+                                               double4 K, const CostParams &cp) {
+  const double d0 = X3[0] - C[0], d1 = X3[1] - C[1], d2 = X3[2] - C[2];
+  const double X = (R[0] * d0 + R[3] * d1) + R[6] * d2;
+  const double Y = (R[1] * d0 + R[4] * d1) + R[7] * d2;
+  const double Z = (R[2] * d0 + R[5] * d1) + R[8] * d2;
+  ObsProj o;
+  o.iz = 1.0 / Z;
+  o.xz = X * o.iz;
+  o.yz = Y * o.iz;
+  const double r0 = cp.sw_repr * ((K.x * o.xz + K.z) - m.x);
+  const double r1 = cp.sw_repr * ((K.y * o.yz + K.w) - m.y);
+  const double hs = huber_scale(cp.hub_repr, r0 * r0 + r1 * r1, o.rho);
+  o.r0 = r0 * hs;
+  o.r1 = r1 * hs;
+  o.w = cp.sw_repr * hs;
+  return o;
+}
+__device__ __forceinline__ double4 load_intr(const double *__restrict__ intr) {
+  return make_double4(ldg1(intr), ldg1(intr + 1), ldg1(intr + 2), ldg1(intr + 3));
+}
+__device__ __forceinline__ void load_pt(const double *__restrict__ pt, int p, double X3[3]) {
+  const double *q = pt + 3 * (size_t)p;
+  X3[0] = ldg1(q);
+  X3[1] = ldg1(q + 1);
+  X3[2] = ldg1(q + 2);
+}
+
+// ------------------------------------------------------------------ linearise (camera-major)
+// 96 B/obs: uv 16 + idx 8 + point 24 read; r 16 + g 32 written (R and centre are per camera: broadcast within an item)
 __global__ void __launch_bounds__(BA_THREADS)
 kf_linearize(int n_obs, const int32_t *__restrict__ cam_idx, const int32_t *__restrict__ pt_idx,
              const double2 *__restrict__ uv, const double *__restrict__ pose, const double *__restrict__ pt,
-             const double *__restrict__ intr, CostParams cp, FPlanes F, double *__restrict__ cost_part, LmState *st,
-             int gate) {
+             const double *__restrict__ geo, const double *__restrict__ intr, CostParams cp, FPlanes F,
+             double *__restrict__ cost_part, LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   __shared__ double red[BA_WARPS + 1];
   const int i = blockIdx.x * BA_THREADS + threadIdx.x;
   double cost = 0.0;
   if (i < n_obs) {
-    const int c = cam_idx[i], p = pt_idx[i];
+    const int c = cam_idx[i];
+    double R[9], X3[3];
+    load_R(geo, c, R);
     const double *P = pose + 7 * (size_t)c;
-    const double q[4] = {ldg1(P), ldg1(P + 1), ldg1(P + 2), ldg1(P + 3)};
-    double R[9];
-    quat_to_R(q, R);
-    const double *X3 = pt + 3 * (size_t)p;
-    const double d0 = ldg1(X3) - ldg1(P + 4), d1 = ldg1(X3 + 1) - ldg1(P + 5), d2 = ldg1(X3 + 2) - ldg1(P + 6);
-    const double X = (R[0] * d0 + R[3] * d1) + R[6] * d2;
-    const double Y = (R[1] * d0 + R[4] * d1) + R[7] * d2;
-    const double Z = (R[2] * d0 + R[5] * d1) + R[8] * d2;
-    const double iz = 1.0 / Z;
-    const double xz = X * iz, yz = Y * iz;
-    const double2 m = lds2(uv + i);
-    double r0 = cp.sw_repr * ((ldg1(intr) * xz + ldg1(intr + 2)) - m.x);
-    double r1 = cp.sw_repr * ((ldg1(intr + 1) * yz + ldg1(intr + 3)) - m.y);
-    double rho0;
-    const double hs = huber_scale(cp.hub_repr, r0 * r0 + r1 * r1, rho0);
-    cost = 0.5 * rho0;
-    r0 *= hs;
-    r1 *= hs;
-    sts2(F.r + i, make_double2(r0, r1));
-    sts2(F.g0 + i, make_double2(xz, yz));
-    sts2(F.g1 + i, make_double2(iz, cp.sw_repr * hs));
-    if (!(isfinite(r0) && isfinite(r1) && isfinite(iz))) st->eval_fail = 1;
+    const double C[3] = {ldg1(P + 4), ldg1(P + 5), ldg1(P + 6)};
+    load_pt(pt, pt_idx[i], X3);
+    const ObsProj o = project_obs(R, C, X3, lds2(uv + i), load_intr(intr), cp);
+    cost = 0.5 * o.rho;
+    sts2(F.r + i, make_double2(o.r0, o.r1));
+    sts4(F.g + i, make_double4(o.xz, o.yz, o.iz, o.w));
+    if (!(isfinite(o.r0) && isfinite(o.r1) && isfinite(o.iz))) st->eval_fail = 1;
   }
-  if (COST) {
-    const double s = block_sum(cost, red);
-    if (threadIdx.x == 0) cost_part[blockIdx.x] = s;
-  }
+  const double s = block_sum(cost, red);
+  if (threadIdx.x == 0) cost_part[blockIdx.x] = s;
 }
 
 // ------------------------------------------------------------------ camera blocks
@@ -214,30 +268,65 @@ kf_cam_blocks(int n_items, const BaItem *__restrict__ items, FPlanes F, const do
   }
 }
 
-// ------------------------------------------------------------------ point blocks
-// V_p (6), g_p (3), clamped LM diagonal; the point's column scale applied once
-__global__ void __launch_bounds__(BA_THREADS)
-kf_pt_blocks(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam, FPlanes F,
-             const double *__restrict__ geo, const double *__restrict__ intr, const double *__restrict__ sp,
-             double *__restrict__ V, double *__restrict__ gp, double *__restrict__ dp, LmOptions lo, const LmState *st,
-             int gate) {
+// ------------------------------------------------------------------ point-major linearisation
+// V_p (6), g_p (3) and the clamped LM diagonal, reduced straight from the projection: no record plane is written and read
+// back.  The point's column scale is applied once.  The tile's cameras (R 9, centre 3) are staged in shared memory as in
+// kf_schur_pass1; STAGED = 0 gathers them from geo and pose.  STORE = 1 also writes the point-major r / g records, which
+// only the implicit solver's product reads.  Algorithmic traffic: 48 B/obs (uv 16, cam and point idx 8, point 24; + 48 B
+// written with STORE) + 72 B/point.
+#define BA_LIN_REC 12
+template <int STORE, int STAGED>
+__global__ void __launch_bounds__(BA_THREADS, 3)
+kf_pt_linearize(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam,
+                const int32_t *__restrict__ pm_pt, const double2 *__restrict__ pm_uv, const double *__restrict__ pose,
+                const double *__restrict__ pt, const double *__restrict__ geo, const int32_t *__restrict__ tile_lo,
+                const int32_t *__restrict__ tile_span, const double *__restrict__ intr, CostParams cp,
+                const double *__restrict__ sp, FPlanes F, double *__restrict__ V, double *__restrict__ gp,
+                double *__restrict__ dp, LmOptions lo, const LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   constexpr int TOBS = 512;
   __shared__ double sm[9 * TOBS];
-  const double fx = ldg1(intr), fy = ldg1(intr + 1);
+  __shared__ __align__(16) double rec[STAGED ? BA_STAGE_CAMS * BA_LIN_REC : 2];
+  int cam_lo = 0;
+  if (STAGED) {
+    cam_lo = tile_lo[blockIdx.x];
+    const int n = tile_span[blockIdx.x];
+    for (int idx = threadIdx.x; idx < n * BA_LIN_REC; idx += BA_THREADS) {
+      const int rc = idx / BA_LIN_REC, k = idx - rc * BA_LIN_REC;
+      const size_t c = (size_t)(cam_lo + rc);
+      rec[idx] = k < 9 ? geo[c * BA_CAMREC + k] : pose[7 * c + 4 + (k - 9)];
+    }
+    __syncthreads();
+  }
+  const double4 K = load_intr(intr);
   tile_point_reduce<9, TOBS>(
       n_pt, pt_rowptr, sm,
       [&](int s, double *v) {
-        const ObsGeo o = load_geo(F, s, fx, fy);
-        const double2 r = lds2(F.r + s);
-        const double *R = geo + (size_t)BA_CAMREC * pm_cam[s];
+        const int c = pm_cam[s];
+        double R[9], C[3], X3[3];
+        if (STAGED) {
+          const double2 *cr = reinterpret_cast<const double2 *>(rec + (c - cam_lo) * BA_LIN_REC);
+          const double2 a = cr[0], b = cr[1], d = cr[2], e = cr[3], f = cr[4], g = cr[5];
+          R[0] = a.x; R[1] = a.y; R[2] = b.x; R[3] = b.y; R[4] = d.x; R[5] = d.y; R[6] = e.x; R[7] = e.y; R[8] = f.x;
+          C[0] = f.y; C[1] = g.x; C[2] = g.y;
+        } else {
+          load_R(geo, c, R);
+          const double *P = pose + 7 * (size_t)c;
+          C[0] = ldg1(P + 4); C[1] = ldg1(P + 5); C[2] = ldg1(P + 6);
+        }
+        load_pt(pt, pm_pt[s], X3);
+        const ObsProj pr = project_obs(R, C, X3, lds2(pm_uv + s), K, cp);
+        if (STORE) {
+          sts2(F.r + s, make_double2(pr.r0, pr.r1));
+          sts4(F.g + s, make_double4(pr.xz, pr.yz, pr.iz, pr.w));
+        }
+        const ObsGeo o = obs_geo(make_double4(pr.xz, pr.yz, pr.iz, pr.w), K.x, K.y);
         const double a = o.wfx * o.iz, b = o.wfy * o.iz;
         double p0[3], p1[3];
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
-          const double r2 = ldg1(R + 3 * k + 2);
-          p0[k] = a * (ldg1(R + 3 * k) - o.xz * r2);
-          p1[k] = b * (ldg1(R + 3 * k + 1) - o.yz * r2);
+          p0[k] = a * (R[3 * k] - o.xz * R[3 * k + 2]);
+          p1[k] = b * (R[3 * k + 1] - o.yz * R[3 * k + 2]);
         }
         v[0] = p0[0] * p0[0] + p1[0] * p1[0];
         v[1] = p0[0] * p0[1] + p1[0] * p1[1];
@@ -246,7 +335,7 @@ kf_pt_blocks(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__r
         v[4] = p0[1] * p0[2] + p1[1] * p1[2];
         v[5] = p0[2] * p0[2] + p1[2] * p1[2];
 #pragma unroll
-        for (int k = 0; k < 3; ++k) v[6 + k] = p0[k] * r.x + p1[k] * r.y;
+        for (int k = 0; k < 3; ++k) v[6 + k] = p0[k] * pr.r0 + p1[k] * pr.r1;
       },
       [&](int p, const double *sum) {
         const double s0 = sp[3 * (size_t)p], s1 = sp[3 * (size_t)p + 1], s2 = sp[3 * (size_t)p + 2];
@@ -304,15 +393,14 @@ kf_point_inverse(int n_pt, const double *__restrict__ V, const double *__restric
 // ------------------------------------------------------------------ pass 1 (point-major)
 //   MODE 0: ts_p = s .* V^-1 (s .* sum_o Jpu^T (Jc x_c))                        (matvec)
 //   MODE 1: y_p  = V^-1 (-g_p - s .* sum_o Jpu^T (Jc y_c)),  ys_p = s .* y_p    (back-substitution)
-// Algorithmic traffic: 36 B/obs (g 32 + cam idx 4) + 80 B/point (V^-1 48 + ts 32).
-// The per-camera operand (s.*x (6), R (9)) of every observation comes from
-// SHARED MEMORY: a tile of 128 consecutive points touches a short run of cameras
-// (tracks are runs of consecutive keyframes, points are numbered by first
-// appearance), so the CTA stages that run once, 144-byte records (bank-conflict
+// Algorithmic traffic: MODE 0 36 B/obs (g 32 + cam idx 4); MODE 1 24 B/obs (uv 16 + cam and point idx 8: g is projected
+// again, by project_obs from the same inputs as kf_pt_linearize, so it is the g the linearisation used); + 80 B/point.
+// The per-camera operand (s.*x (6), R (9), MODE 1 also the centre (3)) of every
+// observation comes from SHARED MEMORY: a tile of 128 consecutive points touches a
+// short run of cameras (tracks are runs of consecutive keyframes, points are numbered
+// by first appearance), so the CTA stages that run once, 144-byte records (bank-conflict
 // free for 8 consecutive cameras).  STAGED = 0 is the fallback for inputs whose
 // tiles span more than BA_STAGE_CAMS cameras: the records are gathered through L1.
-#define BA_STAGE_CAMS 96
-#define BA_STAGE_REC 18
 
 // per point tile: first camera and number of cameras spanned by its observations
 __global__ void __launch_bounds__(BA_THREADS)
@@ -350,8 +438,10 @@ k_tile_cam_range(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t 
 }
 
 template <int MODE, int STAGED>
-__global__ void __launch_bounds__(BA_THREADS)
+__global__ void __launch_bounds__(BA_THREADS, MODE ? 3 : 5)
 kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam, FPlanes F,
+               const int32_t *__restrict__ pm_pt, const double2 *__restrict__ pm_uv, const double *__restrict__ pose,
+               const double *__restrict__ pt, CostParams cp,
                const double *__restrict__ geo, const double *__restrict__ x, const double *__restrict__ camx,
                const int32_t *__restrict__ tile_lo, const int32_t *__restrict__ tile_span, const double *__restrict__ intr,
                const double *__restrict__ Vinv, const double *__restrict__ sp, const double *__restrict__ gp,
@@ -360,19 +450,22 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
   constexpr int TOBS = 512;
   __shared__ double sm[3 * TOBS];
   __shared__ __align__(16) double rec[STAGED ? BA_STAGE_CAMS * BA_STAGE_REC : 2];
-  const double fx = ldg1(intr), fy = ldg1(intr + 1);
+  const double4 K = load_intr(intr);
   int cam_lo = 0;
   if (STAGED) {
+    constexpr int NREC = MODE ? 18 : 16;
     cam_lo = tile_lo[blockIdx.x];
     const int n = tile_span[blockIdx.x];
-    for (int idx = threadIdx.x; idx < n * 16; idx += BA_THREADS) {
-      const int rc = idx >> 4, k = idx & 15;
+    for (int idx = threadIdx.x; idx < n * NREC; idx += BA_THREADS) {
+      const int rc = idx / NREC, k = idx - rc * NREC;
       const size_t c = (size_t)(cam_lo + rc);
-      double v = 0.0;
+      double v;
       if (k < 6)
         v = geo[c * BA_CAMREC + 9 + k] * x[c * 6 + k];
       else if (k < 15)
         v = geo[c * BA_CAMREC + (k - 6)];
+      else
+        v = MODE ? pose[7 * c + 4 + (k - 15)] : 0.0;
       rec[rc * BA_STAGE_REC + k] = v;
     }
     __syncthreads();
@@ -380,19 +473,36 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
   tile_point_reduce<3, TOBS>(
       n_pt, pt_rowptr, sm,
       [&](int s, double *v) {
-        const ObsGeo o = load_geo(F, s, fx, fy);
         const int c = pm_cam[s];
         double2 c0, c1, c2, c3, c4, c5, c6, c7;
+        double C[3];
         if (STAGED) {
           const double2 *cx = reinterpret_cast<const double2 *>(rec + (c - cam_lo) * BA_STAGE_REC);
           c0 = cx[0]; c1 = cx[1]; c2 = cx[2]; c3 = cx[3]; c4 = cx[4]; c5 = cx[5]; c6 = cx[6]; c7 = cx[7];
+          if (MODE == 1) {
+            const double2 c8 = cx[8];
+            C[0] = c7.y; C[1] = c8.x; C[2] = c8.y;
+          }
         } else {
           const double2 *cx = reinterpret_cast<const double2 *>(camx + (size_t)BA_CAMREC * c);
           c0 = ldg2(cx); c1 = ldg2(cx + 1); c2 = ldg2(cx + 2); c3 = ldg2(cx + 3); c4 = ldg2(cx + 4); c5 = ldg2(cx + 5);
           c6 = ldg2(cx + 6); c7 = ldg2(cx + 7);
+          if (MODE == 1) {
+            const double *P = pose + 7 * (size_t)c;
+            C[0] = ldg1(P + 4); C[1] = ldg1(P + 5); C[2] = ldg1(P + 6);
+          }
         }
         const double xx[6] = {c0.x, c0.y, c1.x, c1.y, c2.x, c2.y};
         const double R[9] = {c3.x, c3.y, c4.x, c4.y, c5.x, c5.y, c6.x, c6.y, c7.x};
+        ObsGeo o;
+        if (MODE == 0) {
+          o = load_geo(F, s, K.x, K.y);
+        } else {
+          double X3[3];
+          load_pt(pt, pm_pt[s], X3);
+          const ObsProj pr = project_obs(R, C, X3, lds2(pm_uv + s), K, cp);
+          o = obs_geo(make_double4(pr.xz, pr.yz, pr.iz, pr.w), K.x, K.y);
+        }
         double a0, a1;
         jc_dot(o, xx, a0, a1);
         jp_tmul(o, R, a0, a1, v);
@@ -545,7 +655,7 @@ kf_schur_diag(int n_items, const BaItem *__restrict__ items, const int32_t *__re
 // ------------------------------------------------------------------ model cost change
 __global__ void __launch_bounds__(BA_THREADS)
 kf_model_cost(int n_obs, const int32_t *__restrict__ cam_idx, const int32_t *__restrict__ pt_idx, FPlanes F,
-              const double *__restrict__ camy /* packed (s.*y_c, R) */, const double *__restrict__ intr,
+              const double *__restrict__ geo, const double *__restrict__ yc, const double *__restrict__ intr,
               const double *__restrict__ ys, double *__restrict__ part, const LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   __shared__ double red[BA_WARPS + 1];
@@ -555,11 +665,13 @@ kf_model_cost(int n_obs, const int32_t *__restrict__ cam_idx, const int32_t *__r
   if (i < n_obs) {
     const int c = cam_idx[i], p = pt_idx[i];
     const ObsGeo o = load_geo(F, i, fx, fy);
-    const double2 *cx = reinterpret_cast<const double2 *>(camy + (size_t)BA_CAMREC * c);
-    const double2 c0 = ldg2(cx), c1 = ldg2(cx + 1), c2 = ldg2(cx + 2), c3 = ldg2(cx + 3), c4 = ldg2(cx + 4), c5 = ldg2(cx + 5),
-                  c6 = ldg2(cx + 6), c7 = ldg2(cx + 7);
-    const double y[6] = {c0.x, c0.y, c1.x, c1.y, c2.x, c2.y};
-    const double R[9] = {c3.x, c3.y, c4.x, c4.y, c5.x, c5.y, c6.x, c6.y, c7.x};
+    CamRec cr;
+    load_camrec(geo, c, cr);
+    double y[6];
+    load6(yc + 6 * (size_t)c, y);
+#pragma unroll
+    for (int k = 0; k < 6; ++k) y[k] = cr.s[k] * y[k];
+    const double *R = cr.R;
     double t[3];
     ldg256(ys + 4 * (size_t)p, t[0], t[1], t[2]);
     double a0, a1, b0, b1;

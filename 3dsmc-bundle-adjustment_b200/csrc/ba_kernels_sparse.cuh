@@ -340,16 +340,7 @@ __device__ __forceinline__ void sp_reduce_scatter36(double (&acc)[36], int lane,
   c = (lane & 2) ? c - 3 : 3;
   cnt = (lane & 1) ? (c > 2 ? c - 2 : 0) : (c < 2 ? c : 2);
 }
-__device__ __forceinline__ ObsGeo load_geo_l1(const FPlanes &F, int i, double fx, double fy) {
-  const double2 a = __ldg(F.g0 + i), b = __ldg(F.g1 + i);
-  ObsGeo o;
-  o.xz = a.x;
-  o.yz = a.y;
-  o.iz = b.x;
-  o.wfx = b.y * fx;
-  o.wfy = b.y * fy;
-  return o;
-}
+__device__ __forceinline__ ObsGeo load_geo_l1(const FPlanes &F, int i, double fx, double fy) { return obs_geo(ldg4(F.g + i), fx, fy); }
 // The round-2 kernel: every lane holds the 36 accumulators of the block (238 registers, 8 warps per SM).  Kept only to
 // alternate with k_sp_schur in one process (BA_SPS_SIMT=1, read at create); no solver selects it.
 __global__ void __launch_bounds__(BA_THREADS)
