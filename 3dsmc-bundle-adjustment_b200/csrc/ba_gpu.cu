@@ -129,7 +129,7 @@ struct ba_gpu_ctx {
   Buf sp_cnt, sp_off, sp_keys, sp_vals, sp_keys2, sp_pairs, sp_ukeys, sp_ucnt, sp_nruns, sb_ptr, sb_i, sb_j, row_ucnt, row_tcnt,
       row_ustart, row_tstart, sp_tkeys, sp_tvals, sp_tkeys2, sp_tvals2, ent_ptr, ent, Sblk, ysp, cub_tmp, dsq, row_pq;
   int n_sblk = 0, n_sblk_local = 0, n_ent = 0, pcg_grid = 0, sp_ctas_per_sm = 1;
-  Buf sp_pair_pt, chol_v, chol_linv, chol_lsub, chol_slots;
+  Buf sp_pair_pt, chol_linv, chol_lsub, chol_slots;
   // one LM iteration of the windowed explicit solver as an instantiated CUDA graph (every decision is taken on the
   // device, so the node parameters never change between iterations); upload / set_options mark it stale and the next
   // solve re-captures and updates the executable in place (cudaGraphExecUpdate: destroying and re-instantiating it cost
@@ -137,10 +137,7 @@ struct ba_gpu_ctx {
   cudaGraphExec_t lm_graph = nullptr;
   int64_t lm_graph_launches = 0;
   bool lm_graph_off = false, lm_graph_stale = true;
-  bool spmv6 = false;  // BA_SPMV6=1: six-lanes-per-block product kernel in the launch-per-step PCG / product hook (experiment)
-  bool sps_simt = false;  // BA_SPS_SIMT=1: values of S by k_sp_schur_simt instead of the DMMA kernel (A/B comparisons only)
   bool pdl = false, pdl_off = false;  // programmatic dependent launches inside the windowed LM iteration (BA_NO_PDL=1: off)
-  int legacy_chol = 0;  // BA_LEGACY_CHOL=1: left-looking single-CTA Cholesky, =2: shared-memory L D L^T, =3: grid-barrier blocked substitution (A/B timing only)
   Buf sp_lkeys, sp_gid, sp_gather, sp_gsorted, sp_diag, sp_scal;
   // row-sharded persistent PCG over NVLink peer memory (ba_kernels_dist.cuh)
   Buf my_rows, row_flag, row_pos, ipc_stage;
@@ -171,8 +168,7 @@ struct ba_gpu_ctx {
   Buf spc_xidx, spc_xbuf;
   int spc_nx = 0;
   bool sp_full_next = false;  // the next enqueue_sparse_values() completes ALL of S on every rank (product hook)
-  bool spc_tree = true;         // one persistent launch with dependency counters (BA_SPCHOL_LEVELS=1: one launch per tree level)
-  size_t spc_smem_factor = 0, spc_smem_solve = 0, spc_smem_update = 0;
+  size_t spc_smem_tree = 0, spc_smem_solve = 0;  // dynamic shared memory of k_spchol_tree / k_spchol_solve
   double sym_ms = 0.0;          // host time of the symbolic phase (last upload)
   // sparse Cholesky of the REF / depth-prior / free-intrinsics cost (solver = EXPLICIT_CHOLESKY's linearisation and W / WV,
   // the block-sparse S and the tree instead of the dense S): right-hand-side rows of the tree (5 with the intrinsics border),
@@ -433,13 +429,9 @@ extern "C" int ba_gpu_create(const ba_gpu_options *o, ba_gpu_ctx **out) {
   if ((e = cudaEventCreate(&ctx->ev0)) != cudaSuccess) return bail("cudaEventCreate", e);
   if ((e = cudaEventCreate(&ctx->ev1)) != cudaSuccess) return bail("cudaEventCreate", e);
   if ((e = cudaMallocHost((void **)&ctx->h_st, sizeof(LmState))) != cudaSuccess) return bail("cudaMallocHost", e);
-  ctx->legacy_chol = getenv("BA_LEGACY_CHOL") ? atoi(getenv("BA_LEGACY_CHOL")) : 0;
   ctx->lm_graph_off = getenv("BA_NO_LM_GRAPH") != nullptr;
   ctx->pdl_off = getenv("BA_NO_PDL") != nullptr;
-  ctx->spmv6 = getenv("BA_SPMV6") != nullptr;
-  ctx->sps_simt = getenv("BA_SPS_SIMT") && atoi(getenv("BA_SPS_SIMT")) != 0;
   cudaFuncSetAttribute(k_sp_schur, cudaFuncAttributeMaxDynamicSharedMemorySize, BA_SPS_SMEM);
-  cudaFuncSetAttribute(k_cholesky_solve<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 210 * 1024);
   cudaFuncSetAttribute(k_ldlt_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt_smem_bytes(BA_LDLT_MAX_N));
   cudaFuncSetAttribute(k_ldlt2_solve<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt2_smem_bytes(31));
   cudaFuncSetAttribute(k_ldlt2_solve<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt2_smem_bytes(63));
@@ -447,7 +439,6 @@ extern "C" int ba_gpu_create(const ba_gpu_options *o, ba_gpu_ctx **out) {
   cudaFuncSetAttribute(k_ldlt2_solve<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt2_smem_bytes(127));
   cudaFuncSetAttribute(k_ldlt2_solve<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ldlt2_smem_bytes(BA_LDLT2_MAX_N));
   cudaFuncSetAttribute(k_chol_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_UPD_SMEM);
-  cudaFuncSetAttribute(k_chol_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * CH_NB * CH_LD * 8);
   cudaFuncSetAttribute(k_chol_trsm2, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * CH_NB * CH_LD * 8);
   cudaFuncSetAttribute(k_chol_potrf2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_potrf2_smem_bytes());
   cudaFuncSetAttribute(kt_schur_fused<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem_bytes(2));
@@ -771,10 +762,7 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
          P<int32_t>(ctx->pt_idx), P<int32_t>(ctx->sp_pair_pt));
   {
     int per_sm = 0;
-    if (ctx->sps_simt)
-      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur_simt, BA_THREADS, 0));
-    else
-      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, BA_SPS_SMEM));
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, BA_SPS_SMEM));
     ctx->sp_ctas_per_sm = std::max(1, per_sm);
   }
   RES(sp_ukeys, np8);
@@ -912,11 +900,13 @@ static int build_spchol(ba_gpu_ctx *ctx) {
     if (!v.empty()) CK(cudaMemcpyAsync(b.p, v.data(), v.size() * 4, cudaMemcpyHostToDevice, s));
     return 0;
   };
-  // subtree-to-rank partition: one part per rank (BA_SPCHOL_REPLICATED=1 keeps every rank factorising the whole tree);
-  // on one GPU BA_SPCHOL_PARTS=n runs the n parts one after the other (tests of the queues and of the exchange layout)
-  int want_parts = ctx->n_ranks > 1 ? (getenv("BA_SPCHOL_REPLICATED") ? 1 : ctx->n_ranks)
-                                    : (getenv("BA_SPCHOL_PARTS") ? std::min(BA_MAX_RANKS, std::max(1, atoi(getenv("BA_SPCHOL_PARTS")))) : 1);
-  if (getenv("BA_SPCHOL_LEVELS") || ctx->sp_ref) want_parts = 1;  // (the REF-cost path is single-GPU: one part)
+  // subtree-to-rank partition of the NS LM solve: one part per rank; on one GPU BA_SPCHOL_PARTS=n runs the n parts one after
+  // the other (tests of the queues and of the exchange layout).  One part for the REF-cost solve and for the structure the
+  // covariance builds under another solver: both are single-GPU and run the one-part queue's factor prefix on its own.
+  int want_parts = 1;
+  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG)
+    want_parts = ctx->n_ranks > 1 ? ctx->n_ranks
+                                  : (getenv("BA_SPCHOL_PARTS") ? std::min(BA_MAX_RANKS, std::max(1, atoi(getenv("BA_SPCHOL_PARTS")))) : 1);
   const int R = ctx->spc_nrhs;
   const SpPartition part = spsym_partition(S, want_parts);
   ctx->spc_parts = part.parts;
@@ -994,16 +984,12 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   // (at the front capacity, SPC_CAP_BLOCKS = 770 and SPC_MAX_OWN = 24, the five-row factor front needs 228,160 bytes)
   if (sf > 227 * 1024 || ss > 227 * 1024 || su > 227 * 1024)
     return fail(ctx, BA_ERR_STATE, "sparse Cholesky: front exceeds shared memory (%zu / %zu / %zu bytes)", sf, ss, su);
-  ctx->spc_smem_factor = sf;
+  ctx->spc_smem_tree = std::max(std::max(sf, ss), su);
   ctx->spc_smem_solve = ss;
-  ctx->spc_smem_update = su;
-  if (R > 1) {
-    CK(cudaFuncSetAttribute(k_spchol_factor<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
-    CK(cudaFuncSetAttribute(k_spchol_update<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)su));
-  } else {
-    CK(cudaFuncSetAttribute(k_spchol_factor<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
-    CK(cudaFuncSetAttribute(k_spchol_update<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)su));
-  }
+  if (R > 1)
+    CK(cudaFuncSetAttribute(k_spchol_tree<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->spc_smem_tree));
+  else
+    CK(cudaFuncSetAttribute(k_spchol_tree<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->spc_smem_tree));
   CK(cudaFuncSetAttribute(k_spchol_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
   // work queues of the persistent tree kernel.  Phase A (one queue per part): per level (bottom-up) the factor items of the
   // part's nodes, then their update tiles -- more tiles per node where the part has few nodes on a level.  Phase B: the same
@@ -1011,10 +997,7 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   // holds).  One part: phase A is the whole factorisation and the substitution follows in the same queue (one launch).
   {
     const int P_ = part.parts;
-    // -2: this GPU holds every part.  BA_SPCHOL_ONLY_PART=p on one GPU: the queues rank p of a distributed run would execute
-    // (the other parts' subtree roots count as done, their update matrices are whatever the buffer holds): timing experiments
-    const int only = (ctx->n_ranks == 1 && P_ > 1 && getenv("BA_SPCHOL_ONLY_PART")) ? std::min(P_ - 1, std::max(0, atoi(getenv("BA_SPCHOL_ONLY_PART")))) : -1;
-    const int me = ctx->spc_dist ? ctx->rank : (only >= 0 ? only : -2);
+    const int me = ctx->spc_dist ? ctx->rank : -2;  // (-2: this GPU holds every part)
     auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
     std::vector<int32_t> tiles((size_t)S.n_nodes, 0), q, cnt_init((size_t)3 * S.n_nodes + 16, 0), topcams;
     auto push_factor_levels = [&](int which) {
@@ -1075,12 +1058,6 @@ static int build_spchol(ba_gpu_ctx *ctx) {
         (rc = up(ctx->spc_topcams, topcams)))
       return rc;
     RES(spc_cnt, ((size_t)3 * S.n_nodes + 16) * 4);
-    const size_t st_ = std::max(std::max(sf, ss), su);
-    if (R > 1)
-      CK(cudaFuncSetAttribute(k_spchol_tree<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_));
-    else
-      CK(cudaFuncSetAttribute(k_spchol_tree<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_));
-    ctx->spc_tree = getenv("BA_SPCHOL_LEVELS") == nullptr;
     if (getenv("BA_SPCHOL_DEBUG"))
       fprintf(stderr, "[spchol] rank %d: %d parts%s, top %d nodes / %d cameras (%.1f %% of the work), heaviest part %.1f %%, "
               "exchange %.2f MB, items A %d B %d\n", ctx->rank, P_, ctx->spc_dist ? " (distributed)" : "",
@@ -1269,6 +1246,11 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
                 ctx->n_red);
   if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks > 1)
     return fail(ctx, BA_ERR_UNSUPPORTED, "the explicit solver is single-GPU (windowed problems stay on one GPU)");
+  // the dense substitution (k_chol_solve2) is one cooperative grid of n_sm CTAs, each owning at most CH_S2_OWN tiles of 64 unknowns
+  // (at BA_EXPLICIT_MAX_DIM: 256 tiles, 64 SMs)
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !sp_ref && cdiv(ctx->n_red, CH_NB) > CH_S2_OWN * ctx->n_sm)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky: reduced dimension %d needs %d SMs for its substitution (device has %d)",
+                ctx->n_red, cdiv(cdiv(ctx->n_red, CH_NB), CH_S2_OWN), ctx->n_sm);
   ctx->solver = solver;
   // AUTO on a large NS-mode problem, single GPU: block-sparse explicit S if the co-visibility
   // is sparse enough (decided after the index build, from the pair count), else implicit
@@ -1491,7 +1473,7 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
       return rcs;
     if (tot_pairs <= (double)o.sparse_max_pairs_per_obs * tot_obs && max_pairs <= 2147483647.0) {
       sparse = true;
-      want_chol = getenv("BA_AUTO_PCG") == nullptr;  // AUTO: exact factorisation (the reference's SPARSE_SCHUR) when its fronts fit
+      want_chol = true;  // AUTO: exact factorisation (the reference's SPARSE_SCHUR) when its fronts fit
       ctx->solver = BA_SOLVER_SPARSE_SCHUR_PCG;
     }
   }
@@ -1603,7 +1585,6 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     RES(WV, (no + 1) * 144);
     RES(S, (size_t)ctx->n_red * ctx->n_red * 8 + 64);
     RES(rhs, (size_t)ctx->n_red * 8 + 64);
-    RES(chol_v, (size_t)(ctx->n_red + 64 + 8) * 8);
     // blocked Cholesky: L^-1 of every diagonal tile (kept for the substitution) and the flag-in-data slots of k_chol_solve2
     RES(chol_linv, (size_t)cdiv(ctx->n_red, CH_NB) * CH_NB * CH_NB * 8);
     RES(chol_lsub, (size_t)(cdiv(ctx->n_red, CH_NB) + 1) * CH_NB * CH_NB * 8);  // panel tiles right below the diagonal (look-ahead)
@@ -1875,12 +1856,8 @@ static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int pa
   LmState *st = P<LmState>(ctx->st);
   const int rp = ctx->lo.reset_period;
   if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG && passes == 3) {
-    if (ctx->spmv6)
-      LAUNCH(k_bsr_spmv6, cdiv(ctx->n_cam * 32, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->ent_ptr),
-             P<int2>(ctx->ent), P<double>(ctx->Sblk), v, P<double>(ctx->ysp), st, gate);
-    else
-      LAUNCH(k_bsr_spmv, cdiv(ctx->n_cam * 32, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->ent_ptr),
-             P<int2>(ctx->ent), P<double>(ctx->Sblk), v, P<double>(ctx->ysp), st, gate);
+    LAUNCH(k_bsr_spmv, cdiv(ctx->n_cam * 32, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->ent_ptr), P<int2>(ctx->ent),
+           P<double>(ctx->Sblk), v, P<double>(ctx->ysp), st, gate);
     return ItemRef{P<int32_t>(ctx->ident), P<double>(ctx->ysp)};
   }
   if (ctx->tiled && passes == 3) {
@@ -1937,16 +1914,10 @@ static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
   cudaMemsetAsync(ticket, 0, 4, ctx->stream);
   // (pair records hold canonical observation indices: the kernel reads the CAMERA-major factored planes)
   const int sps_grid = std::min(cdiv(ctx->n_sblk_local, BA_SPS_CHUNK), ctx->n_sm * ctx->sp_ctas_per_sm);
-  if (ctx->sps_simt)
-    LAUNCH(k_sp_schur_simt, sps_grid, BA_THREADS, 0, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
-           P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
-           P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
-           P<double>(ctx->Sblk), ticket, st, gate);
-  else
-    LAUNCH(k_sp_schur, sps_grid, BA_THREADS, BA_SPS_SMEM, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
-           P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
-           P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
-           P<double>(ctx->Sblk), ticket, st, gate);
+  LAUNCH(k_sp_schur, sps_grid, BA_THREADS, BA_SPS_SMEM, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
+         P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
+         P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
+         P<double>(ctx->Sblk), ticket, st, gate);
   if (ctx->n_ranks > 1) {
     if (ctx->spchol && ctx->spc_dist && !ctx->sp_full_next) {
       // distributed factorisation: only the blocks another rank needs from this one (and the top part's) are summed
@@ -1966,8 +1937,8 @@ static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
          P<double>(ctx->Sblk), st, gate);
 }
 
-// exact solve of the reduced camera system by the sparse Cholesky: factorisation bottom-up (one launch per tree level, forward
-// substitution fused), backward substitution top-down.  b / dsq are complete (all-reduced) on every rank: the solve is replicated.
+// exact solve of the reduced camera system by the sparse Cholesky (k_spchol_tree: factorisation bottom-up with the forward
+// substitution fused, backward substitution top-down).  b / dsq are complete (all-reduced) on every rank: the solve is replicated.
 static SpChol spchol_args(ba_gpu_ctx *ctx) {
   SpChol a;
   a.node = P<int32_t>(ctx->spn_node);
@@ -2003,83 +1974,59 @@ static void enqueue_spchol_border(ba_gpu_ctx *ctx, int gate) {
          gate);
   LAUNCH(k_spb_solve, 1, 32, 0, nblk, P<double>(ctx->spb_part), P<double>(ctx->spb_kk), P<double>(ctx->yk), st, gate);
 }
+// one k_spchol_tree launch over the queue items [first, first + n) with ticket counter `slot`.  The launches of one solve share
+// the completion counters; the first (slot 0) brings them back to their state before a solve (spc_cnt_init).
+static void launch_spchol_tree(ba_gpu_ctx *ctx, const SpChol &a, int first, int n, int slot, int gate) {
+  LmState *st = P<LmState>(ctx->st);
+  const int n_nodes = ctx->sym.n_nodes;
+  int *cnt = P<int>(ctx->spc_cnt);
+  if (slot == 0) cudaMemcpyAsync(cnt, ctx->spc_cnt_init.p, ((size_t)3 * n_nodes + 16) * 4, cudaMemcpyDeviceToDevice, ctx->cur);
+  if (n <= 0) return;
+  SpTree t;
+  t.queue = P<int2>(ctx->spc_queue) + first;
+  t.n_items = n;
+  t.tiles = P<int32_t>(ctx->spc_tiles);
+  t.ticket = cnt + slot;
+  t.fdone = cnt + 16;
+  t.udone = t.fdone + n_nodes;
+  t.sdone = t.udone + n_nodes;
+  if (ctx->spc_nrhs > 1)
+    LAUNCH((k_spchol_tree<5>), std::min(ctx->n_sm, n), SPC_THREADS, ctx->spc_smem_tree, a, t, st, gate);
+  else
+    LAUNCH((k_spchol_tree<1>), std::min(ctx->n_sm, n), SPC_THREADS, ctx->spc_smem_tree, a, t, st, gate);
+}
+// the whole linear solve in one persistent launch: dependency counters instead of level barriers.  Partitioned tree: one
+// launch per part for its subtrees (phase A), one for the top part and the backward substitution (phase B).
 static void enqueue_spchol(ba_gpu_ctx *ctx, int gate) {
   LmState *st = P<LmState>(ctx->st);
-  const SpSymbolic &S = ctx->sym;
   const SpChol a = spchol_args(ctx);
-  // every kernel of the chain starts with griddepcontrol.wait (gate_open): programmatic dependent launches let the blocks of
-  // the next launch become resident on idle SMs (the upper tree levels have few nodes) while the previous one still runs
-  if (ctx->spc_tree) {
-    // the whole linear solve in one persistent launch (k_spchol_tree): dependency counters instead of level barriers.
-    // Partitioned tree: one launch for the subtrees (phase A), one for the top part and the backward substitution (phase B).
-    SpTree t;
-    int *cnt = P<int>(ctx->spc_cnt);
-    t.tiles = P<int32_t>(ctx->spc_tiles);
-    t.fdone = cnt + 16;
-    t.udone = t.fdone + S.n_nodes;
-    t.sdone = t.udone + S.n_nodes;
-    cudaMemcpyAsync(cnt, ctx->spc_cnt_init.p, ((size_t)3 * S.n_nodes + 16) * 4, cudaMemcpyDeviceToDevice, ctx->cur);
-    const size_t smem = std::max(std::max(ctx->spc_smem_factor, ctx->spc_smem_solve), ctx->spc_smem_update);
-    auto launch = [&](int first, int n, int slot) {
-      if (n <= 0) return;
-      t.queue = P<int2>(ctx->spc_queue) + first;
-      t.n_items = n;
-      t.ticket = cnt + slot;
-      if (ctx->spc_nrhs > 1)
-        LAUNCH((k_spchol_tree<5>), std::min(ctx->n_sm, n), SPC_THREADS, smem, a, t, st, gate);
-      else
-        LAUNCH((k_spchol_tree<1>), std::min(ctx->n_sm, n), SPC_THREADS, smem, a, t, st, gate);
-    };
-    if (ctx->spc_parts == 1 && ctx->spc_nrhs > 1) {
-      // intrinsics border: the queue's factor / update prefix, the 4 x 4 border system, then the backward substitution
-      launch(0, ctx->spc_qB, 0);
-      enqueue_spchol_border(ctx, gate);
-      phase_mark(ctx, BA_PHASE_FACTOR);
-      launch(ctx->spc_qB, ctx->spc_qB_n, 1);
-      return;
-    }
-    if (ctx->spc_parts == 1) {
-      launch(0, ctx->spc_n_items, 0);
-      phase_mark(ctx, BA_PHASE_FACTOR);
-      return;
-    }
-    if (ctx->spc_dist) cudaMemsetAsync(ctx->spc_U.p, 0, ctx->spc_xchg * 8, ctx->cur);
-    for (int p = 0; p < ctx->spc_parts; ++p) launch(ctx->spc_qA[p], ctx->spc_qA[p + 1] - ctx->spc_qA[p], p);
-    if (ctx->spc_dist && nccl_allreduce(ctx, P<double>(ctx->spc_U), ctx->spc_xchg, false)) ctx->comm_error = true;
-    if (ctx->spc_dist) cudaMemsetAsync(ctx->yc.p, 0, ((size_t)6 * ctx->n_cam + 1) * 8, ctx->cur);
-    launch(ctx->spc_qB, ctx->spc_qB_n, ctx->spc_parts);
-    if (ctx->spc_dist) {
-      // the step: every rank holds the top part's and its own subtrees' cameras; summed over ranks (zeros elsewhere, the top
-      // part kept by rank 0 only) with the failure flag in the extra slot
-      LAUNCH(k_spchol_dist_pre, cdiv(std::max(1, ctx->spc_n_topcams) * 6, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->spc_n_topcams,
-             P<int32_t>(ctx->spc_topcams), ctx->rank, P<double>(ctx->yc), st, gate);
-      if (nccl_allreduce(ctx, P<double>(ctx->yc), (size_t)6 * ctx->n_cam + 1, false)) ctx->comm_error = true;
-      LAUNCH(k_spchol_dist_post, 1, 32, 0, ctx->n_cam, P<double>(ctx->yc), st, gate);
-    }
+  if (ctx->spc_parts == 1 && ctx->spc_nrhs > 1) {
+    // intrinsics border: the queue's factor / update prefix, the 4 x 4 border system, then the backward substitution
+    launch_spchol_tree(ctx, a, 0, ctx->spc_qB, 0, gate);
+    enqueue_spchol_border(ctx, gate);
+    phase_mark(ctx, BA_PHASE_FACTOR);
+    launch_spchol_tree(ctx, a, ctx->spc_qB, ctx->spc_qB_n, 1, gate);
+    return;
+  }
+  if (ctx->spc_parts == 1) {
+    launch_spchol_tree(ctx, a, 0, ctx->spc_n_items, 0, gate);
     phase_mark(ctx, BA_PHASE_FACTOR);
     return;
   }
-  const bool pdl0 = ctx->pdl;
-  ctx->pdl = !ctx->pdl_off;
-  for (int l = 0; l < S.n_levels; ++l) {
-    const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
-    if (ctx->spc_nrhs > 1)
-      LAUNCH((k_spchol_factor<5>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, gate);
-    else
-      LAUNCH((k_spchol_factor<1>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, gate);
-    if (l + 1 < S.n_levels) {  // (roots have no border)
-      const int tiles = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
-      if (ctx->spc_nrhs > 1)
-        LAUNCH((k_spchol_update<5>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, gate);
-      else
-        LAUNCH((k_spchol_update<1>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, gate);
-    }
+  if (ctx->spc_dist) cudaMemsetAsync(ctx->spc_U.p, 0, ctx->spc_xchg * 8, ctx->cur);
+  for (int p = 0; p < ctx->spc_parts; ++p) launch_spchol_tree(ctx, a, ctx->spc_qA[p], ctx->spc_qA[p + 1] - ctx->spc_qA[p], p, gate);
+  if (ctx->spc_dist && nccl_allreduce(ctx, P<double>(ctx->spc_U), ctx->spc_xchg, false)) ctx->comm_error = true;
+  if (ctx->spc_dist) cudaMemsetAsync(ctx->yc.p, 0, ((size_t)6 * ctx->n_cam + 1) * 8, ctx->cur);
+  launch_spchol_tree(ctx, a, ctx->spc_qB, ctx->spc_qB_n, ctx->spc_parts, gate);
+  if (ctx->spc_dist) {
+    // the step: every rank holds the top part's and its own subtrees' cameras; summed over ranks (zeros elsewhere, the top
+    // part kept by rank 0 only) with the failure flag in the extra slot
+    LAUNCH(k_spchol_dist_pre, cdiv(std::max(1, ctx->spc_n_topcams) * 6, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->spc_n_topcams,
+           P<int32_t>(ctx->spc_topcams), ctx->rank, P<double>(ctx->yc), st, gate);
+    if (nccl_allreduce(ctx, P<double>(ctx->yc), (size_t)6 * ctx->n_cam + 1, false)) ctx->comm_error = true;
+    LAUNCH(k_spchol_dist_post, 1, 32, 0, ctx->n_cam, P<double>(ctx->yc), st, gate);
   }
-  if (ctx->spc_nrhs > 1) enqueue_spchol_border(ctx, gate);
   phase_mark(ctx, BA_PHASE_FACTOR);
-  for (int l = S.n_levels - 1; l >= 0; --l)
-    LAUNCH(k_spchol_solve, S.level_ptr[l + 1] - S.level_ptr[l], SPC_THREADS, ctx->spc_smem_solve, a, S.level_ptr[l], st, gate);
-  ctx->pdl = pdl0;
 }
 
 static int poll_state(ba_gpu_ctx *ctx) {
@@ -2239,7 +2186,7 @@ struct ChActive {
 static ChActive chol_active(const ba_gpu_ctx *ctx, int n, int nt, int k) {
   ChActive a;
   const int below = nt - k - 1;
-  if (ctx->ex_band_cams < 0 || getenv("BA_CHOL_DENSE")) {
+  if (ctx->ex_band_cams < 0) {
     a.n_band = below;
     a.bord0 = nt;
     a.n_act = below;
@@ -2374,7 +2321,7 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
          P<int32_t>(ctx->pair_ptr), P<int32_t>(ctx->pair_a), P<int32_t>(ctx->pair_b), P<double>(ctx->W), P<double>(ctx->WV),
          P<double>(ctx->U), P<double>(ctx->dc), P<double>(ctx->S), st, GATE_RUN);
   join(ctx);
-  if (n <= BA_LDLT2_MAX_N && !ctx->legacy_chol) {
+  if (n <= BA_LDLT2_MAX_N) {
     // single CTA, L D L^T with the trailing matrix in registers and the right-hand side as an extra row (ba_kernels_chol.cuh)
 #define LDLT2_LAUNCH(NT)                                                                                                  \
   LAUNCH(k_ldlt2_solve<NT>, 1, 1024, ldlt2_smem_bytes(n), n, P<double>(ctx->S), P<double>(ctx->rhs), ctx->n_cam, ctx->n_free, \
@@ -2387,23 +2334,18 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
       default: LDLT2_LAUNCH(5); break;
     }
 #undef LDLT2_LAUNCH
-  } else if (n <= BA_LDLT_MAX_N && ctx->legacy_chol != 1) {
+  } else if (n <= BA_LDLT_MAX_N) {
     // single CTA, matrix in shared memory, L D L^T with the right-hand side as an extra row (ba_kernels_chol.cuh)
     LAUNCH(k_ldlt_solve, 1, 1024, ldlt_smem_bytes(n), n, P<double>(ctx->S), P<double>(ctx->rhs), ctx->n_cam, ctx->n_free,
-           P<int32_t>(ctx->cam_slot), ctx->nk, P<double>(ctx->yc), P<double>(ctx->yk), st, GATE_RUN);
-  } else if (n <= 160) {
-    const size_t smem = ((size_t)n * n + n + 8) * 8;
-    LAUNCH((k_cholesky_solve<1>), 1, 256, smem, n, P<double>(ctx->S), P<double>(ctx->rhs), ctx->n_cam, ctx->n_free,
            P<int32_t>(ctx->cam_slot), ctx->nk, P<double>(ctx->yc), P<double>(ctx->yk), st, GATE_RUN);
   } else {
     // blocked right-looking Cholesky (ba_kernels_chol.cuh): the reference's global BA with free intrinsics
     const int nt = cdiv(n, CH_NB);
     double *S = P<double>(ctx->S);
     double *Linv = P<double>(ctx->chol_linv);
-    // one GPU: three-stream look-ahead schedule (factor_blocked_lookahead2); otherwise (sharded run, BA_NO_LOOKAHEAD=1, legacy
-    // kernels) the plain right-looking sequence on the solver stream
-    const bool lookahead = ctx->forking && ctx->stream2 && ctx->cur == ctx->stream && ctx->legacy_chol == 0 &&
-                           getenv("BA_NO_LOOKAHEAD") == nullptr;
+    // one GPU: three-stream look-ahead schedule (factor_blocked_lookahead2); otherwise (sharded run, BA_NO_LOOKAHEAD=1) the
+    // plain right-looking sequence on the solver stream
+    const bool lookahead = ctx->forking && ctx->stream2 && ctx->cur == ctx->stream && getenv("BA_NO_LOOKAHEAD") == nullptr;
     if (lookahead) {
       int rcf = factor_blocked_lookahead2(ctx, n, nt, S, Linv, P<double>(ctx->chol_lsub), st);
       ctx->cur = ctx->stream;
@@ -2411,43 +2353,25 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
       if (rcf) return rcf;
     }
     for (int k = 0; k < nt && !lookahead; ++k) {
-      const int below = nt - k - 1;
-      if (ctx->legacy_chol == 1) {
-        LAUNCH(k_chol_potrf, 1, CH_NB, 0, n, S, k, st, GATE_RUN);
-        LAUNCH(k_chol_trsm, below, CH_NB, (size_t)2 * CH_NB * CH_LD * 8, n, S, k, st, GATE_RUN);
-      } else {
-        // diagonal tile: register-resident L D L^T that also yields L^-1; panel: product with L^-1
-        LAUNCH(k_chol_potrf2, 1, 1024, chol_potrf2_smem_bytes(), n, S, Linv + (size_t)k * CH_NB * CH_NB, k, 0, st, GATE_RUN);
-        const ChActive act = chol_active(ctx, n, nt, k);
-        LAUNCH(k_chol_trsm2, act.n_act, 256, (size_t)2 * CH_NB * CH_LD * 8, n, S, Linv + (size_t)k * CH_NB * CH_NB, (double *)nullptr, k,
-               act.n_band, act.bord0, st, GATE_RUN);
-        LAUNCH(k_chol_update, act.n_act * (act.n_act + 1) / 2, 256, CH_UPD_SMEM, n, S, (const double *)nullptr, k, k, 0, act.n_band,
-               act.bord0, st, GATE_RUN);
-        continue;
-      }
-      LAUNCH(k_chol_update, below * (below + 1) / 2, 256, CH_UPD_SMEM, n, S, (const double *)nullptr, k, k, 0, below, nt, st,
-             GATE_RUN);
+      // diagonal tile: register-resident L D L^T that also yields L^-1; panel: product with L^-1
+      LAUNCH(k_chol_potrf2, 1, 1024, chol_potrf2_smem_bytes(), n, S, Linv + (size_t)k * CH_NB * CH_NB, k, 0, st, GATE_RUN);
+      const ChActive act = chol_active(ctx, n, nt, k);
+      LAUNCH(k_chol_trsm2, act.n_act, 256, (size_t)2 * CH_NB * CH_LD * 8, n, S, Linv + (size_t)k * CH_NB * CH_NB, (double *)nullptr, k,
+             act.n_band, act.bord0, st, GATE_RUN);
+      LAUNCH(k_chol_update, act.n_act * (act.n_act + 1) / 2, 256, CH_UPD_SMEM, n, S, (const double *)nullptr, k, k, 0, act.n_band,
+             act.bord0, st, GATE_RUN);
     }
+    // substitution through the stored L_kk^-1 tiles, solved values exchanged as flag-in-data slots (k_chol_solve2; upload
+    // checked that its grid owns every tile)
     int nn = n, n_cam = ctx->n_cam, n_free = ctx->n_free, nk = ctx->nk, gate = GATE_RUN;
-    const double *Sc = S, *rhs = P<double>(ctx->rhs);
+    const double *Sc = S, *Li = Linv, *rhs = P<double>(ctx->rhs);
     double *yc = P<double>(ctx->yc), *yk = P<double>(ctx->yk);
     const int32_t *cam_slot = P<int32_t>(ctx->cam_slot);
-    if (ctx->legacy_chol == 0 && nt <= CH_S2_OWN * ctx->n_sm) {
-      // substitution through the stored L_kk^-1 tiles, solved values exchanged as flag-in-data slots (k_chol_solve2)
-      ChSlot *fwd = P<ChSlot>(ctx->chol_slots), *bwd = fwd + (size_t)nt * CH_NB;
-      CK(cudaMemsetAsync(fwd, 0, (size_t)2 * nt * CH_NB * sizeof(ChSlot), ctx->stream));
-      const double *Li = Linv;
-      void *args[] = {&nn, &Sc, &Li, &rhs, &fwd, &bwd, &n_cam, &n_free, &cam_slot, &nk, &yc, &yk, &st, &gate};
-      CK(cudaLaunchCooperativeKernel((const void *)k_chol_solve2, dim3(ctx->n_sm), dim3(256), args, 0, ctx->stream));
-      ctx->launches++;
-    } else {
-      CK(cudaMemsetAsync(P<char>(ctx->chol_v) + (size_t)(n + 64) * 8, 0, 16, ctx->stream));
-      double *v = P<double>(ctx->chol_v), *ztg = v + n;
-      unsigned int *bar = reinterpret_cast<unsigned int *>(v + n + 64);
-      void *args[] = {&nn, &Sc, &rhs, &v, &ztg, &bar, &n_cam, &n_free, &cam_slot, &nk, &yc, &yk, &st, &gate};
-      CK(cudaLaunchCooperativeKernel((const void *)k_chol_solve, dim3(ctx->n_sm), dim3(256), args, 0, ctx->stream));
-      ctx->launches++;
-    }
+    ChSlot *fwd = P<ChSlot>(ctx->chol_slots), *bwd = fwd + (size_t)nt * CH_NB;
+    CK(cudaMemsetAsync(fwd, 0, (size_t)2 * nt * CH_NB * sizeof(ChSlot), ctx->stream));
+    void *args[] = {&nn, &Sc, &Li, &rhs, &fwd, &bwd, &n_cam, &n_free, &cam_slot, &nk, &yc, &yk, &st, &gate};
+    CK(cudaLaunchCooperativeKernel((const void *)k_chol_solve2, dim3(ctx->n_sm), dim3(256), args, 0, ctx->stream));
+    ctx->launches++;
   }
   return 0;
 }
@@ -3033,38 +2957,8 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
   LAUNCH(k_fill, 1, 32, 0, P<double>(ctx->dsq) + 6 * (size_t)ctx->fixed_cam, (size_t)6, 1.0);
   // factorisation (forward substitution: Z = L^-1 B with the border)
   SpChol a = spchol_args(ctx);
-  if (ctx->spc_tree && ctx->spc_parts == 1) {
-    SpTree t;
-    int *cnt = P<int>(ctx->spc_cnt);
-    t.tiles = P<int32_t>(ctx->spc_tiles);
-    t.fdone = cnt + 16;
-    t.udone = t.fdone + S.n_nodes;
-    t.sdone = t.udone + S.n_nodes;
-    CK(cudaMemcpyAsync(cnt, ctx->spc_cnt_init.p, ((size_t)3 * S.n_nodes + 16) * 4, cudaMemcpyDeviceToDevice, s));
-    const size_t smem = std::max(std::max(ctx->spc_smem_factor, ctx->spc_smem_solve), ctx->spc_smem_update);
-    t.queue = P<int2>(ctx->spc_queue);
-    t.n_items = ctx->spc_qB;
-    t.ticket = cnt;
-    if (ctx->spc_nrhs > 1)
-      LAUNCH((k_spchol_tree<5>), std::min(ctx->n_sm, t.n_items), SPC_THREADS, smem, a, t, st, GATE_RUN);
-    else
-      LAUNCH((k_spchol_tree<1>), std::min(ctx->n_sm, t.n_items), SPC_THREADS, smem, a, t, st, GATE_RUN);
-  } else {
-    for (int l = 0; l < S.n_levels; ++l) {
-      const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
-      if (ctx->spc_nrhs > 1)
-        LAUNCH((k_spchol_factor<5>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, GATE_RUN);
-      else
-        LAUNCH((k_spchol_factor<1>), nodes, SPC_THREADS, ctx->spc_smem_factor, a, S.level_ptr[l], st, GATE_RUN);
-      if (l + 1 < S.n_levels) {
-        const int tiles = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
-        if (ctx->spc_nrhs > 1)
-          LAUNCH((k_spchol_update<5>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, GATE_RUN);
-        else
-          LAUNCH((k_spchol_update<1>), nodes * tiles, SPU_THREADS, ctx->spc_smem_update, a, S.level_ptr[l], tiles, st, GATE_RUN);
-      }
-    }
-  }
+  // (the covariance's structure is always one part: the queue's prefix up to spc_qB is the whole factorisation)
+  launch_spchol_tree(ctx, a, 0, ctx->spc_qB, 0, GATE_RUN);
   LAUNCH(k_cov_pivots, cdiv(6 * ctx->n_cam, BA_THREADS), BA_THREADS, 0, ctx->n_cam, a.perm, P<int32_t>(ctx->sp_diag), a.S, a.dsq,
          a.linv, BA_COV_MIN_PIVOT_RATIO, cp);
   // intrinsics border: T^-1, then X = L^-T Z one column at a time (the backward substitution of the LM step, levels top-down)

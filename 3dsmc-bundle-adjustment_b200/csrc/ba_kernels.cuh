@@ -1968,79 +1968,6 @@ k_explicit_assemble(int n_cam, int n_free, int n, const int32_t *__restrict__ ca
   }
 }
 
-// dense Cholesky A = L L^T and solve, single CTA, left-looking with one thread
-// per row (the summation order of a textbook column Cholesky).  A lives in
-// shared memory when it fits (n <= 160), else in global memory.
-template <int SMEM>
-__global__ void __launch_bounds__(1024)
-k_cholesky_solve(int n, double *__restrict__ Sg, const double *__restrict__ rhs, int n_cam, int n_free,
-                 const int32_t *__restrict__ cam_slot, int nk, double *__restrict__ yc, double *__restrict__ yk, LmState *st,
-                 int gate) {
-  if (!gate_open(st, gate)) return;
-  extern __shared__ double smd[];
-  __shared__ double piv;
-  __shared__ int fail;
-  double *A = SMEM ? smd : Sg;
-  double *bv = SMEM ? smd + (size_t)n * n : nullptr;
-  __shared__ double bsm[1024];
-  if (!SMEM) bv = bsm;
-  const int tid = threadIdx.x, nt = blockDim.x;
-  if (SMEM)
-    for (int k = tid; k < n * n; k += nt) A[k] = Sg[k];
-  if (tid == 0) fail = st->lin_fail;
-  __syncthreads();
-  if (fail) return;
-  for (int j = 0; j < n; ++j) {
-    double s = 0.0;
-    const int i = tid;
-    if (i >= j && i < n) {
-      s = A[(size_t)i * n + j];
-      for (int k = 0; k < j; ++k) s -= A[(size_t)i * n + k] * A[(size_t)j * n + k];
-      if (i == j) {
-        if (!(s > 0.0) || !isfinite(s)) fail = 1;
-        piv = 1.0 / sqrt(s);
-        A[(size_t)j * n + j] = sqrt(s);
-      }
-    }
-    __syncthreads();
-    if (fail) break;
-    if (i > j && i < n) A[(size_t)i * n + j] = s * piv;
-    __syncthreads();
-  }
-  if (fail) {
-    if (tid == 0) st->lin_fail = 1;
-    return;
-  }
-  // forward substitution L z = b
-  double s = (tid < n) ? rhs[tid] : 0.0;
-  for (int k = 0; k < n; ++k) {
-    if (tid == k) bv[k] = s / A[(size_t)k * n + k];
-    __syncthreads();
-    if (tid > k && tid < n) s -= A[(size_t)tid * n + k] * bv[k];
-  }
-  __syncthreads();
-  // back substitution L^T y = z
-  s = (tid < n) ? bv[tid] : 0.0;
-  __syncthreads();
-  for (int k = n - 1; k >= 0; --k) {
-    if (tid == k) bv[k] = s / A[(size_t)k * n + k];
-    __syncthreads();
-    if (tid < k) s -= A[(size_t)k * n + tid] * bv[k];
-  }
-  __syncthreads();
-  for (int c = tid; c < n_cam; c += nt) {
-    const int slot = cam_slot[c];
-#pragma unroll
-    for (int k = 0; k < 6; ++k) {
-      const double v = slot >= 0 ? bv[6 * slot + k] : 0.0;
-      if (!isfinite(v)) st->lin_fail = 1;
-      yc[6 * (size_t)c + k] = v;
-    }
-  }
-  if (tid < 4) yk[tid] = nk ? bv[6 * n_free + tid] : 0.0;
-}
-
-
 // =====================================================================
 // Multi-GPU glue (points sharded across ranks, SURVEY.md 8e): local
 // per-camera sums / scalars are packed into dense buffers that NCCL all-reduces

@@ -11,80 +11,14 @@
 // then k_chol_solve2: blocked forward / backward substitution through the stored L_kk^-1 tiles and the scatter into y_c / y_k.
 // On one GPU the steps are software-pipelined over three streams (ba_gpu.cu: factor_blocked_lookahead2): the diagonal kernel
 // brings its own tile up to date (fused prologue), so it is the only kernel on the critical chain.
-// k_chol_potrf / k_chol_trsm / k_chol_solve are the first versions (BA_LEGACY_CHOL, A/B timing only).
+// The first versions (left-looking diagonal tile, one-thread-per-row panel, substitution with grid barriers) were removed;
+// the timings quoted below for them are the measurements that replaced them.
 // Every sum has a fixed order (no atomics).  == the exact step of Ceres DENSE_SCHUR / SPARSE_SCHUR.
 #pragma once
 #include "ba_kernels.cuh"
 
 #define CH_NB 64
 #define CH_LD (CH_NB + 1)
-
-__global__ void __launch_bounds__(CH_NB)
-k_chol_potrf(int n, double *__restrict__ A, int k, LmState *st, int gate) {
-  if (!gate_open(st, gate) || st->lin_fail) return;
-  __shared__ double T[CH_NB * CH_LD];
-  __shared__ double piv;
-  __shared__ int fail;
-  const int j0 = k * CH_NB, m = min(CH_NB, n - j0), i = threadIdx.x;
-  if (i == 0) fail = 0;
-  for (int r = 0; r < m; ++r)  // row by row: the CTA reads 64 consecutive doubles
-    if (i < m) T[r * CH_LD + i] = i <= r ? A[(size_t)(j0 + r) * n + j0 + i] : 0.0;
-  __syncthreads();
-  for (int j = 0; j < m; ++j) {
-    double s = 0.0;
-    if (i >= j && i < m) {
-      s = T[i * CH_LD + j];
-      for (int q = 0; q < j; ++q) s -= T[i * CH_LD + q] * T[j * CH_LD + q];
-      if (i == j) {
-        if (!(s > 0.0) || !isfinite(s)) fail = 1;
-        piv = 1.0 / sqrt(s);
-        T[j * CH_LD + j] = sqrt(s);
-      }
-    }
-    __syncthreads();
-    if (fail) break;
-    if (i > j && i < m) T[i * CH_LD + j] = s * piv;
-    __syncthreads();
-  }
-  if (fail) {
-    if (i == 0) st->lin_fail = 1;
-    return;
-  }
-  for (int r = 0; r < m; ++r)
-    if (i < m && i <= r) A[(size_t)(j0 + r) * n + j0 + i] = T[r * CH_LD + i];
-}
-
-// rows below the diagonal tile: one thread per row, L_kk broadcast from shared memory
-__global__ void __launch_bounds__(CH_NB)
-k_chol_trsm(int n, double *__restrict__ A, int k, const LmState *st, int gate) {
-  if (!gate_open(st, gate) || st->lin_fail) return;
-  extern __shared__ double sh[];
-  double *L = sh, *X = sh + CH_NB * CH_LD;
-  const int j0 = k * CH_NB, m = min(CH_NB, n - j0);
-  const int r0 = (k + 1 + blockIdx.x) * CH_NB, t = threadIdx.x, row = r0 + t;
-  for (int r = 0; r < m; ++r)
-    if (t < m) L[r * CH_LD + t] = t <= r ? A[(size_t)(j0 + r) * n + j0 + t] : 0.0;
-  for (int r = 0; r < CH_NB; ++r)
-    if (r0 + r < n && t < m) X[r * CH_LD + t] = A[(size_t)(r0 + r) * n + j0 + t];
-  __syncthreads();
-  if (row < n) {
-    for (int j = 0; j < m; ++j) {
-      double s0 = X[t * CH_LD + j], s1 = 0.0, s2 = 0.0, s3 = 0.0;
-      int q = 0;
-      for (; q + 3 < j; q += 4) {  // four partial sums: the dependent-FMA chain is what bounds this loop
-        s0 -= X[t * CH_LD + q] * L[j * CH_LD + q];
-        s1 -= X[t * CH_LD + q + 1] * L[j * CH_LD + q + 1];
-        s2 -= X[t * CH_LD + q + 2] * L[j * CH_LD + q + 2];
-        s3 -= X[t * CH_LD + q + 3] * L[j * CH_LD + q + 3];
-      }
-      for (; q < j; ++q) s0 -= X[t * CH_LD + q] * L[j * CH_LD + q];
-      X[t * CH_LD + j] = ((s0 + s1) + (s2 + s3)) / L[j * CH_LD + j];
-    }
-  }
-  __syncthreads();
-  for (int r = 0; r < CH_NB; ++r)
-    if (r0 + r < n && t < m) A[(size_t)(r0 + r) * n + j0 + t] = X[r * CH_LD + t];
-}
 
 // trailing update with panel k, A_ij -= L_ik L_jk^T, of the lower-triangle tiles (i, j), kmap < j <= i (linear CTA index ->
 // tile), or, with single_col, of the tiles (i, kmap + 1) only.  kmap = k: the whole trailing matrix; the look-ahead
@@ -163,104 +97,6 @@ k_chol_update(int n, double *__restrict__ A, const double *__restrict__ Bsub, in
 // Also rejected: 128 threads with 8 x 4 outputs and both operand tiles transposed in shared memory (LDS.128 operands, 5 instead
 // of 8 shared-memory wavefronts per warp and inner-product step): 7.10 ms against 6.18 ms -- with 12 instead of 24 warps per
 // SM the kernel is bound by latency, not by the LSU / fp64 pipes.)
-// L z = b, L^T y = z, then the scatter of k_cholesky_solve.  Cooperative kernel (one CTA per SM): CTA 0 solves
-// the 64 x 64 diagonal tile in shared memory (column-oriented), a grid barrier publishes the 64 values, all CTAs
-// update the remaining right-hand side (92 MB of L per pass at n = 4798, spread over the grid).  The single-CTA
-// version of this step took 18 ms at n = 4798 -- 60 % of the exact LM step.
-__device__ __forceinline__ void chol_grid_barrier(unsigned int *bar, unsigned int &epoch) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    epoch += gridDim.x;
-    __threadfence();
-    atomicAdd(bar, 1u);
-    while (*((volatile unsigned int *)bar) < epoch) {
-    }
-    __threadfence();
-  }
-  __syncthreads();
-}
-__global__ void __launch_bounds__(256)
-k_chol_solve(int n, const double *__restrict__ A, const double *__restrict__ rhs, double *v /* scratch [n] */,
-             double *zt_g /* [64] */, unsigned int *bar, int n_cam, int n_free, const int32_t *__restrict__ cam_slot, int nk,
-             double *__restrict__ yc, double *__restrict__ yk, LmState *st, int gate) {
-  if (!gate_open(st, gate) || st->lin_fail) return;  // identical on every CTA
-  __shared__ double T[CH_NB * CH_LD];
-  __shared__ double zs[CH_NB];
-  const int tid = threadIdx.x, gtid = blockIdx.x * blockDim.x + tid, nthr = gridDim.x * blockDim.x;
-  const int nt = (n + CH_NB - 1) / CH_NB;
-  unsigned int epoch = 0;
-  for (int i = gtid; i < n; i += nthr) v[i] = rhs[i];
-  chol_grid_barrier(bar, epoch);
-  for (int pass = 0; pass < 2; ++pass) {
-    for (int kk = 0; kk < nt; ++kk) {
-      const int k = pass == 0 ? kk : nt - 1 - kk;
-      const int j0 = k * CH_NB, m = min(CH_NB, n - j0);
-      if (blockIdx.x == 0) {
-        for (int idx = tid; idx < m * CH_NB; idx += blockDim.x) {
-          const int r = idx >> 6, c = idx & 63;
-          if (c <= r && c < m) T[r * CH_LD + c] = A[(size_t)(j0 + r) * n + j0 + c];
-        }
-        if (tid < m) zs[tid] = __ldcg(v + j0 + tid);
-        __syncthreads();
-        if (pass == 0) {
-          for (int j = 0; j < m; ++j) {  // z_j, then eliminate it from the rows below
-            if (tid == 0) zs[j] = zs[j] / T[j * CH_LD + j];
-            __syncthreads();
-            if (tid > j && tid < m) zs[tid] -= T[tid * CH_LD + j] * zs[j];
-            __syncthreads();
-          }
-        } else {
-          for (int j = m - 1; j >= 0; --j) {  // y_j, then eliminate it from the rows above (L^T)
-            if (tid == 0) zs[j] = zs[j] / T[j * CH_LD + j];
-            __syncthreads();
-            if (tid < j) zs[tid] -= T[j * CH_LD + tid] * zs[j];
-            __syncthreads();
-          }
-        }
-        if (tid < m) {
-          zt_g[tid] = zs[tid];
-          v[j0 + tid] = zs[tid];
-        }
-      }
-      chol_grid_barrier(bar, epoch);
-      if (pass == 0) {
-        for (int i = j0 + m + gtid; i < n; i += nthr) {
-          const double *Li = A + (size_t)i * n + j0;
-          double s0 = __ldcg(v + i), s1 = 0.0;
-          int q = 0;
-          for (; q + 1 < m; q += 2) {
-            s0 -= Li[q] * __ldcg(zt_g + q);
-            s1 -= Li[q + 1] * __ldcg(zt_g + q + 1);
-          }
-          if (q < m) s0 -= Li[q] * __ldcg(zt_g + q);
-          v[i] = s0 + s1;
-        }
-      } else {
-        for (int i = gtid; i < j0; i += nthr) {
-          double s0 = __ldcg(v + i), s1 = 0.0;
-          int q = 0;
-          for (; q + 1 < m; q += 2) {
-            s0 -= A[(size_t)(j0 + q) * n + i] * __ldcg(zt_g + q);
-            s1 -= A[(size_t)(j0 + q + 1) * n + i] * __ldcg(zt_g + q + 1);
-          }
-          if (q < m) s0 -= A[(size_t)(j0 + q) * n + i] * __ldcg(zt_g + q);
-          v[i] = s0 + s1;
-        }
-      }
-      chol_grid_barrier(bar, epoch);
-    }
-  }
-  for (int c = gtid; c < n_cam; c += nthr) {
-    const int slot = cam_slot[c];
-#pragma unroll
-    for (int q = 0; q < 6; ++q) {
-      const double x = slot >= 0 ? __ldcg(v + 6 * slot + q) : 0.0;
-      if (!isfinite(x)) st->lin_fail = 1;
-      yc[6 * (size_t)c + q] = x;
-    }
-  }
-  if (gtid < 4) yk[gtid] = nk ? __ldcg(v + 6 * n_free + gtid) : 0.0;
-}
 
 // =====================================================================
 // Windowed problems (n <= BA_LDLT_MAX_N): the whole reduced-system solve in ONE CTA with the matrix in
@@ -273,7 +109,7 @@ k_chol_solve(int n, const double *__restrict__ A, const double *__restrict__ rhs
 //   * the back substitution L^T y = D^-1 w runs in warp 0 with register-resident w (lane l owns rows
 //     l, l+32, ...) and one shuffle broadcast per unknown instead of a CTA barrier.
 // The critical path per column is barrier + 1/d + one fused multiply-add (about 250 cycles) instead of a
-// j-long dependent FMA chain, a square root and two barriers (k_cholesky_solve: 135 us at n = 118).
+// j-long dependent FMA chain, a square root and two barriers (the removed single-CTA column Cholesky: 135 us at n = 118).
 // Every sum has a fixed order.  == the exact step of Ceres DENSE_SCHUR / SPARSE_SCHUR.
 // =====================================================================
 #define BA_LDLT_MAX_N 160
@@ -564,7 +400,7 @@ k_ldlt2_solve(int n, const double *__restrict__ Sg, const double *__restrict__ r
 //  * k_chol_potrf2: the register-resident L D L^T above applied to the m x m diagonal tile (m <= 64) with m extra
 //    rows holding the identity: row m + r ends up as column r of the unit factor's inverse, so the kernel writes
 //    both the Cholesky factor L = Lu D^1/2 (back into A) and L^-1 = D^-1/2 Lu^-1 (into Linv, dense 64 x 64, zeros above
-//    the diagonal) in ~64 barrier steps.  k_chol_potrf (left-looking, one thread per row): 45 us per tile.
+//    the diagonal) in ~64 barrier steps.  The removed left-looking version (one thread per row): 45 us per tile.
 //  * k_chol_trsm2: the panel X = A_ik L^-T as a 64 x 64 x 64 product with L^-1 (256 threads, 4 x 4 outputs each)
 //    instead of one thread per row walking a 64-step substitution with j-long dependent chains (63 us per launch).
 // =====================================================================

@@ -341,104 +341,13 @@ __device__ __forceinline__ void sp_reduce_scatter36(double (&acc)[36], int lane,
   cnt = (lane & 1) ? (c > 2 ? c - 2 : 0) : (c < 2 ? c : 2);
 }
 __device__ __forceinline__ ObsGeo load_geo_l1(const FPlanes &F, int i, double fx, double fy) { return obs_geo(ldg4(F.g + i), fx, fy); }
-// The round-2 kernel: every lane holds the 36 accumulators of the block (238 registers, 8 warps per SM).  Kept only to
-// alternate with k_sp_schur in one process (BA_SPS_SIMT=1, read at create); no solver selects it.
-__global__ void __launch_bounds__(BA_THREADS)
-k_sp_schur_simt(int n_blk, int n_cam, const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ lkeys,
-           const int32_t *__restrict__ gid, const unsigned long long *__restrict__ pairs, const int32_t *__restrict__ pair_pt,
-           FPlanes F, const double *__restrict__ geo, const double *__restrict__ intr, const double *__restrict__ Vs,
-           double *__restrict__ S, int *ticket, const LmState *st, int gate) {
-  if (!gate_open(st, gate)) return;
-  __shared__ int s_chunk, s_next;
-  const int lane = threadIdx.x & 31;
-  const double fx = ldg1(intr), fy = ldg1(intr + 1);
-  for (;;) {
-    __syncthreads();  // every warp is done with the previous chunk's counter
-    if (threadIdx.x == 0) {
-      s_chunk = atomicAdd(ticket, 1);
-      s_next = 0;
-    }
-    __syncthreads();
-    const int c0 = s_chunk * BA_SPS_CHUNK;
-    if (c0 >= n_blk) return;
-    const int cend = c0 + BA_SPS_CHUNK < n_blk ? c0 + BA_SPS_CHUNK : n_blk;
-    for (;;) {
-      int b = 0;
-      if (lane == 0) b = c0 + atomicAdd(&s_next, 1);
-      b = __shfl_sync(BA_FULL, b, 0);
-      if (b >= cend) break;
-      const unsigned long long key = lkeys[b];
-      const int ci = (int)(key / (unsigned long long)n_cam), cj = (int)(key % (unsigned long long)n_cam);
-      CamRec ri, rj;
-      load_camrec(geo, ci, ri);
-      load_camrec(geo, cj, rj);
-      double acc[36];
-#pragma unroll
-      for (int k = 0; k < 36; ++k) acc[k] = 0.0;
-      const int e1 = blk_ptr[b + 1];
-      int e = blk_ptr[b] + lane;
-      unsigned long long pr = 0;
-      int p = 0;
-      if (e < e1) {
-        pr = pairs[e];
-        p = __ldg(pair_pt + e);
-      }
-      while (e < e1) {
-        // the next trip's pair record is fetched before this trip's gathers are consumed
-        const int en = e + 32;
-        unsigned long long prn = 0;
-        int pn = 0;
-        if (en < e1) {
-          prn = pairs[en];
-          pn = __ldg(pair_pt + en);
-        }
-        const int oa = (int)(pr >> 32), ob = (int)(pr & 0xffffffffu);
-        double vs[6];
-#pragma unroll
-        for (int k = 0; k < 6; ++k) vs[k] = ldg1(Vs + 6 * (size_t)p + k);
-        const ObsGeo ga = load_geo_l1(F, oa, fx, fy), gb = load_geo_l1(F, ob, fx, fy);
-        double a0[6], a1[6], pa0[3], pa1[3], b0[6], b1[6], pb0[3], pb1[3];
-        sp_rows(ga, ri.R, a0, a1, pa0, pa1);
-        sp_rows(gb, rj.R, b0, b1, pb0, pb1);
-        double v0[3], v1[3];
-        sym3_mul(vs, pa0, v0);
-        sym3_mul(vs, pa1, v1);
-        const double m00 = v0[0] * pb0[0] + v0[1] * pb0[1] + v0[2] * pb0[2];
-        const double m01 = v0[0] * pb1[0] + v0[1] * pb1[1] + v0[2] * pb1[2];
-        const double m10 = v1[0] * pb0[0] + v1[1] * pb0[1] + v1[2] * pb0[2];
-        const double m11 = v1[0] * pb1[0] + v1[1] * pb1[1] + v1[2] * pb1[2];
-#pragma unroll
-        for (int c = 0; c < 6; ++c) {
-          const double h0 = m00 * b0[c] + m01 * b1[c], h1 = m10 * b0[c] + m11 * b1[c];
-#pragma unroll
-          // (kept as product-sum + add: an fma chain through acc -- two DFMA instead of DMUL + DFMA + DADD -- measured slower,
-          //  1.03 -> 1.13 ms: with two warps per scheduler the longer dependent chain per accumulator costs more than the instruction)
-          for (int r = 0; r < 6; ++r) acc[r * 6 + c] += a0[r] * h0 + a1[r] * h1;
-        }
-        pr = prn;
-        p = pn;
-        e = en;
-      }
-      // column scales (compile-time indices), then the warp sum as a recursive halving: every lane ends up with at most two
-      // COMPLETE entries of the block (37 shuffled doubles instead of the 180 of 36 butterflies; SASS of the butterfly
-      // version: 722 SHFL, a quarter of the instructions of a block with ~155 pairs).  Fixed tree: deterministic.
-#pragma unroll
-      for (int k = 0; k < 36; ++k) acc[k] *= ri.s[k / 6] * rj.s[k % 6];
-      int idx, cnt;
-      sp_reduce_scatter36(acc, lane, idx, cnt);
-      double *Sb = S + 36 * (size_t)gid[b] + idx;
-      if (cnt > 0) Sb[0] = -acc[0];  // k_sp_add_diag puts U on the diagonal blocks
-      if (cnt > 1) Sb[1] = -acc[1];
-    }
-  }
-}
 
 // Per block, S_b = -diag(s_i) [sum_pairs A_p^T H_p] diag(s_j) with A_p = [a0; a1] (2 x 6, rows of Jc in camera i) and
 // H_p = M_p [b0; b1] (2 x 6, the 2x2 core times the rows of Jc in camera j): a dense fp64 contraction of 6 x 2n by 2n x 6,
 // which is what mma.m8n8k4.f64 (DMMA) computes, two pairs per instruction, into an 8 x 8 accumulator (the 6 x 6 block
-// padded) of 2 registers per lane.  The warp walks the block's pairs in trips of 32: lane j stages pair e0 + j -- the
-// same gathers and arithmetic as k_sp_schur_simt -- as 12 double2 (a_t[r], h_t[r]) in its warp's slab, then the warp
-// runs ceil(n / 2) DMMA steps over the slab.  Lanes past the block's end stage zeros, so an odd tail's second pair adds 0.
+// padded) of 2 registers per lane.  The warp walks the block's pairs in trips of 32: lane j gathers pair e0 + j (the point's
+// Vs record and the geometry records of both observations), forms its rows a_t of A_p and h_t of H_p, and stages them as
+// 12 double2 (a_t[r], h_t[r]) in its warp's slab; then the warp runs ceil(n / 2) DMMA steps over the slab.  Lanes past the block's end stage zeros, so an odd tail's second pair adds 0.
 // Every block is summed in one fixed order (pair order, then the steps in order): bit-identical from run to run.
 // Slab: entry q = 6 t + r of pair p at q * BA_SPS_LD + p.  A lane stages with 12 stores of consecutive double2 across the
 // warp, and in step s lane (r = l >> 2, k = l & 3) reads entry (6 (k & 1) + r, 2 s + (k >> 1)) with one 16-byte load; with a
@@ -609,46 +518,6 @@ __device__ __forceinline__ void bsr_row(int r, int lane, const int32_t *__restri
 }
 __device__ __forceinline__ double pick6(const double a[6], int k) {
   return k == 0 ? a[0] : k == 1 ? a[1] : k == 2 ? a[2] : k == 3 ? a[3] : k == 4 ? a[4] : a[5];
-}
-
-// Experimental mapping (BA_SPMV6=1; measurement for the next step of the persistent PCG, DESIGN section 10): a block is shared
-// by SIX lanes -- lane a of a group forms component a of (S_ij x_j), reading one 48-byte block row (or one strided column when
-// the block is used transposed) -- and five groups walk the row's entries.  ~40 registers instead of ~230, so six times as many
-// warps per SM keep loads in flight; the lanes of the same component are added in group order (fixed).
-__global__ void __launch_bounds__(BA_THREADS)
-k_bsr_spmv6(int n_cam, const int32_t *__restrict__ ent_ptr, const int2 *__restrict__ ent, const double *__restrict__ S,
-            const double *__restrict__ x, double *__restrict__ y, const LmState *st, int gate) {
-  if (!gate_open(st, gate)) return;
-  const int r = (blockIdx.x * BA_THREADS + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-  if (r >= n_cam) return;
-  const int g = lane / 6, a = lane - 6 * g;
-  const int b0 = __ldg(ent_ptr + r), e0 = __ldg(ent_ptr + r + 1);
-  double acc = 0.0;
-  if (g < 5) {
-#pragma unroll 4
-    for (int e = b0 + g; e < e0; e += 5) {
-      const int2 en = __ldg(ent + e);
-      const double *B = S + 36 * (size_t)((uint32_t)en.x & 0x7fffffffu);
-      double xv[6], m[6];
-      load6(x + 6 * (size_t)en.y, xv);
-      if ((uint32_t)en.x & 0x80000000u) {
-#pragma unroll
-        for (int k = 0; k < 6; ++k) m[k] = __ldg(B + 6 * k + a);
-      } else {
-        const double2 *row = reinterpret_cast<const double2 *>(B + 6 * a);
-        const double2 m0 = __ldg(row), m1 = __ldg(row + 1), m2 = __ldg(row + 2);
-        m[0] = m0.x; m[1] = m0.y; m[2] = m1.x; m[3] = m1.y; m[4] = m2.x; m[5] = m2.y;
-      }
-      double sdot = 0.0;
-#pragma unroll
-      for (int k = 0; k < 6; ++k) sdot += m[k] * xv[k];
-      acc += sdot;
-    }
-  }
-  double sum = acc;
-#pragma unroll
-  for (int gg = 1; gg < 5; ++gg) sum += __shfl_sync(BA_FULL, acc, (lane + 6 * gg) & 31);
-  if (lane < 6) y[6 * (size_t)r + lane] = sum;
 }
 
 __global__ void __launch_bounds__(BA_THREADS)

@@ -3,8 +3,9 @@
 // (headers/BundleAdjustmentConfig.h:62; ceres::Solve at src/OptimizationUtils.cpp:300) -- the explicit block-sparse
 // S of ba_kernels_sparse.cuh factorised exactly instead of handed to PCG.
 //
-// Supernodal multifrontal Cholesky over the nested-dissection tree built on the host (ba_sparse_symbolic.h):
-//   * ONE thread block per tree node, one launch per tree level (children before parents); nodes of a level are independent.
+// Supernodal multifrontal Cholesky over the nested-dissection tree built on the host (ba_sparse_symbolic.h), as ONE persistent
+// launch (k_spchol_tree, below) that works through a queue of factor, update and solve items with completion counters:
+//   * ONE thread block per factor item (a tree node); a node starts as soon as its children's update matrices are done.
 //   * A node's FRONT PANEL ((own + border) x own cameras, dense, scalar column-major, leading dimension LD = 6 (m + nb))
 //     lives in shared memory for the whole elimination of its m own cameras: assembled from the stored blocks of S
 //     (+ LM damping on the diagonal) minus the children's update matrices (extend-add through the host-built index maps),
@@ -19,10 +20,11 @@
 //     is solved between factorisation and backward substitution (k_spb_reduce / k_spb_solve), and the backward
 //     substitution solves L^T y_c = z - Z y_k.  The symbolic phase, the tree and the supernodes are the same for R = 1, 5.
 //   * The panel goes to HBM/L2 for the backward substitution; the node's update matrix U = L_B L_B^T (+ what its children
-//     pass through) -- two thirds of the multiply-adds, no dependent chain -- is formed by a second launch per level with
-//     several thread blocks per node (k_spchol_update), for the parent's extend-add.
-// Backward substitution: one launch per level, parents before children; L_OO and the stored inverses of the pivot blocks
-// come back into shared memory, the border product is a warp-per-column reduction over the panel in L2.
+//     pass through) -- two thirds of the multiply-adds, no dependent chain -- is formed by several update items per node
+//     (spc_update_node), for the parent's extend-add.
+// Backward substitution: parents before children (solve items of the tree; k_spchol_solve runs one tree level per launch for
+// the covariance's border columns); L_OO and the stored inverses of the pivot blocks come back into shared memory, the
+// border product is a warp-per-column reduction over the panel in L2.
 // Every sum has a fixed order: results are bit-identical from run to run and across ranks.
 #pragma once
 #include "ba_kernels_sparse.cuh"
@@ -168,12 +170,12 @@ __device__ __forceinline__ void spc_wait_ge(const int *flag, int want) {
     __nanosleep(64);
   }
 }
-// (udone / tiles: completion counters of the persistent tree kernel -- the node waits for its children's update matrices only
-//  AFTER it has assembled its stored blocks of S, which do not depend on them; nullptr: one launch per level, nothing to wait for)
+// (udone / tiles: completion counters of k_spchol_tree -- the node waits for its children's update matrices only AFTER it has
+//  assembled its stored blocks of S, which do not depend on them)
 // NR right-hand-side rows (1: b; 5: b and the four border columns), row r of the own cameras at zf[r * C6 ..]
 template <int NR>
 __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool prof_block, LmState *st, double *spc_sm,
-                                                const int *udone = nullptr, const int32_t *tiles = nullptr) {
+                                                const int *udone, const int32_t *tiles) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
   const int k0 = N[SPN_K0], m = N[SPN_M], nb = N[SPN_NB];
@@ -215,7 +217,7 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
       P[(size_t)(6 * en.z + c6) * LD + 6 * en.y + r6] = v;
     }
   }
-  if (udone && tid == 0)
+  if (tid == 0)
     for (int ci = 0; ci < N[SPN_NCHILD]; ++ci) {
       const int ch = a.children[N[SPN_CHILD] + ci];
       spc_wait_ge(udone + ch, tiles[ch]);
@@ -224,7 +226,7 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
   SPC_TICK(0)
   // ---- phase 1b: extend-add of the children (one after the other: fixed order; inside a child the map is injective).
   //      rel is ascending, so the child's border cameras that are OWN cameras of this node come first: only those block
-  //      columns land in the panel (the rest of the child's update matrix passes through to this node's, k_spchol_update)
+  //      columns land in the panel (the rest of the child's update matrix passes through to this node's, spc_update_node)
   for (int ci = 0; ci < N[SPN_NCHILD]; ++ci) {
     const int ch = a.children[N[SPN_CHILD] + ci];
     const int32_t *Cn = a.node + (size_t)ch * SPSYM_NODE_INTS;
@@ -423,23 +425,15 @@ __device__ __forceinline__ void spc_factor_node(const SpChol &a, int id, bool pr
   SPC_TICK(3)
   if (a.prof && prof_block && tid == 0) a.prof[4] += 1;
 }
-template <int NR>
-__global__ void __launch_bounds__(SPC_THREADS, 1)
-k_spchol_factor(SpChol a, int lvl_first, LmState *st, int gate) {
-  if (!gate_open(st, gate)) return;
-  extern __shared__ __align__(16) double spc_sm[];
-  spc_factor_node<NR>(a, a.level_nodes[lvl_first + blockIdx.x], blockIdx.x == 0, st, spc_sm);
-}
 
-// Update matrix of the nodes of one level, after their panels are factorised: U = L_B L_B^T + what the children pass through
-// (block lower triangle, full diagonal blocks) and the right-hand side update ru = L_B z + children.  This is two thirds of a
-// node's multiply-adds and has no dependent chain, so it runs as its own launch with `tiles` thread blocks per node: the upper
-// levels of the tree have fewer nodes than the GPU has SMs.  Every block loads the node's border rows of the panel (L2-resident,
-// just written) into shared memory and takes every tiles-th chunk of the 3 x 6 output pieces.
-#define SPU_THREADS 256
+// Update matrix of a node, after its panel is factorised: U = L_B L_B^T + what the children pass through (block lower
+// triangle, full diagonal blocks) and the right-hand side update ru = L_B z + children.  This is two thirds of a node's
+// multiply-adds and has no dependent chain, so it is split into `tiles` items per node: the upper levels of the tree have
+// fewer nodes than the GPU has SMs.  Every item loads the node's border rows of the panel (L2-resident, just written) into
+// shared memory and takes every tiles-th chunk of the 3 x 6 output pieces.
 inline size_t spc_update_smem(int m, int nb, int R = 1) { return ((size_t)36 * nb * m + 6 * m * R + 8) * 8; }
-// tile `tile` of `tiles` of the update matrix of node `id`, by the calling thread block (NT threads); NR right-hand-side rows
-template <int NT, int NR>
+// tile `tile` of `tiles` of the update matrix of node `id`, by the calling thread block; NR right-hand-side rows
+template <int NR>
 __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int tile, int tiles, double *spc_sm) {
   const int tid = threadIdx.x;
   const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
@@ -451,13 +445,13 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
   {
     const double *Pg = a.panel + 36 * spc_off(N, SPN_PANEL_LO) + C6;
 #pragma unroll 8
-    for (int idx = tid; idx < NB6 * C6; idx += NT) {
+    for (int idx = tid; idx < NB6 * C6; idx += SPC_THREADS) {
       const int c = idx / NB6, r = idx - c * NB6;
       LB[idx] = __ldcg(Pg + (size_t)c * LD + r);  // (L2: written by another thread block of this or the previous launch)
     }
-    for (int i = tid; i < C6; i += NT) zf[i] = __ldcg(a.z + 6 * (size_t)k0 + i);
+    for (int i = tid; i < C6; i += SPC_THREADS) zf[i] = __ldcg(a.z + 6 * (size_t)k0 + i);
     if (NR > 1)
-      for (int i = tid; i < (NR - 1) * C6; i += NT) {
+      for (int i = tid; i < (NR - 1) * C6; i += SPC_THREADS) {
         const int q = i / C6, j = i - q * C6;
         zf[(q + 1) * C6 + j] = __ldcg(a.Zb + 4 * (6 * (size_t)k0 + j) + q);
       }
@@ -466,7 +460,7 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
   double *Ug = a.U + 36 * spc_off(N, SPN_U_LO);
   const int n_items = nb * (nb + 1);
   const int nch = N[SPN_NCHILD];
-  for (int idx = tile * NT + tid; idx < n_items; idx += tiles * NT) {
+  for (int idx = tile * SPC_THREADS + tid; idx < n_items; idx += tiles * SPC_THREADS) {
     int i, j;
     spc_tri(idx >> 1, i, j);
     const int h = idx & 1;
@@ -510,7 +504,7 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
   }
   // rhs updates: row r of the node at ru[6 NR bord + r NB6 ..]
   double *rug = a.ru + 6 * NR * (size_t)N[SPN_BORD];
-  for (int idx = tile * NT + tid; idx < NR * NB6; idx += tiles * NT) {
+  for (int idx = tile * SPC_THREADS + tid; idx < NR * NB6; idx += tiles * SPC_THREADS) {
     const int r = idx / NB6, e = idx - r * NB6;
     const double *zr = zf + r * C6;
     double s = 0.0;
@@ -523,13 +517,6 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
     }
     rug[idx] = s;
   }
-}
-template <int NR>
-__global__ void __launch_bounds__(SPU_THREADS, 1)
-k_spchol_update(SpChol a, int lvl_first, int tiles, LmState *st, int gate) {
-  if (!gate_open(st, gate)) return;
-  extern __shared__ __align__(16) double spc_sm[];
-  spc_update_node<SPU_THREADS, NR>(a, a.level_nodes[lvl_first + blockIdx.x / tiles], blockIdx.x % tiles, tiles, spc_sm);
 }
 
 // backward substitution of one tree level (parents are done): y_O = L_OO^-T (z_O - L_BO^T y_B)
@@ -654,7 +641,7 @@ k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
     } else if (q.y >= 0) {
       if (tid == 0) spc_wait_ge(t.fdone + id, 1);
       __syncthreads();
-      spc_update_node<SPC_THREADS, NR>(a, id, q.y, t.tiles[id], spc_sm);
+      spc_update_node<NR>(a, id, q.y, t.tiles[id], spc_sm);
       __syncthreads();
       if (tid == 0) {
         __threadfence();

@@ -1,12 +1,11 @@
 #!/bin/bash
-# N ranks on one box: multi-GPU parity tests, then the cfg5 bench line with the distributed and the replicated factorisation
+# N ranks on one box: multi-GPU parity tests, then the cfg5 bench line with the distributed factorisation
 cd "$GRAFT_REPO_ROOT" || exit 1
 mkdir -p gpurun_out
 N=$(nvidia-smi -L | wc -l)
 timeout 400 python -m pytest tests/test_gpu_multi.py -m gpu -x -q -k "${MULTI_K:-sparse or auto or implicit}" > gpurun_out/r2_multi_tests_n${N}.log 2>&1; echo rc=$? >> gpurun_out/r2_multi_tests_n${N}.log
 tail -n 5 gpurun_out/r2_multi_tests_n${N}.log
-for mode in ${MODES:-dist repl}; do
-  [ $mode = repl ] && export BA_SPCHOL_REPLICATED=1
+for mode in ${MODES:-dist}; do
   BA_SPCHOL_DEBUG=1 timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 2954$N bench.py --gpus $N --steps 20 --warmup 5 > gpurun_out/r2_bench_cfg5_n${N}_$mode.log 2>&1
   echo "N=$N $mode rc=$?"
   grep "^\[spchol\]" gpurun_out/r2_bench_cfg5_n${N}_$mode.log | head -n 2

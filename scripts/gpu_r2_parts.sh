@@ -1,6 +1,5 @@
 #!/bin/bash
-# partitioned sparse Cholesky on one GPU: bit-identity tests, then what ONE rank of an N-rank run would execute
-# (BA_SPCHOL_ONLY_PART=0: part 0's subtrees + top part + substitution; results are meaningless, the time is the point)
+# partitioned sparse Cholesky on one GPU: bit-identity tests, then the linear solve with N parts run one after the other
 cd "$GRAFT_REPO_ROOT" || exit 1
 mkdir -p gpurun_out
 timeout 300 python -m pytest tests/test_gpu_parity.py -m gpu -x -q -k "spchol" > gpurun_out/r2_parts_tests.log 2>&1; echo rc=$? >> gpurun_out/r2_parts_tests.log
@@ -8,8 +7,6 @@ tail -n 4 gpurun_out/r2_parts_tests.log
 {
 for n in 2 4 8; do
   echo "parts $n (all parts on this GPU)"; BA_SPCHOL_DEBUG=1 BA_SPCHOL_PARTS=$n timeout 120 python scripts/phase_probe.py 5 10 4 2>&1 | tail -n 2
-  echo "parts $n, part 0 only"; BA_SPCHOL_PARTS=$n BA_SPCHOL_ONLY_PART=0 timeout 120 python scripts/phase_probe.py 5 10 4 2>&1 | tail -n 1
-  echo "parts $n, part 1 only"; BA_SPCHOL_PARTS=$n BA_SPCHOL_ONLY_PART=1 timeout 120 python scripts/phase_probe.py 5 10 4 2>&1 | tail -n 1
 done
 } > gpurun_out/r2_parts_probe.log 2>&1
 cat gpurun_out/r2_parts_probe.log

@@ -238,14 +238,15 @@ def test_solve_explicit_window20_ref(solver_cache):
     assert summ.reduced_dim == 6 * 19 + 4 and summ.solver_used == ba_b200.capi.BA_SOLVER_EXPLICIT_CHOLESKY
 
 
-@pytest.mark.parametrize("n_kf", [28, 33, 43, 60, 200])
+@pytest.mark.parametrize("n_kf", [27, 28, 33, 43, 60, 200])
 def test_solve_explicit_blocked_cholesky_ref(n_kf, solver_cache):
     """The reference's global optimisation (windowOptimize over ALL keyframes, REF cost with free intrinsics,
-    src/main.cpp:179-182) beyond the shared-memory Cholesky (n > 160): reduced dimension 6 (n_kf - 1) + 4 = 166 (three
-    tiles, the shortest look-ahead schedule), 196 (last tile of 4 rows), 256 (full tiles only), 358 / 1198 (ragged last
-    tile) -> the blocked dense Cholesky (ba_kernels_chol.cuh: fused diagonal kernel, three-stream look-ahead, flag-in-data
-    substitution).  Exact step: lock step with the oracle's dense Schur at the north-star tolerance 1e-8 (measured worst
-    per-iteration difference over these sizes: 4.6e-12 relative, profiles/r02_chol_tolerance.txt)."""
+    src/main.cpp:179-182) beyond the register-resident L D L^T (n > 159): reduced dimension 6 (n_kf - 1) + 4 = 160 -> the
+    shared-memory L D L^T (k_ldlt_solve, which runs at this size only); 166 (three tiles, the shortest look-ahead schedule),
+    196 (last tile of 4 rows), 256 (full tiles only), 358 / 1198 (ragged last tile) -> the blocked dense Cholesky
+    (ba_kernels_chol.cuh: fused diagonal kernel, three-stream look-ahead, flag-in-data substitution).  Exact step: lock step
+    with the oracle's dense Schur at the north-star tolerance 1e-8 (measured worst per-iteration difference over the blocked
+    sizes: 4.6e-12 relative, profiles/r02_chol_tolerance.txt)."""
     seq = syn.make_tum_sequence(n_kf, 30 * n_kf, 180 * n_kf, seed=21)
     p = syn.window_problem(seq, 0, n_kf - 1).problem
     summ, _ = _compare_solve(p, "REF", 0, 6, solver_cache)
@@ -256,9 +257,7 @@ def test_solve_explicit_blocked_cholesky_ref(n_kf, solver_cache):
 def test_blocked_cholesky_schedules_are_bit_identical(monkeypatch, solver_cache):
     """The three-stream look-ahead schedule (fused diagonal kernel, side buffer for the panel tile below the diagonal,
     flag-in-data substitution) performs the same operations per matrix entry in the same order as the plain right-looking
-    sequence on one stream (BA_NO_LOOKAHEAD=1): every LM iteration's cost and the final state agree bit for bit.
-    Also exercises the first-version kernels (BA_LEGACY_CHOL: left-looking diagonal tile, grid-barrier substitution)
-    against them within round-off."""
+    sequence on one stream (BA_NO_LOOKAHEAD=1): every LM iteration's cost and the final state agree bit for bit."""
     n_kf = 50
     seq = syn.make_tum_sequence(n_kf, 30 * n_kf, 180 * n_kf, seed=5)
     p = syn.window_problem(seq, 0, n_kf - 1).problem   # n = 298: five tiles, ragged last one
@@ -279,10 +278,6 @@ def test_blocked_cholesky_schedules_are_bit_identical(monkeypatch, solver_cache)
     assert a[0].reduced_dim == 6 * (n_kf - 1) + 4 and a[0].num_iterations == b[0].num_iterations >= 3
     assert a[4] == b[4] and a[0].final_cost == b[0].final_cost
     assert np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2]) and np.array_equal(a[3], b[3])
-    monkeypatch.setenv("BA_LEGACY_CHOL", "1")
-    c = run()
-    assert abs(c[0].final_cost - a[0].final_cost) <= 1e-9 * a[0].final_cost
-    assert np.max(np.abs(c[1] - a[1])) < 1e-8
 
 
 def test_solve_to_convergence_ref(solver_cache):
@@ -652,21 +647,6 @@ def test_window_graph_and_device_pairs_are_bit_identical(name):
         assert other[0].final_cost == base[0].final_cost, env
         assert np.array_equal(other[1], base[1]) and np.array_equal(other[2], base[2]) and np.array_equal(other[3], base[3]), env
         assert [t["cost"] for t in other[4]] == [t["cost"] for t in base[4]], env
-
-
-@pytest.mark.parametrize("name", ["cfg1", "window20"])
-def test_window_solver_variants_agree(name):
-    """Register-resident L D L^T (in force) vs the shared-memory L D L^T vs the left-looking Cholesky: three exact
-    solves of the same reduced system; LM traces agree to round-off amplified by the conditioning."""
-    p = _problem(name)
-    base = _explicit_run(p)
-    for mode in ("1", "2"):
-        other = _explicit_run(p, {"BA_LEGACY_CHOL": mode})
-        assert other[0].num_iterations == base[0].num_iterations
-        assert other[0].num_successful == base[0].num_successful
-        assert abs(other[0].final_cost - base[0].final_cost) <= 1e-9 * base[0].final_cost, mode
-        dt, dr = pose_err(other[1], base[1])
-        assert dt < 1e-7 and dr < 1e-7, (mode, dt, dr)
 
 
 def test_window_reupload_updates_graph():

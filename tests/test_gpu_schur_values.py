@@ -1,8 +1,5 @@
 """Values of the block-sparse Schur complement (k_sp_schur, fp64 DMMA): blocks whose pair lists end anywhere in a trip of
-32 pairs and in a DMMA step of two, against the oracle's product and a dense float64 numpy S; bit identity from run to run;
-agreement with the per-lane-accumulator kernel (BA_SPS_SIMT=1)."""
-import os
-
+32 pairs and in a DMMA step of two, against the oracle's product and a dense float64 numpy S; bit identity from run to run."""
 import numpy as np
 import pytest
 
@@ -57,15 +54,6 @@ def dense_schur(p, out):
     return Hcc - np.einsum("pij,pjk->ik", W, np.linalg.solve(V, W.transpose(0, 2, 1)))
 
 
-def make_solver(simt=False, **kw):
-    if simt:
-        os.environ["BA_SPS_SIMT"] = "1"
-    try:
-        return ba_b200.GpuSolver(**kw)
-    finally:
-        os.environ.pop("BA_SPS_SIMT", None)
-
-
 def probe(s, n, radius):
     return np.stack([s.schur_matvec(radius, np.eye(n)[k]) for k in range(n)], axis=1)
 
@@ -74,7 +62,7 @@ def probe(s, n, radius):
 def test_pair_counts_vs_oracle(diag_only):
     p = pair_problem(3, diag_only)
     g, o = mode_opts("NS", solver=3)
-    s = make_solver(**g)
+    s = ba_b200.GpuSolver(**g)
     try:
         s.upload(p)
         rng = np.random.default_rng(7)
@@ -92,7 +80,7 @@ def test_every_block_vs_dense_numpy():
     here (two-view points with short baselines amplify the damping of V): radius 1e16 puts it below 1e-13."""
     p = pair_problem(5)
     g, _ = mode_opts("NS", solver=3)
-    s = make_solver(**g)
+    s = ba_b200.GpuSolver(**g)
     try:
         s.upload(p)
         A = probe(s, 6 * p.n_cam, 1e16)
@@ -116,7 +104,7 @@ def test_same_bits_on_repeat():
     runs = []
     for _ in range(2):
         g, _ = mode_opts("NS", solver=4, max_num_iterations=6)
-        s = make_solver(**g)
+        s = ba_b200.GpuSolver(**g)
         try:
             s.upload(p)
             x = np.random.default_rng(1).normal(size=6 * p.n_cam)
@@ -129,54 +117,3 @@ def test_same_bits_on_repeat():
     assert np.array_equal(y1, y2)
     assert c1 == c2 and t1 == t2
     assert np.array_equal(p1, p2)
-
-
-@pytest.mark.parametrize("name", ["pairs", "cfg3"])
-def test_dmma_matches_simt(name):
-    """Same matrix from both kernels to 1e-12 of each block's norm (different summation order, fp64 both)."""
-    if name == "pairs":
-        p, n_probe = pair_problem(11, diag_only=True), None
-    else:
-        p, n_probe = syn.make_config(3, scale=0.05), 48
-    g, _ = mode_opts("NS", solver=3)
-    mats = []
-    for simt in (True, False):
-        s = make_solver(simt=simt, **g)
-        try:
-            s.upload(p)
-            n = 6 * p.n_cam
-            cols = range(n) if n_probe is None else range(min(n, n_probe))
-            mats.append(np.stack([s.schur_matvec(1e4, np.eye(n)[k]) for k in cols], axis=1))
-        finally:
-            s.close()
-    a, b = mats
-    nc = a.shape[1] // 6
-    for i in range(p.n_cam):
-        for j in range(nc):
-            ba, bb = a[6 * i:6 * i + 6, 6 * j:6 * j + 6], b[6 * i:6 * i + 6, 6 * j:6 * j + 6]
-            nrm = np.max(np.abs(ba))
-            # the diagonal-only camera sees single-view points: U and W V^-1 W^T nearly cancel in its block
-            # (block norm 0.034, difference 3.7e-14 on a B200)
-            tol = 1e-11 if name == "pairs" and i == j == 9 else 1e-12
-            assert np.max(np.abs(ba - bb)) <= tol * nrm, (i, j)
-
-
-def test_dmma_matches_simt_solve():
-    """cfg3 (at --scale 0.1): the exact sparse LM solve with either kernel, same accept sequence, cost to 1e-10."""
-    p = syn.make_config(3, scale=0.1)
-    res = []
-    for simt in (True, False):
-        g, _ = mode_opts("NS", solver=4, max_num_iterations=8, function_tolerance=0.0, parameter_tolerance=0.0,
-                         gradient_tolerance=0.0)
-        s = make_solver(simt=simt, **g)
-        try:
-            s.upload(p)
-            summ = s.solve()
-            res.append((summ.final_cost, [t["step_is_successful"] for t in s.trace()], s.download()[0], summ.solver_used))
-        finally:
-            s.close()
-    (c1, a1, p1, u1), (c2, a2, p2, u2) = res
-    assert u1 == u2 == ba_b200.capi.BA_SOLVER_SPARSE_SCHUR_CHOLESKY
-    assert a1 == a2
-    assert abs(c1 - c2) <= 1e-10 * c1
-    assert np.max(np.abs(p1 - p2)) < 1e-8
