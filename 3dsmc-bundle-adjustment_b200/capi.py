@@ -20,6 +20,7 @@ BA_OK, BA_ERR_INVALID, BA_ERR_CUDA, BA_ERR_STATE, BA_ERR_UNSUPPORTED, BA_ERR_NUM
 BA_SOLVER_AUTO, BA_SOLVER_EXPLICIT_CHOLESKY, BA_SOLVER_IMPLICIT_PCG, BA_SOLVER_SPARSE_SCHUR_PCG = 0, 1, 2, 3
 BA_SOLVER_SPARSE_SCHUR_CHOLESKY = 4
 BA_COV_MIN_PIVOT_RATIO = 1e-9  # ba_gpu_covariance's relative pivot test (include/ba_gpu.h)
+BA_COV_CAMERA, BA_COV_POINT, BA_COV_INTRINSICS = 0, 1, 2  # ba_cov_block kinds
 BA_JAC_AUTO, BA_JAC_PLANES, BA_JAC_FACTORED, BA_JAC_TILED = 0, 1, 2, 3
 BA_KERNEL_LINEARIZE, BA_KERNEL_SCHUR_MATVEC, BA_KERNEL_SCHUR_PASS1, BA_KERNEL_SCHUR_PASS2 = 0, 1, 2, 3
 TERMINATION = {0: "NO_CONVERGENCE", 1: "GRADIENT", 2: "PARAMETER", 3: "FUNCTION", 4: "MIN_RADIUS", 5: "FAILURE"}
@@ -45,6 +46,11 @@ class Options(C.Structure):
     ]
 
 
+class CovBlock(C.Structure):
+    """== ba_cov_block: (kind, index) of a parameter block for ba_gpu_covariance_blocks."""
+    _fields_ = [("kind", C.c_int32), ("index", C.c_int32)]
+
+
 class IterRecord(C.Structure):
     _fields_ = [
         ("iteration", C.c_int32), ("step_is_valid", C.c_int32), ("step_is_successful", C.c_int32),
@@ -68,7 +74,8 @@ EXPORTS = [
     "ba_gpu_upload", "ba_gpu_solve", "ba_gpu_get_trace", "ba_gpu_download", "ba_gpu_eval", "ba_gpu_get_indices",
     "ba_gpu_schur_matvec", "ba_gpu_se3_plus", "ba_gpu_time_kernel", "ba_gpu_launch_count", "ba_gpu_comm_unique_id",
     "ba_gpu_comm_init", "ba_gpu_jacobian_store_used", "ba_gpu_sparse_stats", "ba_gpu_backproject",
-    "ba_gpu_schur_solve", "ba_gpu_spchol_info", "ba_gpu_covariance", "ba_gpu_covariance_pivots", "ba_gpu_phase_times", "ba_gpu_phase_name",
+    "ba_gpu_schur_solve", "ba_gpu_spchol_info", "ba_gpu_covariance", "ba_gpu_covariance_blocks",
+    "ba_gpu_covariance_pivots", "ba_gpu_phase_times", "ba_gpu_phase_name",
     "ba_store_create", "ba_store_destroy", "ba_store_clear", "ba_store_set_keyframe", "ba_store_set_keyframes", "ba_store_set_poses", "ba_store_set_landmarks",
     "ba_store_window_solve",
     "ba_sparse_symbolic_create", "ba_sparse_symbolic_info", "ba_sparse_symbolic_get", "ba_sparse_symbolic_destroy",
@@ -121,6 +128,7 @@ def load():
     L.ba_gpu_spchol_info.argtypes = [vp, C.POINTER(C.c_int64)]
     L.ba_gpu_covariance.argtypes = [vp, c_double_p, c_double_p, c_double_p, c_double_p, C.c_int32, c_int32_p, c_int32_p,
                                     c_double_p]
+    L.ba_gpu_covariance_blocks.argtypes = [vp, C.c_int32, C.POINTER(CovBlock), C.POINTER(CovBlock), c_double_p]
     L.ba_gpu_covariance_pivots.argtypes = [vp, c_double_p]
     L.ba_store_create.argtypes = [vp, C.POINTER(vp)]
     L.ba_store_destroy.argtypes = [vp]

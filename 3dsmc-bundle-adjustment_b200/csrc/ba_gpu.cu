@@ -15,6 +15,7 @@
 #include "ba_kernels_chol.cuh"
 #include "ba_kernels_spchol.cuh"
 #include "ba_kernels_selinv.cuh"
+#include "ba_kernels_covblocks.cuh"
 #include "ba_kernels_store.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -184,6 +185,9 @@ struct ba_gpu_ctx {
   size_t cov_smem = 0;
   Buf cov_Y, cov_X, cov_zq, cov_yscr, cov_Tinv, cov_S, cov_ck, cov_brec, cov_pos, cov_queue, cov_tiles, cov_cnt, cov_cam, cov_ci,
       cov_pt, cov_pin, cov_pout, cov_bad, cov_piv;
+  // ba_gpu_covariance_blocks (ba_kernels_covblocks.cuh), per pass: path entries, forward items, source paths, camera -> source,
+  // requests and their output offsets, F and the carried border rows; per call: the requested points' observations, outputs
+  Buf cb_ent, cb_items, cb_src, cb_cam_src, cb_req, cb_off, cb_F, cb_carry, cb_pts, cb_rng, cb_obs, cb_out;
   double cov_ratio[2] = {0.0, 0.0};  // smallest pivot / diagonal of the last covariance call: cameras, intrinsics (0: none)
   // phase timing of the large-problem solvers: CUDA events on the solver stream at the phase boundaries of every LM
   // iteration of the last solve (a few dozen event records per iteration: < 0.1 % of a multi-millisecond iteration)
@@ -2903,21 +2907,23 @@ static int cov_prepare(ba_gpu_ctx *ctx) {
   return 0;
 }
 
-extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
-                                 int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs) {
-  if (!ctx) return BA_ERR_INVALID;
-  if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_covariance before ba_gpu_upload");
-  if (ctx->n_ranks > 1) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance is single-GPU");
+// preconditions of the covariance calls (`who`: the entry point, for the messages)
+static int cov_check(ba_gpu_ctx *ctx, const char *who) {
+  if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "%s before ba_gpu_upload", who);
+  if (ctx->n_ranks > 1) return fail(ctx, BA_ERR_UNSUPPORTED, "%s is single-GPU", who);
   if (!ctx->depth)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance needs the depth prior: without it (%s cost) the scale is free and the "
-                "Gauss-Newton Hessian is singular", ctx->nk ? "INTR" : "NS");
+    return fail(ctx, BA_ERR_UNSUPPORTED, "%s needs the depth prior: without it (%s cost) the scale is free and the "
+                "Gauss-Newton Hessian is singular", who, ctx->nk ? "INTR" : "NS");
   if (ctx->fixed_cam < 0)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance needs a fixed camera: with fixed_cam < 0 the gauge is free and the "
-                "Gauss-Newton Hessian is singular");
-  if (n_pairs < 0 || (n_pairs > 0 && (!cam_a || !cam_b || !cov_pairs))) return fail(ctx, BA_ERR_INVALID, "bad camera pair list");
-  for (int i = 0; i < n_pairs; ++i)
-    if (cam_a[i] < 0 || cam_a[i] >= ctx->n_cam || cam_b[i] < 0 || cam_b[i] >= ctx->n_cam)
-      return fail(ctx, BA_ERR_INVALID, "camera pair %d (%d, %d) out of range", i, cam_a[i], cam_b[i]);
+    return fail(ctx, BA_ERR_UNSUPPORTED, "%s needs a fixed camera: with fixed_cam < 0 the gauge is free and the "
+                "Gauss-Newton Hessian is singular", who);
+  return 0;
+}
+
+// first half of both covariance calls: relinearisation at radius +inf, the point inverses, W, the border partials, the values
+// of S, the factorisation with the relative pivot test, T^-1 and X = L^-T Z (*X = nullptr with constant intrinsics).  The
+// panels and the stored pivot inverses hold the factor afterwards.
+static int cov_factor(ba_gpu_ctx *ctx, const double **Xout) {
   CK(cudaSetDevice(ctx->device));
   ctx->pdl = false;
   ctx->cur = ctx->stream;
@@ -2981,6 +2987,53 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
     }
     X = P<double>(ctx->cov_X);
   }
+  *Xout = X;
+  return 0;
+}
+
+// after the launches of a covariance call: the failure flags and the pivot test (the ratios are kept for
+// ba_gpu_covariance_pivots)
+static int cov_status(ba_gpu_ctx *ctx, const char *who) {
+  int rc;
+  if ((rc = poll_state(ctx))) return rc;
+  CK(cudaGetLastError());
+  if (ctx->h_st->eval_fail) return fail(ctx, BA_ERR_NUMERIC, "%s: non-finite residual or Jacobian", who);
+  CovPivots piv;
+  CK(cudaMemcpy(&piv, ctx->cov_piv.p, sizeof(piv), cudaMemcpyDeviceToHost));
+  memcpy(&ctx->cov_ratio[0], &piv.min_cam, 8);
+  memcpy(&ctx->cov_ratio[1], &piv.min_border, 8);
+  if (!ctx->nk) ctx->cov_ratio[1] = 0.0;
+  if (piv.bad_point)
+    return fail(ctx, BA_ERR_NUMERIC, "%s: the Hessian is singular: the 3x3 block of a point is singular (a point "
+                "without observations, or one its observations do not fix)", who);
+  if (piv.first_bad) {
+    const int k = ctx->n_cam - piv.first_bad;
+    return fail(ctx, BA_ERR_NUMERIC, "%s: the Hessian is rank-deficient: a pivot of camera %d (elimination position "
+                "%d) is below %g times its diagonal (a camera its observations do not fix, or cameras not connected to the fixed one)",
+                who, ctx->sym.perm[k], k, BA_COV_MIN_PIVOT_RATIO);
+  }
+  if (piv.bad_border)
+    return fail(ctx, BA_ERR_NUMERIC, "%s: the Hessian is rank-deficient: intrinsics pivot %d is below %g times its "
+                "diagonal (the observations do not fix the intrinsics)", who, piv.bad_border - 1, BA_COV_MIN_PIVOT_RATIO);
+  if (ctx->h_st->lin_fail) return fail(ctx, BA_ERR_NUMERIC, "%s: non-positive pivot (the Hessian is not positive definite)", who);
+  return 0;
+}
+
+extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
+                                 int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs) {
+  if (!ctx) return BA_ERR_INVALID;
+  int rc = cov_check(ctx, "ba_gpu_covariance");
+  if (rc) return rc;
+  if (n_pairs < 0 || (n_pairs > 0 && (!cam_a || !cam_b || !cov_pairs))) return fail(ctx, BA_ERR_INVALID, "bad camera pair list");
+  for (int i = 0; i < n_pairs; ++i)
+    if (cam_a[i] < 0 || cam_a[i] >= ctx->n_cam || cam_b[i] < 0 || cam_b[i] >= ctx->n_cam)
+      return fail(ctx, BA_ERR_INVALID, "camera pair %d (%d, %d) out of range", i, cam_a[i], cam_b[i]);
+  const double *X = nullptr;
+  if ((rc = cov_factor(ctx, &X))) return rc;
+  cudaStream_t s = ctx->stream;
+  const SpSymbolic &S = ctx->sym;
+  const size_t nc = (size_t)ctx->n_cam;
+  SpChol a = spchol_args(ctx);
   // selected inversion of A on the pattern of L (overwrites the panels and the update-matrix slots)
   {
     SelInv si;
@@ -3022,27 +3075,7 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
            P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->perm), P<double>(ctx->W), P<double>(ctx->Wk), P<double>(ctx->Vinv),
            P<int32_t>(ctx->ent_ptr), P<int2>(ctx->ent), P<double>(ctx->cov_S), P<double>(ctx->cov_ck), P<double>(ctx->cov_Tinv),
            P<double>(ctx->sp), P<double>(ctx->cov_pt));
-  if ((rc = poll_state(ctx))) return rc;
-  CK(cudaGetLastError());
-  if (ctx->h_st->eval_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-finite residual or Jacobian");
-  CovPivots piv;
-  CK(cudaMemcpy(&piv, cp, sizeof(piv), cudaMemcpyDeviceToHost));
-  memcpy(&ctx->cov_ratio[0], &piv.min_cam, 8);
-  memcpy(&ctx->cov_ratio[1], &piv.min_border, 8);
-  if (!ctx->nk) ctx->cov_ratio[1] = 0.0;
-  if (piv.bad_point)
-    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is singular: the 3x3 block of a point is singular (a point "
-                "without observations, or one its observations do not fix)");
-  if (piv.first_bad) {
-    const int k = ctx->n_cam - piv.first_bad;
-    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is rank-deficient: a pivot of camera %d (elimination position "
-                "%d) is below %g times its diagonal (a camera its observations do not fix, or cameras not connected to the fixed one)",
-                S.perm[k], k, BA_COV_MIN_PIVOT_RATIO);
-  }
-  if (piv.bad_border)
-    return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: the Hessian is rank-deficient: intrinsics pivot %d is below %g times its "
-                "diagonal (the observations do not fix the intrinsics)", piv.bad_border - 1, BA_COV_MIN_PIVOT_RATIO);
-  if (ctx->h_st->lin_fail) return fail(ctx, BA_ERR_NUMERIC, "ba_gpu_covariance: non-positive pivot (the Hessian is not positive definite)");
+  if ((rc = cov_status(ctx, "ba_gpu_covariance"))) return rc;
   int bad = 0;
   CK(cudaMemcpy(&bad, ctx->cov_bad.p, 4, cudaMemcpyDeviceToHost));
   if (bad) return fail(ctx, BA_ERR_INVALID, "ba_gpu_covariance: a requested camera pair shares no point (outside the pattern of S)");
@@ -3059,6 +3092,265 @@ extern "C" int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_c
     for (int i = 0; i < 4; ++i)
       for (int j = 0; j < 4; ++j) cov_intr[4 * i + j] = ti[4 * i + j] * (sk[i] * sk[j]);
   }
+  return BA_OK;
+}
+
+// A pass of ba_gpu_covariance_blocks holds the sources (cameras whose F = L^-1 E is formed) of a run of consecutive requests:
+// at most CB_PASS_SOURCES of them, and at most CB_PASS_BLOCKS 6x6 blocks of F and carried border rows (1.2 GB).  A request
+// whose own sources exceed a cap gets a pass of its own.  The bits of a block do not depend on the split.
+#define CB_PASS_SOURCES 256
+#define CB_PASS_BLOCKS (1ll << 22)
+
+extern "C" int ba_gpu_covariance_blocks(ba_gpu_ctx *ctx, int32_t n, const ba_cov_block *ra, const ba_cov_block *rb, double *out) {
+  if (!ctx) return BA_ERR_INVALID;
+  const char *who = "ba_gpu_covariance_blocks";
+  int rc = cov_check(ctx, who);
+  if (rc) return rc;
+  if (n < 0 || (n > 0 && (!ra || !rb || !out))) return fail(ctx, BA_ERR_INVALID, "%s: bad request list", who);
+  auto valid = [&](const ba_cov_block &k) {
+    return (k.kind == BA_COV_CAMERA && k.index >= 0 && k.index < ctx->n_cam) ||
+           (k.kind == BA_COV_POINT && k.index >= 0 && k.index < ctx->n_pt) || (k.kind == BA_COV_INTRINSICS && k.index == 0);
+  };
+  for (int i = 0; i < n; ++i)
+    if (!valid(ra[i]) || !valid(rb[i]))
+      return fail(ctx, BA_ERR_INVALID, "%s: request %d ((%d, %d), (%d, %d)): unknown kind, or index out of range", who, i, ra[i].kind,
+                  ra[i].index, rb[i].kind, rb[i].index);
+  const double *X = nullptr;
+  if ((rc = cov_factor(ctx, &X)) || (rc = cov_status(ctx, who))) return rc;
+  cudaStream_t s = ctx->stream;
+  const SpSymbolic &S = ctx->sym;
+  auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
+  const int fixed = ctx->fixed_cam, dim[3] = {6, 3, 4};
+  // canonical orientation (camera < point < intrinsics, then index) and output offsets in the caller's order
+  std::vector<int4> req((size_t)n);
+  std::vector<long long> off((size_t)n);
+  long long total = 0;
+  for (int i = 0; i < n; ++i) {
+    int4 q = make_int4(ra[i].kind, ra[i].index, rb[i].kind, rb[i].index);
+    const bool flip = q.x > q.z || (q.x == q.z && q.y > q.w);
+    if (flip) q = make_int4(q.z, q.w, q.x, q.y);
+    req[i] = q;
+    off[i] = total | (flip ? 1ll << 62 : 0);
+    total += dim[q.x] * dim[q.z];
+  }
+  const bool zero_k = ctx->nk == 0;
+  auto constant = [&](const int4 &q) {
+    return (q.x == BA_COV_CAMERA && q.y == fixed) || (q.z == BA_COV_CAMERA && q.w == fixed) ||
+           (zero_k && (q.x == BA_COV_INTRINSICS || q.z == BA_COV_INTRINSICS));
+  };
+  // the cameras that observe the points of camera-point and point-point requests (a small copy of their observation lists)
+  std::vector<int32_t> pts;
+  for (int i = 0; i < n; ++i) {
+    const int4 &q = req[i];
+    if (constant(q)) continue;
+    if (q.x == BA_COV_CAMERA && q.z == BA_COV_POINT) pts.push_back(q.w);
+    if (q.x == BA_COV_POINT && q.z == BA_COV_POINT) {
+      pts.push_back(q.y);
+      pts.push_back(q.w);
+    }
+  }
+  std::sort(pts.begin(), pts.end());
+  pts.erase(std::unique(pts.begin(), pts.end()), pts.end());
+  const int n_rp = (int)pts.size();
+  std::vector<int2> rng((size_t)n_rp);
+  std::vector<int32_t> obs_ptr((size_t)n_rp + 1, 0), obs;
+  if (n_rp > 0) {
+    RES(cb_pts, (size_t)n_rp * 4);
+    RES(cb_rng, (size_t)n_rp * 8);
+    CK(cudaMemcpyAsync(ctx->cb_pts.p, pts.data(), (size_t)n_rp * 4, cudaMemcpyHostToDevice, s));
+    LAUNCH(k_cb_obs_range, cdiv(n_rp, BA_THREADS), BA_THREADS, 0, n_rp, P<int32_t>(ctx->cb_pts), P<int32_t>(ctx->pt_rowptr),
+           P<int2>(ctx->cb_rng));
+    CK(cudaMemcpyAsync(rng.data(), ctx->cb_rng.p, (size_t)n_rp * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (int i = 0; i < n_rp; ++i) obs_ptr[i + 1] = obs_ptr[i] + rng[i].y;
+    const int n_o = obs_ptr[n_rp];
+    std::vector<int32_t> slots((size_t)n_o);
+    for (int i = 0; i < n_rp; ++i)
+      for (int k = 0; k < rng[i].y; ++k) slots[obs_ptr[i] + k] = rng[i].x + k;
+    obs.resize((size_t)n_o);
+    if (n_o > 0) {
+      RES(cb_obs, (size_t)n_o * 8);
+      CK(cudaMemcpyAsync(ctx->cb_obs.p, slots.data(), (size_t)n_o * 4, cudaMemcpyHostToDevice, s));
+      LAUNCH(k_cb_obs_cams, cdiv(n_o, BA_THREADS), BA_THREADS, 0, n_o, P<int32_t>(ctx->cb_obs), P<int32_t>(ctx->pm_cam),
+             P<int32_t>(ctx->cb_obs) + n_o);
+      CK(cudaMemcpyAsync(obs.data(), P<int32_t>(ctx->cb_obs) + n_o, (size_t)n_o * 4, cudaMemcpyDeviceToHost, s));
+      CK(cudaStreamSynchronize(s));
+    }
+  }
+  auto pt_index = [&](int p) { return (int)(std::lower_bound(pts.begin(), pts.end(), p) - pts.begin()); };
+  // tree: node of every position, workspace of a source's path (F: own blocks, carry: border blocks)
+  std::vector<int32_t> node_of((size_t)ctx->n_cam);
+  for (int id = 0; id < S.n_nodes; ++id)
+    for (int k = N_(id, SPN_K0); k < N_(id, SPN_K0) + N_(id, SPN_M); ++k) node_of[k] = id;
+  std::vector<long long> path_blocks((size_t)ctx->n_cam, -1);
+  auto cost = [&](int c) {
+    long long &v = path_blocks[c];
+    if (v < 0) {
+      v = 0;
+      for (int id = node_of[S.pos[c]]; id >= 0; id = N_(id, SPN_PARENT)) v += N_(id, SPN_M) + N_(id, SPN_NB);
+    }
+    return v;
+  };
+  RES(cb_out, (size_t)total * 8 + 16);
+  RES(cb_cam_src, (size_t)ctx->n_cam * 4);
+  size_t fwd_smem = cb_forward_smem(S.max_m);
+  CK(cudaFuncSetAttribute(k_cb_forward, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fwd_smem));
+  std::vector<int32_t> cam_src((size_t)ctx->n_cam, -1);
+  // one pass: the forward substitution of its sources, then its requests
+  auto run_pass = [&](std::vector<int32_t> &src, const std::vector<int> &rq) -> int {
+    std::sort(src.begin(), src.end());
+    const int ns = (int)src.size();
+    std::vector<int32_t> sptr((size_t)ns + 1, 0);
+    std::vector<int4> key;  // (level, node, source, step on the path)
+    for (int i = 0; i < ns; ++i) {
+      int t = 0;
+      for (int id = node_of[S.pos[src[i]]]; id >= 0; id = N_(id, SPN_PARENT), ++t) key.push_back(make_int4(N_(id, SPN_LEVEL), id, i, t));
+      sptr[i + 1] = sptr[i] + t;
+    }
+    std::sort(key.begin(), key.end(), [](const int4 &u, const int4 &v) {
+      return u.x != v.x ? u.x < v.x : u.y != v.y ? u.y < v.y : u.z != v.z ? u.z < v.z : u.w < v.w;
+    });
+    const int ne = (int)key.size();
+    std::vector<int32_t> sent((size_t)ne), ent((size_t)ne * CB_ENT_INTS, 0);
+    for (int e = 0; e < ne; ++e) sent[sptr[key[e].z] + key[e].w] = e;
+    long long fb = 0, cbk = 0;
+    std::vector<int2> items;
+    std::vector<int> lvl_ptr((size_t)S.n_levels + 1, 0);
+    for (int e = 0; e < ne; ++e) {
+      const int4 &k = key[e];
+      int32_t *E = ent.data() + (size_t)e * CB_ENT_INTS;
+      E[0] = k.y;
+      E[1] = k.w > 0 ? sent[sptr[k.z] + k.w - 1] : -1;
+      E[2] = k.w == 0 ? S.pos[src[k.z]] - N_(k.y, SPN_K0) : -1;
+      E[3] = (int32_t)fb;
+      E[4] = (int32_t)cbk;
+      E[5] = k.x;
+      fb += N_(k.y, SPN_M);
+      cbk += N_(k.y, SPN_NB);
+      if (e == 0 || k.y != key[e - 1].y || items.back().y == CB_GROUP) {
+        items.push_back(make_int2(e, 0));
+        lvl_ptr[k.x + 1]++;
+      }
+      items.back().y++;
+    }
+    for (int l = 0; l < S.n_levels; ++l) lvl_ptr[l + 1] += lvl_ptr[l];
+    std::vector<int32_t> paths(sptr);
+    paths.insert(paths.end(), sent.begin(), sent.end());
+    for (int i = 0; i < ns; ++i) cam_src[src[i]] = i;
+    std::vector<int4> preq;
+    std::vector<long long> poff;
+    for (int i : rq) {
+      preq.push_back(req[i]);
+      poff.push_back(off[i]);
+    }
+    RES(cb_ent, (size_t)ne * CB_ENT_INTS * 4);
+    RES(cb_items, items.size() * 8);
+    RES(cb_src, paths.size() * 4);
+    RES(cb_req, preq.size() * 16);
+    RES(cb_off, poff.size() * 8);
+    RES(cb_F, ((size_t)fb + 1) * 288);
+    RES(cb_carry, ((size_t)cbk + 1) * 288);
+    CK(cudaMemcpyAsync(ctx->cb_ent.p, ent.data(), ent.size() * 4, cudaMemcpyHostToDevice, s));
+    if (!items.empty()) CK(cudaMemcpyAsync(ctx->cb_items.p, items.data(), items.size() * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->cb_src.p, paths.data(), paths.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->cb_cam_src.p, cam_src.data(), cam_src.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->cb_req.p, preq.data(), preq.size() * 16, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ctx->cb_off.p, poff.data(), poff.size() * 8, cudaMemcpyHostToDevice, s));
+    const SpChol sa = spchol_args(ctx);
+    CbFwd f;
+    f.node = sa.node;
+    f.rel = sa.rel;
+    f.inv = sa.inv;
+    f.panel = sa.panel;
+    f.linv = sa.linv;
+    f.ent = P<int32_t>(ctx->cb_ent);
+    f.items = P<int2>(ctx->cb_items);
+    f.F = P<double>(ctx->cb_F);
+    f.carry = P<double>(ctx->cb_carry);
+    for (int l = 0; l < S.n_levels; ++l)
+      LAUNCH(k_cb_forward, lvl_ptr[l + 1] - lvl_ptr[l], CB_THREADS, fwd_smem, f, lvl_ptr[l]);
+    CbBlk b;
+    b.ent = f.ent;
+    b.src_ptr = P<int32_t>(ctx->cb_src);
+    b.src_ent = b.src_ptr + ns + 1;
+    b.cam_src = P<int32_t>(ctx->cb_cam_src);
+    b.node = sa.node;
+    b.F = f.F;
+    b.pos = P<int32_t>(ctx->cov_pos);
+    b.X = X;
+    b.Tinv = P<double>(ctx->cov_Tinv);
+    b.nk = ctx->nk;
+    b.n_cam = ctx->n_cam;
+    b.fixed_cam = fixed;
+    b.pt_rowptr = P<int32_t>(ctx->pt_rowptr);
+    b.pm_cam = P<int32_t>(ctx->pm_cam);
+    b.perm = P<int32_t>(ctx->perm);
+    b.W = P<double>(ctx->W);
+    b.Wk = P<double>(ctx->Wk);
+    b.Vinv = P<double>(ctx->Vinv);
+    b.sc = P<double>(ctx->sc);
+    b.sp = P<double>(ctx->sp);
+    b.sk = P<double>(ctx->sk);
+    b.req = P<int4>(ctx->cb_req);
+    b.off = P<long long>(ctx->cb_off);
+    b.n_req = (int)preq.size();
+    b.out = P<double>(ctx->cb_out);
+    LAUNCH(k_cb_blocks, cdiv(b.n_req, CB_WARPS), CB_THREADS, 0, b);
+    CK(cudaStreamSynchronize(s));  // (host vectors die here)
+    for (int i = 0; i < ns; ++i) cam_src[src[i]] = -1;
+    return 0;
+  };
+  // passes: runs of consecutive requests, greedily
+  std::vector<int> stamp((size_t)ctx->n_cam, -1), cur_rq, need;
+  std::vector<int32_t> cur_src, fresh;
+  long long cur_blocks = 0;
+  int pass = 0;
+  for (int i = 0; i < n; ++i) {
+    const int4 &q = req[i];
+    need.clear();
+    auto add_pt = [&](int p) {
+      const int k = pt_index(p);
+      for (int o = obs_ptr[k]; o < obs_ptr[k + 1]; ++o)
+        if (obs[o] != fixed) need.push_back(obs[o]);
+    };
+    if (!constant(q) && q.x == BA_COV_CAMERA && q.z == BA_COV_CAMERA) {
+      need.push_back(q.y);
+      need.push_back(q.w);
+    } else if (!constant(q) && q.x == BA_COV_CAMERA && q.z == BA_COV_POINT) {
+      need.push_back(q.y);
+      add_pt(q.w);
+    } else if (!constant(q) && q.x == BA_COV_POINT && q.z == BA_COV_POINT) {
+      add_pt(q.y);
+      add_pt(q.w);
+    }
+    long long b_new = 0;
+    auto collect = [&]() {
+      fresh.clear();
+      b_new = 0;
+      for (int c : need)
+        if (stamp[c] != pass) {
+          stamp[c] = pass;
+          fresh.push_back(c);
+          b_new += cost(c);
+        }
+    };
+    collect();
+    if (!cur_rq.empty() && !fresh.empty() &&
+        (cur_src.size() + fresh.size() > CB_PASS_SOURCES || cur_blocks + b_new > CB_PASS_BLOCKS)) {
+      if ((rc = run_pass(cur_src, cur_rq))) return rc;
+      cur_src.clear();
+      cur_rq.clear();
+      cur_blocks = 0;
+      ++pass;
+      collect();
+    }
+    cur_src.insert(cur_src.end(), fresh.begin(), fresh.end());
+    cur_blocks += b_new;
+    cur_rq.push_back(i);
+  }
+  if (!cur_rq.empty() && (rc = run_pass(cur_src, cur_rq))) return rc;
+  CK(cudaGetLastError());
+  if (total > 0) CK(cudaMemcpy(out, ctx->cb_out.p, (size_t)total * 8, cudaMemcpyDeviceToHost));
   return BA_OK;
 }
 

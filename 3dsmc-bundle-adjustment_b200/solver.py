@@ -178,6 +178,28 @@ class GpuSolver:
                                                capi.dp(out["pt"]), len(a), capi.ip(a), capi.ip(b), capi.dp(out["pairs"])))
         return out
 
+    def covariance_blocks(self, pairs):
+        """Covariance of any pairs of parameter blocks at the current state (ceres::Covariance::Compute(pairs)), with the
+        conventions and preconditions of covariance().  pairs: [((kind, i), (kind, j)), ...], kind "cam" | "pt" | "intr"
+        (index 0 for the intrinsics) -> a list of arrays, Cov(a, b) of shape (dim a, dim b), dims 6 / 3 / 4.  Camera pairs
+        need not share a point."""
+        kinds = {"cam": capi.BA_COV_CAMERA, "pt": capi.BA_COV_POINT, "intr": capi.BA_COV_INTRINSICS}
+        dims = {"cam": 6, "pt": 3, "intr": 4}
+        pairs = list(pairs)
+        n = len(pairs)
+        a, b = (capi.CovBlock * max(n, 1))(), (capi.CovBlock * max(n, 1))()
+        for i, ((ka, ia), (kb, ib)) in enumerate(pairs):
+            a[i].kind, a[i].index = kinds[ka], int(ia)
+            b[i].kind, b[i].index = kinds[kb], int(ib)
+        sizes = [dims[ka] * dims[kb] for (ka, _), (kb, _) in pairs]
+        out = np.zeros(max(sum(sizes), 1))
+        self._check(self.lib.ba_gpu_covariance_blocks(self._ctx, n, a, b, capi.dp(out)))
+        res, o = [], 0
+        for ((ka, _), (kb, _)), sz in zip(pairs, sizes):
+            res.append(out[o:o + sz].reshape(dims[ka], dims[kb]).copy())
+            o += sz
+        return res
+
     def covariance_pivots(self):
         """Smallest pivot / diagonal ratio of the last covariance() call, also a rejected one: {"cam": camera system,
         "intr": intrinsics (0 when they are constant)}.  covariance() rejects a ratio below capi.BA_COV_MIN_PIVOT_RATIO."""

@@ -220,8 +220,25 @@ int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *rhs, double
 #define BA_COV_MIN_PIVOT_RATIO 1e-9
 int ba_gpu_covariance(ba_gpu_ctx *ctx, double *cov_cam, double *cov_cam_intr, double cov_intr[4 * 4], double *cov_pt,
                       int32_t n_pairs, const int32_t *cam_a, const int32_t *cam_b, double *cov_pairs);
-/* smallest pivot / diagonal ratio of the last ba_gpu_covariance call (also a rejected one): ratio[0] over the camera system,
- * ratio[1] over the intrinsics (0 when they are constant); compare with BA_COV_MIN_PIVOT_RATIO */
+/* Covariance of ANY n pairs of parameter blocks (ceres::Covariance::Compute(pairs), GetCovarianceBlockInTangentSpace):
+ * camera pairs that share no point, camera-point, point-point, camera-intrinsics, intrinsics, and the blocks
+ * ba_gpu_covariance returns.  Same Hessian, conventions and preconditions as ba_gpu_covariance (the same factorisation and
+ * relative pivot test; ba_gpu_covariance_pivots reports this call too), without the selected inversion: with A = L L^T,
+ * (A^-1)_ab = (L^-1 E_a)^T (L^-1 E_b), a dot product over the common part of the two cameras' root paths in the tree.
+ *   a[i], b[i] -> out: Cov(a[i], b[i]), dim(a[i]) x dim(b[i]) row-major (dims 6 / 3 / 4), the blocks back to back in order
+ * A block with the fixed camera, or with constant intrinsics (DEPTH cost), is zero.  The bits of a block do not depend on the
+ * other requests, and Cov(b, a) is exactly Cov(a, b)^T.  A later ba_gpu_solve or ba_gpu_covariance is unaffected.
+ * BA_ERR_INVALID: n < 0, a null array with n > 0, an unknown kind, an index out of range, an intrinsics index other than 0;
+ * otherwise the codes of ba_gpu_covariance.  n == 0 runs the factorisation and its pivot test only. */
+enum { BA_COV_CAMERA = 0, BA_COV_POINT = 1, BA_COV_INTRINSICS = 2 };
+typedef struct ba_cov_block {
+  int32_t kind;  /* BA_COV_* */
+  int32_t index; /* camera or point; 0 for the intrinsics */
+} ba_cov_block;
+int ba_gpu_covariance_blocks(ba_gpu_ctx *ctx, int32_t n, const ba_cov_block *a, const ba_cov_block *b, double *out);
+/* smallest pivot / diagonal ratio of the last ba_gpu_covariance or ba_gpu_covariance_blocks call (also a rejected one):
+ * ratio[0] over the camera system, ratio[1] over the intrinsics (0 when they are constant); compare with
+ * BA_COV_MIN_PIVOT_RATIO */
 int ba_gpu_covariance_pivots(const ba_gpu_ctx *ctx, double ratio[2]);
 /* structure of the sparse Cholesky of the last upload (zeros when another solver is in force): info[0..10] as
  * ba_sparse_symbolic_info, info[11] = host microseconds of the symbolic phase, info[12] = parts of the subtree-to-rank
