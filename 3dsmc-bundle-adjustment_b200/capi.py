@@ -79,7 +79,7 @@ EXPORTS = [
     "ba_store_create", "ba_store_destroy", "ba_store_clear", "ba_store_set_keyframe", "ba_store_set_keyframes", "ba_store_set_poses", "ba_store_set_landmarks",
     "ba_store_window_solve",
     "ba_sparse_symbolic_create", "ba_sparse_symbolic_info", "ba_sparse_symbolic_get", "ba_sparse_symbolic_destroy",
-    "ba_sparse_symbolic_partition",
+    "ba_sparse_symbolic_partition", "ba_sparse_symbolic_queue",
 ]
 
 _LIB = None
@@ -145,6 +145,7 @@ def load():
     L.ba_sparse_symbolic_get.argtypes = [vp, C.c_int32, c_int32_p]
     L.ba_sparse_symbolic_destroy.argtypes = [vp]
     L.ba_sparse_symbolic_partition.argtypes = [vp, C.c_int32, c_int32_p, c_double_p]
+    L.ba_sparse_symbolic_queue.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, c_int32_p] + [c_int32_p] * 5
     L.ba_sparse_symbolic_destroy.restype = None
     for name in EXPORTS:
         if name not in ("ba_gpu_destroy", "ba_gpu_default_options", "ba_gpu_last_error", "ba_gpu_launch_count",

@@ -154,7 +154,7 @@ struct ba_gpu_ctx {
   bool src_on_device = false;   // the arrays handed to the current upload live in device memory (ba_store_window_solve)
   bool spchol = false;          // the block-sparse solver factorises S instead of running PCG
   SpSymbolic sym;               // host-side structure of the last upload
-  Buf spn_node, spn_bord, spn_children, spn_rel, spn_inv, spn_aent, spn_perm, spn_levels;
+  Buf spn_node, spn_bord, spn_children, spn_rel, spn_inv, spn_aent, spn_perm;
   Buf spc_panel, spc_U, spc_z, spc_linv, spc_ypos, spc_prof, spc_queue, spc_tiles, spc_cnt, spc_cnt_init, spc_topcams;
   int spc_n_items = 0;
   // subtree-to-rank partition (spsym_partition): phase A = the subtrees of one part (queue items spc_qA[p] .. spc_qA[p + 1]),
@@ -169,7 +169,7 @@ struct ba_gpu_ctx {
   Buf spc_xidx, spc_xbuf;
   int spc_nx = 0;
   bool sp_full_next = false;  // the next enqueue_sparse_values() completes ALL of S on every rank (product hook)
-  size_t spc_smem_tree = 0, spc_smem_solve = 0;  // dynamic shared memory of k_spchol_tree / k_spchol_solve
+  size_t spc_smem_tree = 0;   // dynamic shared memory of k_spchol_tree
   double sym_ms = 0.0;          // host time of the symbolic phase (last upload)
   // sparse Cholesky of the REF / depth-prior / free-intrinsics cost (solver = EXPLICIT_CHOLESKY's linearisation and W / WV,
   // the block-sparse S and the tree instead of the dense S): right-hand-side rows of the tree (5 with the intrinsics border),
@@ -272,6 +272,13 @@ static T *P(const Buf &b) {
   return reinterpret_cast<T *>(b.p);
 }
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
+// an int32 table into device buffer b, grown as needed (one spare element: an empty table is still a valid pointer)
+static int upload_i32(ba_gpu_ctx *ctx, Buf &b, const std::vector<int32_t> &v) {
+  int rc = buf_reserve(ctx, b, (v.size() + 1) * 4);
+  if (rc) return rc;
+  if (!v.empty()) CK(cudaMemcpyAsync(b.p, v.data(), v.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
 // dense explicit Schur complement: n^2 doubles (2 GiB at the limit), blocked Cholesky above 1024
 #define BA_EXPLICIT_MAX_DIM 16384
 static size_t tile_smem_bytes(int npt) {
@@ -898,12 +905,6 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   if (S.error) return fail(ctx, BA_ERR_STATE, "sparse Cholesky: inconsistent symbolic structure (%d)", S.error);
   if ((double)S.panel_blocks * 288.0 + (double)S.u_blocks * 288.0 > 64e9)
     return fail(ctx, BA_ERR_UNSUPPORTED, "sparse Cholesky: factor would need %.1f GB", ((double)S.panel_blocks + (double)S.u_blocks) * 288e-9);
-  auto up = [&](Buf &b, const std::vector<int32_t> &v) -> int {
-    int rc = buf_reserve(ctx, b, (v.size() + 1) * 4);
-    if (rc) return rc;
-    if (!v.empty()) CK(cudaMemcpyAsync(b.p, v.data(), v.size() * 4, cudaMemcpyHostToDevice, s));
-    return 0;
-  };
   // subtree-to-rank partition of the NS LM solve: one part per rank; on one GPU BA_SPCHOL_PARTS=n runs the n parts one after
   // the other (tests of the queues and of the exchange layout).  One part for the REF-cost solve and for the structure the
   // covariance builds under another solver: both are single-GPU and run the one-part queue's factor prefix on its own.
@@ -963,12 +964,13 @@ static int build_spchol(ba_gpu_ctx *ctx) {
     for (int g = 0; g < n_blk; ++g)
       if (mask[g] != 0.0) xs.push_back(g);
     ctx->spc_nx = (int)xs.size();
-    if ((rc = up(ctx->spc_xidx, xs))) return rc;
+    if ((rc = upload_i32(ctx, ctx->spc_xidx, xs))) return rc;
     RES(spc_xbuf, ((size_t)std::max<size_t>(xs.size(), ((size_t)n_blk + 1) / 36 + 1) + 1) * 288);
   }
-  if ((rc = up(ctx->spn_node, S.node)) || (rc = up(ctx->spn_bord, S.bord)) || (rc = up(ctx->spn_children, S.children)) ||
-      (rc = up(ctx->spn_rel, S.rel)) || (rc = up(ctx->spn_inv, S.inv)) || (rc = up(ctx->spn_aent, S.aent)) ||
-      (rc = up(ctx->spn_perm, S.perm)) || (rc = up(ctx->spn_levels, S.level_nodes)))
+  if ((rc = upload_i32(ctx, ctx->spn_node, S.node)) || (rc = upload_i32(ctx, ctx->spn_bord, S.bord)) ||
+      (rc = upload_i32(ctx, ctx->spn_children, S.children)) || (rc = upload_i32(ctx, ctx->spn_rel, S.rel)) ||
+      (rc = upload_i32(ctx, ctx->spn_inv, S.inv)) || (rc = upload_i32(ctx, ctx->spn_aent, S.aent)) ||
+      (rc = upload_i32(ctx, ctx->spn_perm, S.perm)))
     return rc;
   RES(spc_panel, ((size_t)S.panel_blocks + 1) * 288);
   RES(spc_U, ((size_t)S.u_blocks + (size_t)ru_blocks + 1) * 288);
@@ -989,82 +991,25 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   if (sf > 227 * 1024 || ss > 227 * 1024 || su > 227 * 1024)
     return fail(ctx, BA_ERR_STATE, "sparse Cholesky: front exceeds shared memory (%zu / %zu / %zu bytes)", sf, ss, su);
   ctx->spc_smem_tree = std::max(std::max(sf, ss), su);
-  ctx->spc_smem_solve = ss;
   if (R > 1)
     CK(cudaFuncSetAttribute(k_spchol_tree<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->spc_smem_tree));
   else
     CK(cudaFuncSetAttribute(k_spchol_tree<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->spc_smem_tree));
-  CK(cudaFuncSetAttribute(k_spchol_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
-  // work queues of the persistent tree kernel.  Phase A (one queue per part): per level (bottom-up) the factor items of the
-  // part's nodes, then their update tiles -- more tiles per node where the part has few nodes on a level.  Phase B: the same
-  // for the top part, then the backward substitution level by level top-down (top part first, then the subtrees this GPU
-  // holds).  One part: phase A is the whole factorisation and the substitution follows in the same queue (one launch).
+  // work queues of the persistent tree kernel (spq_cholesky)
   {
-    const int P_ = part.parts;
-    const int me = ctx->spc_dist ? ctx->rank : -2;  // (-2: this GPU holds every part)
-    auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
-    std::vector<int32_t> tiles((size_t)S.n_nodes, 0), q, cnt_init((size_t)3 * S.n_nodes + 16, 0), topcams;
-    auto push_factor_levels = [&](int which) {
-      for (int l = 0; l < S.n_levels; ++l) {
-        int nodes = 0;
-        for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) nodes += part.part[S.level_nodes[e]] == which;
-        if (!nodes) continue;
-        const int t_lvl = std::max(1, std::min(8, ctx->n_sm / nodes));
-        for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-          const int id = S.level_nodes[e];
-          if (part.part[id] != which) continue;
-          tiles[id] = N_(id, SPN_NB) > 0 ? t_lvl : 0;
-          q.push_back(id);
-          q.push_back(-1);
-        }
-        for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-          const int id = S.level_nodes[e];
-          if (part.part[id] != which) continue;
-          for (int t = 0; t < tiles[id]; ++t) {
-            q.push_back(id);
-            q.push_back(t);
-          }
-        }
-      }
-    };
-    auto push_solve_levels = [&](bool top_part) {
-      for (int l = S.n_levels - 1; l >= 0; --l)
-        for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-          const int id = S.level_nodes[e], pr = part.part[id];
-          if (top_part ? pr >= 0 : (pr < 0 || (me != -2 && pr != me))) continue;
-          q.push_back(id);
-          q.push_back(-2);
-        }
-    };
-    for (int p = 0; p < P_; ++p) {
-      ctx->spc_qA[p] = (int)(q.size() / 2);
-      if (me == -2 || p == me) push_factor_levels(p);
-      ctx->spc_qA[p + 1] = (int)(q.size() / 2);
-    }
-    ctx->spc_qB = (int)(q.size() / 2);
-    if (P_ > 1) {
-      push_factor_levels(-1);
-      push_solve_levels(true);
-    }
-    push_solve_levels(false);
-    ctx->spc_qB_n = (int)(q.size() / 2) - ctx->spc_qB;
-    ctx->spc_n_items = (int)(q.size() / 2);
-    // counters before a solve: zero, except "all update tiles done" for the subtree roots other ranks factorise (their
-    // update matrices arrive with the exchange)
-    for (int id = 0; id < S.n_nodes; ++id) {
-      if (part.part[id] < 0)
-        for (int k = 0; k < N_(id, SPN_M); ++k) topcams.push_back(S.perm[N_(id, SPN_K0) + k]);
-      else if (me != -2 && part.part[id] != me)
-        cnt_init[16 + (size_t)S.n_nodes + id] = 1 << 20;
-    }
-    ctx->spc_n_topcams = (int)topcams.size();
-    if ((rc = up(ctx->spc_queue, q)) || (rc = up(ctx->spc_tiles, tiles)) || (rc = up(ctx->spc_cnt_init, cnt_init)) ||
-        (rc = up(ctx->spc_topcams, topcams)))
+    const SpCholQueue Q = spq_cholesky(S, part, ctx->spc_dist ? ctx->rank : -1, ctx->n_sm);
+    std::copy(Q.qA.begin(), Q.qA.end(), ctx->spc_qA);
+    ctx->spc_qB = Q.qB;
+    ctx->spc_qB_n = Q.qB_n;
+    ctx->spc_n_items = Q.n_items();
+    ctx->spc_n_topcams = (int)Q.topcams.size();
+    if ((rc = upload_i32(ctx, ctx->spc_queue, Q.q)) || (rc = upload_i32(ctx, ctx->spc_tiles, Q.tiles)) ||
+        (rc = upload_i32(ctx, ctx->spc_cnt_init, Q.cnt_init)) || (rc = upload_i32(ctx, ctx->spc_topcams, Q.topcams)))
       return rc;
     RES(spc_cnt, ((size_t)3 * S.n_nodes + 16) * 4);
     if (getenv("BA_SPCHOL_DEBUG"))
       fprintf(stderr, "[spchol] rank %d: %d parts%s, top %d nodes / %d cameras (%.1f %% of the work), heaviest part %.1f %%, "
-              "exchange %.2f MB, items A %d B %d\n", ctx->rank, P_, ctx->spc_dist ? " (distributed)" : "",
+              "exchange %.2f MB, items A %d B %d\n", ctx->rank, part.parts, ctx->spc_dist ? " (distributed)" : "",
               (int)std::count(part.part.begin(), part.part.end(), -1), ctx->spc_n_topcams, 100.0 * part.top / std::max(1.0, part.total),
               100.0 * part.heaviest / std::max(1.0, part.total), ctx->spc_xchg * 8e-6, ctx->spc_qB, ctx->spc_qB_n);
   }
@@ -1952,7 +1897,6 @@ static SpChol spchol_args(ba_gpu_ctx *ctx) {
   a.inv = P<int32_t>(ctx->spn_inv);
   a.aent = P<int32_t>(ctx->spn_aent);
   a.perm = P<int32_t>(ctx->spn_perm);
-  a.level_nodes = P<int32_t>(ctx->spn_levels);
   a.S = P<double>(ctx->Sblk);
   a.dsq = P<double>(ctx->dsq);
   a.b = P<double>(ctx->b);
@@ -2836,32 +2780,9 @@ static int cov_prepare(ba_gpu_ctx *ctx) {
   }
   const SpSymbolic &S = ctx->sym;
   auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
-  // queue: levels top-down; per level the prepare items, the product tiles (more per node where the level has few nodes), the
-  // finish items
-  std::vector<int32_t> q, tiles((size_t)S.n_nodes, 0);
+  const SpQueue Q = spq_selinv(S, ctx->n_sm);
   size_t smem = 0;
-  for (int l = S.n_levels - 1; l >= 0; --l) {
-    const int nodes = S.level_ptr[l + 1] - S.level_ptr[l];
-    const int t_lvl = std::max(1, std::min(8, ctx->n_sm / std::max(1, nodes)));
-    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-      const int id = S.level_nodes[e];
-      tiles[id] = N_(id, SPN_NB) > 0 ? t_lvl : 0;
-      smem = std::max(smem, si_smem(N_(id, SPN_M), N_(id, SPN_NB)));
-      q.push_back(id);
-      q.push_back(-1);
-    }
-    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-      const int id = S.level_nodes[e];
-      for (int t = 0; t < tiles[id]; ++t) {
-        q.push_back(id);
-        q.push_back(t);
-      }
-    }
-    for (int e = S.level_ptr[l]; e < S.level_ptr[l + 1]; ++e) {
-      q.push_back(S.level_nodes[e]);
-      q.push_back(-3);
-    }
-  }
+  for (int id = 0; id < S.n_nodes; ++id) smem = std::max(smem, si_smem(N_(id, SPN_M), N_(id, SPN_NB)));
   if (smem > 227 * 1024) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance: a front does not fit shared memory (%zu bytes)", smem);
   // stored block of S -> (node, local row, local column, flags: 1 transposed, 2 diagonal) from the entry table
   std::vector<int32_t> brec((size_t)ctx->n_sblk * 4 + 4, 0);
@@ -2877,15 +2798,10 @@ static int cov_prepare(ba_gpu_ctx *ctx) {
       r[2] = S.aent[4 * (size_t)e + 2];
       r[3] = (code & 0x80000000u ? 1 : 0) | (code & 0x40000000u ? 2 : 0);
     }
-  auto up = [&](Buf &b, const std::vector<int32_t> &v) -> int {
-    int rc2 = buf_reserve(ctx, b, (v.size() + 1) * 4);
-    if (rc2) return rc2;
-    if (!v.empty()) CK(cudaMemcpyAsync(b.p, v.data(), v.size() * 4, cudaMemcpyHostToDevice, s));
-    return 0;
-  };
-  if ((rc = up(ctx->cov_queue, q)) || (rc = up(ctx->cov_tiles, tiles)) || (rc = up(ctx->cov_brec, brec)) || (rc = up(ctx->cov_pos, S.pos)))
+  if ((rc = upload_i32(ctx, ctx->cov_queue, Q.q)) || (rc = upload_i32(ctx, ctx->cov_tiles, Q.tiles)) ||
+      (rc = upload_i32(ctx, ctx->cov_brec, brec)) || (rc = upload_i32(ctx, ctx->cov_pos, S.pos)))
     return rc;
-  ctx->cov_n_items = (int)(q.size() / 2);
+  ctx->cov_n_items = Q.n_items();
   ctx->cov_smem = smem;
   CK(cudaFuncSetAttribute(k_selinv_tree, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const size_t nc = (size_t)ctx->n_cam;
@@ -2967,7 +2883,8 @@ static int cov_factor(ba_gpu_ctx *ctx, const double **Xout) {
   launch_spchol_tree(ctx, a, 0, ctx->spc_qB, 0, GATE_RUN);
   LAUNCH(k_cov_pivots, cdiv(6 * ctx->n_cam, BA_THREADS), BA_THREADS, 0, ctx->n_cam, a.perm, P<int32_t>(ctx->sp_diag), a.S, a.dsq,
          a.linv, BA_COV_MIN_PIVOT_RATIO, cp);
-  // intrinsics border: T^-1, then X = L^-T Z one column at a time (the backward substitution of the LM step, levels top-down)
+  // intrinsics border: T^-1, then X = L^-T Z one column at a time (the backward substitution of the LM step: the solve items
+  // of the queue, one tree launch per column)
   const double *X = nullptr;
   if (ctx->nk) {
     LAUNCH(k_spb_reduce, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->spb_Z), P<double>(ctx->spc_z),
@@ -2982,8 +2899,10 @@ static int cov_factor(ba_gpu_ctx *ctx, const double **Xout) {
     for (int qc = 0; qc < 4; ++qc) {
       LAUNCH(k_cov_zcol, cdiv(6 * ctx->n_cam, BA_THREADS), BA_THREADS, 0, 6 * ctx->n_cam, qc, P<double>(ctx->spb_Z), P<double>(ctx->cov_zq));
       ax.ypos = P<double>(ctx->cov_X) + (size_t)qc * 6 * nc;
-      for (int l = S.n_levels - 1; l >= 0; --l)
-        LAUNCH(k_spchol_solve, S.level_ptr[l + 1] - S.level_ptr[l], SPC_THREADS, ctx->spc_smem_solve, ax, S.level_ptr[l], st, GATE_RUN);
+      // the roots wait on their own fdone, which the factor launch set: between columns only the solve flags go back to zero
+      // (a slot-0 launch would reset every counter), and each column takes a ticket counter of its own
+      if (qc > 0) CK(cudaMemsetAsync(P<int>(ctx->spc_cnt) + 16 + 2 * (size_t)S.n_nodes, 0, (size_t)S.n_nodes * 4, s));
+      launch_spchol_tree(ctx, ax, ctx->spc_qB, ctx->spc_qB_n, 1 + qc, GATE_RUN);
     }
     X = P<double>(ctx->cov_X);
   }
@@ -3956,6 +3875,34 @@ extern "C" int ba_sparse_symbolic_partition(const ba_spsym *h, int32_t parts, in
     work[1] = R.top;
     work[2] = R.heaviest;
   }
+  return R.parts;
+}
+extern "C" int ba_sparse_symbolic_queue(const ba_spsym *h, int32_t which, int32_t parts, int32_t rank, int32_t n_sm, int32_t info[4],
+                                        int32_t *queue, int32_t *tiles, int32_t *qA, int32_t *cnt_init, int32_t *topcams) {
+  if (!h || !info || (which != 0 && which != 1) || parts < 1 || rank >= parts || n_sm < 1) return BA_ERR_INVALID;
+  auto put = [](const std::vector<int32_t> &v, int32_t *dst) {
+    if (dst && !v.empty()) memcpy(dst, v.data(), v.size() * sizeof(int32_t));
+  };
+  if (which == 1) {
+    const SpQueue Q = spq_selinv(h->s, n_sm);
+    info[0] = Q.n_items();
+    info[1] = info[2] = info[3] = 0;
+    put(Q.q, queue);
+    put(Q.tiles, tiles);
+    return 1;
+  }
+  // (as build_spchol: a rank runs its own part only when the partition has one part per rank)
+  const SpPartition R = spsym_partition(h->s, parts);
+  const SpCholQueue Q = spq_cholesky(h->s, R, rank >= 0 && R.parts == parts ? rank : -1, n_sm);
+  info[0] = Q.n_items();
+  info[1] = Q.qB;
+  info[2] = Q.qB_n;
+  info[3] = (int32_t)Q.topcams.size();
+  put(Q.q, queue);
+  put(Q.tiles, tiles);
+  put(Q.qA, qA);
+  put(Q.cnt_init, cnt_init);
+  put(Q.topcams, topcams);
   return R.parts;
 }
 extern "C" int ba_sparse_symbolic_get(const ba_spsym *h, int32_t which, int32_t *dst) {

@@ -11,8 +11,8 @@
 // (same layout), S_BB into the update-matrix slot (dense NB6 x NB6, full).  No L of a node is read after its own inversion
 // (the children read only their own panels and the parent's Sigma front), and the next solve re-factorises.
 // Y goes to a panel-shaped scratch buffer (border rows only).
-// Intrinsics border: X = A^-1 B = L^-T Z (backward substitution, one column at a time, k_spchol_solve), T = C - Z^T Z,
-//     Sigma_kk = T^-1,  Sigma_ck = -X T^-1,  Sigma_cc(a, b) = (A^-1)_ab + X_a T^-1 X_b^T.
+// Intrinsics border: X = A^-1 B = L^-T Z (backward substitution, one column at a time: the solve items of k_spchol_tree),
+//     T = C - Z^T Z, Sigma_kk = T^-1,  Sigma_ck = -X T^-1,  Sigma_cc(a, b) = (A^-1)_ab + X_a T^-1 X_b^T.
 // Points: Sigma_pp = V^-1 + V^-1 (W_p^T Sigma_RR W_p) V^-1 over the observation pairs of the point.
 // Everything is Jacobi-scaled on the device; the outputs are unscaled (Sigma = diag(s) Sigma_s diag(s)).
 // Every sum has a fixed order and no float atomics are used: the results are bit-identical from run to run.
@@ -182,36 +182,26 @@ __device__ __forceinline__ void si_finish(const SelInv &a, int id) {
 //     prepare(n)  its own part (L_OO^-1, Y) at once; the gather of S_BB after finish(parent(n))
 //     tile(n, t)  after prepare(n)
 //     finish(n)   after prepare(n) and every tile of n
-// The queue holds the levels top-down (per level: prepare items, tiles, finish items): every item waits only for items with
-// a smaller queue index, so there is no deadlock whatever the number of resident blocks.
+// The queue holds the levels top-down (per level: prepare items, tiles, finish items; spq_selinv, ba_sparse_symbolic.h): every
+// item waits only for items with a smaller queue index, so there is no deadlock whatever the number of resident blocks
+// (tests/test_tree_queue_order.py checks the order).
 __global__ void __launch_bounds__(SPC_THREADS, 1) k_selinv_tree(SelInv a) {
   extern __shared__ __align__(16) double si_sm[];
   __shared__ int s_item;
   const int tid = threadIdx.x;
   for (;;) {
-    __syncthreads();
-    if (tid == 0) s_item = atomicAdd(a.ticket, 1);
-    __syncthreads();
-    const int it = s_item;
+    const int it = spc_take(a.ticket, &s_item);
     if (it >= a.n_items) return;
     const int2 q = a.queue[it];
     const int id = q.x;
     if (q.y == -1) {
       si_prepare(a, id, si_sm);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicExch(a.pdone + id, 1);
-      }
+      spc_publish(a.pdone + id, false);
     } else if (q.y >= 0) {
       if (tid == 0) spc_wait_ge(a.pdone + id, 1);
       __syncthreads();
       si_tile(a, id, q.y, a.tiles[id], si_sm);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicAdd(a.tdone + id, 1);
-      }
+      spc_publish(a.tdone + id, true);
     } else {
       if (tid == 0) {
         spc_wait_ge(a.pdone + id, 1);  // (a node without tiles -- a root -- has no other path to its own prepare item)
@@ -219,11 +209,7 @@ __global__ void __launch_bounds__(SPC_THREADS, 1) k_selinv_tree(SelInv a) {
       }
       __syncthreads();
       si_finish(a, id);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicExch(a.sdone + id, 1);
-      }
+      spc_publish(a.sdone + id, false);
     }
   }
 }

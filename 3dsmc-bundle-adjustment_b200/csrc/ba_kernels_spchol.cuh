@@ -22,9 +22,9 @@
 //   * The panel goes to HBM/L2 for the backward substitution; the node's update matrix U = L_B L_B^T (+ what its children
 //     pass through) -- two thirds of the multiply-adds, no dependent chain -- is formed by several update items per node
 //     (spc_update_node), for the parent's extend-add.
-// Backward substitution: parents before children (solve items of the tree; k_spchol_solve runs one tree level per launch for
-// the covariance's border columns); L_OO and the stored inverses of the pivot blocks come back into shared memory, the
-// border product is a warp-per-column reduction over the panel in L2.
+// Backward substitution: parents before children (solve items of the tree; the covariance's border columns run the queue's
+// solve items alone, one launch per column); L_OO and the stored inverses of the pivot blocks come back into shared memory,
+// the border product is a warp-per-column reduction over the panel in L2.
 // Every sum has a fixed order: results are bit-identical from run to run and across ranks.
 #pragma once
 #include "ba_kernels_sparse.cuh"
@@ -37,7 +37,7 @@
 #define SPC_MAX_OWN 24
 
 struct SpChol {
-  const int32_t *node, *bord, *children, *rel, *inv, *aent, *perm, *level_nodes;
+  const int32_t *node, *bord, *children, *rel, *inv, *aent, *perm;
   const double *S, *dsq, *b;  // stored upper blocks of S, LM damping D^2 [6 n_cam], right-hand side [6 n_cam] (by camera)
   double *panel, *U, *ru;     // per node: factor panel, update matrix (dense lower incl. full diagonal blocks), rhs update [6 nb]
   double *z, *linv, *ypos;    // by elimination position: forward-substituted rhs [6], inverse pivot blocks [36], solution [6]
@@ -161,7 +161,15 @@ __device__ __forceinline__ void spc_tri(int p, int &i, int &j) {
   j = p - r * (r + 1) / 2;
 }
 
-// factorisation of the front of node `id` by the calling thread block (SPC_THREADS threads, spc_factor_smem bytes at spc_sm)
+// the take / wait / publish steps of the persistent tree kernels (k_spchol_tree, k_selinv_tree).  Take: the next queue item
+// from the ticket counter, between two barriers (the first: the previous item's shared memory is no longer in use).
+__device__ __forceinline__ int spc_take(int *ticket, int *s_item) {
+  __syncthreads();
+  if (threadIdx.x == 0) *s_item = atomicAdd(ticket, 1);
+  __syncthreads();
+  return *s_item;
+}
+// wait (one thread) until a completion counter reaches `want`
 __device__ __forceinline__ void spc_wait_ge(const int *flag, int want) {
   int v;
   for (;;) {
@@ -170,6 +178,19 @@ __device__ __forceinline__ void spc_wait_ge(const int *flag, int want) {
     __nanosleep(64);
   }
 }
+// publish an item: barrier (every thread's writes of the item are issued), device-scope fence, then the counter -- set to 1
+// for the one item of its kind a node has, one more for a tile
+__device__ __forceinline__ void spc_publish(int *counter, bool tile) {
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (tile)
+      atomicAdd(counter, 1);
+    else
+      atomicExch(counter, 1);
+  }
+}
+// factorisation of the front of node `id` by the calling thread block (SPC_THREADS threads, spc_factor_smem bytes at spc_sm)
 // (udone / tiles: completion counters of k_spchol_tree -- the node waits for its children's update matrices only AFTER it has
 //  assembled its stored blocks of S, which do not depend on them)
 // NR right-hand-side rows (1: b; 5: b and the four border columns), row r of the own cameras at zf[r * C6 ..]
@@ -519,7 +540,7 @@ __device__ __forceinline__ void spc_update_node(const SpChol &a, int id, int til
   }
 }
 
-// backward substitution of one tree level (parents are done): y_O = L_OO^-T (z_O - L_BO^T y_B)
+// backward substitution of one node (its parent is done): y_O = L_OO^-T (z_O - L_BO^T y_B)
 __device__ __forceinline__ void spc_solve_node(const SpChol &a, int id, LmState *st, double *spc_sm) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
@@ -586,12 +607,6 @@ __device__ __forceinline__ void spc_solve_node(const SpChol &a, int id, LmState 
     a.yc[6 * (size_t)a.perm[k0 + i / 6] + i % 6] = v;
   }
 }
-__global__ void __launch_bounds__(SPC_THREADS, 1)
-k_spchol_solve(SpChol a, int lvl_first, LmState *st, int gate) {
-  if (!gate_open(st, gate)) return;
-  extern __shared__ __align__(16) double spc_sm[];
-  spc_solve_node(a, a.level_nodes[lvl_first + blockIdx.x], st, spc_sm);
-}
 
 // ---------------------------------------------------------------------------------------------
 // The whole linear solve in ONE launch: a persistent grid (one thread block per SM) works through a queue of items --
@@ -606,6 +621,7 @@ k_spchol_solve(SpChol a, int lvl_first, LmState *st, int gate) {
 // Compared with one launch per tree level this removes 3 x levels launches and, more important, lets a node start as
 // soon as ITS children are done instead of when the slowest node of the level below is: the linear solve is bound by
 // the longest root-to-leaf chain of the tree, not by the sum of the per-level maxima.
+// The queue is built on the host (spq_cholesky, ba_sparse_symbolic.h; tests/test_tree_queue_order.py checks the order).
 // Counters are zeroed by the host before the launch; producers publish with a device-scope fence before the counter
 // update, consumers read other blocks' results through L2 (__ldcg).
 // ---------------------------------------------------------------------------------------------
@@ -623,30 +639,19 @@ k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
   __shared__ int s_item;
   const int tid = threadIdx.x;
   for (;;) {
-    __syncthreads();  // (the previous item's shared memory is no longer in use)
-    if (tid == 0) s_item = atomicAdd(t.ticket, 1);
-    __syncthreads();
-    const int it = s_item;
+    const int it = spc_take(t.ticket, &s_item);
     if (it >= t.n_items) return;
     const int2 q = t.queue[it];
     const int id = q.x;
     const int32_t *N = a.node + (size_t)id * SPSYM_NODE_INTS;
     if (q.y == -1) {
       spc_factor_node<NR>(a, id, it == 0, st, spc_sm, t.udone, t.tiles);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicExch(t.fdone + id, 1);
-      }
+      spc_publish(t.fdone + id, false);
     } else if (q.y >= 0) {
       if (tid == 0) spc_wait_ge(t.fdone + id, 1);
       __syncthreads();
       spc_update_node<NR>(a, id, q.y, t.tiles[id], spc_sm);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicAdd(t.udone + id, 1);
-      }
+      spc_publish(t.udone + id, true);
     } else {
       if (tid == 0) {
         const int par = N[SPN_PARENT];
@@ -657,11 +662,7 @@ k_spchol_tree(SpChol a, SpTree t, LmState *st, int gate) {
       }
       __syncthreads();
       spc_solve_node(a, id, st, spc_sm);
-      __syncthreads();
-      if (tid == 0) {
-        __threadfence();
-        atomicExch(t.sdone + id, 1);
-      }
+      spc_publish(t.sdone + id, false);
     }
   }
 }

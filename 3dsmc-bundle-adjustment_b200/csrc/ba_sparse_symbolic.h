@@ -22,6 +22,7 @@
 #include <stdint.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <vector>
 
 #define SPSYM_NODE_INTS 16
@@ -518,4 +519,92 @@ inline SpPartition spsym_partition(const SpSymbolic &S, int parts) {
     }
   }
   return R;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Work queues of the persistent tree kernels (k_spchol_tree, k_selinv_tree): items (node, kind), kind >= 0 a tile of the
+// node, SPQ_HEAD its factor / prepare item, SPQ_SOLVE, SPQ_FINISH.  The kernels wait on completion counters and cannot
+// deadlock only because every item an item waits for is earlier in the same launch or was done by an earlier launch over the
+// same counters (tests/test_tree_queue_order.py restates the waits and checks this).
+// ---------------------------------------------------------------------------------------------
+enum { SPQ_HEAD = -1, SPQ_SOLVE = -2, SPQ_FINISH = -3 };
+
+struct SpQueue {
+  std::vector<int32_t> q;      // (node, kind) per item
+  std::vector<int32_t> tiles;  // tiles per node (0: no border, or no head item in this queue)
+  int n_items() const { return (int)(q.size() / 2); }
+};
+
+// tiles of the nodes of a level with `nodes` nodes: more where the level has fewer nodes than the GPU has SMs
+inline int spq_level_tiles(int n_sm, int nodes) { return std::max(1, std::min(8, n_sm / std::max(1, nodes))); }
+
+// Appends the levels of the tree, bottom-up or top-down, restricted to the nodes `keep` accepts (levels without such nodes
+// are skipped).  Per level one pass over its nodes per entry of `kinds`: SPQ_HEAD items (they fix the node's tiles), 0 for
+// the tiles 0 .. tiles - 1 of every node, SPQ_SOLVE or SPQ_FINISH items.
+template <class Keep>
+inline void spq_push_levels(const SpSymbolic &S, int n_sm, bool top_down, Keep keep, std::initializer_list<int> kinds, SpQueue &Q) {
+  for (int k = 0; k < S.n_levels; ++k) {
+    const int l = top_down ? S.n_levels - 1 - k : k;
+    const int32_t *b = S.level_nodes.data() + S.level_ptr[l], *e = S.level_nodes.data() + S.level_ptr[l + 1];
+    const int nodes = (int)std::count_if(b, e, keep);
+    if (!nodes) continue;
+    const int t_lvl = spq_level_tiles(n_sm, nodes);
+    for (const int kind : kinds)
+      for (const int32_t *p = b; p < e; ++p) {
+        const int id = *p;
+        if (!keep(id)) continue;
+        if (kind == SPQ_HEAD) Q.tiles[id] = S.node[(size_t)id * SPSYM_NODE_INTS + SPN_NB] > 0 ? t_lvl : 0;
+        for (int t = 0; t < (kind == 0 ? Q.tiles[id] : 1); ++t) {
+          Q.q.push_back(id);
+          Q.q.push_back(kind == 0 ? t : kind);
+        }
+      }
+  }
+}
+
+// Queue of k_spchol_tree for the items rank `me` runs (me < 0: one GPU runs every part).  Phase A, one launch per part p, is
+// [qA[p], qA[p + 1]): the part's factor levels bottom-up, per level the factor items, then their update tiles.  Phase B,
+// [qB, qB + qB_n): the same for the top part, then the backward substitution levels top-down (top part first, then the
+// subtrees this GPU holds).  One part: phase A is the whole factorisation, phase B the backward substitution.
+struct SpCholQueue : SpQueue {
+  std::vector<int32_t> qA;        // parts + 1
+  int qB = 0, qB_n = 0;
+  std::vector<int32_t> cnt_init;  // completion counters before a solve: 16 tickets, then fdone, udone, sdone per node
+  std::vector<int32_t> topcams;   // cameras of the top part
+};
+inline SpCholQueue spq_cholesky(const SpSymbolic &S, const SpPartition &part, int me, int n_sm) {
+  SpCholQueue Q;
+  const int nn = S.n_nodes;
+  Q.tiles.assign((size_t)nn, 0);
+  for (int p = 0; p < part.parts; ++p) {
+    Q.qA.push_back(Q.n_items());
+    if (me < 0 || p == me) spq_push_levels(S, n_sm, false, [&](int id) { return part.part[id] == p; }, {SPQ_HEAD, 0}, Q);
+  }
+  Q.qB = Q.n_items();
+  Q.qA.push_back(Q.qB);
+  if (part.parts > 1) {
+    spq_push_levels(S, n_sm, false, [&](int id) { return part.part[id] < 0; }, {SPQ_HEAD, 0}, Q);
+    spq_push_levels(S, n_sm, true, [&](int id) { return part.part[id] < 0; }, {SPQ_SOLVE}, Q);
+  }
+  spq_push_levels(S, n_sm, true, [&](int id) { return part.part[id] >= 0 && (me < 0 || part.part[id] == me); }, {SPQ_SOLVE}, Q);
+  Q.qB_n = Q.n_items() - Q.qB;
+  // zero, except "all update tiles done" for the subtree roots other ranks factorise (their update matrices arrive with the
+  // exchange)
+  Q.cnt_init.assign((size_t)3 * nn + 16, 0);
+  for (int id = 0; id < nn; ++id) {
+    const int32_t *N = S.node.data() + (size_t)id * SPSYM_NODE_INTS;
+    if (part.part[id] < 0)
+      for (int k = 0; k < N[SPN_M]; ++k) Q.topcams.push_back(S.perm[N[SPN_K0] + k]);
+    else if (me >= 0 && part.part[id] != me)
+      Q.cnt_init[16 + (size_t)nn + id] = 1 << 20;
+  }
+  return Q;
+}
+
+// Queue of k_selinv_tree: the levels top-down, per level the prepare items, the product tiles, the finish items
+inline SpQueue spq_selinv(const SpSymbolic &S, int n_sm) {
+  SpQueue Q;
+  Q.tiles.assign((size_t)S.n_nodes, 0);
+  spq_push_levels(S, n_sm, true, [](int) { return true; }, {SPQ_HEAD, 0, SPQ_FINISH}, Q);
+  return Q;
 }

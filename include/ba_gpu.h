@@ -340,6 +340,13 @@ int ba_sparse_symbolic_get(const ba_spsym *h, int32_t which, int32_t *dst);
  * part[node] = owning rank, -1 = top part (factorised by every rank).  work[0..2] = block operations of the whole tree, of the
  * top part, of the most loaded rank.  Returns the number of parts in force (1: tree too small, the solve stays replicated). */
 int ba_sparse_symbolic_partition(const ba_spsym *h, int32_t parts, int32_t *part, double work[3]);
+/* Work queue of a persistent tree kernel on n_sm SMs (csrc/ba_sparse_symbolic.h): which = 0 the sparse Cholesky's
+ * (spq_cholesky) for `parts` parts and the items rank `rank` runs (-1: one GPU runs every part), which = 1 the selected
+ * inversion's (spq_selinv; parts and rank unused).  info[0..3] = items, then (which = 0) qB, qB_n and the number of top-part
+ * cameras.  Arrays, each may be NULL: queue (node, kind per item; kind >= 0 tile, -1 factor / prepare, -2 solve, -3 finish),
+ * tiles (per node), and for which = 0 qA (parts + 1), cnt_init (3 nodes + 16) and topcams.  Returns the parts in force. */
+int ba_sparse_symbolic_queue(const ba_spsym *h, int32_t which, int32_t parts, int32_t rank, int32_t n_sm, int32_t info[4],
+                             int32_t *queue, int32_t *tiles, int32_t *qA, int32_t *cnt_init, int32_t *topcams);
 
 void ba_sparse_symbolic_destroy(ba_spsym *h);
 

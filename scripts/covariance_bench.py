@@ -5,7 +5,10 @@ Per problem, in one process: an LM solve of --steps exact steps (tolerances disa
 covariance call at the solved state, warmed up, timed --repeats times with a host clock around the call (it returns after a
 device synchronisation and the copies of its outputs) in two variants: cameras + intrinsics only, and with the points.
 Prints JSON lines (device name and power limit first, from nvidia-smi in the same process).
-Usage: python scripts/covariance_bench.py [--steps 10] [--repeats 5] [--sizes 3000,10000] [--out FILE]"""
+--dump DIR also writes every output to DIR/<problem>.npz, for a bitwise comparison of two builds: both covariance variants,
+camera pairs, and ba_gpu_covariance_blocks with every kind of pair (far camera pairs, camera-point, point-point and the
+intrinsics against each).  --closures adds the 120-camera loop-closure problems of tests/irregular_problems.py.
+Usage: python scripts/covariance_bench.py [--steps 10] [--repeats 5] [--sizes 3000,10000] [--out FILE] [--dump DIR] [--closures]"""
 import argparse
 import json
 import os
@@ -22,6 +25,7 @@ import ba_b200  # noqa: E402
 from ref_sparse_bench import cfg3ref, long_sequence  # noqa: E402
 
 OUT = None
+DUMP = None
 
 
 def emit(d):
@@ -30,6 +34,32 @@ def emit(d):
     if OUT:
         with open(OUT, "a") as f:
             f.write(line + "\n")
+
+
+def requests(p, rng):
+    """Camera pairs that share a point (for covariance(pairs=)) and pairs of every kind (for covariance_blocks)."""
+    order = np.argsort(p.pt_idx, kind="stable")
+    cam, pt = p.cam_idx[order], p.pt_idx[order]
+    same = (pt[1:] == pt[:-1]) & (cam[1:] != cam[:-1])
+    co = np.unique(np.sort(np.stack([cam[:-1][same], cam[1:][same]], axis=1), axis=1), axis=0)
+    pairs = co[rng.choice(len(co), size=min(200, len(co)), replace=False)]
+    cams, pts = rng.integers(0, p.n_cam, 12), rng.integers(0, p.n_pt, 12)
+    blocks = [(("cam", 1), ("cam", p.n_cam - 1)), (("cam", 0), ("cam", p.n_cam // 2)), (("intr", 0), ("intr", 0))]
+    blocks += [(("cam", int(a)), ("cam", int(b))) for a, b in zip(cams[:6], cams[6:])]
+    blocks += [(("cam", int(a)), ("pt", int(b))) for a, b in zip(cams, pts)]
+    blocks += [(("pt", int(a)), ("pt", int(b))) for a, b in zip(pts[:6], pts[6:])]
+    blocks += [(("intr", 0), ("cam", int(a))) for a in cams[:4]] + [(("pt", int(a)), ("intr", 0)) for a in pts[:4]]
+    return pairs, blocks
+
+
+def dump(name, s, p):
+    pairs, blocks = requests(p, np.random.default_rng(7))
+    c = s.covariance(points=True, pairs=pairs)
+    out = {k: v for k, v in c.items() if v is not None}
+    out["cameras_intrinsics_cam"] = s.covariance(points=False)["cam"]
+    out["blocks"] = np.concatenate([b.reshape(-1) for b in s.covariance_blocks(blocks)])
+    os.makedirs(DUMP, exist_ok=True)
+    np.savez(os.path.join(DUMP, name + ".npz"), **out)
 
 
 def bench(name, p, steps, repeats):
@@ -50,6 +80,8 @@ def bench(name, p, steps, repeats):
             c = s.covariance(points=points)
             ts.append((time.perf_counter() - t0) * 1e3)
         out[variant + "_ms"] = dict(median=float(np.median(ts)), min=float(np.min(ts)), all=ts)
+    if DUMP:
+        dump(name, s, p)
     out["cov_intr_diag"] = np.diag(c["intr"]).tolist()
     out["cov_cam_trace_median"] = float(np.median(np.trace(c["cam"], axis1=1, axis2=2)))
     s.close()
@@ -57,14 +89,16 @@ def bench(name, p, steps, repeats):
 
 
 def main():
-    global OUT
+    global OUT, DUMP
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--repeats", type=int, default=5)
     ap.add_argument("--sizes", default="3000,10000")
     ap.add_argument("--out", default=None)
+    ap.add_argument("--dump", metavar="DIR", default=None)
+    ap.add_argument("--closures", action="store_true")
     a = ap.parse_args()
-    OUT = a.out
+    OUT, DUMP = a.out, a.dump
     try:
         smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
                              text=True, timeout=30).stdout.strip()
@@ -72,6 +106,11 @@ def main():
         smi = "nvidia-smi unavailable: %s" % e
     emit(dict(what="device", nvidia_smi=smi))
     bench("cfg3ref", cfg3ref(), a.steps, a.repeats)
+    if a.closures:
+        sys.path.insert(0, os.path.join(ROOT, "tests"))
+        import irregular_problems
+        for case in "abc":
+            bench("closure_" + case, irregular_problems.closure_problem(case), a.steps, a.repeats)
     for n_kf in [int(x) for x in a.sizes.split(",") if x]:
         bench("ref_sequence_%d" % n_kf, long_sequence(n_kf), a.steps, a.repeats)
 

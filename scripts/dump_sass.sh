@@ -7,7 +7,7 @@ cd "$(dirname "$0")/.." || exit 1
 SO=3dsmc-bundle-adjustment_b200/libba_gpu.so
 ROUND=${1:-r02}
 shift
-KERNELS=${*:-k_sp_schur k_spchol_tree k_spchol_solve kf_cam_blocks kf_schur_pass1 kf_linearize k_linearize}
+KERNELS=${*:-k_sp_schur k_spchol_tree kf_cam_blocks kf_schur_pass1 kf_linearize k_linearize}
 for k in $KERNELS; do
   if [ "$ROUND" = r02 ]; then pat="$k"; else pat="Function : _Z[0-9]+${k}[^_]"; fi
   cuobjdump -sass $SO | awk -v k="$pat" '/Function :/{p=($0 ~ k)} p' |

@@ -35,6 +35,12 @@ class Symbolic:
             work = np.zeros(3)
             got = lib.ba_sparse_symbolic_partition(h, parts, ba_b200.capi.ip(part), ba_b200.capi.dp(work))
             self.partitions[parts] = (got, part[:self.n_nodes].copy(), work.copy())
+        self.queues = {}
+        for n_sm in (148, 5):  # (a B200, and few SMs: more tiles per node on the upper levels)
+            self.queues[("selinv", n_sm)] = _queue(lib, h, self.n_nodes, 1, 1, -1, n_sm)
+            for parts in (1, 2, 3, 4, 8):  # work queues of k_spchol_tree: one GPU running every part, then each rank's own
+                for rank in range(-1, parts if parts > 1 else 0):
+                    self.queues[("chol", parts, rank, n_sm)] = _queue(lib, h, self.n_nodes, 0, parts, rank, n_sm)
         lib.ba_sparse_symbolic_destroy(h)
         self.node = self.node.reshape(-1, NI)
         self.aent = self.aent.reshape(-1, 4)
@@ -46,6 +52,26 @@ class Symbolic:
         return dict(nodes=self.n_nodes, levels=self.n_levels, max_m=int(m.max()), max_nb=int(nb.max()), mean_m=float(m.mean()),
                     mean_nb=float(nb.mean()), max_front=self.info[5], panel_MB=self.info[3] * 288 / 1e6, u_MB=self.info[4] * 288 / 1e6,
                     gflop=self.info[9] / 1e9, crit_blocks=self.info[10], level_sizes=lev.tolist())
+
+
+def _queue(lib, h, nn, which, parts, rank, n_sm):
+    """One work queue through the C-ABI (ba_sparse_symbolic_queue): dict of items (n x 2: node, kind), tiles, and for the sparse
+    Cholesky the parts in force, qA, qB, qB_n, cnt_init, topcams."""
+    ip = ba_b200.capi.ip
+    info = np.zeros(4, dtype=np.int32)
+    got = lib.ba_sparse_symbolic_queue(h, which, parts, rank, n_sm, ip(info), None, None, None, None, None)
+    if got < 1:
+        raise RuntimeError("ba_sparse_symbolic_queue rc=%d" % got)
+    q = np.zeros(2 * max(1, info[0]), dtype=np.int32)
+    tiles = np.zeros(max(1, nn), dtype=np.int32)
+    qA = np.zeros(got + 1, dtype=np.int32)
+    cnt = np.zeros(3 * nn + 16, dtype=np.int32)
+    top = np.zeros(max(1, info[3]), dtype=np.int32)
+    lib.ba_sparse_symbolic_queue(h, which, parts, rank, n_sm, ip(info), ip(q), ip(tiles), ip(qA), ip(cnt), ip(top))
+    out = dict(items=q[:2 * info[0]].reshape(-1, 2), tiles=tiles[:nn])
+    if which == 0:
+        out.update(parts=got, qA=qA, qB=int(info[1]), qB_n=int(info[2]), cnt_init=cnt, topcams=top[:info[3]])
+    return out
 
 
 def covisibility_blocks(cam_idx, pt_idx, n_cam, fixed_cam):
