@@ -1328,11 +1328,13 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   RES(q, nc * 48);
   RES(Minv, nc * 288);
   RES(pc_lin, (size_t)ctx->nblk_obs * 8);
-  RES(pc_cand, (size_t)ctx->nblk_obs * 8);
-  RES(pc_mcc, (size_t)ctx->nblk_obs * 8);
+  // model cost change / candidate cost partials: per observation block, or per point tile (kf_step_eval)
+  RES(pc_cand, (size_t)(ctx->fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
+  RES(pc_mcc, (size_t)(ctx->fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
   RES(pe_gmax, (size_t)ctx->nblk_ent * 8);
   RES(pe_xn, (size_t)ctx->nblk_ent * 8);
-  RES(pe_step, (size_t)ctx->nblk_ent * 8);
+  // step norm partials: per entry block, or per block of cameras + intrinsics (k_candidate) followed by one per point tile
+  RES(pe_step, (size_t)(ctx->fact ? cdiv(n_cam + 1, BA_THREADS) + ctx->n_tiles : ctx->nblk_ent) * 8);
   RES(pcam_rho, (size_t)ctx->nblk_cam * 8);
   RES(pcam_bb, (size_t)ctx->nblk_cam * 8);
   RES(pcam_pq, (size_t)ctx->nblk_cam * 8);
@@ -1824,16 +1826,14 @@ static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int pa
     const double *intr = P<double>(ctx->intr);
     if (passes & 1) {
       if (ctx->staged) {
-        LAUNCH((kf_schur_pass1<0, 1>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-               ctx->Fp_, (const int32_t *)nullptr, (const double2 *)nullptr, (const double *)nullptr, (const double *)nullptr,
-               ctx->cp, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
-               P<double>(ctx->Vinv), P<double>(ctx->sp), (const double *)nullptr, (double *)nullptr, P<double>(ctx->ts), st, gate);
+        LAUNCH((kf_schur_pass1<1>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
+               ctx->Fp_, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
+               P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->ts), st, gate);
       } else {
         LAUNCH(k_pack_camx, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, v, P<double>(ctx->geo), P<double>(ctx->camx), st, gate);
-        LAUNCH((kf_schur_pass1<0, 0>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-               ctx->Fp_, (const int32_t *)nullptr, (const double2 *)nullptr, (const double *)nullptr, (const double *)nullptr,
-               ctx->cp, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
-               P<double>(ctx->Vinv), P<double>(ctx->sp), (const double *)nullptr, (double *)nullptr, P<double>(ctx->ts), st, gate);
+        LAUNCH((kf_schur_pass1<0>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
+               ctx->Fp_, P<double>(ctx->geo), v, P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr,
+               P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->ts), st, gate);
       }
     }
     if (passes & 2)
@@ -2332,52 +2332,64 @@ static int enqueue_lm_iteration(ba_gpu_ctx *ctx) {
   int rc = ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY ? solve_implicit(ctx) : solve_explicit(ctx);
   if (rc) return rc;
   phase_mark(ctx, BA_PHASE_SUBSTITUTION);
+  // step evaluation: back-substitution y = (y_c, y_p), the model cost change, the candidate x+ and its cost
+  int nblk_mcc = ctx->nblk_obs, nblk_step = ctx->nblk_ent;
   if (ctx->fact) {
-    const double *intr = P<double>(ctx->intr);
-    // (pass 1 projects every observation again instead of reading point-major records; the camera run staged as in the product)
-#define BACKSUB(STAGED)                                                                                                         \
-  LAUNCH((kf_schur_pass1<1, STAGED>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr),                      \
-         P<int32_t>(ctx->pm_cam), ctx->Fp_, P<int32_t>(ctx->pm_pt), P<double2>(ctx->pm_uv), P<double>(ctx->pose),             \
-         P<double>(ctx->pt), ctx->cp, P<double>(ctx->geo), P<double>(ctx->yc), P<double>(ctx->camx), P<int32_t>(ctx->tile_lo), \
-         P<int32_t>(ctx->tile_span), intr, P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->gp), P<double>(ctx->yp),  \
-         P<double>(ctx->ys), st, GATE_RUN)
+    // the candidate cameras and intrinsics first (no points: entries [0, n_cam]); then one point-major pass over the tiles does
+    // the rest (camera run staged in shared memory)
+    const int nblk_cc = cdiv(ctx->n_cam + 1, BA_THREADS);
+    LAUNCH(k_candidate, nblk_cc, BA_THREADS, 0, ctx->n_cam, 0, K, ctx->fixed_cam, P<double>(ctx->pose), P<double>(ctx->pt),
+           P<double>(ctx->intr), P<double>(ctx->yc), P<double>(ctx->yp), P<double>(ctx->yk), P<double>(ctx->sc), P<double>(ctx->sp),
+           P<double>(ctx->sk), P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c), P<double>(ctx->pe_step), st,
+           GATE_RUN, ctx->rank == 0 ? 1.0 : 0.0);
+#define STEP_EVAL(STAGED)                                                                                                      \
+  LAUNCH((kf_step_eval<STAGED>), ctx->n_tiles, BA_THREADS, 0, ctx->n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),   \
+         P<int32_t>(ctx->pm_pt), P<double2>(ctx->pm_uv), P<double>(ctx->pose), P<double>(ctx->pt), ctx->cp, P<double>(ctx->geo), \
+         P<double>(ctx->yc), P<double>(ctx->camx), P<double>(ctx->pose_c), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span),  \
+         P<double>(ctx->intr), P<double>(ctx->intr_c), P<double>(ctx->Vinv), P<double>(ctx->sp), P<double>(ctx->gp),             \
+         P<double>(ctx->yp), P<double>(ctx->ys), P<double>(ctx->pt_c), P<double>(ctx->pc_mcc), P<double>(ctx->pe_step), nblk_cc, \
+         P<double>(ctx->pc_cand), st, GATE_RUN)
     if (ctx->staged) {
-      BACKSUB(1);
+      STEP_EVAL(1);
     } else {
       LAUNCH(k_pack_camx, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->yc), P<double>(ctx->geo), P<double>(ctx->camx),
              st, GATE_RUN);
-      BACKSUB(0);
+      STEP_EVAL(0);
     }
-#undef BACKSUB
-    LAUNCH(kf_model_cost, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx), ctx->Fc_,
-           P<double>(ctx->geo), P<double>(ctx->yc), intr, P<double>(ctx->ys), P<double>(ctx->pc_mcc), st, GATE_RUN);
-  } else
-  DISPATCH_DK(D, K, {
-    // back-substitution y_p = V^-1 (-g_p - W^T y_c)
-    LAUNCH((k_schur_pass1<DD, KK, 1>), ctx->pl_tiles, BA_THREADS, 0, ctx->n_pt, ctx->pl_tile_pts, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-           ctx->Jp_, P<double>(ctx->yc), P<double>(ctx->yk), P<double>(ctx->Vinv), P<double>(ctx->gp), P<double>(ctx->yp), st,
-           GATE_RUN, 0);
-    fork_side(ctx);  // the model cost change does not depend on the candidate point
-    LAUNCH((k_model_cost<DD, KK>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
-           ctx->Jc_, P<double>(ctx->yc), P<double>(ctx->yp), P<double>(ctx->yk), P<double>(ctx->pc_mcc), st, GATE_RUN);
-    fork_main(ctx);
-  });
-  if (!ctx->forking) phase_mark(ctx, BA_PHASE_BACKSUB);
-  LAUNCH(k_candidate, ctx->nblk_ent, BA_THREADS, 0, ctx->n_cam, ctx->n_pt, K, ctx->fixed_cam, P<double>(ctx->pose), P<double>(ctx->pt),
-         P<double>(ctx->intr), P<double>(ctx->yc), P<double>(ctx->yp), P<double>(ctx->yk), P<double>(ctx->sc), P<double>(ctx->sp),
-         P<double>(ctx->sk), P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c), P<double>(ctx->pe_step), st,
-         GATE_RUN, ctx->rank == 0 ? 1.0 : 0.0);
-  DISPATCH_D(D, {
-    LAUNCH((k_cost<DD>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
-           P<double2>(ctx->uv), P<double>(ctx->depthv), P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c),
-           ctx->cp, P<double>(ctx->pc_cand), st, GATE_RUN);
-  });
-  join(ctx);
-  phase_mark(ctx, ctx->forking ? BA_PHASE_BACKSUB : BA_PHASE_CANDIDATE);
+#undef STEP_EVAL
+    nblk_mcc = ctx->n_tiles;
+    nblk_step = nblk_cc + ctx->n_tiles;
+    // (one kernel does both phases' work: all of it is reported as back-substitution, the candidate phase is empty)
+    phase_mark(ctx, BA_PHASE_BACKSUB);
+    phase_mark(ctx, BA_PHASE_CANDIDATE);
+  } else {
+    DISPATCH_DK(D, K, {
+      // back-substitution y_p = V^-1 (-g_p - W^T y_c)
+      LAUNCH((k_schur_pass1<DD, KK, 1>), ctx->pl_tiles, BA_THREADS, 0, ctx->n_pt, ctx->pl_tile_pts, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
+             ctx->Jp_, P<double>(ctx->yc), P<double>(ctx->yk), P<double>(ctx->Vinv), P<double>(ctx->gp), P<double>(ctx->yp), st,
+             GATE_RUN, 0);
+      fork_side(ctx);  // the model cost change does not depend on the candidate point
+      LAUNCH((k_model_cost<DD, KK>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
+             ctx->Jc_, P<double>(ctx->yc), P<double>(ctx->yp), P<double>(ctx->yk), P<double>(ctx->pc_mcc), st, GATE_RUN);
+      fork_main(ctx);
+    });
+    if (!ctx->forking) phase_mark(ctx, BA_PHASE_BACKSUB);
+    LAUNCH(k_candidate, ctx->nblk_ent, BA_THREADS, 0, ctx->n_cam, ctx->n_pt, K, ctx->fixed_cam, P<double>(ctx->pose), P<double>(ctx->pt),
+           P<double>(ctx->intr), P<double>(ctx->yc), P<double>(ctx->yp), P<double>(ctx->yk), P<double>(ctx->sc), P<double>(ctx->sp),
+           P<double>(ctx->sk), P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c), P<double>(ctx->pe_step), st,
+           GATE_RUN, ctx->rank == 0 ? 1.0 : 0.0);
+    DISPATCH_D(D, {
+      LAUNCH((k_cost<DD>), ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
+             P<double2>(ctx->uv), P<double>(ctx->depthv), P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c),
+             ctx->cp, P<double>(ctx->pc_cand), st, GATE_RUN);
+    });
+    join(ctx);
+    phase_mark(ctx, ctx->forking ? BA_PHASE_BACKSUB : BA_PHASE_CANDIDATE);
+  }
   sync_flags(ctx);
   {
     const double *const parts[3] = {P<double>(ctx->pc_mcc), P<double>(ctx->pe_step), P<double>(ctx->pc_cand)};
-    const int nblks[3] = {ctx->nblk_obs, ctx->nblk_ent, ctx->nblk_obs};
+    const int nblks[3] = {nblk_mcc, nblk_step, nblk_mcc};
     PartRef grp[3];
     reduce_scalar_group(ctx, 3, parts, nblks, 3, GATE_RUN, grp);
     const PartRef rm = grp[0], rs = grp[1], rc2 = grp[2];

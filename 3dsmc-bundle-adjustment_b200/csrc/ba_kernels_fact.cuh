@@ -18,12 +18,12 @@
 // Layout and readers:
 //   geo  per camera: R (from k_cam_geo, the one R every projection uses) and s_c.
 //   Fc_  camera-major r / g, written by kf_linearize; read by kf_cam_blocks,
-//        kf_schur_pass2, kf_schur_diag, kf_model_cost and k_sp_schur.
+//        kf_schur_pass2, kf_schur_diag and k_sp_schur.
 //   Fp_  point-major r / g, only for the implicit solver (its PCG product runs
-//        kf_schur_pass1<0, .> every iteration); filled by kf_pt_linearize<1, .>.
+//        kf_schur_pass1 every iteration); filled by kf_pt_linearize<1, .>.
 //        The block-sparse solvers neither allocate nor fill it: kf_pt_linearize<0, .>
-//        reduces V, g_p straight from the projection, and the back-substitution
-//        kf_schur_pass1<1, .> projects again.  All projections go through
+//        reduces V, g_p straight from the projection, and the step evaluation
+//        kf_step_eval projects again.  All projections go through
 //        project_obs with R from geo, so a recomputed g equals the stored one bit for bit.
 #pragma once
 #include "ba_kernels.cuh"
@@ -36,7 +36,8 @@ struct FPlanes {
 // per-camera record, 16 doubles = one 128-byte line: R (9, row-major), s (6, zero
 // for the constant pose :299 so that its Jacobian columns vanish), pad
 #define BA_CAMREC 16
-// shared-memory staging of a point tile's camera run (kf_pt_linearize, kf_schur_pass1): at most BA_STAGE_CAMS cameras
+// shared-memory staging of a point tile's camera run (kf_pt_linearize, kf_schur_pass1, kf_step_eval): at most BA_STAGE_CAMS
+// cameras
 #define BA_STAGE_CAMS 96
 #define BA_STAGE_REC 18
 struct CamRec {
@@ -391,16 +392,15 @@ kf_point_inverse(int n_pt, const double *__restrict__ V, const double *__restric
 }
 
 // ------------------------------------------------------------------ pass 1 (point-major)
-//   MODE 0: ts_p = s .* V^-1 (s .* sum_o Jpu^T (Jc x_c))                        (matvec)
-//   MODE 1: y_p  = V^-1 (-g_p - s .* sum_o Jpu^T (Jc y_c)),  ys_p = s .* y_p    (back-substitution)
-// Algorithmic traffic: MODE 0 36 B/obs (g 32 + cam idx 4); MODE 1 24 B/obs (uv 16 + cam and point idx 8: g is projected
-// again, by project_obs from the same inputs as kf_pt_linearize, so it is the g the linearisation used); + 80 B/point.
-// The per-camera operand (s.*x (6), R (9), MODE 1 also the centre (3)) of every
+//   ts_p = s .* V^-1 (s .* sum_o Jpu^T (Jc x_c))      (the implicit solver's matvec)
+// Algorithmic traffic: 36 B/obs (g 32 + cam idx 4) + 80 B/point.
+// The per-camera operand (s.*x (6), R (9)) of every
 // observation comes from SHARED MEMORY: a tile of 128 consecutive points touches a
 // short run of cameras (tracks are runs of consecutive keyframes, points are numbered
 // by first appearance), so the CTA stages that run once, 144-byte records (bank-conflict
 // free for 8 consecutive cameras).  STAGED = 0 is the fallback for inputs whose
 // tiles span more than BA_STAGE_CAMS cameras: the records are gathered through L1.
+// kf_step_eval (below) stages the same way.
 
 // per point tile: first camera and number of cameras spanned by its observations
 __global__ void __launch_bounds__(BA_THREADS)
@@ -437,15 +437,13 @@ k_tile_cam_range(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t 
   }
 }
 
-template <int MODE, int STAGED>
-__global__ void __launch_bounds__(BA_THREADS, MODE ? 3 : 5)
+template <int STAGED>
+__global__ void __launch_bounds__(BA_THREADS, 5)
 kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam, FPlanes F,
-               const int32_t *__restrict__ pm_pt, const double2 *__restrict__ pm_uv, const double *__restrict__ pose,
-               const double *__restrict__ pt, CostParams cp,
                const double *__restrict__ geo, const double *__restrict__ x, const double *__restrict__ camx,
                const int32_t *__restrict__ tile_lo, const int32_t *__restrict__ tile_span, const double *__restrict__ intr,
-               const double *__restrict__ Vinv, const double *__restrict__ sp, const double *__restrict__ gp,
-               double *__restrict__ out, double *__restrict__ out_s, const LmState *st, int gate) {
+               const double *__restrict__ Vinv, const double *__restrict__ sp, double *__restrict__ out_s, const LmState *st,
+               int gate) {
   if (!gate_open(st, gate)) return;
   constexpr int TOBS = 512;
   __shared__ double sm[3 * TOBS];
@@ -453,7 +451,7 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
   const double4 K = load_intr(intr);
   int cam_lo = 0;
   if (STAGED) {
-    constexpr int NREC = MODE ? 18 : 16;
+    constexpr int NREC = 16;
     cam_lo = tile_lo[blockIdx.x];
     const int n = tile_span[blockIdx.x];
     for (int idx = threadIdx.x; idx < n * NREC; idx += BA_THREADS) {
@@ -465,7 +463,7 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
       else if (k < 15)
         v = geo[c * BA_CAMREC + (k - 6)];
       else
-        v = MODE ? pose[7 * c + 4 + (k - 15)] : 0.0;
+        v = 0.0;
       rec[rc * BA_STAGE_REC + k] = v;
     }
     __syncthreads();
@@ -475,34 +473,17 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
       [&](int s, double *v) {
         const int c = pm_cam[s];
         double2 c0, c1, c2, c3, c4, c5, c6, c7;
-        double C[3];
         if (STAGED) {
           const double2 *cx = reinterpret_cast<const double2 *>(rec + (c - cam_lo) * BA_STAGE_REC);
           c0 = cx[0]; c1 = cx[1]; c2 = cx[2]; c3 = cx[3]; c4 = cx[4]; c5 = cx[5]; c6 = cx[6]; c7 = cx[7];
-          if (MODE == 1) {
-            const double2 c8 = cx[8];
-            C[0] = c7.y; C[1] = c8.x; C[2] = c8.y;
-          }
         } else {
           const double2 *cx = reinterpret_cast<const double2 *>(camx + (size_t)BA_CAMREC * c);
           c0 = ldg2(cx); c1 = ldg2(cx + 1); c2 = ldg2(cx + 2); c3 = ldg2(cx + 3); c4 = ldg2(cx + 4); c5 = ldg2(cx + 5);
           c6 = ldg2(cx + 6); c7 = ldg2(cx + 7);
-          if (MODE == 1) {
-            const double *P = pose + 7 * (size_t)c;
-            C[0] = ldg1(P + 4); C[1] = ldg1(P + 5); C[2] = ldg1(P + 6);
-          }
         }
         const double xx[6] = {c0.x, c0.y, c1.x, c1.y, c2.x, c2.y};
         const double R[9] = {c3.x, c3.y, c4.x, c4.y, c5.x, c5.y, c6.x, c6.y, c7.x};
-        ObsGeo o;
-        if (MODE == 0) {
-          o = load_geo(F, s, K.x, K.y);
-        } else {
-          double X3[3];
-          load_pt(pt, pm_pt[s], X3);
-          const ObsProj pr = project_obs(R, C, X3, lds2(pm_uv + s), K, cp);
-          o = obs_geo(make_double4(pr.xz, pr.yz, pr.iz, pr.w), K.x, K.y);
-        }
+        const ObsGeo o = load_geo(F, s, K.x, K.y);
         double a0, a1;
         jc_dot(o, xx, a0, a1);
         jp_tmul(o, R, a0, a1, v);
@@ -515,15 +496,7 @@ kf_schur_pass1(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *_
         double b[3], t[3];
 #pragma unroll
         for (int k = 0; k < 3; ++k) b[k] = s[k] * sum[k];
-        if (MODE == 1) {
-#pragma unroll
-          for (int k = 0; k < 3; ++k) b[k] = -gp[3 * (size_t)p + k] - b[k];
-        }
         sym3_mul(vi, b, t);
-        if (MODE == 1) {
-#pragma unroll
-          for (int k = 0; k < 3; ++k) out[3 * (size_t)p + k] = t[k];
-        }
         // pre-scaled copy, padded to 32 bytes: one 256-bit gather per observation in pass 2
         double4 *o4 = reinterpret_cast<double4 *>(out_s) + p;
         *o4 = make_double4(s[0] * t[0], s[1] * t[1], s[2] * t[2], 0.0);
@@ -652,35 +625,178 @@ kf_schur_diag(int n_items, const BaItem *__restrict__ items, const int32_t *__re
   }
 }
 
-// ------------------------------------------------------------------ model cost change
-__global__ void __launch_bounds__(BA_THREADS)
-kf_model_cost(int n_obs, const int32_t *__restrict__ cam_idx, const int32_t *__restrict__ pt_idx, FPlanes F,
-              const double *__restrict__ geo, const double *__restrict__ yc, const double *__restrict__ intr,
-              const double *__restrict__ ys, double *__restrict__ part, const LmState *st, int gate) {
+// ------------------------------------------------------------------ step evaluation
+// One point-major pass over a tile of BA_TILE_PTS points evaluates the LM step:
+//   1. back-substitution  y_p = V^-1 (-g_p - s .* sum_o Jpu^T (Jc y_c)),  ys_p = s .* y_p  (J rebuilt by project_obs from
+//      the inputs of kf_pt_linearize, so it is the J the linearisation used);
+//   2. candidate point  pt_c = p + y_p .* s_p  and its share of |x+ - x|^2;
+//   3. per observation, the model cost term m (r + m / 2), m = Jc (s_c .* y_c) + Jp ys_p (r and J projected again: the
+//      bits kf_linearize stored), and the candidate cost rho / 2 at (pose_c, pt_c) (k_cost's arithmetic): two more loops
+//      over the tile's observations, whose indices and measurements then come from L2.
+// The candidate cameras pose_c come first (k_candidate over the cameras and the intrinsics entry only).  Per-tile partials of
+// the three sums (fixed-order block sums, no atomics) go to part_mcc, part_step[step_off + tile] and part_cand.  The camera
+// run is staged as in kf_schur_pass1: s.*y_c, R and centre (18 doubles), and the candidate camera's R(q+) and centre (12);
+// STAGED = 0 gathers s.*y_c and R from camx (k_pack_camx), the centre from pose, and forms R(q+) per observation.
+// Algorithmic traffic: 24 B/obs (uv 16, cam and point idx 8) + 224 B/point (pt 24, V^-1 48, s_p 24, g_p 24 read; y_p 24,
+// ys_p 32, pt_c 24 written; the tile's points once more through L2 are not counted).
+#define BA_CAND_REC 12
+template <int STAGED>
+__global__ void __launch_bounds__(BA_THREADS, 3)
+kf_step_eval(int n_pt, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam,
+             const int32_t *__restrict__ pm_pt, const double2 *__restrict__ pm_uv, const double *__restrict__ pose,
+             const double *__restrict__ pt, CostParams cp, const double *__restrict__ geo, const double *__restrict__ yc,
+             const double *__restrict__ camx, const double *__restrict__ pose_c, const int32_t *__restrict__ tile_lo,
+             const int32_t *__restrict__ tile_span, const double *__restrict__ intr, const double *__restrict__ intr_c,
+             const double *__restrict__ Vinv, const double *__restrict__ sp, const double *__restrict__ gp,
+             double *__restrict__ yp, double *__restrict__ ys, double *__restrict__ pt_c, double *__restrict__ part_mcc,
+             double *__restrict__ part_step, int step_off, double *__restrict__ part_cand, const LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
+  constexpr int TOBS = 512, PREC = 9;  // per point of the tile, after the reduction: X (3), ys (3), pt_c (3)
+  static_assert(PREC * BA_TILE_PTS <= 3 * TOBS, "point records reuse the reduction buffer");
+  __shared__ double sm[3 * TOBS];
+  __shared__ __align__(16) double rec[STAGED ? BA_STAGE_CAMS * BA_STAGE_REC : 2];
+  __shared__ __align__(16) double recc[STAGED ? BA_STAGE_CAMS * BA_CAND_REC : 2];
   __shared__ double red[BA_WARPS + 1];
-  const int i = blockIdx.x * BA_THREADS + threadIdx.x;
-  const double fx = ldg1(intr), fy = ldg1(intr + 1);
-  double acc = 0.0;
-  if (i < n_obs) {
-    const int c = cam_idx[i], p = pt_idx[i];
-    const ObsGeo o = load_geo(F, i, fx, fy);
-    CamRec cr;
-    load_camrec(geo, c, cr);
-    double y[6];
-    load6(yc + 6 * (size_t)c, y);
-#pragma unroll
-    for (int k = 0; k < 6; ++k) y[k] = cr.s[k] * y[k];
-    const double *R = cr.R;
-    double t[3];
-    ldg256(ys + 4 * (size_t)p, t[0], t[1], t[2]);
-    double a0, a1, b0, b1;
-    jc_dot(o, y, a0, a1);
-    jp_dot(o, R, t, b0, b1);
-    const double m0 = a0 + b0, m1 = a1 + b1;
-    const double2 r = lds2(F.r + i);
-    acc = m0 * (r.x + m0 / 2.0) + m1 * (r.y + m1 / 2.0);
+  const double4 K = load_intr(intr);
+  int cam_lo = 0;
+  if (STAGED) {
+    cam_lo = tile_lo[blockIdx.x];
+    const int n = tile_span[blockIdx.x];
+    for (int idx = threadIdx.x; idx < n * BA_STAGE_REC; idx += BA_THREADS) {
+      const int rc = idx / BA_STAGE_REC, k = idx - rc * BA_STAGE_REC;
+      const size_t c = (size_t)(cam_lo + rc);
+      double v;
+      if (k < 6)
+        v = geo[c * BA_CAMREC + 9 + k] * yc[c * 6 + k];
+      else if (k < 15)
+        v = geo[c * BA_CAMREC + (k - 6)];
+      else
+        v = pose[7 * c + 4 + (k - 15)];
+      rec[idx] = v;
+    }
+    for (int rc = threadIdx.x; rc < n; rc += BA_THREADS) {
+      const double *P = pose_c + 7 * (size_t)(cam_lo + rc);
+      const double q[4] = {P[0], P[1], P[2], P[3]};
+      double *o = recc + rc * BA_CAND_REC;
+      quat_to_R(q, o);
+      o[9] = P[4]; o[10] = P[5]; o[11] = P[6];
+    }
+    __syncthreads();
   }
-  const double s = block_sum(acc, red);
-  if (threadIdx.x == 0) part[blockIdx.x] = s;
+  // the current camera of observation s: s.*y_c, R, centre
+  auto cam = [&](int c, double xx[6], double R[9], double C[3]) {
+    double2 c0, c1, c2, c3, c4, c5, c6, c7;
+    if (STAGED) {
+      const double2 *cx = reinterpret_cast<const double2 *>(rec + (c - cam_lo) * BA_STAGE_REC);
+      c0 = cx[0]; c1 = cx[1]; c2 = cx[2]; c3 = cx[3]; c4 = cx[4]; c5 = cx[5]; c6 = cx[6]; c7 = cx[7];
+      const double2 c8 = cx[8];
+      C[0] = c7.y; C[1] = c8.x; C[2] = c8.y;
+    } else {
+      const double2 *cx = reinterpret_cast<const double2 *>(camx + (size_t)BA_CAMREC * c);
+      c0 = ldg2(cx); c1 = ldg2(cx + 1); c2 = ldg2(cx + 2); c3 = ldg2(cx + 3); c4 = ldg2(cx + 4); c5 = ldg2(cx + 5);
+      c6 = ldg2(cx + 6); c7 = ldg2(cx + 7);
+      const double *P = pose + 7 * (size_t)c;
+      C[0] = ldg1(P + 4); C[1] = ldg1(P + 5); C[2] = ldg1(P + 6);
+    }
+    xx[0] = c0.x; xx[1] = c0.y; xx[2] = c1.x; xx[3] = c1.y; xx[4] = c2.x; xx[5] = c2.y;
+    R[0] = c3.x; R[1] = c3.y; R[2] = c4.x; R[3] = c4.y; R[4] = c5.x; R[5] = c5.y; R[6] = c6.x; R[7] = c6.y; R[8] = c7.x;
+  };
+  const int p0 = blockIdx.x * BA_TILE_PTS, p1 = min(n_pt, p0 + BA_TILE_PTS);
+  tile_point_reduce<3, TOBS>(
+      n_pt, pt_rowptr, sm,
+      [&](int s, double *v) {
+        double xx[6], R[9], C[3], X3[3];
+        cam(pm_cam[s], xx, R, C);
+        load_pt(pt, pm_pt[s], X3);
+        const ObsProj pr = project_obs(R, C, X3, lds2(pm_uv + s), K, cp);
+        const ObsGeo o = obs_geo(make_double4(pr.xz, pr.yz, pr.iz, pr.w), K.x, K.y);
+        double a0, a1;
+        jc_dot(o, xx, a0, a1);
+        jp_tmul(o, R, a0, a1, v);
+      },
+      [&](int p, const double *sum) {
+        double vi[6];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) vi[k] = Vinv[6 * (size_t)p + k];
+        const double s[3] = {sp[3 * (size_t)p], sp[3 * (size_t)p + 1], sp[3 * (size_t)p + 2]};
+        double b[3], t[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) b[k] = s[k] * sum[k];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) b[k] = -gp[3 * (size_t)p + k] - b[k];
+        sym3_mul(vi, b, t);
+        // the point's record for the loops below; the candidate point with k_candidate's arithmetic
+        double *q = sm + PREC * (p - p0);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          yp[3 * (size_t)p + k] = t[k];
+          const double x = pt[3 * (size_t)p + k];
+          const double c = fma(t[k], s[k], x);  // (contracted as in k_candidate; s * t, rounded, is also formed below)
+          pt_c[3 * (size_t)p + k] = c;
+          q[k] = x;
+          q[3 + k] = s[k] * t[k];
+          q[6 + k] = c;
+        }
+        // pre-scaled copy, padded to 32 bytes: one 256-bit gather per observation in pass 2
+        *(reinterpret_cast<double4 *>(ys) + p) = make_double4(q[3], q[4], q[5], 0.0);
+      });
+  __syncthreads();
+  // the tile's share of |x+ - x|^2, written before the observation loops so that it holds no register through them
+  double sn = 0.0;
+  if (p0 + (int)threadIdx.x < p1) {
+    const double *q = sm + PREC * threadIdx.x;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const double df = q[k] - q[6 + k];
+      sn += df * df;
+    }
+  }
+  sn = block_sum(sn, red);
+  if (threadIdx.x == 0) part_step[step_off + blockIdx.x] = sn;
+  // model cost change and candidate cost over the tile's observations: two loops, so that neither holds the other's
+  // camera in registers (one loop spills at 80 registers)
+  const double4 Kc = load_intr(intr_c);
+  double mcc = 0.0, cand = 0.0;
+  for (int s = pt_rowptr[p0] + threadIdx.x, o1 = pt_rowptr[p1]; s < o1; s += BA_THREADS) {
+    const int c = pm_cam[s];
+    const double *q = sm + PREC * (pm_pt[s] - p0);
+    const double2 m = ldg2(pm_uv + s);
+    double xx[6], R[9], C[3];
+    cam(c, xx, R, C);
+    {
+      const double X3[3] = {q[0], q[1], q[2]}, t[3] = {q[3], q[4], q[5]};
+      const ObsProj pr = project_obs(R, C, X3, m, K, cp);
+      const ObsGeo o = obs_geo(make_double4(pr.xz, pr.yz, pr.iz, pr.w), K.x, K.y);
+      double a0, a1, b0, b1;
+      jc_dot(o, xx, a0, a1);
+      jp_dot(o, R, t, b0, b1);
+      const double m0 = a0 + b0, m1 = a1 + b1;
+      mcc += m0 * (pr.r0 + m0 / 2.0) + m1 * (pr.r1 + m1 / 2.0);
+    }
+  }
+  for (int s = pt_rowptr[p0] + threadIdx.x, o1 = pt_rowptr[p1]; s < o1; s += BA_THREADS) {
+    const int c = pm_cam[s];
+    const double *q = sm + PREC * (pm_pt[s] - p0);
+    const double2 m = ldg2(pm_uv + s);
+    double Rc[9], Cc[3];
+    if (STAGED) {
+      const double2 *cx = reinterpret_cast<const double2 *>(recc + (c - cam_lo) * BA_CAND_REC);
+      const double2 a = cx[0], b = cx[1], d = cx[2], e = cx[3], f = cx[4], g = cx[5];
+      Rc[0] = a.x; Rc[1] = a.y; Rc[2] = b.x; Rc[3] = b.y; Rc[4] = d.x; Rc[5] = d.y; Rc[6] = e.x; Rc[7] = e.y; Rc[8] = f.x;
+      Cc[0] = f.y; Cc[1] = g.x; Cc[2] = g.y;
+    } else {
+      const double *P = pose_c + 7 * (size_t)c;
+      const double q[4] = {ldg1(P), ldg1(P + 1), ldg1(P + 2), ldg1(P + 3)};
+      quat_to_R(q, Rc);
+      Cc[0] = ldg1(P + 4); Cc[1] = ldg1(P + 5); Cc[2] = ldg1(P + 6);
+    }
+    const double Xc[3] = {q[6], q[7], q[8]};
+    cand += 0.5 * project_obs(Rc, Cc, Xc, m, Kc, cp).rho;
+  }
+  const double s_mcc = block_sum(mcc, red);
+  const double s_cand = block_sum(cand, red);
+  if (threadIdx.x == 0) {
+    part_mcc[blockIdx.x] = s_mcc;
+    part_cand[blockIdx.x] = s_cand;
+  }
 }
