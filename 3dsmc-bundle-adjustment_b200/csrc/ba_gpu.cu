@@ -82,6 +82,27 @@ struct Buf {
   size_t cap = 0;
 };
 
+// How an LM step is solved, decided by ba_gpu_upload alone (and reset by every upload); the predicates after ba_gpu_ctx
+// are the only readers of its combinations.
+enum LinSolve {
+  LIN_DENSE,            // explicit Schur complement, dense Cholesky (windows, REF up to BA_EXPLICIT_MAX_DIM)
+  LIN_SPARSE_BORDERED,  // block-sparse S from the planes store, sparse Cholesky with the intrinsics border (REF / DEPTH / INTR)
+  LIN_SPARSE_CHOL,      // block-sparse S from the factored store, sparse Cholesky (NS)
+  LIN_SPARSE_PCG,       // block-sparse S from the factored store, PCG (NS)
+  LIN_IMPLICIT_PCG      // matrix-free Schur product, PCG
+};
+enum PcgForm {
+  PCG_NONE,         // no PCG: a Cholesky solves the step
+  PCG_STEPS,        // one launch per PCG step, the host polls the PCG controller
+  PCG_PERSISTENT,   // the whole PCG solve in one cooperative launch (block-sparse S)
+  PCG_ROW_SHARDED   // persistent, the product row-sharded over the ranks through NVLink peer memory (block-sparse S)
+};
+struct SolvePlan {
+  LinSolve lin = LIN_DENSE;
+  PcgForm pcg = PCG_NONE;
+  int store = BA_JAC_PLANES;  // BA_JAC_PLANES / _FACTORED / _TILED
+};
+
 struct ba_gpu_ctx {
   ba_gpu_options opt;
   int device = 0, n_sm = 148;
@@ -102,7 +123,8 @@ struct ba_gpu_ctx {
   // sizes
   int n_cam = 0, n_pt = 0, n_obs = 0, fixed_cam = -1, n_free = 0, n_items = 0;
   int depth = 0, nk = 0;  // cost-model switches in force
-  int solver = 0, n_red = 0;
+  SolvePlan plan;
+  int n_red = 0;
   int nblk_obs = 0, nblk_ent = 0, nblk_cam = 0, nblk_pt = 0, n_tiles = 0, nblk_item = 0, pl_tile_pts = BA_TILE_PTS, pl_tiles = 0;
   CostParams cp;
   LmOptions lo;
@@ -116,14 +138,12 @@ struct ba_gpu_ctx {
   // Jacobian planes (materialised store) / factored store
   Buf jcm, jpm;
   JPlanes Jc_, Jp_;
-  bool fact = false, planes_ready = false;
+  bool planes_ready = false;
   Buf fcm, fpm, geo, camx, Vs, ts, tgs, ys, tile_lo, tile_span;
   bool staged = false;
-  bool fp_store = false;  // point-major r / g records (Fp_) are kept: only the implicit solver's product reads them
   FPlanes Fc_, Fp_;
   // tile-fused product (ba_kernels_tile.cuh)
   Buf tmeta, tseg, tout, taux, tm_cam, tm_pt, tm_uv, ftm, cam_tmin, cam_tmax, tcnt, tpart_ptr, part6t;
-  bool tiled = false;
   int tile_npt = 0, n_tparts = 0;
   double2 *Tg0 = nullptr, *Tg1 = nullptr;
   // explicit block-sparse Schur complement (ba_kernels_sparse.cuh)
@@ -147,12 +167,10 @@ struct ba_gpu_ctx {
   int xch_ncam = 0;
   void *xch_peer[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   PcgFan fan;
-  bool dist_pcg = false;
   int n_my_rows = 0, dist_grid = 0;
   long long n_pairs = 0;
   // exact sparse Cholesky of S (ba_sparse_symbolic.h / ba_kernels_spchol.cuh)
   bool src_on_device = false;   // the arrays handed to the current upload live in device memory (ba_store_window_solve)
-  bool spchol = false;          // the block-sparse solver factorises S instead of running PCG
   SpSymbolic sym;               // host-side structure of the last upload
   Buf spn_node, spn_bord, spn_children, spn_rel, spn_inv, spn_aent, spn_perm;
   Buf spc_panel, spc_U, spc_z, spc_linv, spc_ypos, spc_prof, spc_queue, spc_tiles, spc_cnt, spc_cnt_init, spc_topcams;
@@ -171,10 +189,9 @@ struct ba_gpu_ctx {
   bool sp_full_next = false;  // the next enqueue_sparse_values() completes ALL of S on every rank (product hook)
   size_t spc_smem_tree = 0;   // dynamic shared memory of k_spchol_tree
   double sym_ms = 0.0;          // host time of the symbolic phase (last upload)
-  // sparse Cholesky of the REF / depth-prior / free-intrinsics cost (solver = EXPLICIT_CHOLESKY's linearisation and W / WV,
-  // the block-sparse S and the tree instead of the dense S): right-hand-side rows of the tree (5 with the intrinsics border),
-  // B by camera [24 n_cam], Z = L^-1 B by position [24 n_cam], the corner C + b_k [20], the per-CTA border partials
-  bool sp_ref = false;
+  // bordered sparse Cholesky (LIN_SPARSE_BORDERED: the dense solver's linearisation and W / WV, the block-sparse S and the tree
+  // instead of the dense S): right-hand-side rows of the tree (5 with the intrinsics border), B by camera [24 n_cam],
+  // Z = L^-1 B by position [24 n_cam], the corner C + b_k [20], the per-CTA border partials
   int spc_nrhs = 1;
   Buf spb_B, spb_Z, spb_kk, spb_part;
   // covariance (ba_gpu_covariance, ba_kernels_selinv.cuh), built by the first call after an upload: selected-inversion queue,
@@ -225,6 +242,34 @@ struct ba_gpu_ctx {
   int64_t collectives = 0;
   bool comm_error = false;
 };
+
+// what the plan implies, for everything that reads it
+static bool plan_factored(const SolvePlan &p) { return p.store != BA_JAC_PLANES; }
+// point-major r / g records (Fp_): only the matrix-free product reads them (the block-sparse solvers reduce the point blocks
+// straight from the projection and project again in the back-substitution)
+static bool plan_point_records(const SolvePlan &p) { return plan_factored(p) && p.lin == LIN_IMPLICIT_PCG; }
+// block-sparse S in force: built from the factored store in NS mode (k_sp_schur), from the planes store with the border
+static bool plan_sparse_ns(const SolvePlan &p) { return p.lin == LIN_SPARSE_CHOL || p.lin == LIN_SPARSE_PCG; }
+static bool plan_sparse_s(const SolvePlan &p) { return p.lin == LIN_SPARSE_BORDERED || plan_sparse_ns(p); }
+// supernodal tree of the LM solve in force
+static bool plan_tree(const SolvePlan &p) { return p.lin == LIN_SPARSE_BORDERED || p.lin == LIN_SPARSE_CHOL; }
+static int plan_solver_used(const SolvePlan &p) {
+  switch (p.lin) {
+    case LIN_DENSE: return BA_SOLVER_EXPLICIT_CHOLESKY;
+    case LIN_SPARSE_PCG: return BA_SOLVER_SPARSE_SCHUR_PCG;
+    case LIN_IMPLICIT_PCG: return BA_SOLVER_IMPLICIT_PCG;
+    default: return BA_SOLVER_SPARSE_SCHUR_CHOLESKY;
+  }
+}
+// the host polls inside the PCG loop (the launch-per-step form polls its controller, the row-sharded one reads its abort flag)
+static bool plan_host_polls_pcg(const SolvePlan &p) { return p.pcg == PCG_STEPS || p.pcg == PCG_ROW_SHARDED; }
+// CUDA-event phase times of ba_gpu_solve: the large-problem solvers
+static bool plan_phase_times(const SolvePlan &p) { return p.lin != LIN_DENSE; }
+// windowed dense solve on one GPU (single-CTA factorisation, every kernel a small gated one): the LM iteration is a captured
+// graph with programmatic dependent launches
+static bool plan_windowed(const ba_gpu_ctx *ctx) {
+  return ctx->plan.lin == LIN_DENSE && ctx->n_ranks == 1 && ctx->n_red > 0 && ctx->n_red <= BA_LDLT_MAX_N;
+}
 
 static thread_local std::string g_create_err;
 
@@ -517,9 +562,7 @@ extern "C" int ba_gpu_set_options(ba_gpu_ctx *ctx, const ba_gpu_options *o) {
 extern "C" int64_t ba_gpu_launch_count(const ba_gpu_ctx *ctx) { return ctx ? ctx->launches : 0; }
 extern "C" int ba_gpu_sparse_stats(const ba_gpu_ctx *ctx, int64_t *n_pairs, int32_t *n_blocks, int32_t *n_entries) {
   if (!ctx || !ctx->uploaded) return BA_ERR_STATE;
-  // block-sparse S in force: the NS solvers (PCG and Cholesky: ctx->solver == SPARSE_SCHUR_PCG) and the sparse Cholesky with
-  // depth prior / free intrinsics (ctx->sp_ref)
-  const bool sp = ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG || ctx->sp_ref;
+  const bool sp = plan_sparse_s(ctx->plan);
   if (n_pairs) *n_pairs = sp ? ctx->n_pairs : 0;
   if (n_blocks) *n_blocks = sp ? ctx->n_sblk : 0;
   if (n_entries) *n_entries = sp ? ctx->n_ent : 0;
@@ -527,7 +570,7 @@ extern "C" int ba_gpu_sparse_stats(const ba_gpu_ctx *ctx, int64_t *n_pairs, int3
 }
 extern "C" int ba_gpu_jacobian_store_used(const ba_gpu_ctx *ctx) {
   if (!ctx || !ctx->uploaded) return BA_ERR_STATE;
-  return ctx->tiled ? BA_JAC_TILED : (ctx->fact ? BA_JAC_FACTORED : BA_JAC_PLANES);
+  return ctx->plan.store;
 }
 
 // ------------------------------------------------------------------ upload
@@ -883,9 +926,10 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
 }
 
 // symbolic phase of the exact sparse Cholesky (host: ordering, elimination tree, supernodes, maps) from the block structure of
-// the last build_sparse_structure(); uploads the integer tables and sizes the numeric buffers.  BA_ERR_UNSUPPORTED when a front
-// cannot fit one SM's shared memory (co-visibility without a sequential structure): the caller keeps PCG then.
-static int build_spchol(ba_gpu_ctx *ctx) {
+// the last build_sparse_structure(), split into want_parts subtree parts, with nrhs right-hand-side rows (5 with the intrinsics
+// border); uploads the integer tables and sizes the numeric buffers.  BA_ERR_UNSUPPORTED when a front cannot fit one SM's shared
+// memory (co-visibility without a sequential structure): AUTO keeps PCG then.
+static int build_spchol(ba_gpu_ctx *ctx, int want_parts, int nrhs) {
   cudaStream_t s = ctx->stream;
   const int n_cam = ctx->n_cam, n_blk = ctx->n_sblk;
   std::vector<int32_t> bi((size_t)n_blk + 1), bj((size_t)n_blk + 1);
@@ -905,14 +949,8 @@ static int build_spchol(ba_gpu_ctx *ctx) {
   if (S.error) return fail(ctx, BA_ERR_STATE, "sparse Cholesky: inconsistent symbolic structure (%d)", S.error);
   if ((double)S.panel_blocks * 288.0 + (double)S.u_blocks * 288.0 > 64e9)
     return fail(ctx, BA_ERR_UNSUPPORTED, "sparse Cholesky: factor would need %.1f GB", ((double)S.panel_blocks + (double)S.u_blocks) * 288e-9);
-  // subtree-to-rank partition of the NS LM solve: one part per rank; on one GPU BA_SPCHOL_PARTS=n runs the n parts one after
-  // the other (tests of the queues and of the exchange layout).  One part for the REF-cost solve and for the structure the
-  // covariance builds under another solver: both are single-GPU and run the one-part queue's factor prefix on its own.
-  int want_parts = 1;
-  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG)
-    want_parts = ctx->n_ranks > 1 ? ctx->n_ranks
-                                  : (getenv("BA_SPCHOL_PARTS") ? std::min(BA_MAX_RANKS, std::max(1, atoi(getenv("BA_SPCHOL_PARTS")))) : 1);
-  const int R = ctx->spc_nrhs;
+  ctx->spc_nrhs = nrhs;
+  const int R = nrhs;
   const SpPartition part = spsym_partition(S, want_parts);
   ctx->spc_parts = part.parts;
   ctx->spc_dist = ctx->n_ranks > 1 && part.parts == ctx->n_ranks;
@@ -1014,16 +1052,15 @@ static int build_spchol(ba_gpu_ctx *ctx) {
               100.0 * part.heaviest / std::max(1.0, part.total), ctx->spc_xchg * 8e-6, ctx->spc_qB, ctx->spc_qB_n);
   }
   CK(cudaStreamSynchronize(s));  // host vectors of this call die here
-  ctx->spchol = true;
   return 0;
 }
 
 // exchange buffers of the row-sharded PCG: one cudaMalloc per rank, handles all-gathered through NCCL,
-// peers mapped with cudaIpcOpenMemHandle (NVLink peer access)
-static int setup_dist_pcg(ba_gpu_ctx *ctx) {
+// peers mapped with cudaIpcOpenMemHandle (NVLink peer access); *ok: every rank can run the row-sharded PCG
+static int setup_dist_pcg(ba_gpu_ctx *ctx, bool *ok_out) {
   const int n_cam = ctx->n_cam, n_wb = cdiv(n_cam, 32), N = ctx->n_ranks;
   cudaStream_t s = ctx->stream;
-  ctx->dist_pcg = false;
+  *ok_out = false;
   if (N > BA_MAX_RANKS) return 0;
   // layout (16-byte slots): q[2][6n] pq[2][n] slice[2][n_slices] | epoch (u64) abort (int)
   const size_t n6 = (size_t)6 * n_cam, n_slices = (size_t)cdiv(n_cam, BA_PQ_SLICE);
@@ -1115,7 +1152,19 @@ static int setup_dist_pcg(ba_gpu_ctx *ctx) {
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pcg_sparse_dist, BA_THREADS, (size_t)BA_WARPS * BA_PCG_SMEM_PER_WARP));
     ctx->dist_grid = per_sm > 0 ? ctx->n_sm : 0;
   }
-  ctx->dist_pcg = ctx->dist_grid > 0;
+  *ok_out = ctx->dist_grid > 0;
+  return 0;
+}
+
+// buffers of the bordered system: W and WV per observation, B and Z = L^-1 B by camera, the corner, the per-CTA border partials
+static int reserve_bordered(ba_gpu_ctx *ctx) {
+  const size_t no = (size_t)ctx->n_obs, nc = (size_t)ctx->n_cam;
+  RES(W, (no + 1) * 144);
+  RES(WV, (no + 1) * 144);
+  RES(spb_B, nc * 192 + 64);
+  RES(spb_Z, nc * 192 + 64);
+  RES(spb_kk, 20 * 8);
+  RES(spb_part, (size_t)(ctx->nblk_cam + 1) * 14 * 8);
   return 0;
 }
 
@@ -1136,6 +1185,59 @@ struct UploadProf {
   }
 };
 
+// (a) of the upload's plan, from the options and the sizes before any allocation: the solve path and the store as far as they
+// are known, or the first rule the options break.  The NS sparse Cholesky is tentative until its symbolic phase.
+static int plan_from_options(ba_gpu_ctx *ctx, SolvePlan *plan) {
+  const ba_gpu_options &o = ctx->opt;
+  int solver = o.solver == BA_SOLVER_SPARSE_SCHUR_CHOLESKY ? BA_SOLVER_SPARSE_SCHUR_PCG : o.solver;
+  // depth prior and / or free intrinsics through the sparse Cholesky: when asked for, and under AUTO when free intrinsics
+  // take the problem past the dense explicit limit.  It keeps the dense solver's linearisation (planes store, W / WV) and
+  // replaces the dense S by the block-sparse one; the four intrinsics columns become a border of the tree's solve.
+  const bool bordered = (o.use_depth_prior || o.optimize_intrinsics) &&
+                        (o.solver == BA_SOLVER_SPARSE_SCHUR_CHOLESKY ||
+                         (o.solver == BA_SOLVER_AUTO && ctx->nk && ctx->n_red > BA_EXPLICIT_MAX_DIM && ctx->n_ranks == 1));
+  if (bordered) {
+    if (ctx->n_ranks > 1)
+      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics is single-GPU");
+    if (o.jacobian_store == BA_JAC_FACTORED || o.jacobian_store == BA_JAC_TILED)
+      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics reads the planes Jacobian store");
+    solver = BA_SOLVER_EXPLICIT_CHOLESKY;
+  }
+  if (solver == BA_SOLVER_AUTO)
+    solver = (ctx->n_red <= o.explicit_max_dim || ctx->nk) ? BA_SOLVER_EXPLICIT_CHOLESKY : BA_SOLVER_IMPLICIT_PCG;
+  if ((solver == BA_SOLVER_IMPLICIT_PCG || solver == BA_SOLVER_SPARSE_SCHUR_PCG) && ctx->nk)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "optimize_intrinsics needs the explicit solver (as ITERATIVE_SCHUR needs points only)");
+  if (solver == BA_SOLVER_SPARSE_SCHUR_PCG && o.use_depth_prior)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "the block-sparse Schur solver needs NS mode (no depth prior, fixed intrinsics)");
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !bordered && ctx->n_red > BA_EXPLICIT_MAX_DIM)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d)", BA_EXPLICIT_MAX_DIM,
+                ctx->n_red);
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks > 1)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "the explicit solver is single-GPU (windowed problems stay on one GPU)");
+  // the dense substitution (k_chol_solve2) is one cooperative grid of n_sm CTAs, each owning at most CH_S2_OWN tiles of 64 unknowns
+  // (at BA_EXPLICIT_MAX_DIM: 256 tiles, 64 SMs)
+  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !bordered && cdiv(ctx->n_red, CH_NB) > CH_S2_OWN * ctx->n_sm)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky: reduced dimension %d needs %d SMs for its substitution (device has %d)",
+                ctx->n_red, cdiv(cdiv(ctx->n_red, CH_NB), CH_S2_OWN), ctx->n_sm);
+  const bool sparse = solver == BA_SOLVER_SPARSE_SCHUR_PCG;
+  const bool can_fact = ((solver == BA_SOLVER_IMPLICIT_PCG || sparse) && !o.use_depth_prior && !o.optimize_intrinsics);
+  if (sparse && o.jacobian_store == BA_JAC_PLANES)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "the block-sparse Schur solver rebuilds its blocks from the factored store");
+  if (o.jacobian_store == BA_JAC_FACTORED && !can_fact)
+    return fail(ctx, BA_ERR_UNSUPPORTED, "the factored Jacobian store needs NS mode (no depth prior, fixed intrinsics) + implicit PCG");
+  *plan = SolvePlan{};
+  if (bordered)
+    plan->lin = LIN_SPARSE_BORDERED;
+  else if (solver == BA_SOLVER_EXPLICIT_CHOLESKY)
+    plan->lin = LIN_DENSE;
+  else if (sparse)
+    plan->lin = o.solver == BA_SOLVER_SPARSE_SCHUR_CHOLESKY ? LIN_SPARSE_CHOL : LIN_SPARSE_PCG;
+  else
+    plan->lin = LIN_IMPLICIT_PCG;
+  plan->store = can_fact && o.jacobian_store != BA_JAC_PLANES ? BA_JAC_FACTORED : BA_JAC_PLANES;
+  return 0;
+}
+
 extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7, int32_t fixed_cam, int32_t n_pt,
                              const double *pt3, int32_t n_obs, const int32_t *cam_idx, const int32_t *pt_idx,
                              const double *uv2, const double *depth, const double intr4[4], const double intr_prior4[4]) {
@@ -1143,6 +1245,7 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   ctx->pdl = false;
   UploadProf prof;
   ctx->uploaded = false;
+  ctx->plan = SolvePlan{};
   ctx->lm_graph_stale = true;
   ctx->linearized = false;
   ctx->cov_ready = false;
@@ -1162,56 +1265,12 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   ctx->depth = o.use_depth_prior ? 1 : 0;
   ctx->nk = o.optimize_intrinsics ? 4 : 0;
   ctx->n_red = 6 * ctx->n_free + ctx->nk;
-  int solver = o.solver;
-  // the exact sparse Cholesky shares the block-sparse S machinery of the PCG variant; ctx->spchol switches the linear solve
-  bool want_chol = solver == BA_SOLVER_SPARSE_SCHUR_CHOLESKY;
-  if (want_chol) solver = BA_SOLVER_SPARSE_SCHUR_PCG;
-  ctx->spchol = false;
-  // depth prior and / or free intrinsics through the sparse Cholesky: when asked for, and under AUTO when free intrinsics
-  // take the problem past the dense explicit limit.  It keeps the explicit solver's linearisation (planes store, W / WV) and
-  // replaces the dense S by the block-sparse one; the four intrinsics columns become a border of the tree's solve.
-  const bool sp_ref = (o.use_depth_prior || o.optimize_intrinsics) &&
-                      (want_chol || (solver == BA_SOLVER_AUTO && ctx->nk && ctx->n_red > BA_EXPLICIT_MAX_DIM && ctx->n_ranks == 1));
-  ctx->sp_ref = sp_ref;
-  // right-hand-side rows of the tree, decided by THIS upload (a context reused after set_options must not keep the border of an
-  // earlier REF problem: the NS path is the one-row tree)
-  ctx->spc_nrhs = sp_ref && ctx->nk ? 5 : 1;
-  if (sp_ref) {
-    if (ctx->n_ranks > 1)
-      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics is single-GPU");
-    if (o.jacobian_store == BA_JAC_FACTORED || o.jacobian_store == BA_JAC_TILED)
-      return fail(ctx, BA_ERR_UNSUPPORTED, "the sparse Cholesky with depth prior / free intrinsics reads the planes Jacobian store");
-    solver = BA_SOLVER_EXPLICIT_CHOLESKY;
-    want_chol = false;
-  }
-  if (solver == BA_SOLVER_AUTO)
-    solver = (ctx->n_red <= o.explicit_max_dim || ctx->nk) ? BA_SOLVER_EXPLICIT_CHOLESKY : BA_SOLVER_IMPLICIT_PCG;
-  if ((solver == BA_SOLVER_IMPLICIT_PCG || solver == BA_SOLVER_SPARSE_SCHUR_PCG) && ctx->nk)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "optimize_intrinsics needs the explicit solver (as ITERATIVE_SCHUR needs points only)");
-  if (solver == BA_SOLVER_SPARSE_SCHUR_PCG && o.use_depth_prior)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "the block-sparse Schur solver needs NS mode (no depth prior, fixed intrinsics)");
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !sp_ref && ctx->n_red > BA_EXPLICIT_MAX_DIM)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d)", BA_EXPLICIT_MAX_DIM,
-                ctx->n_red);
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && ctx->n_ranks > 1)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "the explicit solver is single-GPU (windowed problems stay on one GPU)");
-  // the dense substitution (k_chol_solve2) is one cooperative grid of n_sm CTAs, each owning at most CH_S2_OWN tiles of 64 unknowns
-  // (at BA_EXPLICIT_MAX_DIM: 256 tiles, 64 SMs)
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && !sp_ref && cdiv(ctx->n_red, CH_NB) > CH_S2_OWN * ctx->n_sm)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky: reduced dimension %d needs %d SMs for its substitution (device has %d)",
-                ctx->n_red, cdiv(cdiv(ctx->n_red, CH_NB), CH_S2_OWN), ctx->n_sm);
-  ctx->solver = solver;
-  // AUTO on a large NS-mode problem, single GPU: block-sparse explicit S if the co-visibility
-  // is sparse enough (decided after the index build, from the pair count), else implicit
-  const bool auto_large = o.solver == BA_SOLVER_AUTO && solver == BA_SOLVER_IMPLICIT_PCG && !o.use_depth_prior &&
-                          o.jacobian_store != BA_JAC_PLANES;
-  bool sparse = solver == BA_SOLVER_SPARSE_SCHUR_PCG;
-  const bool can_fact = ((solver == BA_SOLVER_IMPLICIT_PCG || sparse) && !o.use_depth_prior && !o.optimize_intrinsics);
-  if (sparse && o.jacobian_store == BA_JAC_PLANES)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "the block-sparse Schur solver rebuilds its blocks from the factored store");
-  if (o.jacobian_store == BA_JAC_FACTORED && !can_fact)
-    return fail(ctx, BA_ERR_UNSUPPORTED, "the factored Jacobian store needs NS mode (no depth prior, fixed intrinsics) + implicit PCG");
-  ctx->fact = can_fact && o.jacobian_store != BA_JAC_PLANES;
+  // the plan in three steps: (a) from the options and the sizes, (b) after the index build, (c) after the symbolic phase
+  SolvePlan plan;
+  int rc = plan_from_options(ctx, &plan);
+  if (rc) return rc;
+  ctx->plan = plan;
+  const bool fact = plan_factored(plan);
   ctx->planes_ready = false;
 
   const int64_t N = o.n_obs_total > 0 ? o.n_obs_total : (int64_t)n_obs;
@@ -1278,14 +1337,14 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   RES(item_cnt, (nc + 1) * 4);
   RES(cam_slot, nc * 4);
   const size_t n_pad = (no + 31) / 32 * 32 + 32;
-  if (!ctx->fact) {
+  if (!fact) {
     int rcp = ensure_planes(ctx);
     if (rcp) return rcp;
   } else {
     RES(fcm, n_pad * 48);
     ctx->Fc_.r = P<double2>(ctx->fcm);
     ctx->Fc_.g = reinterpret_cast<double4 *>(P<double2>(ctx->fcm) + n_pad);  // (n_pad is a multiple of 32: 32-byte aligned)
-    ctx->Fp_ = FPlanes{nullptr, nullptr};  // (allocated below once the solver is known)
+    ctx->Fp_ = FPlanes{nullptr, nullptr};  // (allocated below once the solve path is known)
     RES(geo, nc * BA_CAMREC * 8);
     RES(camx, nc * BA_CAMREC * 8);
     RES(Vs, np * 48);
@@ -1329,12 +1388,12 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   RES(Minv, nc * 288);
   RES(pc_lin, (size_t)ctx->nblk_obs * 8);
   // model cost change / candidate cost partials: per observation block, or per point tile (kf_step_eval)
-  RES(pc_cand, (size_t)(ctx->fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
-  RES(pc_mcc, (size_t)(ctx->fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
+  RES(pc_cand, (size_t)(fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
+  RES(pc_mcc, (size_t)(fact ? ctx->n_tiles : ctx->nblk_obs) * 8);
   RES(pe_gmax, (size_t)ctx->nblk_ent * 8);
   RES(pe_xn, (size_t)ctx->nblk_ent * 8);
   // step norm partials: per entry block, or per block of cameras + intrinsics (k_candidate) followed by one per point tile
-  RES(pe_step, (size_t)(ctx->fact ? cdiv(n_cam + 1, BA_THREADS) + ctx->n_tiles : ctx->nblk_ent) * 8);
+  RES(pe_step, (size_t)(fact ? cdiv(n_cam + 1, BA_THREADS) + ctx->n_tiles : ctx->nblk_ent) * 8);
   RES(pcam_rho, (size_t)ctx->nblk_cam * 8);
   RES(pcam_bb, (size_t)ctx->nblk_cam * 8);
   RES(pcam_pq, (size_t)ctx->nblk_cam * 8);
@@ -1403,7 +1462,7 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   RES(items, (size_t)(h_items + 1) * sizeof(BaItem));
   LAUNCH(k_item_fill, ctx->nblk_cam, BA_THREADS, 0, n_cam, item_obs, P<int32_t>(ctx->cam_rowptr), P<int32_t>(ctx->item_ptr),
          P<BaItem>(ctx->items));
-  if (ctx->fact) {
+  if (fact) {
     // camera span of every point tile -> shared-memory staging of pass 1
     CK(cudaMemsetAsync(ctx->err_flag.p, 0, 16, s));
     LAUNCH(k_tile_cam_range, ctx->n_tiles, BA_THREADS, 0, n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
@@ -1413,56 +1472,25 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     CK(cudaStreamSynchronize(s));
     ctx->staged = h_span <= BA_STAGE_CAMS;
   }
-  ctx->tiled = false;
-  if (auto_large) {
+  // (b) AUTO on a large NS problem: block-sparse S if the co-visibility is sparse enough (decided from the pair count, the same
+  // on every rank), factorised exactly (the reference's SPARSE_SCHUR) when its fronts fit; else matrix-free
+  if (o.solver == BA_SOLVER_AUTO && ctx->plan.lin == LIN_IMPLICIT_PCG && fact) {
     long long n_pairs = 0;
     int rcs = sparse_count_pairs(ctx, &n_pairs);
     if (rcs) return rcs;
-    double tot_pairs = (double)n_pairs, tot_obs = (double)n_obs, max_pairs = (double)n_pairs;  // same decision on every rank
+    double tot_pairs = (double)n_pairs, tot_obs = (double)n_obs, max_pairs = (double)n_pairs;
     if ((rcs = allreduce_host_scalar(ctx, &tot_pairs, false)) || (rcs = allreduce_host_scalar(ctx, &tot_obs, false)) ||
         (rcs = allreduce_host_scalar(ctx, &max_pairs, true)))
       return rcs;
-    if (tot_pairs <= (double)o.sparse_max_pairs_per_obs * tot_obs && max_pairs <= 2147483647.0) {
-      sparse = true;
-      want_chol = true;  // AUTO: exact factorisation (the reference's SPARSE_SCHUR) when its fronts fit
-      ctx->solver = BA_SOLVER_SPARSE_SCHUR_PCG;
-    }
+    if (tot_pairs <= (double)o.sparse_max_pairs_per_obs * tot_obs && max_pairs <= 2147483647.0) ctx->plan.lin = LIN_SPARSE_CHOL;
   }
-  if (sparse) {
-    prof.stamp("to sparse");
-    int rcs = build_sparse_structure(ctx);
-    if (rcs) return rcs;
-    prof.stamp("sparse structure");
-    if (want_chol) {
-      rcs = build_spchol(ctx);
-      if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) rcs = 0;  // falls back to PCG on the same S
-      if (rcs) return rcs;
-      prof.stamp("symbolic + tables");
-    }
-    ctx->dist_pcg = false;
-    if (!ctx->spchol && ctx->n_ranks > 1 && o.persistent_pcg == 1 && (rcs = setup_dist_pcg(ctx))) return rcs;
-  }
-  // point-major records: only the implicit solver's product reads them (the block-sparse solvers, AUTO's included, reduce
-  // the point blocks straight from the projection and project again in the back-substitution)
-  ctx->fp_store = ctx->fact && !sparse;
-  if (ctx->fp_store) {
+  if (plan_point_records(ctx->plan)) {
     RES(fpm, n_pad * 48);
     ctx->Fp_.r = P<double2>(ctx->fpm);
     ctx->Fp_.g = reinterpret_cast<double4 *>(P<double2>(ctx->fpm) + n_pad);
   }
-  if (sp_ref) {
-    prof.stamp("to sparse");
-    int rcs = build_sparse_structure(ctx);
-    if (!rcs) rcs = build_spchol(ctx);
-    if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) {
-      const std::string why = ctx->err;
-      return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d), and the sparse "
-                  "Cholesky cannot take it: %s", BA_EXPLICIT_MAX_DIM, ctx->n_red, why.c_str());
-    }
-    if (rcs) return rcs;
-    prof.stamp("sparse structure + symbolic");
-  }
-  if (ctx->fact && !sparse && o.jacobian_store != BA_JAC_FACTORED && ctx->n_tiles > 0) {
+  // then the store: the matrix-free product takes the tiled one where the tile bounds hold
+  if (fact && ctx->plan.lin == LIN_IMPLICIT_PCG && o.jacobian_store != BA_JAC_FACTORED && ctx->n_tiles > 0) {
     // tile-fused product: tile metadata, then (if the locality bounds hold) the tile-camera-major store
     RES(tmeta, (size_t)ctx->n_tiles * sizeof(TileMeta));
     CK(cudaMemsetAsync(ctx->err_flag.p, 0, 16, s));
@@ -1510,8 +1538,47 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
       CK(cudaStreamSynchronize(s));
       ctx->n_tparts = h_parts;
       RES(part6t, (size_t)(h_parts + 1) * 48);
-      ctx->tiled = true;
+      ctx->plan.store = BA_JAC_TILED;
     }
+  }
+  // (c) the symbolic phase: the NS sparse Cholesky, or PCG on the same S when its fronts do not fit under AUTO; then the PCG form
+  if (plan_sparse_ns(ctx->plan)) {
+    prof.stamp("to sparse");
+    int rcs = build_sparse_structure(ctx);
+    if (rcs) return rcs;
+    prof.stamp("sparse structure");
+    if (ctx->plan.lin == LIN_SPARSE_CHOL) {
+      // subtree-to-rank partition: one part per rank; on one GPU BA_SPCHOL_PARTS=n runs the n parts one after the other
+      // (tests of the queues and of the exchange layout)
+      const char *env_parts = getenv("BA_SPCHOL_PARTS");
+      const int parts = ctx->n_ranks > 1 ? ctx->n_ranks : (env_parts ? std::min(BA_MAX_RANKS, std::max(1, atoi(env_parts))) : 1);
+      rcs = build_spchol(ctx, parts, 1);
+      if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) {
+        rcs = 0;
+        ctx->plan.lin = LIN_SPARSE_PCG;
+      }
+      if (rcs) return rcs;
+      prof.stamp("symbolic + tables");
+    }
+    if (ctx->plan.lin == LIN_SPARSE_PCG) {
+      bool sharded = false;
+      if (ctx->n_ranks > 1 && o.persistent_pcg == 1 && (rcs = setup_dist_pcg(ctx, &sharded))) return rcs;
+      ctx->plan.pcg = sharded ? PCG_ROW_SHARDED : (o.persistent_pcg && ctx->pcg_grid > 0) ? PCG_PERSISTENT : PCG_STEPS;
+    }
+  }
+  if (ctx->plan.lin == LIN_IMPLICIT_PCG) ctx->plan.pcg = PCG_STEPS;
+  if (ctx->plan.lin == LIN_SPARSE_BORDERED) {
+    // (one part: the bordered solve is single-GPU and runs the one-part queue's factor prefix on its own)
+    prof.stamp("to sparse");
+    int rcs = build_sparse_structure(ctx);
+    if (!rcs) rcs = build_spchol(ctx, 1, ctx->nk ? 5 : 1);
+    if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) {
+      const std::string why = ctx->err;
+      return fail(ctx, BA_ERR_UNSUPPORTED, "dense explicit Cholesky supports reduced dimension <= %d (got %d), and the sparse "
+                  "Cholesky cannot take it: %s", BA_EXPLICIT_MAX_DIM, ctx->n_red, why.c_str());
+    }
+    if (rcs) return rcs;
+    prof.stamp("sparse structure + symbolic");
   }
   RES(part_blk, (size_t)(h_items + 1) * 61 * 8);
   RES(part6, (size_t)(h_items + 1) * 6 * 8);
@@ -1521,17 +1588,12 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   LAUNCH(k_fill, cdiv(6 * n_cam, 256), 256, 0, P<double>(ctx->one_c), (size_t)6 * nc, 1.0);
   LAUNCH(k_fill, cdiv(3 * n_pt, 256), 256, 0, P<double>(ctx->one_p), (size_t)3 * np, 1.0);
   LAUNCH(k_fill, 1, 256, 0, P<double>(ctx->one_k), (size_t)4, 1.0);
-  if (solver == BA_SOLVER_EXPLICIT_CHOLESKY && sp_ref) {
+  if (ctx->plan.lin == LIN_SPARSE_BORDERED) {
     // no dense S, no pair list: the block-sparse structure of build_sparse_structure() holds S
-    RES(W, (no + 1) * 144);
-    RES(WV, (no + 1) * 144);
-    RES(spb_B, nc * 192 + 64);
-    RES(spb_Z, nc * 192 + 64);
-    RES(spb_kk, 20 * 8);
-    RES(spb_part, (size_t)(ctx->nblk_cam + 1) * 14 * 8);
+    if ((rc = reserve_bordered(ctx))) return rc;
     CK(cudaMemsetAsync(ctx->yk.p, 0, 32, s));  // (no intrinsics: y_k stays 0)
     prof.stamp("rest");
-  } else if (solver == BA_SOLVER_EXPLICIT_CHOLESKY) {
+  } else if (ctx->plan.lin == LIN_DENSE) {
     RES(W, (no + 1) * 144);
     RES(WV, (no + 1) * 144);
     RES(S, (size_t)ctx->n_red * ctx->n_red * 8 + 64);
@@ -1684,7 +1746,7 @@ static void enqueue_linearize(ba_gpu_ctx *ctx, int gate, const double *sc, const
   // from_candidate (planes path): read the accepted candidate x+ directly while k_accept copies it into x on the side stream
   const double *xpose = P<double>(from_candidate ? ctx->pose_c : ctx->pose), *xpt = P<double>(from_candidate ? ctx->pt_c : ctx->pt),
                *xintr = P<double>(from_candidate ? ctx->intr_c : ctx->intr);
-  if (ctx->fact && !force_planes) {
+  if (plan_factored(ctx->plan) && !force_planes) {
     const double *intr = P<double>(ctx->intr);
     LAUNCH(k_cam_geo, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam, P<double>(ctx->pose), sc, P<double>(ctx->geo), st,
            gate);
@@ -1695,13 +1757,13 @@ static void enqueue_linearize(ba_gpu_ctx *ctx, int gate, const double *sc, const
          P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->pm_pt), P<double2>(ctx->pm_uv), P<double>(ctx->pose), P<double>(ctx->pt),    \
          P<double>(ctx->geo), P<int32_t>(ctx->tile_lo), P<int32_t>(ctx->tile_span), intr, ctx->cp, sp, ctx->Fp_,               \
          P<double>(ctx->V), P<double>(ctx->gp), P<double>(ctx->dp), ctx->lo, st, gate)
-    if (ctx->fp_store) {
+    if (plan_point_records(ctx->plan)) {
       if (ctx->staged) PT_LIN(1, 1); else PT_LIN(1, 0);
     } else {
       if (ctx->staged) PT_LIN(0, 1); else PT_LIN(0, 0);
     }
 #undef PT_LIN
-    if (ctx->tiled)
+    if (ctx->plan.store == BA_JAC_TILED)
       LAUNCH(kt_linearize, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->tm_cam), P<int32_t>(ctx->tm_pt),
              P<double2>(ctx->tm_uv), P<double>(ctx->pose), P<double>(ctx->pt), intr, ctx->cp, ctx->Tg0, ctx->Tg1, st, gate);
     fork_main(ctx);
@@ -1783,7 +1845,7 @@ static void enqueue_iteration_zero(ba_gpu_ctx *ctx, bool begin_loop = true) {
 // one implicit-Schur product: part6 <- sum Jc^T (alpha Jc v - Jp t), t <- pass 1 of v
 static void enqueue_point_inverse(ba_gpu_ctx *ctx, int gate) {
   LmState *st = P<LmState>(ctx->st);
-  if (ctx->fact)
+  if (plan_factored(ctx->plan))
     LAUNCH(kf_point_inverse, ctx->nblk_pt, BA_THREADS, 0, ctx->n_pt, P<double>(ctx->V), P<double>(ctx->dp), P<double>(ctx->gp),
            P<double>(ctx->sp), P<double>(ctx->Vinv), P<double>(ctx->Vs), P<double>(ctx->tgs), st, gate);
   else
@@ -1806,12 +1868,12 @@ static void launch_fused(ba_gpu_ctx *ctx, const double *v, int gate) {
 static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int passes = 3) {
   LmState *st = P<LmState>(ctx->st);
   const int rp = ctx->lo.reset_period;
-  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG && passes == 3) {
+  if (plan_sparse_ns(ctx->plan) && passes == 3) {
     LAUNCH(k_bsr_spmv, cdiv(ctx->n_cam * 32, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->ent_ptr), P<int2>(ctx->ent),
            P<double>(ctx->Sblk), v, P<double>(ctx->ysp), st, gate);
     return ItemRef{P<int32_t>(ctx->ident), P<double>(ctx->ysp)};
   }
-  if (ctx->tiled && passes == 3) {
+  if (ctx->plan.store == BA_JAC_TILED && passes == 3) {
     switch (ctx->tile_npt) {
       case 2: launch_fused<2>(ctx, v, gate); break;
       case 3: launch_fused<3>(ctx, v, gate); break;
@@ -1822,7 +1884,7 @@ static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int pa
     return ItemRef{P<int32_t>(ctx->tpart_ptr), P<double>(ctx->part6t)};
   }
   const ItemRef items_ref{P<int32_t>(ctx->item_ptr), P<double>(ctx->part6)};
-  if (ctx->fact) {
+  if (plan_factored(ctx->plan)) {
     const double *intr = P<double>(ctx->intr);
     if (passes & 1) {
       if (ctx->staged) {
@@ -1856,7 +1918,7 @@ static ItemRef enqueue_matvec(ba_gpu_ctx *ctx, const double *v, int gate, int pa
 // every rank fills the blocks of its own points into the common structure, the values are all-reduced,
 // then the (already reduced) camera blocks U go onto the diagonal.
 static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
-  if (ctx->solver != BA_SOLVER_SPARSE_SCHUR_PCG) return;
+  if (!plan_sparse_ns(ctx->plan)) return;
   LmState *st = P<LmState>(ctx->st);
   if (ctx->n_ranks > 1) cudaMemsetAsync(ctx->Sblk.p, 0, (size_t)ctx->n_sblk * 288, ctx->stream);
   int *ticket = reinterpret_cast<int *>(P<char>(ctx->pcg_bar) + 16);
@@ -1868,7 +1930,7 @@ static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
          P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
          P<double>(ctx->Sblk), ticket, st, gate);
   if (ctx->n_ranks > 1) {
-    if (ctx->spchol && ctx->spc_dist && !ctx->sp_full_next) {
+    if (ctx->plan.lin == LIN_SPARSE_CHOL && ctx->spc_dist && !ctx->sp_full_next) {
       // distributed factorisation: only the blocks another rank needs from this one (and the top part's) are summed
       if (ctx->spc_nx > 0) {
         LAUNCH(k_sp_xpack, cdiv(ctx->spc_nx * 36, BA_THREADS), BA_THREADS, 0, ctx->spc_nx, P<int32_t>(ctx->spc_xidx), P<double>(ctx->Sblk),
@@ -1990,7 +2052,7 @@ static void enqueue_pcg_iteration(ba_gpu_ctx *ctx, int it) {
   const int rp = ctx->lo.reset_period;
   const int reset = (rp > 0 && (it % rp) == 0) ? 1 : 0;
   LAUNCH(k_pcg_dir, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<double>(ctx->z), P<double>(ctx->p), st, GATE_PCG);
-  const bool replicated = ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG;  // S is complete on every rank: no exchange in PCG
+  const bool replicated = ctx->plan.lin == LIN_SPARSE_PCG;  // S is complete on every rank: no exchange in PCG
   ItemRef ir = enqueue_matvec(ctx, P<double>(ctx->p), GATE_PCG);
   if (!replicated) ir = reduce_items<6>(ctx, ir.part, ctx->red6, GATE_PCG, ir.ptr);
   LAUNCH(k_pcg_q, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, ir.ptr, ir.part, P<double>(ctx->dc), P<double>(ctx->p),
@@ -2007,15 +2069,15 @@ static void enqueue_pcg_iteration(ba_gpu_ctx *ctx, int it) {
   }
 }
 
-// reduced system solve by implicit Schur + block-Jacobi PCG; host polls the
-// device-side PCG controller every poll_interval iterations
-static int solve_implicit(ba_gpu_ctx *ctx) {
+// prologue of solve_sparse_chol and solve_pcg: the item partials of the reduced right-hand side (part6), the Jacobi blocks of
+// the matrix-free product (part21), then the values of the block-sparse S
+static void enqueue_reduced_rhs(ba_gpu_ctx *ctx) {
   LmState *st = P<LmState>(ctx->st);
-  if (ctx->fact) {
+  if (plan_factored(ctx->plan)) {
     const double *intr = P<double>(ctx->intr);
     LAUNCH(kf_schur_pass2, ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), P<int32_t>(ctx->pt_idx), ctx->Fc_,
            P<double>(ctx->geo), intr, P<double>(ctx->gc), P<double>(ctx->tgs), 0.0, P<double>(ctx->part6), st, GATE_RUN);
-    if (ctx->solver != BA_SOLVER_SPARSE_SCHUR_PCG)  // the block-sparse solver reads the diagonal blocks of S itself
+    if (!plan_sparse_ns(ctx->plan))  // the block-sparse solvers read the diagonal blocks of S themselves
     LAUNCH(kf_schur_diag, ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), P<int32_t>(ctx->pt_idx), ctx->Fc_,
            P<double>(ctx->geo), intr, P<double>(ctx->Vs), P<double>(ctx->part21), st, GATE_RUN);
   } else
@@ -2028,18 +2090,28 @@ static int solve_implicit(ba_gpu_ctx *ctx) {
   });
   phase_mark(ctx, BA_PHASE_RHS);
   enqueue_sparse_values(ctx, GATE_RUN);
-  // (the exact solve does not branch on the failure flags; the ranks agree on them after it, before the step is judged)
-  if (!ctx->spchol) sync_flags(ctx);
+}
+
+// exact step by the NS sparse Cholesky: b and the damping, then the factorisation and the two substitutions (yc written by the
+// last kernels).  The exact solve does not branch on the failure flags; the ranks agree on them after it, before the step is judged.
+static int solve_sparse_chol(ba_gpu_ctx *ctx) {
+  LmState *st = P<LmState>(ctx->st);
+  enqueue_reduced_rhs(ctx);
   phase_mark(ctx, BA_PHASE_SCHUR);
-  if (ctx->spchol) {
-    // exact step: b and the damping, then the factorisation and the two substitutions (yc written by the last kernels)
-    ItemRef i6c = reduce_items<6>(ctx, P<double>(ctx->part6), ctx->red6, GATE_RUN);
-    LAUNCH(k_spchol_rhs, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, i6c.ptr, i6c.part, P<double>(ctx->gc), P<double>(ctx->dc),
-           P<double>(ctx->b), P<double>(ctx->dsq), st, GATE_RUN, 0);
-    enqueue_spchol(ctx, GATE_RUN);
-    return 0;
-  }
-  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG) {
+  ItemRef i6c = reduce_items<6>(ctx, P<double>(ctx->part6), ctx->red6, GATE_RUN);
+  LAUNCH(k_spchol_rhs, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, i6c.ptr, i6c.part, P<double>(ctx->gc), P<double>(ctx->dc),
+         P<double>(ctx->b), P<double>(ctx->dsq), st, GATE_RUN, 0);
+  enqueue_spchol(ctx, GATE_RUN);
+  return 0;
+}
+
+// reduced system by block-Jacobi PCG on the block-sparse S or the matrix-free product, in the form plan.pcg names
+static int solve_pcg(ba_gpu_ctx *ctx) {
+  LmState *st = P<LmState>(ctx->st);
+  enqueue_reduced_rhs(ctx);
+  sync_flags(ctx);
+  phase_mark(ctx, BA_PHASE_SCHUR);
+  if (ctx->plan.lin == LIN_SPARSE_PCG) {
     LAUNCH(k_sp_minv, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->sp_diag), P<double>(ctx->Sblk), P<double>(ctx->dc),
            P<double>(ctx->Minv), P<double>(ctx->dsq), st, GATE_RUN);
   } else {
@@ -2052,7 +2124,7 @@ static int solve_implicit(ba_gpu_ctx *ctx) {
          P<double>(ctx->b), P<double>(ctx->x), P<double>(ctx->r), P<double>(ctx->z), P<double>(ctx->pcam_rho),
          P<double>(ctx->pcam_bb), st, GATE_RUN);
   LAUNCH(k_pcg_start, 1, BA_THREADS, 0, ctx->nblk_cam, P<double>(ctx->pcam_bb), P<double>(ctx->pcam_rho), st, GATE_RUN);
-  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG && ctx->opt.persistent_pcg == 1 && ctx->dist_pcg) {
+  if (ctx->plan.pcg == PCG_ROW_SHARDED) {
     // persistent PCG with the product row-sharded over the ranks, exchange through flag-in-data slots in
     // NVLink peer memory inside the kernel (ba_kernels_dist.cuh)
     cudaMemsetAsync(ctx->pcg_bar.p, 0, 16, ctx->stream);
@@ -2079,7 +2151,7 @@ static int solve_implicit(ba_gpu_ctx *ctx) {
     if (h_abort) return fail(ctx, BA_ERR_COMM, "row-sharded PCG: a peer GPU did not deliver its slots within 4 s");
     return 0;
   }
-  if (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG && ctx->opt.persistent_pcg && ctx->pcg_grid > 0) {
+  if (ctx->plan.pcg == PCG_PERSISTENT) {
     // the whole PCG solve in one cooperative launch (ba_kernels_sparse.cuh)
     cudaMemsetAsync(ctx->pcg_bar.p, 0, 16, ctx->stream);  // (profile counters at +64 accumulate over the solve)
     int n_cam = ctx->n_cam;
@@ -2100,6 +2172,7 @@ static int solve_implicit(ba_gpu_ctx *ctx) {
            GATE_RUN);
     return 0;
   }
+  // PCG_STEPS: the host polls the device-side PCG controller every poll_interval iterations
   const int batch = std::max(1, ctx->opt.poll_interval);
   int it = 1;
   for (;;) {
@@ -2196,11 +2269,9 @@ static int factor_blocked_lookahead2(ba_gpu_ctx *ctx, int n, int nt, double *S, 
   return 0;
 }
 
-static int solve_explicit(ba_gpu_ctx *ctx) {
+// the point-block inverses and W / WV of every observation: the prologue of solve_dense and solve_sparse_bordered
+static void enqueue_obs_W(ba_gpu_ctx *ctx) {
   LmState *st = P<LmState>(ctx->st);
-  const int n = ctx->n_red;
-  if (n == 0) return 0;
-  if (!ctx->sp_ref) cudaMemsetAsync(ctx->S.p, 0, (size_t)n * n * 8, ctx->stream);
   // side stream: point-block inverses (k_obs_W re-derives the inverse it needs), then -- once W is there -- borders +
   // right-hand side; main stream: W, then the camera-camera blocks (disjoint parts of S)
   fork_side(ctx);
@@ -2212,37 +2283,50 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
            P<double>(ctx->dp), P<double>(ctx->W), P<double>(ctx->WV), st, GATE_RUN);
   });
   side_after_main(ctx);
-  if (ctx->sp_ref) {
-    // sparse Cholesky: side stream -- camera-side vectors, then b_c, B, C and b_k by camera; main stream -- the blocks of S
-    if (ctx->nk) {
-      LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
-             P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
-             P<double>(ctx->part_ex), ctx->n_pt, P<double>(ctx->Vinv), P<double>(ctx->part_kk), st, GATE_RUN);
-      LAUNCH((k_spb_assemble<4>), cdiv(ctx->n_cam * 30 + 14, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
-             P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
-             P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
-             P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
-    } else {
-      LAUNCH((k_explicit_cam<0>), ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), P<int32_t>(ctx->pt_idx),
-             P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk), P<double>(ctx->part_ex), st, GATE_RUN);
-      LAUNCH((k_spb_assemble<0>), cdiv(ctx->n_cam * 6, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
-             P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
-             P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
-             P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
-    }
-    fork_main(ctx);
-    LAUNCH(k_sp_schur_planes, cdiv(ctx->n_sblk * 32, BA_THREADS), BA_THREADS, 0, ctx->n_sblk, P<int32_t>(ctx->sb_ptr),
-           P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->Sblk), st, GATE_RUN);
-    LAUNCH(k_sp_add_diag, cdiv(ctx->n_cam * 36, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->sp_diag), P<double>(ctx->U),
-           P<double>(ctx->Sblk), st, GATE_RUN);
-    join(ctx);
-    phase_mark(ctx, BA_PHASE_SCHUR);
-    // LM damping of the camera columns (b is already assembled), then factorisation, border and substitutions
-    LAUNCH(k_spchol_rhs, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->item_ptr), P<double>(ctx->part6), P<double>(ctx->gc),
-           P<double>(ctx->dc), P<double>(ctx->b), P<double>(ctx->dsq), st, GATE_RUN, 1);
-    enqueue_spchol(ctx, GATE_RUN);
-    return 0;
+}
+
+// bordered sparse Cholesky: the dense solver's W / WV, the block-sparse S and the tree instead of the dense S
+static int solve_sparse_bordered(ba_gpu_ctx *ctx) {
+  LmState *st = P<LmState>(ctx->st);
+  if (ctx->n_red == 0) return 0;
+  enqueue_obs_W(ctx);
+  // sparse Cholesky: side stream -- camera-side vectors, then b_c, B, C and b_k by camera; main stream -- the blocks of S
+  if (ctx->nk) {
+    LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
+           P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
+           P<double>(ctx->part_ex), ctx->n_pt, P<double>(ctx->Vinv), P<double>(ctx->part_kk), st, GATE_RUN);
+    LAUNCH((k_spb_assemble<4>), cdiv(ctx->n_cam * 30 + 14, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
+           P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
+           P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
+           P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
+  } else {
+    LAUNCH((k_explicit_cam<0>), ctx->nblk_item, BA_THREADS, 0, ctx->n_items, P<BaItem>(ctx->items), P<int32_t>(ctx->pt_idx),
+           P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk), P<double>(ctx->part_ex), st, GATE_RUN);
+    LAUNCH((k_spb_assemble<0>), cdiv(ctx->n_cam * 6, BA_THREADS), BA_THREADS, 0, ctx->n_cam, ctx->fixed_cam,
+           P<int32_t>(ctx->item_ptr), P<double>(ctx->part_ex), ctx->nblk_pt, P<double>(ctx->part_kk), P<double>(ctx->gc),
+           P<double>(ctx->Uck), P<double>(ctx->Ukk), P<double>(ctx->gk), P<double>(ctx->dk), P<double>(ctx->b),
+           P<double>(ctx->spb_B), P<double>(ctx->spb_kk), st, GATE_RUN);
   }
+  fork_main(ctx);
+  LAUNCH(k_sp_schur_planes, cdiv(ctx->n_sblk * 32, BA_THREADS), BA_THREADS, 0, ctx->n_sblk, P<int32_t>(ctx->sb_ptr),
+         P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->Sblk), st, GATE_RUN);
+  LAUNCH(k_sp_add_diag, cdiv(ctx->n_cam * 36, BA_THREADS), BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->sp_diag), P<double>(ctx->U),
+         P<double>(ctx->Sblk), st, GATE_RUN);
+  join(ctx);
+  phase_mark(ctx, BA_PHASE_SCHUR);
+  // LM damping of the camera columns (b is already assembled), then factorisation, border and substitutions
+  LAUNCH(k_spchol_rhs, ctx->nblk_cam, BA_THREADS, 0, ctx->n_cam, P<int32_t>(ctx->item_ptr), P<double>(ctx->part6), P<double>(ctx->gc),
+         P<double>(ctx->dc), P<double>(ctx->b), P<double>(ctx->dsq), st, GATE_RUN, 1);
+  enqueue_spchol(ctx, GATE_RUN);
+  return 0;
+}
+
+static int solve_dense(ba_gpu_ctx *ctx) {
+  LmState *st = P<LmState>(ctx->st);
+  const int n = ctx->n_red;
+  if (n == 0) return 0;
+  cudaMemsetAsync(ctx->S.p, 0, (size_t)n * n * 8, ctx->stream);
+  enqueue_obs_W(ctx);
   if (ctx->nk) {
     LAUNCH(k_explicit_cam_kk, ctx->nblk_item + ctx->nblk_pt, BA_THREADS, 0, ctx->nblk_item, ctx->n_items, P<BaItem>(ctx->items),
            P<int32_t>(ctx->pt_idx), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->tg), P<double>(ctx->Wk),
@@ -2327,14 +2411,23 @@ static int solve_explicit(ba_gpu_ctx *ctx) {
 static int enqueue_lm_iteration(ba_gpu_ctx *ctx) {
   LmState *st = P<LmState>(ctx->st);
   const int D = ctx->depth, K = ctx->nk;
-  if (ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY) enqueue_point_inverse(ctx, GATE_RUN);  // (explicit: inside solve_explicit)
+  // (the dense and the bordered solve run the point inverses on the side stream, next to W)
+  const bool own_inverse = ctx->plan.lin == LIN_DENSE || ctx->plan.lin == LIN_SPARSE_BORDERED;
+  if (!own_inverse) enqueue_point_inverse(ctx, GATE_RUN);
   phase_mark(ctx, BA_PHASE_POINT_INVERSE);
-  int rc = ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY ? solve_implicit(ctx) : solve_explicit(ctx);
+  int rc = 0;
+  switch (ctx->plan.lin) {
+    case LIN_DENSE: rc = solve_dense(ctx); break;
+    case LIN_SPARSE_BORDERED: rc = solve_sparse_bordered(ctx); break;
+    case LIN_SPARSE_CHOL: rc = solve_sparse_chol(ctx); break;
+    case LIN_SPARSE_PCG:
+    case LIN_IMPLICIT_PCG: rc = solve_pcg(ctx); break;
+  }
   if (rc) return rc;
   phase_mark(ctx, BA_PHASE_SUBSTITUTION);
   // step evaluation: back-substitution y = (y_c, y_p), the model cost change, the candidate x+ and its cost
   int nblk_mcc = ctx->nblk_obs, nblk_step = ctx->nblk_ent;
-  if (ctx->fact) {
+  if (plan_factored(ctx->plan)) {
     // the candidate cameras and intrinsics first (no points: entries [0, n_cam]); then one point-major pass over the tiles does
     // the rest (camera run staged in shared memory)
     const int nblk_cc = cdiv(ctx->n_cam + 1, BA_THREADS);
@@ -2399,7 +2492,7 @@ static int enqueue_lm_iteration(ba_gpu_ctx *ctx) {
   }
   phase_mark(ctx, BA_PHASE_CONTROL);
   // accepted: x <- x+, relinearise (all gated on the device-side decision)
-  const bool overlap_accept = ctx->forking && !ctx->fact;  // windowed explicit path
+  const bool overlap_accept = ctx->forking && !plan_factored(ctx->plan);  // windowed dense path
   if (overlap_accept) fork_side(ctx);
   LAUNCH(k_accept, ctx->nblk_ent, BA_THREADS, 0, ctx->n_cam, ctx->n_pt, P<double>(ctx->pose), P<double>(ctx->pt), P<double>(ctx->intr),
          P<double>(ctx->pose_c), P<double>(ctx->pt_c), P<double>(ctx->intr_c), st, GATE_ACCEPTED);
@@ -2429,11 +2522,10 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   ctx->cur = ctx->stream;
   const int64_t l0 = ctx->launches;
   CK(cudaEventRecord(ctx->ev0, ctx->stream));
-  // windowed explicit solver on one GPU (single-CTA solve: every kernel is a small gated kernel): programmatic dependent launches
-  const bool pdl = !ctx->pdl_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && !ctx->sp_ref && ctx->n_ranks == 1 && ctx->n_red > 0 &&
-                   ctx->n_red <= BA_LDLT_MAX_N;
+  const bool windowed = plan_windowed(ctx);
+  const bool pdl = !ctx->pdl_off && windowed;
   ctx->pdl = pdl;
-  ctx->ph_on = (ctx->solver != BA_SOLVER_EXPLICIT_CHOLESKY || ctx->sp_ref) && getenv("BA_NO_PHASE_TIMES") == nullptr;
+  ctx->ph_on = plan_phase_times(ctx->plan) && getenv("BA_NO_PHASE_TIMES") == nullptr;
   ctx->ph_n = 0;
   phase_mark(ctx, BA_PHASE_START);
   enqueue_iteration_zero(ctx);
@@ -2441,10 +2533,8 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   ctx->pdl = false;
   const int poll = std::max(1, ctx->opt.poll_interval);
   int rc = 0;
-  // windowed explicit solver on one GPU: the ~26 small kernels of an LM iteration (two streams, fork / join) are
-  // captured once per upload and replayed
-  const bool graphed = !ctx->lm_graph_off && ctx->solver == BA_SOLVER_EXPLICIT_CHOLESKY && !ctx->sp_ref && ctx->n_ranks == 1 &&
-                       ctx->n_red > 0 && ctx->n_red <= BA_LDLT_MAX_N;
+  // windowed: the ~26 small kernels of an LM iteration (two streams, fork / join) are captured once per upload and replayed
+  const bool graphed = !ctx->lm_graph_off && windowed;
   for (int it = 1;; ++it) {
     if (graphed) {
       if (!ctx->lm_graph || ctx->lm_graph_stale) {
@@ -2490,10 +2580,7 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
     // flag after every solve; every other path takes all decisions on the device, so the host only looks at the controller
     // state every poll_interval iterations and keeps the launch queue full in between (a host synchronisation per LM
     // iteration left the GPU idle while the ~60 launches of the next iteration were being enqueued).
-    const bool host_in_loop = ctx->solver == BA_SOLVER_IMPLICIT_PCG ||
-                              (ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG && !ctx->spchol &&
-                               (ctx->dist_pcg || !(ctx->opt.persistent_pcg && ctx->pcg_grid > 0)));
-    if (!host_in_loop && (it % poll) != 0 && it <= ctx->lo.max_num_iterations) continue;
+    if (!plan_host_polls_pcg(ctx->plan) && (it % poll) != 0 && it <= ctx->lo.max_num_iterations) continue;
     rc = poll_state(ctx);
     if (rc) return rc;
     if (ctx->h_st->done) break;
@@ -2520,7 +2607,7 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   s.initial_cost = h.initial_cost;
   s.final_cost = h.x_cost;
   s.total_linear_iters = h.total_lin_iters;
-  s.solver_used = ctx->spchol ? BA_SOLVER_SPARSE_SCHUR_CHOLESKY : ctx->solver;
+  s.solver_used = plan_solver_used(ctx->plan);
   s.reduced_dim = ctx->n_red;
   s.solve_ms = ms;
   s.kernel_launches = ctx->launches - l0;
@@ -2529,7 +2616,7 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
   if (nt) CK(cudaMemcpy(ctx->h_trace.data(), ctx->trace.p, (size_t)nt * sizeof(BaIterRec), cudaMemcpyDeviceToHost));
   ctx->last_summary = s;
   if (summary) *summary = s;
-  if (getenv("BA_SPCHOL_PROF") && ctx->spchol) {
+  if (getenv("BA_SPCHOL_PROF") && plan_tree(ctx->plan)) {
     unsigned long long pr[8];
     cudaMemcpy(pr, ctx->spc_prof.p, 64, cudaMemcpyDeviceToHost);
     cudaMemset(ctx->spc_prof.p, 0, 64);
@@ -2537,7 +2624,7 @@ extern "C" int ba_gpu_solve(ba_gpu_ctx *ctx, ba_gpu_summary *summary) {
     fprintf(stderr, "[BA_SPCHOL_PROF] us per factor launch (thread block 0, %llu launches): assemble S %.2f | extend-add %.2f | factor loop %.2f | "
                     "write panel %.2f\n", pr[4], pr[0] / n / 1e3, pr[1] / n / 1e3, pr[2] / n / 1e3, pr[3] / n / 1e3);
   }
-  if (getenv("BA_PCG_PROF") && ctx->pcg_bar.p && ctx->solver == BA_SOLVER_SPARSE_SCHUR_PCG) {
+  if (getenv("BA_PCG_PROF") && ctx->pcg_bar.p && plan_sparse_ns(ctx->plan)) {
     unsigned long long pr[6];
     cudaMemcpy(pr, P<unsigned long long>(ctx->pcg_bar) + 8, 48, cudaMemcpyDeviceToHost);
     cudaMemset(P<unsigned long long>(ctx->pcg_bar) + 8, 0, 48);
@@ -2713,7 +2800,7 @@ extern "C" int ba_gpu_schur_matvec(ba_gpu_ctx *ctx, double radius, const double 
   if (!ctx || !x || !y) return BA_ERR_INVALID;
   if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_schur_matvec before ba_gpu_upload");
   if (ctx->nk) return fail(ctx, BA_ERR_UNSUPPORTED, "implicit Schur product needs optimize_intrinsics = 0");
-  if (ctx->sp_ref) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_matvec with the sparse Cholesky needs NS mode");
+  if (ctx->plan.lin == LIN_SPARSE_BORDERED) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_matvec with the sparse Cholesky needs NS mode");
   CK(cudaSetDevice(ctx->device));
   ctx->sp_full_next = true;  // (the product needs every block of S on every rank)
   int rc = prepare_linear_system(ctx, radius);
@@ -2739,8 +2826,8 @@ extern "C" int ba_gpu_schur_matvec(ba_gpu_ctx *ctx, double radius, const double 
 extern "C" int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *rhs, double *y) {
   if (!ctx || !rhs || !y) return BA_ERR_INVALID;
   if (!ctx->uploaded) return fail(ctx, BA_ERR_STATE, "ba_gpu_schur_solve before ba_gpu_upload");
-  if (!ctx->spchol) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs the sparse Cholesky solver");
-  if (ctx->sp_ref) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs NS mode (no depth prior, fixed intrinsics)");
+  if (!plan_tree(ctx->plan)) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs the sparse Cholesky solver");
+  if (ctx->plan.lin == LIN_SPARSE_BORDERED) return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_schur_solve needs NS mode (no depth prior, fixed intrinsics)");
   CK(cudaSetDevice(ctx->device));
   int rc = prepare_linear_system(ctx, radius);
   if (rc) return rc;
@@ -2765,30 +2852,23 @@ extern "C" int ba_gpu_schur_solve(ba_gpu_ctx *ctx, double radius, const double *
 
 // ------------------------------------------------------------------ covariance
 // structure of ba_gpu_covariance, once per upload: under another solver (dense explicit, matrix-free PCG) the block structure and the symbolic tree
-// that solver = 4 builds (the sp_ref branch of the upload); then the selected-inversion queue, the block -> front records and
+// that solver = 4 builds (LIN_SPARSE_BORDERED); then the selected-inversion queue, the block -> front records and
 // the scratch buffers.  Growing buffers a captured LM-iteration graph may point at marks that graph stale.
 static int cov_prepare(ba_gpu_ctx *ctx) {
   if (ctx->cov_ready) return 0;
   cudaStream_t s = ctx->stream;
   int rc;
-  if (!ctx->sp_ref) {
+  if (!plan_tree(ctx->plan)) {
     ctx->lm_graph_stale = true;
     if ((rc = build_sparse_structure(ctx))) return rc;
-    ctx->spc_nrhs = ctx->nk ? 5 : 1;
-    rc = build_spchol(ctx);
-    ctx->spchol = false;  // (the LM solve of this context stays the dense explicit one)
+    rc = build_spchol(ctx, 1, ctx->nk ? 5 : 1);
     if (rc == BA_ERR_UNSUPPORTED) {
       const std::string why = ctx->err;
       return fail(ctx, BA_ERR_UNSUPPORTED, "ba_gpu_covariance: %s", why.c_str());
     }
     if (rc) return rc;
-    const size_t nc = (size_t)ctx->n_cam;
-    RES(W, ((size_t)ctx->n_obs + 1) * 144);  // (the matrix-free PCG, AUTO on a large DEPTH problem, has no per-observation W)
-    RES(WV, ((size_t)ctx->n_obs + 1) * 144);
-    RES(spb_B, nc * 192 + 64);
-    RES(spb_Z, nc * 192 + 64);
-    RES(spb_kk, 20 * 8);
-    RES(spb_part, (size_t)(ctx->nblk_cam + 1) * 14 * 8);
+    // (the matrix-free PCG, AUTO on a large DEPTH problem, has no per-observation W)
+    if ((rc = reserve_bordered(ctx))) return rc;
   }
   const SpSymbolic &S = ctx->sym;
   auto N_ = [&](int id, int f) { return S.node[(size_t)id * SPSYM_NODE_INTS + f]; };
@@ -3295,7 +3375,7 @@ extern "C" int ba_gpu_covariance_pivots(const ba_gpu_ctx *ctx, double ratio[2]) 
 extern "C" int ba_gpu_spchol_info(const ba_gpu_ctx *ctx, int64_t info[24]) {
   if (!ctx || !info) return BA_ERR_INVALID;
   memset(info, 0, 24 * sizeof(int64_t));
-  if (!ctx->uploaded || !ctx->spchol) return BA_OK;
+  if (!ctx->uploaded || !plan_tree(ctx->plan)) return BA_OK;
   const SpSymbolic &s = ctx->sym;
   info[0] = s.n_cam; info[1] = s.n_nodes; info[2] = s.n_levels; info[3] = s.panel_blocks; info[4] = s.u_blocks;
   info[5] = s.max_front_blocks; info[6] = s.max_m; info[7] = s.max_nb; info[8] = s.max_children;
@@ -3424,7 +3504,7 @@ extern "C" int ba_gpu_time_kernel(ba_gpu_ctx *ctx, int32_t which, int32_t warmup
   LmState *st = P<LmState>(ctx->st);
   LAUNCH(k_clear_done, 1, 1, 0, st);
   // the two-pass product of the factored store reads the point-major records, which only the implicit solver keeps
-  const bool two_pass = !ctx->fact || ctx->fp_store;
+  const bool two_pass = !plan_factored(ctx->plan) || plan_point_records(ctx->plan);
   if ((which == BA_KERNEL_SCHUR_PASS1 || which == BA_KERNEL_SCHUR_PASS2) && !two_pass)
     return fail(ctx, BA_ERR_UNSUPPORTED, "the two-pass product runs with the implicit solver only (solver = 2)");
   if (which != BA_KERNEL_LINEARIZE) {
@@ -3435,7 +3515,7 @@ extern "C" int ba_gpu_time_kernel(ba_gpu_ctx *ctx, int32_t which, int32_t warmup
   const size_t flush_n = (size_t)512 * 1024 * 1024 / 8;  // 512 MiB > 126 MB L2
   if (flush_l2) RES(flush, flush_n * 8);
   auto one = [&]() {
-    if (which == BA_KERNEL_LINEARIZE && ctx->fact) {
+    if (which == BA_KERNEL_LINEARIZE && plan_factored(ctx->plan)) {
       LAUNCH(kf_linearize, ctx->nblk_obs, BA_THREADS, 0, ctx->n_obs, P<int32_t>(ctx->cam_idx), P<int32_t>(ctx->pt_idx),
              P<double2>(ctx->uv), P<double>(ctx->pose), P<double>(ctx->pt), P<double>(ctx->geo), P<double>(ctx->intr), ctx->cp,
              ctx->Fc_, P<double>(ctx->pc_lin), st, GATE_RUN);

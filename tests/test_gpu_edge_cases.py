@@ -105,7 +105,9 @@ def test_single_camera_window():
 
 def test_auto_policy():
     """AUTO: dense explicit for windows, block-sparse S factorised exactly for large sequential NS problems, implicit
-    when the co-visibility is dense (pairs per observation above the threshold)."""
+    when the co-visibility is dense (pairs per observation above the threshold).  Then the whole table of cost mode x solver x
+    Jacobian store on three problems: the upload's return code, the solver and store in force, and whether the block-sparse S
+    and the supernodal tree exist."""
     s = _solver()
     try:
         s.upload(syn.make_config(1))
@@ -126,6 +128,107 @@ def test_auto_policy():
     try:
         s.upload(p)
         assert s.solve().solver_used == cap.BA_SOLVER_IMPLICIT_PCG
+    finally:
+        s.close()
+    # every cost mode x solver x Jacobian store on a window, on the sequence above and on wide co-visibility
+    seq = p.copy()
+    seq.depth = syn.camera_point(seq.pose7[seq.cam_idx], seq.pt3[seq.pt_idx])[:, 2].copy()  # (for the depth-prior modes)
+    problems = [("cfg1", syn.make_config(1), {}, True), ("seq", seq, dict(explicit_max_dim=36), True),
+                ("wide", _wide_covisibility(), {}, False)]
+    wrong = []
+    for name, prob, kw, fronts_fit in problems:
+        tiles_ok = _tiles_fit(prob)
+        for mode in ("NS", "DEPTH", "INTR", "REF"):
+            for solver in range(5):
+                for store in range(4):
+                    n_red = 6 * (prob.n_cam - 1) + (4 if mode in ("INTR", "REF") else 0)
+                    want = _expected_plan(mode, solver, store, n_red, kw.get("explicit_max_dim", 160), fronts_fit, tiles_ok)
+                    wrong += _check_plan(prob, mode, solver, store, kw, want, (name, mode, solver, store))
+    assert not wrong, "\n".join(wrong)
+
+
+def _wide_covisibility(n_cam=800, n_pt=4000, seed=5):
+    """Every point is seen by three random cameras of 800: few observation pairs per observation, so AUTO builds the block-sparse
+    S on an NS problem, but the co-visibility is so wide that no front of its Cholesky fits shared memory.  The cameras sit on
+    a plane and look along +z at points 20 to 40 m away."""
+    rng = np.random.default_rng(seed)
+    K = syn.K_TUM.copy()
+    truth = np.zeros((n_cam, 7))
+    truth[:, 3] = 1.0
+    truth[:, 4:6] = rng.uniform(-2.0, 2.0, (n_cam, 2))
+    truth_pt = np.stack([rng.uniform(-3, 3, n_pt), rng.uniform(-2, 2, n_pt), rng.uniform(20, 40, n_pt)], axis=1)
+    cam = np.concatenate([rng.choice(n_cam, 3, replace=False) for _ in range(n_pt)])
+    lm = np.repeat(np.arange(n_pt), 3)
+    order = np.lexsort((lm, cam))
+    cam, lm = cam[order], lm[order]
+    uv, z = syn.project(truth[cam], truth_pt[lm], K)
+    uv = uv + 0.5 * rng.standard_normal(uv.shape)
+    pose = truth.copy()
+    pose[1:, 4:] += 0.01 * rng.standard_normal((n_cam - 1, 3))
+    pt = truth_pt + 0.05 * rng.standard_normal(truth_pt.shape)
+    return ba_b200.BAProblem(pose, pt, cam.astype(np.int32), lm.astype(np.int32), uv, z + 0.01 * rng.standard_normal(z.shape),
+                             K, None, 0)
+
+
+def _tiles_fit(p, tile_pts=128, max_span=64, max_obs=2048):
+    """The tiled store's bounds (BA_JAC_TILED): every tile of 128 consecutive points spans <= 64 cameras and holds <= 2048
+    observations."""
+    tile = p.pt_idx // tile_pts
+    for t in np.unique(tile):
+        c = p.cam_idx[tile == t]
+        if c.max() - c.min() + 1 > max_span or c.size > max_obs:
+            return False
+    return True
+
+
+def _expected_plan(mode, solver, store, n_red, explicit_max_dim, fronts_fit, tiles_ok):
+    """(upload return code, solver_used, jacobian_store_used) by the rules of include/ba_gpu.h for one GPU below the dense
+    limit (BA_SOLVER_* and BA_JAC_* comments; AUTO's pair threshold holds on these problems)."""
+    U = cap.BA_ERR_UNSUPPORTED
+    depth, intr = mode in ("DEPTH", "REF"), mode in ("INTR", "REF")
+    if solver == 4 and (depth or intr):        # the bordered sparse Cholesky: planes store only
+        if store in (cap.BA_JAC_FACTORED, cap.BA_JAC_TILED) or not fronts_fit:
+            return U, None, None
+        return 0, 4, cap.BA_JAC_PLANES
+    s = solver
+    if s == 0:
+        s = 1 if (n_red <= explicit_max_dim or intr) else 2
+    if s in (2, 3, 4) and intr:                 # points-only solvers
+        return U, None, None
+    if s in (3, 4) and depth:                   # the block-sparse solvers need NS mode
+        return U, None, None
+    if s == 1:                                  # dense: planes store (FACTORED needs NS + PCG, TILED falls back)
+        return (U, None, None) if store == cap.BA_JAC_FACTORED else (0, 1, cap.BA_JAC_PLANES)
+    if s == 2 and depth:                        # matrix-free with depth prior: planes store
+        return (U, None, None) if store == cap.BA_JAC_FACTORED else (0, 2, cap.BA_JAC_PLANES)
+    if store == cap.BA_JAC_PLANES:              # NS: the block-sparse solvers rebuild S from the factored store
+        return (U, None, None) if s in (3, 4) else (0, 2, cap.BA_JAC_PLANES)
+    if s == 2 and solver == 0:                  # AUTO on a large NS problem with sparse co-visibility: block-sparse S,
+        return 0, 4 if fronts_fit else 3, cap.BA_JAC_FACTORED   # factorised when the fronts fit, else PCG
+    if s == 2:                                  # matrix-free: tiled where the tile bounds hold
+        if tiles_ok and store != cap.BA_JAC_FACTORED:
+            return 0, 2, cap.BA_JAC_TILED
+        return (U, None, None) if store == cap.BA_JAC_TILED else (0, 2, cap.BA_JAC_FACTORED)
+    if s == 4 and not fronts_fit:
+        return U, None, None
+    return 0, s, cap.BA_JAC_FACTORED
+
+
+def _check_plan(prob, mode, solver, store, kw, want, case):
+    g, _ = mode_opts(mode, solver=solver, jacobian_store=store, max_num_iterations=1, **kw)
+    s = _solver(**g)
+    try:
+        try:
+            s.upload(prob)
+        except ba_b200.BAError as e:
+            return [] if e.code == want[0] else [f"{case}: upload rc {e.code} ({e}), expected {want}"]
+        if want[0] != 0:
+            return [f"{case}: upload succeeded, expected rc {want[0]}"]
+        used, store_used = s.solve().solver_used, s.jacobian_store_used()
+        sparse_s, tree = s.sparse_stats()[1] > 0, bool(s.spchol_info())
+        got = (used, store_used, sparse_s, tree)
+        exp = (want[1], want[2], want[1] in (3, 4), want[1] == 4)
+        return [] if got == exp else [f"{case}: (solver_used, store, sparse S, tree) {got}, expected {exp}"]
     finally:
         s.close()
 
