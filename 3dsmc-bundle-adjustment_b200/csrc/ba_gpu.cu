@@ -170,7 +170,6 @@ struct ba_gpu_ctx {
   int n_my_rows = 0, dist_grid = 0;
   long long n_pairs = 0;
   // exact sparse Cholesky of S (ba_sparse_symbolic.h / ba_kernels_spchol.cuh)
-  bool src_on_device = false;   // the arrays handed to the current upload live in device memory (ba_store_window_solve)
   SpSymbolic sym;               // host-side structure of the last upload
   Buf spn_node, spn_bord, spn_children, spn_rel, spn_inv, spn_aent, spn_perm;
   Buf spc_panel, spc_U, spc_z, spc_linv, spc_ypos, spc_prof, spc_queue, spc_tiles, spc_cnt, spc_cnt_init, spc_topcams;
@@ -225,10 +224,12 @@ struct ba_gpu_ctx {
   // multi-GPU staging (dense per-camera sums, scalars, identity item_ptr)
   Buf red_blk, red6, red21, scal, ident;
   // explicit solver
-  Buf W, WV, S, rhs, blk_i, blk_j, blk_cam, pair_ptr, pair_a, pair_b;
-  Buf ex_keys, ex_keys2, ex_vals, ex_vals2, blk_cnt;  // device-built pair list (windows)
-  int n_blk = 0;
-  int ex_band_cams = -1;  // largest camera-slot distance of a non-empty block of the dense explicit S (-1: unknown = dense)
+  Buf W, WV, S, rhs;
+  // block table of k_schur_pairs (build_dense_blocks): the blocks of build_pair_blocks() (sp_ukeys, sb_ptr, count sp_nruns), then
+  // n_xdiag empty diagonal blocks (keys sp_xdiag); n_blk CTAs are launched
+  Buf sp_xdiag;
+  int n_blk = 0, n_xdiag = 0;
+  int ex_band_cams = -1;  // largest camera-slot distance of a block of the dense explicit S (-1: dense; set for the blocked factorisation)
   // controller
   Buf st, trace;
   LmState *h_st = nullptr;  // pinned
@@ -612,87 +613,6 @@ __global__ void k_slots(int n_cam, int fixed_cam, int32_t *slot) {
   if (c < n_cam) slot[c] = (c == fixed_cam) ? -1 : (fixed_cam >= 0 && c > fixed_cam ? c - 1 : c);
 }
 
-// host-side pair list of the explicit Schur complement: for every block pair
-// (i <= j) of free-camera slots the (obs_a, obs_b) pairs that share a point, in
-// point-major order.  Pure index plumbing; values never touch the host.
-static int build_pair_list(ba_gpu_ctx *ctx, const int32_t *cam_idx, const int32_t *pt_idx) {
-  const int n_obs = ctx->n_obs, n_pt = ctx->n_pt, nf = ctx->n_free;
-  std::vector<int32_t> rowptr((size_t)n_pt + 1, 0), perm((size_t)n_obs);
-  for (int i = 0; i < n_obs; ++i) rowptr[pt_idx[i] + 1]++;
-  for (int p = 0; p < n_pt; ++p) rowptr[p + 1] += rowptr[p];
-  {
-    std::vector<int32_t> cur(rowptr.begin(), rowptr.end() - 1);
-    for (int i = 0; i < n_obs; ++i) perm[cur[pt_idx[i]]++] = i;
-  }
-  auto slot = [&](int c) { return c == ctx->fixed_cam ? -1 : (ctx->fixed_cam >= 0 && c > ctx->fixed_cam ? c - 1 : c); };
-  const size_t nb_all = (size_t)nf * (nf + 1) / 2;
-  auto bidx = [&](int i, int j) { return (size_t)i * nf - (size_t)i * (i - 1) / 2 + (j - i); };
-  std::vector<int64_t> cnt(nb_all + 1, 0);
-  for (int p = 0; p < n_pt; ++p)
-    for (int a = rowptr[p]; a < rowptr[p + 1]; ++a) {
-      const int sa = slot(cam_idx[perm[a]]);
-      if (sa < 0) continue;
-      for (int b = rowptr[p]; b < rowptr[p + 1]; ++b) {
-        const int sb = slot(cam_idx[perm[b]]);
-        if (sb < sa) continue;
-        cnt[bidx(sa, sb) + 1]++;
-      }
-    }
-  // keep every diagonal block (damping only when a camera has no observation)
-  std::vector<int32_t> bi, bj, bc, pptr;
-  std::vector<int64_t> start(nb_all, -1);
-  int64_t total = 0;
-  std::vector<int> slot_cam(nf);
-  for (int c = 0; c < ctx->n_cam; ++c)
-    if (slot(c) >= 0) slot_cam[slot(c)] = c;
-  for (int i = 0; i < nf; ++i)
-    for (int j = i; j < nf; ++j) {
-      const size_t k = bidx(i, j);
-      if (cnt[k + 1] == 0 && i != j) continue;
-      start[k] = total;
-      bi.push_back(i);
-      bj.push_back(j);
-      bc.push_back(slot_cam[i]);
-      pptr.push_back((int32_t)total);
-      total += cnt[k + 1];
-    }
-  if (total > 0x7fffffff) return fail(ctx, BA_ERR_UNSUPPORTED, "explicit Schur pair list too large");
-  pptr.push_back((int32_t)total);
-  std::vector<int32_t> pa((size_t)total), pb((size_t)total);
-  std::vector<int64_t> cur(start);
-  for (int p = 0; p < n_pt; ++p)
-    for (int a = rowptr[p]; a < rowptr[p + 1]; ++a) {
-      const int sa = slot(cam_idx[perm[a]]);
-      if (sa < 0) continue;
-      for (int b = rowptr[p]; b < rowptr[p + 1]; ++b) {
-        const int sb = slot(cam_idx[perm[b]]);
-        if (sb < sa) continue;
-        const int64_t w = cur[bidx(sa, sb)]++;
-        pa[w] = perm[a];
-        pb[w] = perm[b];
-      }
-    }
-  ctx->n_blk = (int)bi.size();
-  ctx->ex_band_cams = 0;
-  for (size_t b = 0; b < bi.size(); ++b) ctx->ex_band_cams = std::max(ctx->ex_band_cams, bj[b] - bi[b]);
-  RES(blk_i, bi.size() * 4);
-  RES(blk_j, bi.size() * 4);
-  RES(blk_cam, bi.size() * 4);
-  RES(pair_ptr, pptr.size() * 4);
-  RES(pair_a, pa.size() * 4);
-  RES(pair_b, pb.size() * 4);
-  CK(cudaMemcpyAsync(ctx->blk_i.p, bi.data(), bi.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->blk_j.p, bj.data(), bj.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->blk_cam.p, bc.data(), bc.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->pair_ptr.p, pptr.data(), pptr.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-  if (total) {
-    CK(cudaMemcpyAsync(ctx->pair_a.p, pa.data(), pa.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->pair_b.p, pb.data(), pb.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-  }
-  CK(cudaStreamSynchronize(ctx->stream));  // host vectors die here
-  return 0;
-}
-
 // materialised Jacobian planes, allocated on demand (always for the explicit /
 // REF path; lazily for the un-scaled evaluation hook when the store is factored)
 static int ensure_planes(ba_gpu_ctx *ctx) {
@@ -727,80 +647,32 @@ static int allreduce_host_scalar(ba_gpu_ctx *ctx, double *v, bool is_max) {
   CK(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
-// pair list of the dense explicit solver, device-built (windowed problems: the host loop of build_pair_list()
-// plus its six host->device copies were the largest part of ba_gpu_upload).  Every block of the upper triangle is
-// listed; k_schur_pairs skips the empty off-diagonal ones.
-static int build_pair_list_device(ba_gpu_ctx *ctx) {
-  const int n_pt = ctx->n_pt, nf = ctx->n_free;
-  const int nb_all = nf * (nf + 1) / 2;
-  cudaStream_t s = ctx->stream;
-  RES(sp_cnt, ((size_t)n_pt + 2) * 8);
-  RES(sp_off, ((size_t)n_pt + 2) * 8);
-  LAUNCH(k_sp_count, cdiv(n_pt + 1, BA_THREADS), BA_THREADS, 0, n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-         ctx->fixed_cam, P<long long>(ctx->sp_cnt));
-  CUBCALL(cub::DeviceScan::ExclusiveSum, P<long long>(ctx->sp_cnt), P<long long>(ctx->sp_off), n_pt + 1);
-  long long n_pairs = 0;
-  CK(cudaMemcpyAsync(&n_pairs, P<long long>(ctx->sp_off) + n_pt, 8, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  if (n_pairs > 0x7fffffffLL) return fail(ctx, BA_ERR_UNSUPPORTED, "explicit Schur pair list too large");
-  const size_t np1 = (size_t)n_pairs + 1;
-  RES(ex_keys, np1 * 4);
-  RES(ex_keys2, np1 * 4);
-  RES(ex_vals, np1 * 8);
-  RES(ex_vals2, np1 * 8);
-  RES(blk_cnt, ((size_t)nb_all + 2) * 4);
-  RES(blk_i, ((size_t)nb_all + 1) * 4);
-  RES(blk_j, ((size_t)nb_all + 1) * 4);
-  RES(blk_cam, ((size_t)nb_all + 1) * 4);
-  RES(pair_ptr, ((size_t)nb_all + 2) * 4);
-  RES(pair_a, np1 * 4);
-  RES(pair_b, np1 * 4);
-  CK(cudaMemsetAsync(ctx->blk_cnt.p, 0, ((size_t)nb_all + 2) * 4, s));
-  LAUNCH(k_ex_emit, ctx->nblk_pt, BA_THREADS, 0, n_pt, nf, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam), P<int32_t>(ctx->perm),
-         ctx->fixed_cam, P<long long>(ctx->sp_off), P<uint32_t>(ctx->ex_keys), P<unsigned long long>(ctx->ex_vals),
-         P<int32_t>(ctx->blk_cnt));
-  if (n_pairs > 0) {
-    int bits = 1;
-    while (bits < 31 && (1 << bits) < nb_all) ++bits;
-    CUBCALL(cub::DeviceRadixSort::SortPairs, P<uint32_t>(ctx->ex_keys), P<uint32_t>(ctx->ex_keys2),
-            P<unsigned long long>(ctx->ex_vals), P<unsigned long long>(ctx->ex_vals2), (int)n_pairs, 0, bits);
-  }
-  LAUNCH(k_exclusive_scan, 1, 1024, 0, nb_all, P<int32_t>(ctx->blk_cnt), P<int32_t>(ctx->pair_ptr));
-  LAUNCH(k_ex_finish, cdiv(std::max((int)n_pairs, nf * nf), BA_THREADS), BA_THREADS, 0, (int)n_pairs,
-         P<unsigned long long>(ctx->ex_vals2), P<int32_t>(ctx->pair_a), P<int32_t>(ctx->pair_b), nf, ctx->fixed_cam,
-         P<int32_t>(ctx->blk_i), P<int32_t>(ctx->blk_j), P<int32_t>(ctx->blk_cam));
-  ctx->n_blk = nb_all;
-  ctx->ex_band_cams = -1;  // (windows: every block of the upper triangle is listed; at most 7 tiles anyway)
-  return 0;
-}
-
-static int sparse_count_pairs(ba_gpu_ctx *ctx, long long *n_pairs_out) {
+// observation pairs per point and their total, read into ctx->n_pairs by the caller's next stream synchronisation (the
+// upload's index build: AUTO's pair count and build_pair_blocks)
+static int count_pairs(ba_gpu_ctx *ctx) {
   const int n_pt = ctx->n_pt;
-  cudaStream_t s = ctx->stream;
   RES(sp_cnt, ((size_t)n_pt + 2) * 8);
   RES(sp_off, ((size_t)n_pt + 2) * 8);
   LAUNCH(k_sp_count, cdiv(n_pt + 1, BA_THREADS), BA_THREADS, 0, n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
          ctx->fixed_cam, P<long long>(ctx->sp_cnt));
   CUBCALL(cub::DeviceScan::ExclusiveSum, P<long long>(ctx->sp_cnt), P<long long>(ctx->sp_off), n_pt + 1);
-  CK(cudaMemcpyAsync(n_pairs_out, P<long long>(ctx->sp_off) + n_pt, 8, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
+  CK(cudaMemcpyAsync(&ctx->n_pairs, P<long long>(ctx->sp_off) + n_pt, 8, cudaMemcpyDeviceToHost, ctx->stream));
   return 0;
 }
-static int build_sparse_structure(ba_gpu_ctx *ctx) {
+// largest block count of the pair blocks: one block per camera pair (i <= j) at most, one pair each at least
+static long long pair_block_bound(const ba_gpu_ctx *ctx) {
+  return std::min(ctx->n_pairs, (long long)ctx->n_cam * (ctx->n_cam + 1) / 2);
+}
+// (a) pair blocks (after count_pairs): the pairs of every block (i <= j) of S in point-major order (sp_pairs), the blocks' keys
+// (sp_ukeys) and their pair ranges (sb_ptr; past the last block every range is empty).  Every Schur complement sums over this
+// structure.  The block count stays on the device (sp_nruns) until read_pair_blocks().
+static int build_pair_blocks(ba_gpu_ctx *ctx) {
   const int n_pt = ctx->n_pt, n_cam = ctx->n_cam;
   cudaStream_t s = ctx->stream;
   typedef unsigned long long u64;
-  RES(sp_cnt, ((size_t)n_pt + 2) * 8);
-  RES(sp_off, ((size_t)n_pt + 2) * 8);
-  LAUNCH(k_sp_count, cdiv(n_pt + 1, BA_THREADS), BA_THREADS, 0, n_pt, P<int32_t>(ctx->pt_rowptr), P<int32_t>(ctx->pm_cam),
-         ctx->fixed_cam, P<long long>(ctx->sp_cnt));
-  CUBCALL(cub::DeviceScan::ExclusiveSum, P<long long>(ctx->sp_cnt), P<long long>(ctx->sp_off), n_pt + 1);
-  long long n_pairs = 0;
-  CK(cudaMemcpyAsync(&n_pairs, P<long long>(ctx->sp_off) + n_pt, 8, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
+  const long long n_pairs = ctx->n_pairs;
   if (n_pairs > 0x7fffffffLL) return fail(ctx, BA_ERR_UNSUPPORTED, "sparse Schur: %lld observation pairs (limit 2^31-1)", n_pairs);
-  ctx->n_pairs = n_pairs;
-  const size_t np8 = ((size_t)n_pairs + 1) * 8;
+  const size_t np8 = ((size_t)n_pairs + 1) * 8, nbound = (size_t)pair_block_bound(ctx);
   RES(sp_keys, np8);
   RES(sp_vals, np8);
   RES(sp_keys2, np8);
@@ -811,31 +683,28 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
   while (bits < 64 && ((u64)1 << bits) < (u64)n_cam * (u64)n_cam) ++bits;
   CUBCALL(cub::DeviceRadixSort::SortPairs, P<u64>(ctx->sp_keys), P<u64>(ctx->sp_keys2), P<u64>(ctx->sp_vals), P<u64>(ctx->sp_pairs),
           (int)n_pairs, 0, bits);
-  RES(sp_pair_pt, ((size_t)n_pairs + 1) * 4);
-  LAUNCH(k_sp_pair_points, (int)((n_pairs + BA_THREADS - 1) / BA_THREADS), BA_THREADS, 0, n_pairs, P<u64>(ctx->sp_pairs),
-         P<int32_t>(ctx->pt_idx), P<int32_t>(ctx->sp_pair_pt));
-  {
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, BA_SPS_SMEM));
-    ctx->sp_ctas_per_sm = std::max(1, per_sm);
-  }
-  RES(sp_ukeys, np8);
-  RES(sp_ucnt, ((size_t)n_pairs + 2) * 4);
+  RES(sp_ukeys, (nbound + 1) * 8);
+  RES(sp_ucnt, (nbound + 2) * 4);
   RES(sp_nruns, 16);
-  CUBCALL(cub::DeviceRunLengthEncode::Encode, P<u64>(ctx->sp_keys2), P<u64>(ctx->sp_ukeys), P<int32_t>(ctx->sp_ucnt),
-          P<int32_t>(ctx->sp_nruns), (int)n_pairs);
+  CK(cudaMemsetAsync(ctx->sp_ucnt.p, 0, (nbound + 2) * 4, s));  // (counts past the last block stay 0)
+  CK(cudaMemsetAsync(ctx->sp_nruns.p, 0, 4, s));
+  if (n_pairs > 0)
+    CUBCALL(cub::DeviceRunLengthEncode::Encode, P<u64>(ctx->sp_keys2), P<u64>(ctx->sp_ukeys), P<int32_t>(ctx->sp_ucnt),
+            P<int32_t>(ctx->sp_nruns), (int)n_pairs);
+  // (+ n_cam entries: the dense solver's table runs up to n_cam entries past the last block, build_dense_blocks)
+  RES(sb_ptr, (nbound + n_cam + 2) * 4);
+  CUBCALL(cub::DeviceScan::ExclusiveSum, P<int32_t>(ctx->sp_ucnt), P<int32_t>(ctx->sb_ptr), (int)nbound + 1);
+  return 0;
+}
+// the block count of build_pair_blocks() on the host; point-sharded, the block list every rank shares (sp_ukeys, n_sblk) and
+// the rank's own blocks in it (sp_lkeys, sp_gid, n_sblk_local)
+static int read_pair_blocks(ba_gpu_ctx *ctx) {
+  cudaStream_t s = ctx->stream;
+  typedef unsigned long long u64;
   int32_t n_blk = 0;
   CK(cudaMemcpyAsync(&n_blk, ctx->sp_nruns.p, 4, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  if (n_pairs == 0) n_blk = 0;
-  // pair list pointers of the LOCAL blocks
   ctx->n_sblk_local = n_blk;
-  RES(sb_ptr, ((size_t)n_blk + 2) * 4);
-  CK(cudaMemsetAsync(P<int32_t>(ctx->sp_ucnt) + n_blk, 0, 4, s));
-  CUBCALL(cub::DeviceScan::ExclusiveSum, P<int32_t>(ctx->sp_ucnt), P<int32_t>(ctx->sb_ptr), n_blk + 1);
-  RES(sp_lkeys, ((size_t)n_blk + 1) * 8);
-  RES(sp_gid, ((size_t)n_blk + 1) * 4);
-  CK(cudaMemcpyAsync(ctx->sp_lkeys.p, ctx->sp_ukeys.p, (size_t)n_blk * 8, cudaMemcpyDeviceToDevice, s));
   if (ctx->n_ranks > 1) {
     // point-sharded: every rank holds the blocks its own points touch.  The block structure must be the
     // same everywhere (S is all-reduced, PCG runs replicated): all-gather the key lists, sort, unique.
@@ -844,6 +713,9 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
     if (rcm) return rcm;
     const size_t slot = (size_t)mx + 1, all = slot * ctx->n_ranks;
     if (all > 0x7fffffffull) return fail(ctx, BA_ERR_UNSUPPORTED, "sparse Schur: too many blocks to gather");
+    RES(sp_lkeys, ((size_t)n_blk + 1) * 8);
+    RES(sp_gid, ((size_t)n_blk + 1) * 4);
+    CK(cudaMemcpyAsync(ctx->sp_lkeys.p, ctx->sp_ukeys.p, (size_t)n_blk * 8, cudaMemcpyDeviceToDevice, s));
     RES(sp_gather, (all + 1) * 8);
     RES(sp_gsorted, (all + 1) * 8);
     CK(cudaMemsetAsync(P<u64>(ctx->sp_gather) + slot * ctx->rank, 0xff, slot * 8, s));
@@ -862,10 +734,17 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
     n_blk = n_all - 1;  // the padding key ~0 sorts last (every rank pads at least one slot)
     LAUNCH(k_sp_lookup, cdiv(ctx->n_sblk_local, BA_THREADS), BA_THREADS, 0, ctx->n_sblk_local, P<u64>(ctx->sp_lkeys), n_blk,
            P<u64>(ctx->sp_ukeys), P<int32_t>(ctx->sp_gid));
-  } else {
-    LAUNCH(k_iota, cdiv(n_blk + 1, 256), 256, 0, n_blk + 1, P<int32_t>(ctx->sp_gid));
   }
   ctx->n_sblk = n_blk;
+  CK(cudaGetLastError());
+  return 0;
+}
+// (b) rows of the block-sparse S (after build_pair_blocks): the transposed entries, every camera row's entries (ent_ptr / ent),
+// the PCG row order, the diagonal blocks, the values Sblk and the PCG scratch
+static int build_rows(ba_gpu_ctx *ctx) {
+  const int n_cam = ctx->n_cam, n_blk = ctx->n_sblk;
+  cudaStream_t s = ctx->stream;
+  typedef unsigned long long u64;
   const size_t nb = (size_t)n_blk;
   RES(sb_i, (nb + 1) * 4);
   RES(sb_j, (nb + 1) * 4);
@@ -925,8 +804,43 @@ static int build_sparse_structure(ba_gpu_ctx *ctx) {
   return 0;
 }
 
+// block table of k_schur_pairs (dense solver, after build_pair_blocks): the structure's blocks (count on the device), then an
+// empty entry for the diagonal block of every free camera without an observation (sp_xdiag; cam_ptr: the camera CSR on the host;
+// U + D^2 only).  The blocked factorisation reads the block keys back for its band (largest camera-slot distance of a block) and
+// launches exactly the table; the single-CTA factorisations (windows) read nothing back and launch the table's bound, the CTAs
+// past the table return.
+static int build_dense_blocks(ba_gpu_ctx *ctx, const std::vector<int32_t> &cam_ptr) {
+  typedef unsigned long long u64;
+  const int n_cam = ctx->n_cam, fixed = ctx->fixed_cam, nf = ctx->n_free;
+  cudaStream_t s = ctx->stream;
+  std::vector<u64> xdiag;
+  for (int c = 0; c < n_cam; ++c)
+    if (c != fixed && cam_ptr[c + 1] == cam_ptr[c]) xdiag.push_back((u64)c * n_cam + c);
+  const int m = (int)xdiag.size();
+  ctx->n_xdiag = m;
+  RES(sp_xdiag, ((size_t)m + 1) * 8);
+  if (m > 0) CK(cudaMemcpyAsync(ctx->sp_xdiag.p, xdiag.data(), (size_t)m * 8, cudaMemcpyHostToDevice, s));
+  ctx->ex_band_cams = -1;
+  if (ctx->n_red <= BA_LDLT_MAX_N) {
+    ctx->n_blk = (int)std::min((long long)nf * (nf + 1) / 2, pair_block_bound(ctx) + m);
+  } else {
+    int rc = read_pair_blocks(ctx);
+    if (rc) return rc;
+    const int nb = ctx->n_sblk;
+    std::vector<u64> k((size_t)nb + 1);
+    if (nb > 0) CK(cudaMemcpyAsync(k.data(), ctx->sp_ukeys.p, (size_t)nb * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    auto slot = [&](int c) { return fixed >= 0 && c > fixed ? c - 1 : c; };
+    ctx->ex_band_cams = 0;
+    for (int b = 0; b < nb; ++b)
+      ctx->ex_band_cams = std::max(ctx->ex_band_cams, slot((int)(k[b] % (u64)n_cam)) - slot((int)(k[b] / (u64)n_cam)));
+    ctx->n_blk = nb + m;
+  }
+  return 0;
+}
+
 // symbolic phase of the exact sparse Cholesky (host: ordering, elimination tree, supernodes, maps) from the block structure of
-// the last build_sparse_structure(), split into want_parts subtree parts, with nrhs right-hand-side rows (5 with the intrinsics
+// the last build_rows(), split into want_parts subtree parts, with nrhs right-hand-side rows (5 with the intrinsics
 // border); uploads the integer tables and sizes the numeric buffers.  BA_ERR_UNSUPPORTED when a front cannot fit one SM's shared
 // memory (co-visibility without a sequential structure): AUTO keeps PCG then.
 static int build_spchol(ba_gpu_ctx *ctx, int want_parts, int nrhs) {
@@ -1451,9 +1365,18 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   LAUNCH(k_exclusive_scan, 1, 1024, 0, n_cam, P<int32_t>(ctx->item_cnt), P<int32_t>(ctx->item_ptr));
   LAUNCH(k_slots, ctx->nblk_cam, BA_THREADS, 0, n_cam, ctx->fixed_cam, P<int32_t>(ctx->cam_slot));
   LAUNCH(k_iota, cdiv(n_cam + 1, 256), 256, 0, n_cam + 1, P<int32_t>(ctx->ident));
+  // every plan that builds the pair blocks, and AUTO's choice between the sparse and the matrix-free solve, needs the pair count
+  if (ctx->plan.lin != LIN_IMPLICIT_PCG || (o.solver == BA_SOLVER_AUTO && fact)) {
+    if ((rc = count_pairs(ctx))) return rc;
+  }
   int32_t h_items = 0, h_err = 0;
   CK(cudaMemcpyAsync(&h_items, P<int32_t>(ctx->item_ptr) + n_cam, 4, cudaMemcpyDeviceToHost, s));
   CK(cudaMemcpyAsync(&h_err, ctx->err_flag.p, 4, cudaMemcpyDeviceToHost, s));
+  std::vector<int32_t> h_cam_ptr;  // (the dense solver's cameras without observations, build_dense_blocks)
+  if (ctx->plan.lin == LIN_DENSE) {
+    h_cam_ptr.resize(nc + 1);
+    CK(cudaMemcpyAsync(h_cam_ptr.data(), ctx->cam_rowptr.p, (nc + 1) * 4, cudaMemcpyDeviceToHost, s));
+  }
   CK(cudaStreamSynchronize(s));
   if (h_err) return fail(ctx, BA_ERR_INVALID, "observation indices out of range or cam_idx not non-decreasing");
   prof.stamp("index build + sync");
@@ -1475,10 +1398,8 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   // (b) AUTO on a large NS problem: block-sparse S if the co-visibility is sparse enough (decided from the pair count, the same
   // on every rank), factorised exactly (the reference's SPARSE_SCHUR) when its fronts fit; else matrix-free
   if (o.solver == BA_SOLVER_AUTO && ctx->plan.lin == LIN_IMPLICIT_PCG && fact) {
-    long long n_pairs = 0;
-    int rcs = sparse_count_pairs(ctx, &n_pairs);
-    if (rcs) return rcs;
-    double tot_pairs = (double)n_pairs, tot_obs = (double)n_obs, max_pairs = (double)n_pairs;
+    int rcs;
+    double tot_pairs = (double)ctx->n_pairs, tot_obs = (double)n_obs, max_pairs = (double)ctx->n_pairs;
     if ((rcs = allreduce_host_scalar(ctx, &tot_pairs, false)) || (rcs = allreduce_host_scalar(ctx, &tot_obs, false)) ||
         (rcs = allreduce_host_scalar(ctx, &max_pairs, true)))
       return rcs;
@@ -1544,8 +1465,22 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   // (c) the symbolic phase: the NS sparse Cholesky, or PCG on the same S when its fronts do not fit under AUTO; then the PCG form
   if (plan_sparse_ns(ctx->plan)) {
     prof.stamp("to sparse");
-    int rcs = build_sparse_structure(ctx);
+    int rcs = build_pair_blocks(ctx);
+    if (!rcs) rcs = read_pair_blocks(ctx);
+    if (!rcs) rcs = build_rows(ctx);
     if (rcs) return rcs;
+    // k_sp_schur's inputs: on one GPU the own blocks are the whole list (identity ids); the point of every pair (one level less
+    // in the dependent-load chain)
+    if (ctx->n_ranks == 1) {
+      RES(sp_gid, ((size_t)ctx->n_sblk + 1) * 4);
+      LAUNCH(k_iota, cdiv(ctx->n_sblk + 1, 256), 256, 0, ctx->n_sblk + 1, P<int32_t>(ctx->sp_gid));
+    }
+    RES(sp_pair_pt, ((size_t)ctx->n_pairs + 1) * 4);
+    LAUNCH(k_sp_pair_points, (int)((ctx->n_pairs + BA_THREADS - 1) / BA_THREADS), BA_THREADS, 0, ctx->n_pairs,
+           P<unsigned long long>(ctx->sp_pairs), P<int32_t>(ctx->pt_idx), P<int32_t>(ctx->sp_pair_pt));
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sp_schur, BA_THREADS, BA_SPS_SMEM));
+    ctx->sp_ctas_per_sm = std::max(1, per_sm);
     prof.stamp("sparse structure");
     if (ctx->plan.lin == LIN_SPARSE_CHOL) {
       // subtree-to-rank partition: one part per rank; on one GPU BA_SPCHOL_PARTS=n runs the n parts one after the other
@@ -1570,7 +1505,9 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   if (ctx->plan.lin == LIN_SPARSE_BORDERED) {
     // (one part: the bordered solve is single-GPU and runs the one-part queue's factor prefix on its own)
     prof.stamp("to sparse");
-    int rcs = build_sparse_structure(ctx);
+    int rcs = build_pair_blocks(ctx);
+    if (!rcs) rcs = read_pair_blocks(ctx);
+    if (!rcs) rcs = build_rows(ctx);
     if (!rcs) rcs = build_spchol(ctx, 1, ctx->nk ? 5 : 1);
     if (rcs == BA_ERR_UNSUPPORTED && o.solver == BA_SOLVER_AUTO) {
       const std::string why = ctx->err;
@@ -1589,7 +1526,7 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
   LAUNCH(k_fill, cdiv(3 * n_pt, 256), 256, 0, P<double>(ctx->one_p), (size_t)3 * np, 1.0);
   LAUNCH(k_fill, 1, 256, 0, P<double>(ctx->one_k), (size_t)4, 1.0);
   if (ctx->plan.lin == LIN_SPARSE_BORDERED) {
-    // no dense S, no pair list: the block-sparse structure of build_sparse_structure() holds S
+    // no dense S: the block-sparse structure of build_pair_blocks() and build_rows() holds S
     if ((rc = reserve_bordered(ctx))) return rc;
     CK(cudaMemsetAsync(ctx->yk.p, 0, 32, s));  // (no intrinsics: y_k stays 0)
     prof.stamp("rest");
@@ -1603,14 +1540,8 @@ extern "C" int ba_gpu_upload(ba_gpu_ctx *ctx, int32_t n_cam, const double *pose7
     RES(chol_lsub, (size_t)(cdiv(ctx->n_red, CH_NB) + 1) * CH_NB * CH_NB * 8);  // panel tiles right below the diagonal (look-ahead)
     RES(chol_slots, (size_t)2 * cdiv(ctx->n_red, CH_NB) * CH_NB * sizeof(ChSlot));
     prof.stamp("rest");
-    // windows: device-built pair list; the global REF problem keeps the host-built list of NON-EMPTY blocks
-    // (320 k mostly empty blocks at 800 keyframes)
-    const bool dev_pairs = ctx->n_free <= 64 && (ctx->src_on_device || getenv("BA_HOST_PAIRS") == nullptr);
-    if (!dev_pairs && ctx->src_on_device)
-      return fail(ctx, BA_ERR_UNSUPPORTED, "device-resident windows are limited to 65 keyframes (the pair list of larger explicit problems is host-built)");
-    int rc = dev_pairs ? build_pair_list_device(ctx) : build_pair_list(ctx, cam_idx, pt_idx);
-    if (rc) return rc;
-    prof.stamp("pair list");
+    if ((rc = build_pair_blocks(ctx)) || (rc = build_dense_blocks(ctx, h_cam_ptr))) return rc;
+    prof.stamp("pair blocks");
   }
   prof.flush();
   CK(cudaGetLastError());
@@ -1926,7 +1857,7 @@ static void enqueue_sparse_values(ba_gpu_ctx *ctx, int gate) {
   // (pair records hold canonical observation indices: the kernel reads the CAMERA-major factored planes)
   const int sps_grid = std::min(cdiv(ctx->n_sblk_local, BA_SPS_CHUNK), ctx->n_sm * ctx->sp_ctas_per_sm);
   LAUNCH(k_sp_schur, sps_grid, BA_THREADS, BA_SPS_SMEM, ctx->n_sblk_local, ctx->n_cam, P<int32_t>(ctx->sb_ptr),
-         P<unsigned long long>(ctx->sp_lkeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
+         P<unsigned long long>(ctx->n_ranks > 1 ? ctx->sp_lkeys : ctx->sp_ukeys), P<int32_t>(ctx->sp_gid), P<unsigned long long>(ctx->sp_pairs),
          P<int32_t>(ctx->sp_pair_pt), ctx->Fc_, P<double>(ctx->geo), P<double>(ctx->intr), P<double>(ctx->Vs),
          P<double>(ctx->Sblk), ticket, st, gate);
   if (ctx->n_ranks > 1) {
@@ -2345,13 +2276,15 @@ static int solve_dense(ba_gpu_ctx *ctx) {
   }
   fork_main(ctx);
   if (ctx->n_blk <= 4 * ctx->n_sm)
-    LAUNCH(k_schur_pairs<28>, ctx->n_blk, 28 * 36, 0, n, P<int32_t>(ctx->blk_i), P<int32_t>(ctx->blk_j), P<int32_t>(ctx->blk_cam),
-         P<int32_t>(ctx->pair_ptr), P<int32_t>(ctx->pair_a), P<int32_t>(ctx->pair_b), P<double>(ctx->W), P<double>(ctx->WV),
-         P<double>(ctx->U), P<double>(ctx->dc), P<double>(ctx->S), st, GATE_RUN);
+    LAUNCH(k_schur_pairs<28>, ctx->n_blk, 28 * 36, 0, n, ctx->n_cam, ctx->fixed_cam, P<int32_t>(ctx->sp_nruns),
+           P<unsigned long long>(ctx->sp_ukeys), P<int32_t>(ctx->sb_ptr), P<unsigned long long>(ctx->sp_xdiag), ctx->n_xdiag,
+           P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->U),
+           P<double>(ctx->dc), P<double>(ctx->S), st, GATE_RUN);
   else
-    LAUNCH(k_schur_pairs<7>, ctx->n_blk, 7 * 36, 0, n, P<int32_t>(ctx->blk_i), P<int32_t>(ctx->blk_j), P<int32_t>(ctx->blk_cam),
-         P<int32_t>(ctx->pair_ptr), P<int32_t>(ctx->pair_a), P<int32_t>(ctx->pair_b), P<double>(ctx->W), P<double>(ctx->WV),
-         P<double>(ctx->U), P<double>(ctx->dc), P<double>(ctx->S), st, GATE_RUN);
+    LAUNCH(k_schur_pairs<7>, ctx->n_blk, 7 * 36, 0, n, ctx->n_cam, ctx->fixed_cam, P<int32_t>(ctx->sp_nruns),
+           P<unsigned long long>(ctx->sp_ukeys), P<int32_t>(ctx->sb_ptr), P<unsigned long long>(ctx->sp_xdiag), ctx->n_xdiag,
+           P<unsigned long long>(ctx->sp_pairs), P<double>(ctx->W), P<double>(ctx->WV), P<double>(ctx->U),
+           P<double>(ctx->dc), P<double>(ctx->S), st, GATE_RUN);
   join(ctx);
   if (n <= BA_LDLT2_MAX_N) {
     // single CTA, L D L^T with the trailing matrix in registers and the right-hand side as an extra row (ba_kernels_chol.cuh)
@@ -2860,7 +2793,13 @@ static int cov_prepare(ba_gpu_ctx *ctx) {
   int rc;
   if (!plan_tree(ctx->plan)) {
     ctx->lm_graph_stale = true;
-    if ((rc = build_sparse_structure(ctx))) return rc;
+    if (ctx->plan.lin == LIN_IMPLICIT_PCG) {
+      if ((rc = count_pairs(ctx))) return rc;
+      CK(cudaStreamSynchronize(s));
+      if ((rc = build_pair_blocks(ctx))) return rc;
+    }
+    if (!plan_sparse_s(ctx->plan) && (rc = read_pair_blocks(ctx))) return rc;
+    if ((rc = build_rows(ctx))) return rc;
     rc = build_spchol(ctx, 1, ctx->nk ? 5 : 1);
     if (rc == BA_ERR_UNSUPPORTED) {
       const std::string why = ctx->err;
@@ -3875,10 +3814,8 @@ extern "C" int ba_store_window_solve(ba_store *st, int32_t kf_i, int32_t kf_f, c
   if (n_obs_out) *n_obs_out = n_obs;
   *n_pt_out = n_pt;
   if (n_pt > lm_cap) return fail(ctx, BA_ERR_INVALID, "store: %d landmarks in the window, caller's capacity %d", n_pt, lm_cap);
-  ctx->src_on_device = true;
   rc = ba_gpu_upload(ctx, n_cam, (const double *)st->w_pose.p, 0, n_pt, (const double *)st->w_pt3.p, n_obs, (const int32_t *)st->w_cam.p,
                      (const int32_t *)st->w_pt.p, (const double *)st->w_uv.p, (const double *)st->w_depth.p, intr4, intr_prior4);
-  ctx->src_on_device = false;
   if (rc) return rc;
   st->ms[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
   auto t_ph = std::chrono::steady_clock::now();

@@ -1848,36 +1848,41 @@ k_explicit_cam_kk(int nb_item, int n_items, const BaItem *__restrict__ items, co
     d_k_explicit_kk(blockIdx.x - nb_item, n_pt, Wk, Vinv, tg, part_kk, st, gate);
 }
 
-// camera-camera blocks: one CTA per block pair (i <= j) of the pair list;
+// camera-camera blocks: one CTA per block (ci <= cj) of the block-sparse pair structure (keys ci * n_cam + cj, pair
+// ranges blk_ptr, pairs (ia << 32) | ib in point-major order, *n_keys blocks), then n_xdiag empty diagonal blocks of free
+// cameras without observations (keys xdiag); CTAs past the table return.
 // thread = (entry of the 6x6 block, slice of the pair run); fixed-order
 // reduction over the slices in shared memory.
-//   S_ij = [i==j] (U_i + D_i^2) - sum_{(a,b)} WV_a W_b^T
+//   S_ij = [i==j] (U_i + D_i^2) - sum_{(a,b)} WV_a W_b^T        (i, j: camera slots)
 // SLICES = 28 (1008 threads) when the blocks are few and their pair runs long (windows), 7 otherwise
 template <int SLICES>
-__global__ void __launch_bounds__(SLICES * 36)
-k_schur_pairs(int n, const int32_t *__restrict__ blk_i, const int32_t *__restrict__ blk_j,
-              const int32_t *__restrict__ blk_cam_i, const int32_t *__restrict__ pair_ptr,
-              const int32_t *__restrict__ pair_a, const int32_t *__restrict__ pair_b, const double *__restrict__ W,
+__global__ void __launch_bounds__(SLICES * 36, 2048 / (SLICES * 36))  // (32 registers: 2 / 8 CTAs per SM)
+k_schur_pairs(int n, int n_cam, int fixed_cam, const int32_t *__restrict__ n_keys, const unsigned long long *__restrict__ keys,
+              const int32_t *__restrict__ blk_ptr, const unsigned long long *__restrict__ xdiag, int n_xdiag,
+              const unsigned long long *__restrict__ pairs, const double *__restrict__ W,
               const double *__restrict__ WV, const double *__restrict__ U, const double *__restrict__ dc,
               double *__restrict__ S, const LmState *st, int gate) {
   if (!gate_open(st, gate)) return;
   __shared__ double sm[SLICES * 36];
   const int blk = blockIdx.x;
-  // device-built block table lists the whole upper triangle: an off-diagonal block without pairs stays zero
-  if (pair_ptr[blk] == pair_ptr[blk + 1] && blk_i[blk] != blk_j[blk]) return;
+  // (blk_ptr holds an entry for every launched CTA: the range loads go out together with the block count)
+  const int nk = *n_keys, p0 = blk_ptr[blk], p1 = blk_ptr[blk + 1];
+  if (blk >= nk + n_xdiag) return;
+  const bool own = blk < nk;
   const int e = threadIdx.x % 36, sl = threadIdx.x / 36;
   const int row = e / 6, col = e % 6;
   // the loop is bound by the index -> block gather latency: four pairs per round, all index loads issued before
   // the first block load; the slice's partial is (even pairs) + (odd pairs), a fixed order
   double acc0 = 0.0, acc1 = 0.0;
-  const int k1 = pair_ptr[blk + 1];
-  for (int k = pair_ptr[blk] + sl; k < k1; k += 4 * SLICES) {
+  const int k1 = own ? p1 : 0;
+  for (int k = (own ? p0 : 0) + sl; k < k1; k += 4 * SLICES) {
     int ia[4], ib[4];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const int kk = k + u * SLICES;
-      ia[u] = kk < k1 ? pair_a[kk] : -1;
-      ib[u] = kk < k1 ? pair_b[kk] : 0;
+      const int2 v = kk < k1 ? reinterpret_cast<const int2 *>(pairs)[kk] : make_int2(0, -1);  // (low word ib, high word ia)
+      ia[u] = v.y;
+      ib[u] = v.x;
     }
     double t[4];
 #pragma unroll
@@ -1900,10 +1905,11 @@ k_schur_pairs(int n, const int32_t *__restrict__ blk_i, const int32_t *__restric
     double s = 0.0;
 #pragma unroll
     for (int q = 0; q < SLICES; ++q) s += sm[q * 36 + e];
-    const int i = blk_i[blk], j = blk_j[blk];
+    const uint32_t key = (uint32_t)(own ? keys[blk] : xdiag[blk - nk]);  // (dense S: n_cam <= BA_EXPLICIT_MAX_DIM / 6, so n_cam^2 < 2^32)
+    const int c = (int)(key / (uint32_t)n_cam), cj = (int)(key % (uint32_t)n_cam);
+    const int i = fixed_cam >= 0 && c > fixed_cam ? c - 1 : c, j = fixed_cam >= 0 && cj > fixed_cam ? cj - 1 : cj;
     double v = -s;
     if (i == j) {
-      const int c = blk_cam_i[blk];
       v += U[36 * (size_t)c + e];
       if (row == col) {
         const double D = sqrt(dc[6 * (size_t)c + row] / st->radius);

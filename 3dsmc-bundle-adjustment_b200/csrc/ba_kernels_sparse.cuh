@@ -17,6 +17,7 @@
 //             by key => the pair list of every block, in point-major order
 //             (the fixed summation order of the block)
 //   blocks  : the distinct keys (upper triangle incl. diagonal), blk_ptr into pairs
+//             (pairs + blocks are also the structure k_schur_pairs sums the dense explicit S over)
 //   rows    : per camera the entries (block, transposed?) in ascending column order
 // Values: one warp per block walks its pair list; Jacobian entries are rebuilt from
 // the factored point-major store (ba_kernels_fact.cuh).
@@ -69,71 +70,6 @@ k_sp_emit(int n_pt, int n_cam, const int32_t *__restrict__ pt_rowptr, const int3
         vals[w] = ((unsigned long long)ib << 32) | ia;
         ++w;
       }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Pair list of the DENSE explicit solver (windowed problems), built on the device instead of by the host loop
-// of build_pair_list(): same enumeration as k_sp_emit, keyed by the dense upper-triangle index of the camera
-// SLOT pair, values = the two CANONICAL (camera-major) observation indices; the per-block counts come from
-// integer atomics (the counts, not the order, so the result is deterministic), the order inside a block from the
-// stable radix sort = ascending point, as the host loop produces.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ int ex_slot(int c, int fixed_cam) { return c == fixed_cam ? -1 : (fixed_cam >= 0 && c > fixed_cam ? c - 1 : c); }
-__device__ __forceinline__ int ex_bidx(int i, int j, int nf) { return i * nf - i * (i - 1) / 2 + (j - i); }
-
-__global__ void __launch_bounds__(BA_THREADS)
-k_ex_emit(int n_pt, int nf, const int32_t *__restrict__ pt_rowptr, const int32_t *__restrict__ pm_cam,
-          const int32_t *__restrict__ perm, int fixed_cam, const long long *__restrict__ off, uint32_t *__restrict__ keys,
-          unsigned long long *__restrict__ vals, int32_t *blk_cnt) {
-  const int p = blockIdx.x * BA_THREADS + threadIdx.x;
-  if (p >= n_pt) return;
-  long long w = off[p];
-  const int b0 = pt_rowptr[p], e0 = pt_rowptr[p + 1];
-  for (int a = b0; a < e0; ++a) {
-    const int sa = ex_slot(pm_cam[a], fixed_cam);
-    if (sa < 0) continue;
-    const unsigned oa = (unsigned)perm[a];
-    for (int b = a; b < e0; ++b) {
-      const int sb = ex_slot(pm_cam[b], fixed_cam);
-      if (sb < 0) continue;
-      // cameras ascend inside a point's run (stable sort of a camera-major list): sa <= sb
-      const int key = ex_bidx(sa, sb, nf);
-      const unsigned ob = (unsigned)perm[b];
-      keys[w] = (uint32_t)key;
-      vals[w] = ((unsigned long long)oa << 32) | ob;
-      ++w;
-      int n = 1;
-      if (sa == sb && a != b) {  // same camera twice: the diagonal block also needs W_b V^-1 W_a^T
-        keys[w] = (uint32_t)key;
-        vals[w] = ((unsigned long long)ob << 32) | oa;
-        ++w;
-        n = 2;
-      }
-      atomicAdd(&blk_cnt[key], n);
-    }
-  }
-}
-
-// sorted values -> pair_a / pair_b; block table of the dense upper triangle (every block listed; empty
-// off-diagonal ones are skipped by k_schur_pairs)
-__global__ void __launch_bounds__(BA_THREADS)
-k_ex_finish(int n_pairs, const unsigned long long *__restrict__ vals, int32_t *__restrict__ pair_a, int32_t *__restrict__ pair_b,
-            int nf, int fixed_cam, int32_t *__restrict__ blk_i, int32_t *__restrict__ blk_j, int32_t *__restrict__ blk_cam) {
-  const int t = blockIdx.x * BA_THREADS + threadIdx.x;
-  if (t < n_pairs) {
-    const unsigned long long v = vals[t];
-    pair_a[t] = (int32_t)(v >> 32);
-    pair_b[t] = (int32_t)(v & 0xffffffffu);
-  }
-  if (t < nf * nf) {
-    const int i = t / nf, j = t - i * nf;
-    if (j >= i) {
-      const int k = ex_bidx(i, j, nf);
-      blk_i[k] = i;
-      blk_j[k] = j;
-      blk_cam[k] = (fixed_cam >= 0 && i >= fixed_cam) ? i + 1 : i;
     }
   }
 }

@@ -687,7 +687,7 @@ __global__ void k_spchol_dist_post(int n_cam, const double *yc, LmState *st, int
 // ---------------------------------------------------------------------------------------------
 // Sparse Cholesky of the REF / DEPTH / INTR cost (depth prior and / or free intrinsics, planes store): the explicit path's
 // per-observation W = Jc^T Jp and WV = W V^-1 (k_obs_W, already Jacobi-scaled) summed into the device-built block structure
-// (build_sparse_structure), the camera-intrinsics border B, the corner C and the right-hand side assembled by camera, and the
+// (build_pair_blocks), the camera-intrinsics border B, the corner C and the right-hand side assembled by camera, and the
 // 4 x 4 border system solved between the forward and the backward substitution.
 // ---------------------------------------------------------------------------------------------
 // values of S from the planes: one warp per block, S_b = -sum_pairs WV_a W_b^T in the fixed pair order of the block

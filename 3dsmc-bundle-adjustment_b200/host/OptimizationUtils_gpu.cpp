@@ -76,7 +76,6 @@ namespace {
 int window_optimize_store(const ba_gpu_options &opt, int kf_i, int kf_f, vector<KeyFrame> &keyframes, Map3D &map,
                           const Vector4d &intrinsics_initial, Vector4d &intrinsics_optimized) {
   const int n_cam = kf_f - kf_i + 1;
-  if (n_cam > 65) return -1;  // (larger explicit problems build their pair list on the host)
   const auto t_begin = std::chrono::steady_clock::now();
   int rc = g_ctx.ctx ? ba_gpu_set_options(g_ctx.ctx, &opt) : ba_gpu_create(&opt, &g_ctx.ctx);
   if (rc == BA_OK && !g_store.st) rc = ba_store_create(g_ctx.ctx, &g_store.st);

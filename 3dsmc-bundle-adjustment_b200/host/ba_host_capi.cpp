@@ -85,8 +85,8 @@ int ba_host_window_optimize(int n_kf, double *pose7, const int32_t *kf_ptr, cons
 // global optimisation over all keyframes instead (:178-182).  Containers are built once (as the tracking front end
 // would have left them); every window is warm-started by the previous ones.  fixed_iterations != 0 switches the
 // tolerances off, so that every call runs exactly max_num_iterations LM iterations (throughput measurement).
-// out_ms[6]: accumulated host wall clock -- total, container walk + frame change, ba_gpu_upload, ba_gpu_solve,
-// ba_gpu_download, write-back.  Returns the number of windowOptimize calls, or -1 if one failed.
+// out_ms[7]: accumulated host wall clock -- total, container walk + frame change, ba_gpu_upload, ba_gpu_solve,
+// ba_gpu_download, write-back -- and the number of calls the device-resident store solved.  Returns the number of windowOptimize calls, or -1 if one failed.
 int ba_host_sliding_sequence(int n_kf, double *pose7, const int32_t *kf_ptr, const int32_t *lm, const float *uv,
                              const double *depth, int n_lm, const int32_t *lm_id, double *lm_pt, int window_size,
                              int frame_frequency, int do_global, int max_num_iterations, int fixed_iterations,
@@ -135,7 +135,7 @@ int ba_host_sliding_sequence(int n_kf, double *pose7, const int32_t *kf_ptr, con
   ceresGlobalProblem gp;
   gp.options.max_num_iterations = max_num_iterations;
   Vector4d i0(intr0[0], intr0[1], intr0[2], intr0[3]), io(intr[0], intr[1], intr[2], intr[3]);
-  double ms[6] = {0, 0, 0, 0, 0, 0};
+  double ms[7] = {0, 0, 0, 0, 0, 0, 0};
   int64_t lm_iterations = 0;
   int calls = 0;
   bool ok = true;
@@ -150,6 +150,7 @@ int ba_host_sliding_sequence(int n_kf, double *pose7, const int32_t *kf_ptr, con
     ms[3] += last.ms_solve;
     ms[4] += last.ms_download;
     ms[5] += last.ms_writeback;
+    if (ok && last.cam_idx.empty() && last.admissible_obs > 0) ms[6] += 1;  // (the store path keeps no host index arrays)
     lm_iterations += last.summary.num_iterations;
     ++calls;
   };

@@ -19,7 +19,7 @@ const BaHostLastProblem &ba_host_last_problem();
 // measurement only: tolerances off, so that every call runs exactly options.max_num_iterations LM iterations
 void ba_host_fixed_iterations(bool on);
 // Device-resident keyframe / landmark store (SURVEY.md 8f row N1; ba_store_* of include/ba_gpu.h) behind windowOptimize: on =
-// windows of up to 65 keyframes upload only the keyframes that are new or whose global_points_map grew since the last
+// windows upload only the keyframes that are new or whose global_points_map grew since the last
 // call, and enumerate / change frames on the device; off (default) = every call walks and uploads the whole window.
 // Assumes what holds in the reference's main loop: between two calls only new keyframes / landmarks appear, a keyframe's
 // map only GROWS (src/Map3D.cpp:52-53, 73), and world points are changed by windowOptimize alone.  Calling it (on or off)

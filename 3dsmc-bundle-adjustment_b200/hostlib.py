@@ -54,7 +54,7 @@ def sliding_sequence(seq, window_size, frame_frequency=10, max_num_iterations=75
     lm_id = np.arange(pt.shape[0], dtype=np.int32)
     intr0 = np.array(seq.K if intrinsics_initial is None else intrinsics_initial, dtype=np.float64)
     intr = np.array(seq.K if intrinsics_optimized is None else intrinsics_optimized, dtype=np.float64)
-    ms = np.zeros(6)
+    ms = np.zeros(7)
     n_it = C.c_int64(0)
     rc = L.ba_host_sliding_sequence(n_kf, _ptr(pose, C.c_double), _ptr(kf_ptr, C.c_int32), _ptr(lm, C.c_int32), _ptr(uv, C.c_float),
                                     _ptr(depth, C.c_double), int(pt.shape[0]), _ptr(lm_id, C.c_int32), _ptr(pt, C.c_double),
@@ -68,4 +68,5 @@ def sliding_sequence(seq, window_size, frame_frequency=10, max_num_iterations=75
     if intrinsics_optimized is not None:
         intrinsics_optimized[:] = intr
     keys = ("total", "extract", "upload", "solve", "download", "write_back")
-    return {"windows": rc, "lm_iterations": int(n_it.value), "ms": dict(zip(keys, ms.tolist())), "intrinsics": intr}
+    return {"windows": rc, "lm_iterations": int(n_it.value), "ms": dict(zip(keys, ms.tolist())), "intrinsics": intr,
+            "store_windows": int(ms[6])}

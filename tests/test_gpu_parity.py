@@ -637,11 +637,11 @@ def _explicit_run(p, env=None, iters=8, **kw):
 
 @pytest.mark.parametrize("name", ["cfg1", "window20"])
 def test_window_graph_and_device_pairs_are_bit_identical(name):
-    """The CUDA-graph replay of the LM iteration and the device-built pair list change HOW the work is enqueued /
-    indexed, not the arithmetic: results must equal the direct-enqueue / host-built-list run bit for bit."""
+    """The CUDA-graph replay of the LM iteration and the two-stream fork change HOW the work is enqueued, not the
+    arithmetic: results must equal the direct-enqueue / single-stream run bit for bit."""
     p = _problem(name)
     base = _explicit_run(p)
-    for env in ({"BA_NO_LM_GRAPH": "1"}, {"BA_HOST_PAIRS": "1"}, {"BA_NO_FORK": "1"}):
+    for env in ({"BA_NO_LM_GRAPH": "1"}, {"BA_NO_FORK": "1"}):
         other = _explicit_run(p, env)
         assert other[0].num_iterations == base[0].num_iterations
         assert other[0].final_cost == base[0].final_cost, env

@@ -189,23 +189,26 @@ def test_no_raw_pointer_se3_constructor_anywhere():
 
 # ---------------------------------------------------------------- device-resident store (SURVEY.md 8f row N1)
 @pytest.mark.gpu
-@pytest.mark.parametrize("growing", [False, True], ids=["complete-maps", "maps-grow-between-windows"])
-def test_device_store_sliding_windows_bit_identical(growing):
+@pytest.mark.parametrize("growing, window", [(False, 20), (True, 20), (False, 70)],
+                         ids=["complete-maps", "maps-grow-between-windows", "complete-maps-window70"])
+def test_device_store_sliding_windows_bit_identical(growing, window):
     """The reference's schedule (a 20-keyframe window every 10 keyframes, warm-started) through the compiled drop-in, once
     with every window walked and uploaded in full and once through the device-resident store (only new / grown keyframes
     and new landmarks are uploaded; enumeration and frame changes on the device): poses, landmarks and intrinsics must
     be equal BIT FOR BIT after the whole sequence.  With growing maps the second half of every keyframe's map arrives with
-    the next keyframe (the "old_frame" inserts of src/Map3D.cpp:52): such a keyframe is uploaded twice."""
+    the next keyframe (the "old_frame" inserts of src/Map3D.cpp:52): such a keyframe is uploaded twice.  70-keyframe
+    windows take the blocked dense factorisation."""
     hostlib = ba_b200.hostlib
     out = []
     for store in (False, True):
         seq = syn.make_config(2, scale=0.1)   # 80 keyframes, 8000 landmarks
         intr = seq.K.copy()
-        r = hostlib.sliding_sequence(seq, 20, 10, max_num_iterations=6, fixed_iterations=True, intrinsics_optimized=intr,
+        r = hostlib.sliding_sequence(seq, window, 10, max_num_iterations=6, fixed_iterations=True, intrinsics_optimized=intr,
                                      device_store=store, growing_maps=growing)
         out.append((seq.pose.copy(), seq.pt.copy(), intr.copy(), r))
     a, b = out
-    assert a[3]["windows"] == b[3]["windows"] == 7 and a[3]["lm_iterations"] == b[3]["lm_iterations"]
+    assert a[3]["windows"] == b[3]["windows"] == (80 - window) // 10 + 1 and a[3]["lm_iterations"] == b[3]["lm_iterations"]
+    assert a[3]["store_windows"] == 0 and b[3]["store_windows"] == b[3]["windows"]   # every window of the second run took the store
     assert np.array_equal(a[0], b[0]), float(np.max(np.abs(a[0] - b[0])))
     assert np.array_equal(a[1], b[1]), float(np.max(np.abs(a[1] - b[1])))
     assert np.array_equal(a[2], b[2])
